@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- station-pair cross-correlation throughput of the B200 TDOA engine.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): 3 stations x 100 s x 2 Msps dual-frequency uint8 IQ
 captures (200 000 000 samples = 400 MB per station, blocks ref/target/ref), simulator.go
@@ -33,6 +33,7 @@ Beside the headline the line carries
 from __future__ import annotations
 
 import argparse
+import hashlib
 import json
 import os
 import subprocess
@@ -73,6 +74,22 @@ def true_delays():
     d = np.array([np.linalg.norm(tx - llh_to_ecef(*s)) for s in STATION_LLH])
     k = np.rint(d / C_LIGHT * FS).astype(int)
     return k - k.min()
+
+
+# ----------------------------------------------------------------------------- --dump-outputs
+def record_arrays(prefix: str, records: np.ndarray) -> dict:
+    """One array per field of a peak-record table (PEAK_DTYPE): <prefix>_lag, <prefix>_corr, ..."""
+    return {f"{prefix}_{name}": records[name] for name in records.dtype.names}
+
+
+def dump_outputs(directory: str, arrays: dict) -> None:
+    """DIR/<name>.npy for every array: float32 where the engine returns float32, float64 otherwise
+    (integers and flags convert exactly), so that two builds can be compared output for output."""
+    out = Path(directory)
+    out.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        np.save(out / f"{name}.npy", a.astype(np.float32 if a.dtype == np.float32 else np.float64))
 
 
 # ----------------------------------------------------------------------------- clocks
@@ -122,7 +139,9 @@ class ClockSampler:
 def synth_captures_gpu(torch, device, block: int, seed: int):
     """Mode-B captures generated on the GPU (setup only, never timed): FM of box-car
     filtered Gaussian audio, amplitude 0.5, integer delays from the station geometry,
-    AWGN sigma 0.02, quantised as simulator.go:150-160.  Returns uint8 tensors [3][6*block]."""
+    AWGN sigma 0.02, quantised as simulator.go:150-160.  Returns uint8 tensors [3][6*block].
+    The same seed gives the same bytes on every run: the two prefix sums run on the host in index
+    order, because CUDA's floating-point cumsum may add its tiles in a different order each run."""
     g = torch.Generator(device=device)
     delays = true_delays()
     pad = int(delays.max()) + 64
@@ -130,10 +149,10 @@ def synth_captures_gpu(torch, device, block: int, seed: int):
     def fm(n, sd, dev):
         g.manual_seed(sd)
         a = torch.randn(n + 64, device=device, generator=g)
-        cs = torch.cumsum(a, 0)
+        cs = torch.cumsum(a.cpu(), 0).to(device)
         a = (cs[64:] - cs[:-64]) / 64.0          # 64-tap box-car audio
         a = a / a.abs().max()
-        ph = torch.cumsum(a.double(), 0) * (2 * np.pi * dev / FS)
+        ph = torch.cumsum(a.double().cpu(), 0).to(device) * (2 * np.pi * dev / FS)
         ph = torch.remainder(ph, 2 * np.pi).float()
         return 0.5 * torch.cos(ph), 0.5 * torch.sin(ph)
 
@@ -315,7 +334,7 @@ def sharded_block(args, torch, dist, T, device, local, rank, world):
         # both pair loops in one call: the windows of both kinds are dealt over the ranks as one list (tdoa_xcorr_windows)
         return eng.xcorr_windows(0, SHARD_W, nw_r, nw_t, SHARD_W)
 
-    steps, warm = max(1, min(args.steps, 5)), 3
+    steps, warm = args.steps, 3
     for _ in range(warm):
         r, t = step()
     if world > 1:
@@ -361,7 +380,7 @@ def sharded_block(args, torch, dist, T, device, local, rank, world):
     eng.close()
     del caps
     torch.cuda.empty_cache()
-    return out
+    return out, {**record_arrays("sharded_ref", r), **record_arrays("sharded_tgt", t)}
 
 
 def sharded_oracle_sample(caps, block, tgt_table, nw_t, window=7, pairs=((0, 1), (3, 9))):
@@ -473,11 +492,13 @@ def main_ours(args):
         dist.init_process_group("nccl", device_id=device)
 
     if args.only_sharded:   # profiling aid: the sharded configs[3] block alone
-        shard = sharded_block(args, torch, dist, T, device, local, rank, world)
+        shard, shard_out = sharded_block(args, torch, dist, T, device, local, rank, world)
         if world > 1:
             dist.barrier()
             dist.destroy_process_group()
         if rank == 0:
+            if args.dump_outputs:
+                dump_outputs(args.dump_outputs, shard_out)
             OUT.emit(json.dumps({"sharded": shard}))
         return 0
 
@@ -489,6 +510,10 @@ def main_ours(args):
     pinned = [T.host_alloc(nbytes) for _ in range(3)]
     for k in range(3):
         pinned[k].array[:] = caps[k].cpu().numpy()
+    digest = hashlib.sha256()
+    for pb in pinned:
+        digest.update(pb.array)
+    inputs_sha256 = digest.hexdigest()   # equal digests: two runs (or two builds) worked on the same captures
 
     eng = T.Engine(T.MODE_BINARY, chunk_samples=0, device=local, use_fft=1)
     eng.set_stream(torch.cuda.current_stream().cuda_stream)
@@ -521,12 +546,11 @@ def main_ours(args):
         # loop, TGT pair loop, time / range differences, solveTDOA, queued on the device without
         # an intermediate host synchronisation; records and fix come back to the host
         r = eng.process(STATION_LLH)
-        ref, tgt, pos, status = r["ref"], r["tgt"], r["position"], r["status"]
         if world > 1:
             # the path's single collective (SURVEY.md 8e): every rank's peak records
-            rec = torch.from_numpy(np.concatenate([ref, tgt]).view(np.uint8).copy()).to(device, non_blocking=True)
+            rec = torch.from_numpy(np.concatenate([r["ref"], r["tgt"]]).view(np.uint8).copy()).to(device, non_blocking=True)
             dist.all_gather(gather_out, rec)
-        return ref, tgt, pos, status
+        return r
 
     def step_e2e():
         # host buffers in: the three captures sit in pinned host memory (tdoa_host_alloc);
@@ -546,7 +570,8 @@ def main_ours(args):
         torch.cuda.synchronize()
 
     # correctness of the benchmarked path on this very input (not timed)
-    ref, tgt, pos, status = step_resident()
+    r0 = step_resident()
+    ref, tgt, pos, status = r0["ref"], r0["tgt"], r0["position"], r0["status"]
     want = [int(delays[j] - delays[i]) for i, j in pairs]
     got_r, got_t = [int(x) for x in ref["lag"]], [int(x) for x in tgt["lag"]]
     clamp = [max(w, 0) for w in want]  # the reference searches non-negative lags only
@@ -572,7 +597,7 @@ def main_ours(args):
         collecting[0] = collect_stats
         e0.record()
         for _ in range(steps):
-            fn()
+            last = fn()
         e1.record()
         collecting[0] = False
         sync_all()
@@ -580,17 +605,19 @@ def main_ours(args):
         t = torch.tensor([ms], device=device, dtype=torch.float64)
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        return float(t.item()), eng.stats()["launches_total"] - l0
+        return float(t.item()), eng.stats()["launches_total"] - l0, last
 
     # clocks are sampled over both timed regions (nvidia-smi answers in ~100 ms, the
     # resident region alone is shorter than that at the default step count)
     with ClockSampler(local) as clocks:
-        ms_res, launches = timed(step_resident, args.steps, args.warmup)
-        ms_e2e, _ = timed(step_e2e, max(1, args.steps), max(3, args.warmup) if args.warmup else 0)
-        ms_serial, _ = timed(step_serial, args.steps, args.warmup, collect_stats=True)
+        ms_res, launches, last_res = timed(step_resident, args.steps, args.warmup)
+        ms_e2e, _, _ = timed(step_e2e, args.steps, max(3, args.warmup) if args.warmup else 0)
+        ms_serial, _, _ = timed(step_serial, args.steps, args.warmup, collect_stats=True)
+    dumped = {**record_arrays("ref", last_res["ref"]), **record_arrays("tgt", last_res["tgt"]),
+              **{k: last_res[k] for k in ("time_differences", "range_differences", "position", "status", "iters")}}
 
     t_step = ms_res / args.steps / 1e3
-    t_e2e = ms_e2e / max(1, args.steps) / 1e3
+    t_e2e = ms_e2e / args.steps / 1e3
     value = world * pair_samples / t_step / 1e6
     e2e_value = world * pair_samples / t_e2e / 1e6
 
@@ -657,7 +684,7 @@ def main_ours(args):
         line = {
             "metric": "station-pair xcorr throughput", "value": value, "unit": "pair-Msamples/s", "n_gpus": world,
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": t_step * 1e3, "higher_is_better": True,
-            "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
+            "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic", "inputs_sha256": inputs_sha256,
             "config": dict(WORKLOAD_CONFIG, samples_per_station=n_samp,
                            parallelism=f"{world} rank(s), one capture set per rank, no data-path collective; "
                                        "one all_gather of 192-byte peak records per step" if world > 1 else "1 GPU"),
@@ -694,12 +721,15 @@ def main_ours(args):
     # BASELINE configs[3] as one job over the N GPUs (every rank takes part)
     shard = None
     if not args.no_sharded:
-        shard = sharded_block(args, torch, dist, T, device, local, rank, world)
+        shard, shard_out = sharded_block(args, torch, dist, T, device, local, rank, world)
+        dumped.update(shard_out)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
     rc = 0
     if line is not None:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, dumped)
         line["sharded"] = shard
         if world == 1 and not args.no_cpu_restatement:
             line["cpu_restatement"] = cpu_restatement()
@@ -757,7 +787,14 @@ def main():
     ap.add_argument("--shard-check", action="store_true", help="run the oracle sample of the sharded block at N > 1 too")
     ap.add_argument("--no-oracle-check", action="store_true", help="skip the CPU oracle at full size (parity_check.oracle_at_size)")
     ap.add_argument("--no-cpu-restatement", action="store_true", help="skip the C restatement baselines (cpu_restatement)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (peak records, time / range differences, fix, "
+                         "sharded tables) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's outputs (--impl ours)")
     with OnlyJsonOnStdout() as OUT:
         if args.impl == "reference":
             return main_reference(args)
