@@ -220,6 +220,62 @@ TDOA_API int tdoa_process(tdoa_engine *e, const double *stations_llh, tdoa_peak 
                           double *time_diffs, double *range_diffs, double *fix_llh, int32_t *fix_status,
                           int32_t *fix_iters);
 
+/* ---- windowed ProcessTDOA: one fix per TGT window (no reference equivalent; engine-defined).
+ * BINARY and EXTENDED modes (SOURCE has no REF correction, processor.go:853).  Window arguments as
+ * tdoa_xcorr_windows; P = S(S-1)/2 pairs i<j.
+ *  - Window time: the capture-sample index of the window's centre, start + (len - 1) / 2 mapped into the
+ *    capture of the pair's FIRST station i (b = nsamp_i / 3, g = guard_samples): REF sample k is at k when
+ *    k < b, else at 2b + g + (k - b); TGT sample k at b + g + k.  A REF window with samples in both block 1
+ *    and block 3 has no single time and takes no part in the fit.
+ *  - A record is usable unless it is EMPTY or EDGE, or margin < min_margin (min_margin = 0: no margin
+ *    test).  Its value y = lag + frac, in capture samples.
+ *  - REF fit per pair: least-squares line y = a + beta (t - t_mean) through the usable REF windows, sums in
+ *    f64 in window order; one window: beta = 0; none: the pair is used in no TGT window.  ref_max_residual
+ *    > 0: one refit without the windows whose |residual| from the first line exceeds it (none left: no fit).
+ *    ref_fit[p] = {REF lag at the centre of station i's block 2 (b + (b - 1) / 2; 0 without a fit), beta
+ *    (samples per sample = ppm * 1e-6), windows used}.
+ *  - Range difference of (TGT window w, pair p): (y_tgt / fs - (a + beta (t_w - t_mean)) / fs) * c, plus
+ *    |x_ref - s_j| - |x_ref - s_i| when has_ref_tx (the REF transmitter is not equidistant from i and j);
+ *    NaN and pair_used = 0 unless the TGT record is usable and the pair has a fit.  With whole blocks as
+ *    windows (win_len = hop = b, guard 0), no drift and no REF position this is tdoa_process's range
+ *    difference with chunk_samples = 0: exactly in BINARY, within 1e-3 samples in EXTENDED (the whole-signal
+ *    frac and the mean of two block fracs need not agree).
+ *  - Fix per TGT window: tdoa_solve_ls over the used pairs only (dims 2 or 3; start init_llh, or the mean
+ *    of the stations); rms over the used pairs.  fix_status 0 ok, 1 degenerate, 2 too few measurements
+ *    (fewer than dims used pairs, or used pairs touching fewer than dims + 1 stations; no iteration, the
+ *    start point is returned). */
+typedef struct {
+    int32_t dims;              /* 2 or 3 (3 needs >= 4 stations)                                  */
+    float min_margin;          /* records below this margin are not used; 0 = off                 */
+    double ref_max_residual;   /* samples; > 0: one refit without REF outliers; 0 = off           */
+    int32_t has_ref_tx;        /* 1: ref_tx_llh is the REF transmitter (geometric term)           */
+    int32_t has_init;          /* 1: init_llh is the least-squares start of every window          */
+    double ref_tx_llh[3];
+    double init_llh[3];
+} tdoa_window_opts;
+
+/* Captures -> REF and TGT tables -> range differences -> one fix per TGT window.  The tables are those
+ * tdoa_xcorr_windows gives for the same arguments, bit for bit (on a multi-GPU engine dealt and gathered
+ * the same way); the fix stage reads them where the pair loops left them in device memory.  On one GPU the
+ * pair loops make their checks as tdoa_xcorr_windows does; on a multi-GPU engine the call is collective and
+ * every rank runs the fix stage on its own gathered tables (no second collective), so every rank returns
+ * everything.  ref_out[n_ref * P], tgt_out[n_tgt * P], ref_fit[P][3], range_diffs[n_tgt][P],
+ * pair_used[n_tgt][P], fix_rms[n_tgt], fix_iters[n_tgt] may be NULL; fix_llh[n_tgt][3], fix_status[n_tgt]
+ * may not.  Refused (TDOA_E_INVALID): SOURCE mode, S < 3 or S > 64, dims not 2 or 3, dims 3 with S < 4,
+ * n_ref_windows < 1, n_tgt_windows < 1, bad window arguments. */
+TDOA_API int tdoa_process_windows(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts *o,
+                                  int64_t win_start, int64_t win_len, int32_t n_ref_windows, int32_t n_tgt_windows,
+                                  int64_t hop, tdoa_peak *ref_out, tdoa_peak *tgt_out, double *ref_fit,
+                                  double *range_diffs, uint8_t *pair_used, double *fix_llh, double *fix_rms,
+                                  int32_t *fix_status, int32_t *fix_iters);
+/* The same fix stage from host tables (e.g. kept from earlier tdoa_xcorr_windows calls); the window times
+ * come from the captures the engine holds.  Same arguments and refusals; ref_in / tgt_in may not be NULL. */
+TDOA_API int tdoa_window_fixes(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts *o,
+                               int64_t win_start, int64_t win_len, int32_t n_ref_windows, int32_t n_tgt_windows,
+                               int64_t hop, const tdoa_peak *ref_in, const tdoa_peak *tgt_in, double *ref_fit,
+                               double *range_diffs, uint8_t *pair_used, double *fix_llh, double *fix_rms,
+                               int32_t *fix_status, int32_t *fix_iters);
+
 /* crossCorrelate seam (processor.go:619-643): two host complex64 slices
  * (interleaved re,im), returns (delay, correlation).  Empty input -> (0, 0.0). */
 TDOA_API int tdoa_cross_correlate(tdoa_engine *e, const float *sig1_c64, int64_t n1,
@@ -329,7 +385,8 @@ typedef struct {
     float ms_demod;           /* fused unpack + power + FM discriminator launches */
     float ms_boxcar;          /* small box-car (DC subtract + low-pass + power)   */
     float ms_cand;            /* exact re-evaluation of the candidate lags        */
-    float reserved0;
+    float ms_fix;             /* fix stage of the last tdoa_process_windows / tdoa_window_fixes
+                                 (REF fit, range differences, least-squares fixes)  */
     int64_t demod_launches, demod_samples;
     int64_t boxcar_launches, boxcar_samples;
     int64_t cand_launches, cand_pair_samples;

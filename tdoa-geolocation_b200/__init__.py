@@ -21,6 +21,9 @@ from ._native import (  # noqa: F401
     load_library,
     host_alloc,
     comm_unique_id,
+    PEAK_DTYPE,
+    PEAK_EDGE,
+    PEAK_EMPTY,
 )
 from .processor import Station, TDOAProcessor  # noqa: F401
 from . import sharding  # noqa: F401
@@ -28,5 +31,5 @@ from . import analyzer  # noqa: F401
 
 __all__ = [
     "Engine", "TdoaError", "Peak", "MODE_SOURCE", "MODE_BINARY", "MODE_EXTENDED", "KIND_REF", "KIND_TGT",
-    "default_config", "library_path", "load_library", "host_alloc", "comm_unique_id", "Station", "TDOAProcessor", "sharding", "analyzer",
+    "default_config", "library_path", "load_library", "host_alloc", "comm_unique_id", "PEAK_DTYPE", "PEAK_EDGE", "PEAK_EMPTY", "Station", "TDOAProcessor", "sharding", "analyzer",
 ]

@@ -23,7 +23,7 @@ ERRORS = {-1: "TDOA_E_INVALID", -2: "TDOA_E_NODEVICE", -3: "TDOA_E_CUDA", -4: "T
 # every symbol include/tdoa_b200.h declares (tests check the library exports them all)
 ABI_SYMBOLS = [
     "tdoa_default_config", "tdoa_create", "tdoa_destroy", "tdoa_last_error", "tdoa_host_alloc", "tdoa_host_free",
-    "tdoa_load_u8", "tdoa_load_file", "tdoa_load_u8_pinned", "tdoa_load_u8_device", "tdoa_unpack", "tdoa_preprocess", "tdoa_xcorr", "tdoa_xcorr_device", "tdoa_xcorr_windows", "tdoa_process", "tdoa_xcorr_info", "tdoa_analyze",
+    "tdoa_load_u8", "tdoa_load_file", "tdoa_load_u8_pinned", "tdoa_load_u8_device", "tdoa_unpack", "tdoa_preprocess", "tdoa_xcorr", "tdoa_xcorr_device", "tdoa_xcorr_windows", "tdoa_process", "tdoa_process_windows", "tdoa_window_fixes", "tdoa_xcorr_info", "tdoa_analyze",
     "tdoa_cross_correlate", "tdoa_baselines", "tdoa_solve", "tdoa_solve_binary", "tdoa_solve_ls", "tdoa_grid", "tdoa_get_stats", "tdoa_stream",
     "tdoa_set_stream", "tdoa_synchronize", "tdoa_selftest",
     "tdoa_comm_unique_id", "tdoa_comm_init", "tdoa_comm_rank", "tdoa_shard_windows",
@@ -74,12 +74,18 @@ class SignalQuality(C.Structure):
         return {k: getattr(self, k) for k, _ in self._fields_}
 
 
+class WindowOpts(C.Structure):
+    _fields_ = [("dims", C.c_int32), ("min_margin", C.c_float), ("ref_max_residual", C.c_double),
+                ("has_ref_tx", C.c_int32), ("has_init", C.c_int32), ("ref_tx_llh", C.c_double * 3),
+                ("init_llh", C.c_double * 3)]
+
+
 class Stats(C.Structure):
     _fields_ = [
         ("launches_total", C.c_int64), ("launches_last", C.c_int64), ("ms_preprocess", C.c_float),
         ("ms_fft", C.c_float), ("ms_exact", C.c_float), ("ms_total", C.c_float), ("fft_launches", C.c_int64),
         ("ms_fft_seg", C.c_float), ("fft_pair_samples", C.c_int64), ("brute_pairs", C.c_int64),
-        ("ms_demod", C.c_float), ("ms_boxcar", C.c_float), ("ms_cand", C.c_float), ("reserved0", C.c_float),
+        ("ms_demod", C.c_float), ("ms_boxcar", C.c_float), ("ms_cand", C.c_float), ("ms_fix", C.c_float),
         ("demod_launches", C.c_int64), ("demod_samples", C.c_int64),
         ("boxcar_launches", C.c_int64), ("boxcar_samples", C.c_int64),
         ("cand_launches", C.c_int64), ("cand_pair_samples", C.c_int64),
@@ -144,6 +150,8 @@ def load_library():
     L.tdoa_analyze.argtypes = [vp, i32, i32, vp, vp]
     L.tdoa_xcorr_device.argtypes = [vp, i32, i64, i64, i32, i64, vp]
     L.tdoa_xcorr_windows.argtypes = [vp, i64, i64, i32, i32, i64, vp, vp]
+    L.tdoa_process_windows.argtypes = [vp, vp, C.POINTER(WindowOpts), i64, i64, i32, i32, i64] + [vp] * 9
+    L.tdoa_window_fixes.argtypes = [vp, vp, C.POINTER(WindowOpts), i64, i64, i32, i32, i64] + [vp] * 9
     L.tdoa_cross_correlate.argtypes = [vp, vp, i64, vp, i64, C.POINTER(PeakStruct)]
     L.tdoa_baselines.argtypes = [vp, vp, i32, vp]
     L.tdoa_solve.argtypes = [vp, vp, i32, vp, i32, i32, vp, vp, vp]
@@ -442,6 +450,52 @@ class Engine:
                                            C.byref(status), C.byref(iters)))
         return {"ref": ref, "tgt": tgt, "time_differences": td, "range_differences": rd, "position": fix,
                 "status": int(status.value), "iters": int(iters.value)}
+
+    def _windows(self, fn, stations_llh, win_start, win_len, n_ref_windows, n_tgt_windows, hop, tables, dims,
+                 min_margin, ref_max_residual, ref_tx_llh, init_llh) -> dict:
+        st = np.ascontiguousarray(stations_llh, dtype=np.float64).reshape(-1, 3)
+        if st.shape[0] != self.n_stations:
+            raise ValueError(f"stations_llh has {st.shape[0]} rows, the engine holds {self.n_stations} stations")
+        o = WindowOpts(dims=dims, min_margin=min_margin, ref_max_residual=ref_max_residual,
+                       has_ref_tx=ref_tx_llh is not None, has_init=init_llh is not None)
+        if ref_tx_llh is not None:
+            o.ref_tx_llh[:] = [float(v) for v in ref_tx_llh]
+        if init_llh is not None:
+            o.init_llh[:] = [float(v) for v in init_llh]
+        P, nt = self.n_pairs, max(n_tgt_windows, 0)
+        ref_fit, rd = np.zeros((P, 3), np.float64), np.zeros((nt, P), np.float64)
+        used = np.zeros((nt, P), np.uint8)
+        fix, rms = np.zeros((nt, 3), np.float64), np.zeros(nt, np.float64)
+        status, iters = np.zeros(nt, np.int32), np.zeros(nt, np.int32)
+        self._check(fn(self._h, _ptr(st), C.byref(o), win_start, win_len, n_ref_windows, n_tgt_windows, hop,
+                       *[_ptr(t) for t in tables], _ptr(ref_fit), _ptr(rd), _ptr(used), _ptr(fix), _ptr(rms),
+                       _ptr(status), _ptr(iters)))
+        return {"ref_fit": ref_fit, "range_differences": rd, "pair_used": used.astype(bool), "position": fix,
+                "rms": rms, "status": status, "iters": iters}
+
+    def process_windows(self, stations_llh, win_start: int, win_len: int, n_ref_windows: int, n_tgt_windows: int,
+                        hop: int, dims: int = 2, min_margin: float = 0.0, ref_max_residual: float = 0.0,
+                        ref_tx_llh=None, init_llh=None) -> dict:
+        """Windowed ProcessTDOA (tdoa_process_windows): REF and TGT tables as xcorr_windows gives them, the REF
+        lag's linear track per pair (ref_fit: lag at block 2's centre, drift in samples per sample, windows
+        used), range differences and the used mask per (TGT window, pair), one least-squares fix per TGT window
+        (status 0 ok, 1 degenerate, 2 too few measurements).  ref_tx_llh: the REF transmitter's position, whose
+        geometric range difference is added back."""
+        ref = np.zeros((max(n_ref_windows, 0), self.n_pairs), PEAK_DTYPE)
+        tgt = np.zeros((max(n_tgt_windows, 0), self.n_pairs), PEAK_DTYPE)
+        out = self._windows(self._lib.tdoa_process_windows, stations_llh, win_start, win_len, n_ref_windows,
+                            n_tgt_windows, hop, (ref, tgt), dims, min_margin, ref_max_residual, ref_tx_llh, init_llh)
+        out["ref"], out["tgt"] = ref, tgt
+        return out
+
+    def window_fixes(self, stations_llh, win_start: int, win_len: int, ref, tgt, hop: int, dims: int = 2,
+                     min_margin: float = 0.0, ref_max_residual: float = 0.0, ref_tx_llh=None, init_llh=None) -> dict:
+        """The fix stage of process_windows on given tables (tdoa_window_fixes): ref[n_ref][P], tgt[n_tgt][P] of
+        PEAK_DTYPE, e.g. kept from xcorr_windows; window times come from the captures the engine holds."""
+        ref = np.ascontiguousarray(ref, PEAK_DTYPE).reshape(-1, self.n_pairs)
+        tgt = np.ascontiguousarray(tgt, PEAK_DTYPE).reshape(-1, self.n_pairs)
+        return self._windows(self._lib.tdoa_window_fixes, stations_llh, win_start, win_len, ref.shape[0], tgt.shape[0],
+                             hop, (ref, tgt), dims, min_margin, ref_max_residual, ref_tx_llh, init_llh)
 
     def solve_ls(self, stations_llh, range_diffs, init_llh=None, dims: int = 2):
         """Levenberg-Marquardt fix over all pair range differences (engine-defined, SURVEY 8f-4).

@@ -28,6 +28,7 @@ UNITS = [
     ("seqsum.cu", ["-fmad=false"]),
     ("xcorr_exact.cu", ["-fmad=false"]),
     ("solve.cu", ["-fmad=false"]),
+    ("window_fix.cu", ["-fmad=false"]),
     ("analyze.cu", ["-fmad=false"]),
     ("xcorr_fft.cu", []),
     ("xcorr_tile.cu", []),

@@ -178,6 +178,10 @@ int window_lengths(tdoa_engine *e, int32_t kind, int64_t win_start, int64_t win_
                    std::vector<i64> &len);
 int xcorr_core(tdoa_engine *e, int32_t kind, int64_t win_start, const std::vector<i64> &len, int32_t n_windows,
                int64_t hop, PeakRec *d_out, Pending *pend);
+// tdoa_xcorr / tdoa_xcorr_device as one call; d_table (device, n_windows * P, out may then be nullptr): the
+// records are also left there, past the call's end (tdoa_process_windows)
+int xcorr_impl(tdoa_engine *e, int32_t kind, int64_t win_start, int64_t win_len, int32_t n_windows, int64_t hop,
+               tdoa_peak *out, bool out_is_device, PeakRec *d_table = nullptr);
 
 // ---- more than one GPU (engine_multi.cu)
 // windows dealt over the ranks of the engine's communicator, records gathered: true if it took the call

@@ -1344,12 +1344,12 @@ int xcorr_core(tdoa_engine *e, int32_t kind, int64_t win_start, const std::vecto
 }
 
 int xcorr_impl(tdoa_engine *e, int32_t kind, int64_t win_start, int64_t win_len, int32_t n_windows, int64_t hop,
-               tdoa_peak *out, bool out_is_device)
+               tdoa_peak *out, bool out_is_device, PeakRec *d_table)
 {
     if (!e) return TDOA_E_INVALID;
     int rc = begin_call(e);
     if (rc) return rc;
-    if (!out) return fail(e, TDOA_E_INVALID, "tdoa_xcorr: out is NULL");
+    if (!out && !d_table) return fail(e, TDOA_E_INVALID, "tdoa_xcorr: out is NULL");
     std::vector<i64> len;
     if ((rc = window_lengths(e, kind, win_start, win_len, n_windows, hop, len))) return rc;
     // more than one GPU: windows dealt over the ranks, records gathered (engine_multi.cu)
@@ -1357,6 +1357,7 @@ int xcorr_impl(tdoa_engine *e, int32_t kind, int64_t win_start, int64_t win_len,
     const int S = e->cfg.n_stations, P = S * (S - 1) / 2;
     PeakRec *d_out = nullptr;
     if (out_is_device) d_out = reinterpret_cast<PeakRec *>(out);
+    else if (d_table) d_out = d_table;
     else if ((rc = alloc_t(e, &d_out, (size_t)n_windows * P))) return rc;
     stats_reset(e);
     cudaEventRecord(e->ev[0], e->stream);
@@ -1397,7 +1398,7 @@ int xcorr_impl(tdoa_engine *e, int32_t kind, int64_t win_start, int64_t win_len,
         if (ok) {
             e->info_first[kind] = h_first;
             fill_info(e, kind, pend[0].sigs, h_stats[0].data(), S);
-            std::memcpy(out, h_pk.data(), h_pk.size() * sizeof(PeakRec));
+            if (out) std::memcpy(out, h_pk.data(), h_pk.size() * sizeof(PeakRec));
             done = true;
         } else {
             spans_collect(e);
@@ -1406,7 +1407,7 @@ int xcorr_impl(tdoa_engine *e, int32_t kind, int64_t win_start, int64_t win_len,
     if (!done) {
         if ((rc = xcorr_core(e, kind, win_start, len, n_windows, hop, d_out, nullptr))) return rc;
         cudaEventRecord(e->ev[4], e->stream);
-        if (!out_is_device)
+        if (!out_is_device && out)
             CU(cudaMemcpyAsync(out, d_out, (size_t)n_windows * P * sizeof(tdoa_peak), cudaMemcpyDeviceToHost, e->stream));
     }
     rc = end_call(e, !out_is_device);

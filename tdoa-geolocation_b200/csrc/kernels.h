@@ -175,8 +175,17 @@ void launch_solve(const double *d_llh, const double *d_rd, int n_sets, int rd_st
 void launch_solve_binary(const double *d_llh, const double *d_rd, int n_rd, double *d_out_llh, int *d_info, double *d_trace,
                          cudaStream_t st);
 void launch_solve_ls(const double *d_llh, int n_st, const double *d_rd, int n_sets, int rd_stride, const double *d_init,
-                     int dims, double *d_out_llh, double *d_rms, int *d_status, int *d_iters, cudaStream_t st);
+                     int dims, double *d_out_llh, double *d_rms, int *d_status, int *d_iters, cudaStream_t st,
+                     const uint8_t *d_used = nullptr);   // d_used[set * rd_stride + p]: pair p takes part
 int solve_ls_max_stations();
+// ---- window_fix.cu (tdoa_process_windows / tdoa_window_fixes): the REF drift fit per pair and the
+// range differences per (TGT window, pair); the fix is launch_solve_ls with the used mask
+void launch_window_ref_fit(const PeakRec *d_ref, int n_ref, int n_st, const double *d_t_ref, const double *d_t_mid,
+                           const double *d_llh, const double *d_ref_tx, float min_margin, double max_resid, double *d_fit,
+                           double *d_ref_fit, cudaStream_t st);
+void launch_window_rd(const PeakRec *d_tgt, int n_tgt, int n_st, const double *d_t_tgt, const double *d_fit, float min_margin,
+                      double fs, double *d_rd, uint8_t *d_used, cudaStream_t st);
+constexpr int kWindowFitDoubles = 5;   // per pair: a, beta, t_mean, windows used, geometric term
 void launch_range_diffs(const PeakRec *d_ref, const PeakRec *d_tgt, int n_pairs, double fs, int mode, double *d_td,
                         double *d_rd, cudaStream_t st);
 void launch_grid_cells(const double *d_llh, int n_st, const double *d_grid_desc, int nlat, int nlon,

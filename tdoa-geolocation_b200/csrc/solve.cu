@@ -5,26 +5,12 @@
 // (:151-163), solveTDOA (:932-1020) and ecefToLatLon (:1023-1045).  All f64, written
 // in the reference's operation order.  The grid solve has no reference equivalent
 // (oracle: orc_grid_solve).
+#include "geodesy.cuh"
 #include "kernels.h"
 
 namespace tdoa {
 
 namespace {
-
-constexpr double kA = 6378137.0;
-constexpr double kF = 1.0 / 298.257223563;
-constexpr double kPi = 3.14159265358979323846;
-
-__device__ void llh_to_ecef(double lat, double lon, double elev, double *xyz)
-{
-    const double e2 = 2 * kF - kF * kF;
-    const double lr = lat * kPi / 180, lo = lon * kPi / 180;
-    const double sl = sin(lr), cl = cos(lr), so = sin(lo), co = cos(lo);
-    const double N = kA / sqrt(1 - e2 * sl * sl);
-    xyz[0] = (N + elev) * cl * co;
-    xyz[1] = (N + elev) * cl * so;
-    xyz[2] = (N * (1 - e2) + elev) * sl;
-}
 
 __device__ void ecef_to_llh(double x, double y, double z, double *llh)
 {
@@ -189,11 +175,14 @@ __global__ void k_solve_binary(const double *llh, const double *rd, int n_rd, do
 //   the unit vector from station k to x;  (J'J + lambda diag(J'J)) d = -J'f;  a step is
 //   taken only if it lowers sum f^2 (lambda / 3), else lambda * 4, at most 8 tries;
 //   stop after 60 iterations, when no try succeeds, or when |d| < 1e-6 m.
+// used (may be nullptr): per set and pair, 0 leaves the pair out of the cost, the normal equations
+// and the rms; fewer than `dims` used pairs, or used pairs touching fewer than dims + 1 stations,
+// give status 2 with the start point and no iteration (tdoa_process_windows).
 struct LsPoint {
     double lat, lon, h;  // degrees, degrees, metres
 };
 
-__device__ double ls_cost(const double *s_st, int n_st, const double *rd, const LsPoint &p, double *r_out)
+__device__ double ls_cost(const double *s_st, int n_st, const double *rd, const uint8_t *used, const LsPoint &p, double *r_out)
 {
     double x[3];
     llh_to_ecef(p.lat, p.lon, p.h, x);
@@ -205,6 +194,7 @@ __device__ double ls_cost(const double *s_st, int n_st, const double *rd, const 
     int q = 0;
     for (int i = 0; i < n_st; i++)
         for (int j = i + 1; j < n_st; j++, q++) {
+            if (used && !used[q]) continue;
             const double f = (r_out[j] - r_out[i]) - rd[q];
             c += f * f;
         }
@@ -246,7 +236,8 @@ __device__ bool ls_step(const double (&A)[3][3], const double (&b)[3], double la
 constexpr int kLsMaxStations = 64;
 
 __global__ void k_solve_ls(const double *llh, int n_st, const double *rd_all, int n_sets, int rd_stride,
-                           const double *init_llh, int dims, double *out_llh, double *out_rms, int *status, int *iters)
+                           const double *init_llh, int dims, double *out_llh, double *out_rms, int *status, int *iters,
+                           const uint8_t *used_all)
 {
     extern __shared__ double s_st[];  // station ECEF
     for (int k = threadIdx.x; k < n_st; k += blockDim.x) llh_to_ecef(llh[3 * k], llh[3 * k + 1], llh[3 * k + 2], s_st + 3 * k);
@@ -254,7 +245,8 @@ __global__ void k_solve_ls(const double *llh, int n_st, const double *rd_all, in
     const int set = blockIdx.x * blockDim.x + threadIdx.x;
     if (set >= n_sets) return;
     const double *rd = rd_all + (size_t)set * rd_stride;
-    const int P = n_st * (n_st - 1) / 2;
+    const uint8_t *used = used_all ? used_all + (size_t)set * rd_stride : nullptr;
+    int P = n_st * (n_st - 1) / 2;
     const double e2 = 2 * kF - kF * kF;
     LsPoint p;
     if (init_llh) {
@@ -264,9 +256,26 @@ __global__ void k_solve_ls(const double *llh, int n_st, const double *rd_all, in
         for (int k = 0; k < n_st; k++) { p.lat += llh[3 * k]; p.lon += llh[3 * k + 1]; p.h += llh[3 * k + 2]; }
         p.lat /= n_st; p.lon /= n_st; p.h /= n_st;
     }
+    if (used) {   // too few measurements: no iteration
+        int n_used = 0, q = 0;
+        unsigned long long touched = 0ull;
+        for (int i = 0; i < n_st; i++)
+            for (int j = i + 1; j < n_st; j++, q++)
+                if (used[q]) { n_used++; touched |= (1ull << i) | (1ull << j); }
+        if (n_used < dims || __popcll(touched) < dims + 1) {
+            out_llh[3 * set] = p.lat;
+            out_llh[3 * set + 1] = p.lon;
+            out_llh[3 * set + 2] = p.h;
+            if (out_rms) out_rms[set] = 0.0;
+            status[set] = 2;
+            if (iters) iters[set] = 0;
+            return;
+        }
+        P = n_used;
+    }
     double r[kLsMaxStations], g[kLsMaxStations][3];
     double lambda = 1e-3;
-    double cost = ls_cost(s_st, n_st, rd, p, r);
+    double cost = ls_cost(s_st, n_st, rd, used, p, r);
     int it = 0, st = 0;
     for (; it < 60; it++) {
         const double lr = p.lat * kPi / 180, lo = p.lon * kPi / 180;
@@ -285,6 +294,7 @@ __global__ void k_solve_ls(const double *llh, int n_st, const double *rd_all, in
         int q = 0;
         for (int i = 0; i < n_st; i++)
             for (int j = i + 1; j < n_st; j++, q++) {
+                if (used && !used[q]) continue;
                 const double f = (r[j] - r[i]) - rd[q];
                 const double row[3] = {g[j][0] - g[i][0], g[j][1] - g[i][1], g[j][2] - g[i][2]};
                 for (int a = 0; a < 3; a++) {
@@ -301,7 +311,7 @@ __global__ void k_solve_ls(const double *llh, int n_st, const double *rd_all, in
             c.lon = p.lon + d[0] / ((Nr + p.h) * cl) * 180.0 / kPi;
             if (dims == 3) c.h = p.h + d[2];
             double rc[kLsMaxStations];
-            const double cc = ls_cost(s_st, n_st, rd, c, rc);
+            const double cc = ls_cost(s_st, n_st, rd, used, c, rc);
             if (cc < cost) {
                 p = c; cost = cc; moved = true;
                 for (int k = 0; k < n_st; k++) r[k] = rc[k];
@@ -497,11 +507,12 @@ void launch_range_diffs(const PeakRec *d_ref, const PeakRec *d_tgt, int n_pairs,
 int solve_ls_max_stations() { return kLsMaxStations; }
 
 void launch_solve_ls(const double *d_llh, int n_st, const double *d_rd, int n_sets, int rd_stride, const double *d_init,
-                     int dims, double *d_out_llh, double *d_rms, int *d_status, int *d_iters, cudaStream_t st)
+                     int dims, double *d_out_llh, double *d_rms, int *d_status, int *d_iters, cudaStream_t st,
+                     const uint8_t *d_used)
 {
     if (n_sets <= 0) return;
     k_solve_ls<<<(n_sets + 31) / 32, 32, 3 * n_st * sizeof(double), st>>>(d_llh, n_st, d_rd, n_sets, rd_stride, d_init, dims,
-                                                                       d_out_llh, d_rms, d_status, d_iters);
+                                                                       d_out_llh, d_rms, d_status, d_iters, d_used);
 }
 
 // ---------------------------------------------------------------- grid multilateration, ranked

@@ -1,0 +1,355 @@
+// window_fix.cu -- from window tables to range differences, one fix per TGT window
+// (tdoa_process_windows, tdoa_window_fixes; no reference equivalent; restated in tests/window_oracle.py).
+//
+// An RTL-SDR's sample clock is off by ppm, so the lag between two collectors drifts linearly over
+// the capture (1 ppm of relative rate = 2 samples per second at 2 Msps).  The reference correlates
+// the REF blocks 1 and 3 as one signal, which evaluates the REF lag at block 2's centre: right for a
+// TGT correlation over the whole of block 2, but a 1 s TGT window 16 s from that centre keeps
+// 33 samples (5 km) of error per ppm.  Here the REF lag's linear track is fitted per pair across the
+// REF windows and evaluated at each TGT window's time:
+//   k_window_ref_fit  one thread per pair: least-squares line y = a + beta (t - t_mean) through the
+//                     usable REF windows (sums in f64, window order), one optional refit without the
+//                     windows whose residual exceeds max_resid, the REF transmitter's geometric term
+//   k_window_rd       one thread per (TGT window, pair): rd = (y_tgt / fs - y_ref(t_w) / fs) * c
+//                     (+ the geometric term) and the used mask that k_solve_ls reads.
+// Window times and the usable test are stated in include/tdoa_b200.h (tdoa_process_windows).
+#include <cuda_runtime.h>
+
+#include <cmath>
+#include <vector>
+
+#include "engine_internal.h"
+#include "geodesy.cuh"
+
+using namespace tdoa;
+
+namespace tdoa {
+
+namespace {
+
+constexpr double kC = 299792458.0;
+
+__device__ __forceinline__ bool record_usable(const PeakRec &r, float min_margin)
+{
+    if (r.flags & (TDOA_PEAK_EMPTY | TDOA_PEAK_EDGE)) return false;
+    return !(min_margin > 0.f && r.margin < min_margin);
+}
+
+__device__ __forceinline__ double record_lag(const PeakRec &r) { return (double)r.lag + (double)r.frac; }
+
+// pair p = (i, j), i < j lexicographic
+__device__ __forceinline__ void pair_stations(int p, int n_st, int &i, int &j)
+{
+    int rem = p;
+    i = 0;
+    while (rem >= n_st - 1 - i) { rem -= n_st - 1 - i; i++; }
+    j = i + 1 + rem;
+}
+
+// least-squares line through the REF windows of pair p that pass the usable test, the time test (a window
+// with samples in blocks 1 and 3 has no time: NaN) and -- refit -- |y - line0(t)| <= max_resid
+struct Line { double a, beta, t_mean; int n; };
+
+__device__ Line fit_line(const PeakRec *ref, int n_ref, int P, int p, const double *t_ref, int n_st, int i, float min_margin,
+                         const Line *line0, double max_resid)
+{
+    auto take = [&](int w, double &t, double &y) -> bool {
+        const PeakRec r = ref[(size_t)w * P + p];
+        t = t_ref[(size_t)w * n_st + i];
+        if (!record_usable(r, min_margin) || isnan(t)) return false;
+        y = record_lag(r);
+        return !line0 || !(fabs(y - (line0->a + line0->beta * (t - line0->t_mean))) > max_resid);
+    };
+    int n = 0;
+    double st = 0.0, sy = 0.0;
+    for (int w = 0; w < n_ref; w++) {
+        double t, y;
+        if (take(w, t, y)) { n++; st += t; sy += y; }
+    }
+    Line L{0.0, 0.0, 0.0, n};
+    if (n == 0) return L;
+    L.t_mean = st / n;
+    L.a = sy / n;
+    double stt = 0.0, sty = 0.0;
+    for (int w = 0; w < n_ref; w++) {
+        double t, y;
+        if (take(w, t, y)) {
+            const double dt = t - L.t_mean;
+            stt += dt * dt;
+            sty += dt * (y - L.a);
+        }
+    }
+    if (n > 1 && stt > 0.0) L.beta = sty / stt;
+    return L;
+}
+
+__global__ void k_window_ref_fit(const PeakRec *ref, int n_ref, int n_st, const double *t_ref, const double *t_mid,
+                                 const double *llh, const double *ref_tx, float min_margin, double max_resid, double *fit,
+                                 double *ref_fit)
+{
+    const int P = n_st * (n_st - 1) / 2;
+    const int p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= P) return;
+    int i, j;
+    pair_stations(p, n_st, i, j);
+    Line L = fit_line(ref, n_ref, P, p, t_ref, n_st, i, min_margin, nullptr, 0.0);
+    if (max_resid > 0.0 && L.n > 0) {
+        const Line L0 = L;
+        L = fit_line(ref, n_ref, P, p, t_ref, n_st, i, min_margin, &L0, max_resid);
+    }
+    double geo = 0.0;
+    if (ref_tx) {
+        double x[3], a[3], b[3];
+        llh_to_ecef(ref_tx[0], ref_tx[1], ref_tx[2], x);
+        llh_to_ecef(llh[3 * i], llh[3 * i + 1], llh[3 * i + 2], a);
+        llh_to_ecef(llh[3 * j], llh[3 * j + 1], llh[3 * j + 2], b);
+        const double ri = sqrt((x[0] - a[0]) * (x[0] - a[0]) + (x[1] - a[1]) * (x[1] - a[1]) + (x[2] - a[2]) * (x[2] - a[2]));
+        const double rj = sqrt((x[0] - b[0]) * (x[0] - b[0]) + (x[1] - b[1]) * (x[1] - b[1]) + (x[2] - b[2]) * (x[2] - b[2]));
+        geo = rj - ri;
+    }
+    double *f = fit + (size_t)kWindowFitDoubles * p;
+    f[0] = L.a; f[1] = L.beta; f[2] = L.t_mean; f[3] = (double)L.n; f[4] = geo;
+    if (ref_fit) {
+        ref_fit[3 * p] = L.n > 0 ? L.a + L.beta * (t_mid[i] - L.t_mean) : 0.0;
+        ref_fit[3 * p + 1] = L.beta;
+        ref_fit[3 * p + 2] = (double)L.n;
+    }
+}
+
+__global__ void k_window_rd(const PeakRec *tgt, int n_tgt, int n_st, const double *t_tgt, const double *fit, float min_margin,
+                            double fs, double *rd, uint8_t *used)
+{
+    const int P = n_st * (n_st - 1) / 2;
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n_tgt * P) return;
+    const int w = k / P, p = k - w * P;
+    int i, j;
+    pair_stations(p, n_st, i, j);
+    const double *f = fit + (size_t)kWindowFitDoubles * p;
+    const PeakRec r = tgt[k];
+    const bool ok = f[3] > 0.0 && record_usable(r, min_margin);
+    double v = __longlong_as_double(0x7ff8000000000000ll);   // NaN: pair not used in this window
+    if (ok) {
+        const double y_ref = f[0] + f[1] * (t_tgt[(size_t)w * n_st + i] - f[2]);
+        // k_range_diffs' order: dt = y_tgt / fs - y_ref / fs, rd = dt * c
+        v = (record_lag(r) / fs - y_ref / fs) * kC + f[4];
+    }
+    rd[k] = v;
+    used[k] = ok ? 1 : 0;
+}
+
+}  // namespace
+
+void launch_window_ref_fit(const PeakRec *d_ref, int n_ref, int n_st, const double *d_t_ref, const double *d_t_mid,
+                           const double *d_llh, const double *d_ref_tx, float min_margin, double max_resid, double *d_fit,
+                           double *d_ref_fit, cudaStream_t st)
+{
+    const int P = n_st * (n_st - 1) / 2;
+    if (P > 0)
+        k_window_ref_fit<<<(P + 63) / 64, 64, 0, st>>>(d_ref, n_ref, n_st, d_t_ref, d_t_mid, d_llh, d_ref_tx, min_margin,
+                                                       max_resid, d_fit, d_ref_fit);
+}
+
+void launch_window_rd(const PeakRec *d_tgt, int n_tgt, int n_st, const double *d_t_tgt, const double *d_fit, float min_margin,
+                      double fs, double *d_rd, uint8_t *d_used, cudaStream_t st)
+{
+    const int n = n_tgt * (n_st * (n_st - 1) / 2);
+    if (n > 0) k_window_rd<<<(n + 127) / 128, 128, 0, st>>>(d_tgt, n_tgt, n_st, d_t_tgt, d_fit, min_margin, fs, d_rd, d_used);
+}
+
+// ---------------------------------------------------------------- host side
+
+namespace {
+
+// what the fix stage needs besides the tables: window times per (window, station), block-2 centres
+struct WinTimes {
+    int n_ref = 0, n_tgt = 0;
+    std::vector<double> t_ref, t_tgt, t_mid;
+    std::vector<ShardPart> parts;   // per kind: window lengths as the pair loops take them
+};
+
+// make_view's mapping is the one place that knows where a window lies in the capture
+double window_time(const Station &s, int kind, i64 start, i64 len, i64 guard)
+{
+    const SigSrc v = make_view(s, kind, start, len, guard);
+    if (s.nsamp / 3 > 0 && v.run0_len < len) return NAN;   // REF window across blocks 1 and 3
+    return (double)v.run0_start + 0.5 * (double)(len - 1);
+}
+
+int window_check(tdoa_engine *e, const char *fn, const double *stations_llh, const tdoa_window_opts *o, int64_t win_start,
+                 int64_t win_len, int32_t n_ref, int32_t n_tgt, int64_t hop, const double *fix_llh, const int32_t *fix_status,
+                 WinTimes &T)
+{
+    const int S = e->cfg.n_stations;
+    if (!stations_llh || !o || !fix_llh || !fix_status) return fail(e, TDOA_E_INVALID, "%s: NULL argument", fn);
+    if (e->cfg.mode == TDOA_MODE_SOURCE)
+        return fail(e, TDOA_E_INVALID, "%s: SOURCE mode has no REF correction (processor.go:853)", fn);
+    if (S < 3 || S > solve_ls_max_stations())
+        return fail(e, TDOA_E_INVALID, "%s: 3..%d stations, got %d", fn, solve_ls_max_stations(), S);
+    if (o->dims != 2 && o->dims != 3) return fail(e, TDOA_E_INVALID, "%s: dims must be 2 or 3, got %d", fn, o->dims);
+    if (o->dims == 3 && S < 4) return fail(e, TDOA_E_INVALID, "%s: dims 3 needs at least 4 stations", fn);
+    if (n_ref < 1 || n_tgt < 1)
+        return fail(e, TDOA_E_INVALID, "%s: need >= 1 REF and >= 1 TGT window, got %d and %d", fn, n_ref, n_tgt);
+    T.n_ref = n_ref; T.n_tgt = n_tgt;
+    T.parts.assign(2, ShardPart{});
+    int rc;
+    for (int kind = 0; kind < 2; kind++) {
+        ShardPart &Q = T.parts[kind];
+        Q.kind = kind; Q.win_start = win_start; Q.hop = hop;
+        Q.n_windows = kind == TDOA_KIND_REF ? n_ref : n_tgt;
+        if ((rc = window_lengths(e, kind, win_start, win_len, Q.n_windows, hop, Q.len))) return rc;
+        std::vector<double> &t = kind == TDOA_KIND_REF ? T.t_ref : T.t_tgt;
+        t.resize((size_t)Q.n_windows * S);
+        for (int w = 0; w < Q.n_windows; w++)
+            for (int st = 0; st < S; st++)
+                t[(size_t)w * S + st] = window_time(e->stations[st], kind, win_start + (i64)w * hop, Q.len[st], e->cfg.guard_samples);
+    }
+    T.t_mid.resize(S);
+    for (int st = 0; st < S; st++) {
+        const i64 b = e->stations[st].nsamp / 3;
+        T.t_mid[st] = (double)b + 0.5 * (double)(b - 1);
+    }
+    return TDOA_OK;
+}
+
+// the fix stage on device tables, queued on the engine's stream inside the caller's begin_call / end_call;
+// the station table, times and options ride in the descriptor frame
+int fix_stage(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts *o, const WinTimes &T, const PeakRec *d_ref,
+              const PeakRec *d_tgt, double *ref_fit, double *range_diffs, uint8_t *pair_used, double *fix_llh, double *fix_rms,
+              int32_t *fix_status, int32_t *fix_iters)
+{
+    const int S = e->cfg.n_stations, P = S * (S - 1) / 2, nt = T.n_tgt;
+    int rc;
+    const double *d_llh = nullptr, *d_t_ref = nullptr, *d_t_tgt = nullptr, *d_t_mid = nullptr, *d_ref_tx = nullptr,
+                 *d_init = nullptr;
+    if ((rc = upload(e, std::vector<double>(stations_llh, stations_llh + (size_t)3 * S), &d_llh)) ||
+        (rc = upload(e, T.t_ref, &d_t_ref)) || (rc = upload(e, T.t_tgt, &d_t_tgt)) || (rc = upload(e, T.t_mid, &d_t_mid)))
+        return rc;
+    if (o->has_ref_tx && (rc = upload(e, std::vector<double>(o->ref_tx_llh, o->ref_tx_llh + 3), &d_ref_tx))) return rc;
+    if (o->has_init) {
+        std::vector<double> init((size_t)3 * nt);
+        for (int w = 0; w < nt; w++)
+            for (int k = 0; k < 3; k++) init[(size_t)3 * w + k] = o->init_llh[k];
+        if ((rc = upload(e, init, &d_init))) return rc;
+    }
+    double *d_fit = nullptr, *d_ref_fit = nullptr, *d_rd = nullptr, *d_fix = nullptr, *d_rms = nullptr;
+    uint8_t *d_used = nullptr;
+    int *d_status = nullptr, *d_iters = nullptr;
+    if ((rc = alloc_t(e, &d_fit, (size_t)kWindowFitDoubles * P)) || (rc = alloc_t(e, &d_ref_fit, (size_t)3 * P)) ||
+        (rc = alloc_t(e, &d_rd, (size_t)nt * P)) || (rc = alloc_t(e, &d_used, (size_t)nt * P)) ||
+        (rc = alloc_t(e, &d_fix, (size_t)3 * nt)) || (rc = alloc_t(e, &d_rms, (size_t)nt)) ||
+        (rc = alloc_t(e, &d_status, (size_t)nt)) || (rc = alloc_t(e, &d_iters, (size_t)nt)))
+        return rc;
+    CU(cudaEventRecord(e->ev[1], e->stream));
+    launch_window_ref_fit(d_ref, T.n_ref, S, d_t_ref, d_t_mid, d_llh, d_ref_tx, o->min_margin, o->ref_max_residual, d_fit,
+                          d_ref_fit, e->stream);
+    launch_window_rd(d_tgt, nt, S, d_t_tgt, d_fit, o->min_margin, e->cfg.sample_rate, d_rd, d_used, e->stream);
+    launch_solve_ls(d_llh, S, d_rd, nt, P, d_init, o->dims, d_fix, d_rms, d_status, d_iters, e->stream, d_used);
+    count_launch(e, 3);
+    CU(cudaEventRecord(e->ev[2], e->stream));
+    CU(cudaGetLastError());
+    auto back = [&](void *dst, const void *src, size_t bytes) -> int {
+        if (dst) CU(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, e->stream));
+        return TDOA_OK;
+    };
+    if ((rc = back(ref_fit, d_ref_fit, (size_t)3 * P * sizeof(double))) ||
+        (rc = back(range_diffs, d_rd, (size_t)nt * P * sizeof(double))) || (rc = back(pair_used, d_used, (size_t)nt * P)) ||
+        (rc = back(fix_llh, d_fix, (size_t)3 * nt * sizeof(double))) || (rc = back(fix_rms, d_rms, (size_t)nt * sizeof(double))) ||
+        (rc = back(fix_status, d_status, (size_t)nt * sizeof(int32_t))) ||
+        (rc = back(fix_iters, d_iters, (size_t)nt * sizeof(int32_t))))
+        return rc;
+    return TDOA_OK;
+}
+
+int finish_fix_stage(tdoa_engine *e)
+{
+    const int rc = end_call(e, true);
+    if (rc) return rc;
+    float t = 0.f;
+    cudaEventElapsedTime(&t, e->ev[1], e->ev[2]);
+    e->st.ms_fix = t;
+    return TDOA_OK;
+}
+
+// the two device tables of tdoa_process_windows: they outlive the pair loops' calls
+struct Tables {
+    cudaStream_t st;
+    PeakRec *ref = nullptr, *tgt = nullptr;
+    ~Tables()
+    {
+        if (ref) cudaFreeAsync(ref, st);
+        if (tgt) cudaFreeAsync(tgt, st);
+    }
+};
+
+}  // namespace
+
+}  // namespace tdoa
+
+extern "C" {
+
+int tdoa_window_fixes(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts *o, int64_t win_start, int64_t win_len,
+                      int32_t n_ref_windows, int32_t n_tgt_windows, int64_t hop, const tdoa_peak *ref_in, const tdoa_peak *tgt_in,
+                      double *ref_fit, double *range_diffs, uint8_t *pair_used, double *fix_llh, double *fix_rms,
+                      int32_t *fix_status, int32_t *fix_iters)
+{
+    if (!e) return TDOA_E_INVALID;
+    int rc = begin_call(e);
+    if (rc) return rc;
+    WinTimes T;
+    if ((rc = window_check(e, "tdoa_window_fixes", stations_llh, o, win_start, win_len, n_ref_windows, n_tgt_windows, hop,
+                           fix_llh, fix_status, T)))
+        return rc;
+    if (!ref_in || !tgt_in) return fail(e, TDOA_E_INVALID, "tdoa_window_fixes: a table is NULL");
+    const int S = e->cfg.n_stations, P = S * (S - 1) / 2;
+    PeakRec *d_ref = nullptr, *d_tgt = nullptr;
+    if ((rc = alloc_t(e, &d_ref, (size_t)n_ref_windows * P)) || (rc = alloc_t(e, &d_tgt, (size_t)n_tgt_windows * P))) return rc;
+    CU(cudaMemcpyAsync(d_ref, ref_in, (size_t)n_ref_windows * P * sizeof(PeakRec), cudaMemcpyHostToDevice, e->stream));
+    CU(cudaMemcpyAsync(d_tgt, tgt_in, (size_t)n_tgt_windows * P * sizeof(PeakRec), cudaMemcpyHostToDevice, e->stream));
+    if ((rc = fix_stage(e, stations_llh, o, T, d_ref, d_tgt, ref_fit, range_diffs, pair_used, fix_llh, fix_rms, fix_status,
+                        fix_iters)))
+        return rc;
+    return finish_fix_stage(e);
+}
+
+int tdoa_process_windows(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts *o, int64_t win_start,
+                         int64_t win_len, int32_t n_ref_windows, int32_t n_tgt_windows, int64_t hop, tdoa_peak *ref_out,
+                         tdoa_peak *tgt_out, double *ref_fit, double *range_diffs, uint8_t *pair_used, double *fix_llh,
+                         double *fix_rms, int32_t *fix_status, int32_t *fix_iters)
+{
+    if (!e) return TDOA_E_INVALID;
+    int rc = begin_call(e);
+    if (rc) return rc;
+    WinTimes T;
+    if ((rc = window_check(e, "tdoa_process_windows", stations_llh, o, win_start, win_len, n_ref_windows, n_tgt_windows, hop,
+                           fix_llh, fix_status, T)))
+        return rc;
+    const int S = e->cfg.n_stations, P = S * (S - 1) / 2;
+    Tables tab{e->stream};
+    CU(cudaMallocAsync(reinterpret_cast<void **>(&tab.ref), (size_t)n_ref_windows * P * sizeof(PeakRec), e->stream));
+    CU(cudaMallocAsync(reinterpret_cast<void **>(&tab.tgt), (size_t)n_tgt_windows * P * sizeof(PeakRec), e->stream));
+    const bool sharded = multi_wants(e, n_ref_windows + n_tgt_windows);
+    if (sharded) {   // the tables tdoa_xcorr_windows gathers, left on this rank's device
+        T.parts[TDOA_KIND_REF].out = reinterpret_cast<tdoa_peak *>(tab.ref);
+        T.parts[TDOA_KIND_TGT].out = reinterpret_cast<tdoa_peak *>(tab.tgt);
+        for (ShardPart &Q : T.parts) Q.out_is_device = true;
+        if ((rc = xcorr_sharded(e, T.parts))) return rc;
+    } else {         // tdoa_xcorr_windows on one GPU: the REF pair loop, then the TGT pair loop
+        if ((rc = xcorr_impl(e, TDOA_KIND_REF, win_start, win_len, n_ref_windows, hop, ref_out, false, tab.ref)) ||
+            (rc = xcorr_impl(e, TDOA_KIND_TGT, win_start, win_len, n_tgt_windows, hop, tgt_out, false, tab.tgt)))
+            return rc;
+    }
+    if ((rc = begin_call(e))) return rc;
+    if (sharded) {
+        if (ref_out)
+            CU(cudaMemcpyAsync(ref_out, tab.ref, (size_t)n_ref_windows * P * sizeof(PeakRec), cudaMemcpyDeviceToHost, e->stream));
+        if (tgt_out)
+            CU(cudaMemcpyAsync(tgt_out, tab.tgt, (size_t)n_tgt_windows * P * sizeof(PeakRec), cudaMemcpyDeviceToHost, e->stream));
+    }
+    if ((rc = fix_stage(e, stations_llh, o, T, tab.ref, tab.tgt, ref_fit, range_diffs, pair_used, fix_llh, fix_rms, fix_status,
+                        fix_iters)))
+        return rc;
+    return finish_fix_stage(e);
+}
+
+}  // extern "C"
