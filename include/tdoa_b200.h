@@ -275,6 +275,30 @@ TDOA_API int tdoa_window_fixes(tdoa_engine *e, const double *stations_llh, const
                                int64_t hop, const tdoa_peak *ref_in, const tdoa_peak *tgt_in, double *ref_fit,
                                double *range_diffs, uint8_t *pair_used, double *fix_llh, double *fix_rms,
                                int32_t *fix_status, int32_t *fix_iters);
+/* Grid-seeded windowed fixes: as tdoa_process_windows / tdoa_window_fixes, with each TGT window's
+ * least-squares fix started from the arg-min of tdoa_grid_masked over grid_desc (7 doubles, as
+ * tdoa_grid) with that window's range differences and used pairs -- computed on the device between the
+ * range differences and the fix, in the same stream and without another host synchronisation.  A window
+ * the least-squares step refuses (status 2) is not searched: seed_index -1, seed_cost NaN, and it keeps
+ * the start it has without a grid.  Every other window starts at its arg-min cell (lat, lon, the grid's
+ * elevation); dims 3 solves the height from there.  The ranked arg-min is checked after the call's one
+ * synchronisation; a candidate table that overflowed, or a searched window without a survivor, reruns the
+ * grid on every cell and the fixes before anything is returned, so the results are those of evaluating
+ * every cell.  seed_llh[n_tgt][3], seed_cost[n_tgt], seed_index[n_tgt] may be NULL.  Refused
+ * (TDOA_E_INVALID): what the base calls refuse, a NULL grid_desc, more than 16 stations, an empty or too
+ * large grid.  ms_fix covers the grid. */
+TDOA_API int tdoa_process_windows_grid(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts *o,
+                                       int64_t win_start, int64_t win_len, int32_t n_ref_windows,
+                                       int32_t n_tgt_windows, int64_t hop, const double *grid_desc, tdoa_peak *ref_out,
+                                       tdoa_peak *tgt_out, double *ref_fit, double *range_diffs, uint8_t *pair_used,
+                                       double *fix_llh, double *fix_rms, int32_t *fix_status, int32_t *fix_iters,
+                                       double *seed_llh, double *seed_cost, int64_t *seed_index);
+TDOA_API int tdoa_window_fixes_grid(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts *o,
+                                    int64_t win_start, int64_t win_len, int32_t n_ref_windows, int32_t n_tgt_windows,
+                                    int64_t hop, const double *grid_desc, const tdoa_peak *ref_in,
+                                    const tdoa_peak *tgt_in, double *ref_fit, double *range_diffs, uint8_t *pair_used,
+                                    double *fix_llh, double *fix_rms, int32_t *fix_status, int32_t *fix_iters,
+                                    double *seed_llh, double *seed_cost, int64_t *seed_index);
 
 /* crossCorrelate seam (processor.go:619-643): two host complex64 slices
  * (interleaved re,im), returns (delay, correlation).  Empty input -> (0, 0.0). */
@@ -321,6 +345,16 @@ TDOA_API int tdoa_solve_binary(tdoa_engine *e, const double *stations_llh, int32
 TDOA_API int tdoa_grid(tdoa_engine *e, const double *stations_llh, int32_t n_stations,
                        const double *grid_desc, const double *range_diffs, int32_t n_sets,
                        int32_t rd_stride, double *out_llh, double *out_cost, int64_t *out_index);
+/* The same arg-min over a subset of the pairs of each set (no reference equivalent): the
+ * cost is the sum above over the pairs with used[set * rd_stride + p] != 0 only, in the
+ * same order; an unused slot is never read (NaN there is fine).  A set with no used pair
+ * has no arg-min: out_index -1, out_cost NaN, out_llh NaN.  used == NULL is tdoa_grid
+ * exactly.  Ranked as tdoa_grid (the bracket of the expanded cost loses the unused pairs'
+ * terms), with the same fall-back to evaluating every cell; same refusals as tdoa_grid. */
+TDOA_API int tdoa_grid_masked(tdoa_engine *e, const double *stations_llh, int32_t n_stations,
+                              const double *grid_desc, const double *range_diffs, const uint8_t *used,
+                              int32_t n_sets, int32_t rd_stride, double *out_llh, double *out_cost,
+                              int64_t *out_index);
 
 /* Least-squares fix over ALL S(S-1)/2 range differences (SURVEY.md 8f rank 4; no reference
  * equivalent -- solveTDOA uses two of three measurements, freezes Z and stops after ten
@@ -386,7 +420,8 @@ typedef struct {
     float ms_boxcar;          /* small box-car (DC subtract + low-pass + power)   */
     float ms_cand;            /* exact re-evaluation of the candidate lags        */
     float ms_fix;             /* fix stage of the last tdoa_process_windows / tdoa_window_fixes
-                                 (REF fit, range differences, least-squares fixes)  */
+                                 (REF fit, range differences, grid seed of the _grid
+                                 calls, least-squares fixes)                        */
     int64_t demod_launches, demod_samples;
     int64_t boxcar_launches, boxcar_samples;
     int64_t cand_launches, cand_pair_samples;

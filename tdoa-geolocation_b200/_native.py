@@ -23,8 +23,8 @@ ERRORS = {-1: "TDOA_E_INVALID", -2: "TDOA_E_NODEVICE", -3: "TDOA_E_CUDA", -4: "T
 # every symbol include/tdoa_b200.h declares (tests check the library exports them all)
 ABI_SYMBOLS = [
     "tdoa_default_config", "tdoa_create", "tdoa_destroy", "tdoa_last_error", "tdoa_host_alloc", "tdoa_host_free",
-    "tdoa_load_u8", "tdoa_load_file", "tdoa_load_u8_pinned", "tdoa_load_u8_device", "tdoa_unpack", "tdoa_preprocess", "tdoa_xcorr", "tdoa_xcorr_device", "tdoa_xcorr_windows", "tdoa_process", "tdoa_process_windows", "tdoa_window_fixes", "tdoa_xcorr_info", "tdoa_analyze",
-    "tdoa_cross_correlate", "tdoa_baselines", "tdoa_solve", "tdoa_solve_binary", "tdoa_solve_ls", "tdoa_grid", "tdoa_get_stats", "tdoa_stream",
+    "tdoa_load_u8", "tdoa_load_file", "tdoa_load_u8_pinned", "tdoa_load_u8_device", "tdoa_unpack", "tdoa_preprocess", "tdoa_xcorr", "tdoa_xcorr_device", "tdoa_xcorr_windows", "tdoa_process", "tdoa_process_windows", "tdoa_window_fixes", "tdoa_process_windows_grid", "tdoa_window_fixes_grid", "tdoa_xcorr_info", "tdoa_analyze",
+    "tdoa_cross_correlate", "tdoa_baselines", "tdoa_solve", "tdoa_solve_binary", "tdoa_solve_ls", "tdoa_grid", "tdoa_grid_masked", "tdoa_get_stats", "tdoa_stream",
     "tdoa_set_stream", "tdoa_synchronize", "tdoa_selftest",
     "tdoa_comm_unique_id", "tdoa_comm_init", "tdoa_comm_rank", "tdoa_shard_windows",
 ]
@@ -152,12 +152,15 @@ def load_library():
     L.tdoa_xcorr_windows.argtypes = [vp, i64, i64, i32, i32, i64, vp, vp]
     L.tdoa_process_windows.argtypes = [vp, vp, C.POINTER(WindowOpts), i64, i64, i32, i32, i64] + [vp] * 9
     L.tdoa_window_fixes.argtypes = [vp, vp, C.POINTER(WindowOpts), i64, i64, i32, i32, i64] + [vp] * 9
+    L.tdoa_process_windows_grid.argtypes = [vp, vp, C.POINTER(WindowOpts), i64, i64, i32, i32, i64] + [vp] * 13
+    L.tdoa_window_fixes_grid.argtypes = [vp, vp, C.POINTER(WindowOpts), i64, i64, i32, i32, i64] + [vp] * 13
     L.tdoa_cross_correlate.argtypes = [vp, vp, i64, vp, i64, C.POINTER(PeakStruct)]
     L.tdoa_baselines.argtypes = [vp, vp, i32, vp]
     L.tdoa_solve.argtypes = [vp, vp, i32, vp, i32, i32, vp, vp, vp]
     L.tdoa_solve_binary.argtypes = [vp, vp, i32, vp, i32, vp, C.POINTER(i32), C.POINTER(i32), C.POINTER(i32), C.POINTER(i32), vp]
     L.tdoa_solve_ls.argtypes = [vp, vp, i32, vp, i32, i32, vp, i32, vp, vp, vp, vp]
     L.tdoa_grid.argtypes = [vp, vp, i32, vp, vp, i32, i32, vp, vp, vp]
+    L.tdoa_grid_masked.argtypes = [vp, vp, i32, vp, vp, vp, i32, i32, vp, vp, vp]
     L.tdoa_get_stats.argtypes = [vp, C.POINTER(Stats)]
     L.tdoa_stream.argtypes = [vp]
     L.tdoa_stream.restype = vp
@@ -452,7 +455,7 @@ class Engine:
                 "status": int(status.value), "iters": int(iters.value)}
 
     def _windows(self, fn, stations_llh, win_start, win_len, n_ref_windows, n_tgt_windows, hop, tables, dims,
-                 min_margin, ref_max_residual, ref_tx_llh, init_llh) -> dict:
+                 min_margin, ref_max_residual, ref_tx_llh, init_llh, grid=None) -> dict:
         st = np.ascontiguousarray(stations_llh, dtype=np.float64).reshape(-1, 3)
         if st.shape[0] != self.n_stations:
             raise ValueError(f"stations_llh has {st.shape[0]} rows, the engine holds {self.n_stations} stations")
@@ -467,35 +470,52 @@ class Engine:
         used = np.zeros((nt, P), np.uint8)
         fix, rms = np.zeros((nt, 3), np.float64), np.zeros(nt, np.float64)
         status, iters = np.zeros(nt, np.int32), np.zeros(nt, np.int32)
-        self._check(fn(self._h, _ptr(st), C.byref(o), win_start, win_len, n_ref_windows, n_tgt_windows, hop,
+        if grid is None:
+            self._check(fn(self._h, _ptr(st), C.byref(o), win_start, win_len, n_ref_windows, n_tgt_windows, hop,
+                           *[_ptr(t) for t in tables], _ptr(ref_fit), _ptr(rd), _ptr(used), _ptr(fix), _ptr(rms),
+                           _ptr(status), _ptr(iters)))
+            return {"ref_fit": ref_fit, "range_differences": rd, "pair_used": used.astype(bool), "position": fix,
+                    "rms": rms, "status": status, "iters": iters}
+        gd = np.ascontiguousarray(grid, dtype=np.float64).reshape(-1)
+        if gd.size != 7:
+            raise ValueError(f"grid must be 7 numbers (lat0, lon0, dlat, dlon, nlat, nlon, elev), got {gd.size}")
+        seed, seed_cost, seed_index = np.zeros((nt, 3), np.float64), np.zeros(nt, np.float64), np.zeros(nt, np.int64)
+        self._check(fn(self._h, _ptr(st), C.byref(o), win_start, win_len, n_ref_windows, n_tgt_windows, hop, _ptr(gd),
                        *[_ptr(t) for t in tables], _ptr(ref_fit), _ptr(rd), _ptr(used), _ptr(fix), _ptr(rms),
-                       _ptr(status), _ptr(iters)))
+                       _ptr(status), _ptr(iters), _ptr(seed), _ptr(seed_cost), _ptr(seed_index)))
         return {"ref_fit": ref_fit, "range_differences": rd, "pair_used": used.astype(bool), "position": fix,
-                "rms": rms, "status": status, "iters": iters}
+                "rms": rms, "status": status, "iters": iters, "seed": seed, "seed_cost": seed_cost,
+                "seed_index": seed_index}
 
     def process_windows(self, stations_llh, win_start: int, win_len: int, n_ref_windows: int, n_tgt_windows: int,
                         hop: int, dims: int = 2, min_margin: float = 0.0, ref_max_residual: float = 0.0,
-                        ref_tx_llh=None, init_llh=None) -> dict:
+                        ref_tx_llh=None, init_llh=None, grid=None) -> dict:
         """Windowed ProcessTDOA (tdoa_process_windows): REF and TGT tables as xcorr_windows gives them, the REF
         lag's linear track per pair (ref_fit: lag at block 2's centre, drift in samples per sample, windows
         used), range differences and the used mask per (TGT window, pair), one least-squares fix per TGT window
         (status 0 ok, 1 degenerate, 2 too few measurements).  ref_tx_llh: the REF transmitter's position, whose
-        geometric range difference is added back."""
+        geometric range difference is added back.  grid = (lat0, lon0, dlat, dlon, nlat, nlon, elev): each window's
+        fix starts from the masked grid arg-min of its used pairs (tdoa_process_windows_grid); the result gains
+        seed (the start cell), seed_cost and seed_index (-1 and NaN for a window with status 2)."""
         ref = np.zeros((max(n_ref_windows, 0), self.n_pairs), PEAK_DTYPE)
         tgt = np.zeros((max(n_tgt_windows, 0), self.n_pairs), PEAK_DTYPE)
-        out = self._windows(self._lib.tdoa_process_windows, stations_llh, win_start, win_len, n_ref_windows,
-                            n_tgt_windows, hop, (ref, tgt), dims, min_margin, ref_max_residual, ref_tx_llh, init_llh)
+        fn = self._lib.tdoa_process_windows if grid is None else self._lib.tdoa_process_windows_grid
+        out = self._windows(fn, stations_llh, win_start, win_len, n_ref_windows, n_tgt_windows, hop, (ref, tgt), dims,
+                            min_margin, ref_max_residual, ref_tx_llh, init_llh, grid)
         out["ref"], out["tgt"] = ref, tgt
         return out
 
     def window_fixes(self, stations_llh, win_start: int, win_len: int, ref, tgt, hop: int, dims: int = 2,
-                     min_margin: float = 0.0, ref_max_residual: float = 0.0, ref_tx_llh=None, init_llh=None) -> dict:
+                     min_margin: float = 0.0, ref_max_residual: float = 0.0, ref_tx_llh=None, init_llh=None,
+                     grid=None) -> dict:
         """The fix stage of process_windows on given tables (tdoa_window_fixes): ref[n_ref][P], tgt[n_tgt][P] of
-        PEAK_DTYPE, e.g. kept from xcorr_windows; window times come from the captures the engine holds."""
+        PEAK_DTYPE, e.g. kept from xcorr_windows; window times come from the captures the engine holds.  grid: as
+        process_windows (tdoa_window_fixes_grid)."""
         ref = np.ascontiguousarray(ref, PEAK_DTYPE).reshape(-1, self.n_pairs)
         tgt = np.ascontiguousarray(tgt, PEAK_DTYPE).reshape(-1, self.n_pairs)
-        return self._windows(self._lib.tdoa_window_fixes, stations_llh, win_start, win_len, ref.shape[0], tgt.shape[0],
-                             hop, (ref, tgt), dims, min_margin, ref_max_residual, ref_tx_llh, init_llh)
+        fn = self._lib.tdoa_window_fixes if grid is None else self._lib.tdoa_window_fixes_grid
+        return self._windows(fn, stations_llh, win_start, win_len, ref.shape[0], tgt.shape[0], hop, (ref, tgt), dims,
+                             min_margin, ref_max_residual, ref_tx_llh, init_llh, grid)
 
     def solve_ls(self, stations_llh, range_diffs, init_llh=None, dims: int = 2):
         """Levenberg-Marquardt fix over all pair range differences (engine-defined, SURVEY 8f-4).
@@ -519,7 +539,9 @@ class Engine:
             return out[0], float(rms[0]), int(status[0]), int(iters[0])
         return out, rms, status, iters
 
-    def grid(self, stations_llh, grid_desc, range_diffs):
+    def grid(self, stations_llh, grid_desc, range_diffs, used=None):
+        """Dense grid arg-min per set (tdoa_grid); used[set][p] (same shape as range_diffs): only the pairs with
+        used != 0 enter the cost (tdoa_grid_masked; a set with no used pair gives index -1, cost and cell NaN)."""
         st = np.ascontiguousarray(stations_llh, dtype=np.float64).reshape(-1, 3)
         gd = np.ascontiguousarray(grid_desc, dtype=np.float64)
         rd = np.ascontiguousarray(range_diffs, dtype=np.float64)
@@ -529,8 +551,13 @@ class Engine:
         out = np.zeros((n, 3), np.float64)
         cost = np.zeros(n, np.float64)
         idx = np.zeros(n, np.int64)
-        self._check(self._lib.tdoa_grid(self._h, _ptr(st), st.shape[0], _ptr(gd), _ptr(rd), n, stride, _ptr(out),
-                                        _ptr(cost), _ptr(idx)))
+        if used is None:
+            self._check(self._lib.tdoa_grid(self._h, _ptr(st), st.shape[0], _ptr(gd), _ptr(rd), n, stride, _ptr(out),
+                                            _ptr(cost), _ptr(idx)))
+        else:
+            u = np.ascontiguousarray(np.asarray(used).astype(np.uint8).reshape(n, stride))
+            self._check(self._lib.tdoa_grid_masked(self._h, _ptr(st), st.shape[0], _ptr(gd), _ptr(rd), _ptr(u), n, stride,
+                                                   _ptr(out), _ptr(cost), _ptr(idx)))
         if single:
             return out[0], float(cost[0]), int(idx[0])
         return out, cost, idx

@@ -164,6 +164,9 @@ int span_begin(tdoa_engine *e, int tag);
 void span_end(tdoa_engine *e, int idx);
 void spans_collect(tdoa_engine *e);   // the stream must be idle
 
+// ---- grid multilateration (engine.cu): the argument checks every grid entry point shares
+int grid_check(tdoa_engine *e, const char *fn, int n_stations, const double *grid_desc);
+
 // ---- signal views and lazy loads (engine_pipeline.cu)
 i64 signal_length(const Station &s, int kind, i64 guard);
 SigSrc make_view(const Station &s, int kind, i64 start, i64 len, i64 guard);

@@ -235,6 +235,23 @@ __device__ bool ls_step(const double (&A)[3][3], const double (&b)[3], double la
 
 constexpr int kLsMaxStations = 64;
 
+// The status-2 rule of a masked fix (k_solve_ls) and of the grid seed (k_grid_rows): the number of used pairs, or -1
+// when there are fewer than `dims` of them or they touch fewer than dims + 1 stations (dims = 0: no used pair).
+__host__ __device__ __forceinline__ int ls_used_pairs(const uint8_t *used, int n_st, int dims)
+{
+    int n_used = 0, q = 0;
+    unsigned long long touched = 0ull;
+    for (int i = 0; i < n_st; i++)
+        for (int j = i + 1; j < n_st; j++, q++)
+            if (used[q]) { n_used++; touched |= (1ull << i) | (1ull << j); }
+#ifdef __CUDA_ARCH__
+    const int n_touched = __popcll(touched);
+#else
+    const int n_touched = __builtin_popcountll(touched);
+#endif
+    return (n_used < dims || n_touched < dims + 1) ? -1 : n_used;
+}
+
 __global__ void k_solve_ls(const double *llh, int n_st, const double *rd_all, int n_sets, int rd_stride,
                            const double *init_llh, int dims, double *out_llh, double *out_rms, int *status, int *iters,
                            const uint8_t *used_all)
@@ -257,12 +274,8 @@ __global__ void k_solve_ls(const double *llh, int n_st, const double *rd_all, in
         p.lat /= n_st; p.lon /= n_st; p.h /= n_st;
     }
     if (used) {   // too few measurements: no iteration
-        int n_used = 0, q = 0;
-        unsigned long long touched = 0ull;
-        for (int i = 0; i < n_st; i++)
-            for (int j = i + 1; j < n_st; j++, q++)
-                if (used[q]) { n_used++; touched |= (1ull << i) | (1ull << j); }
-        if (n_used < dims || __popcll(touched) < dims + 1) {
+        const int n_used = ls_used_pairs(used, n_st, dims);
+        if (n_used < 0) {
             out_llh[3 * set] = p.lat;
             out_llh[3 * set + 1] = p.lon;
             out_llh[3 * set + 2] = p.h;
@@ -337,8 +350,17 @@ __global__ void k_solve_ls(const double *llh, int n_st, const double *rd_all, in
 // terms added in pair order (as orc_grid_solve); arg-min, lowest linear index wins ties.
 // The S ranges of a cell do not depend on the set, so one thread computes them once
 // and sweeps every set; per-CTA minima go to scratch and a second kernel reduces them.
+// Masked statement (tdoa_grid_masked, the windowed seed): the sum runs over the pairs with used[p] != 0 only, in the
+// same order; an unused slot is never read (NaN there is fine); a set that is not searched -- no used pair, or the
+// windowed fix's status-2 rule -- has no arg-min: index -1, cost NaN, out_llh left as it was.  used == NULL is the
+// unmasked statement, and the kernels' kMasked = false instantiations are the unmasked kernels unchanged.
 constexpr int kGridThreads = 128;
 constexpr int kMaxStations = 16;
+constexpr int kMaxPairs = kMaxStations * (kMaxStations - 1) / 2;
+// a set's row of the ranked table: c[16], sum rd^2, 2 sum |rd|, unused pairs m, searched (1 / 0); a masked row then
+// holds the m unused pairs as one byte each, i * 16 + j, in pair order
+constexpr int kRankTab = 20;
+constexpr int kRankTabMasked = kRankTab + (kMaxPairs + 7) / 8 + 1;   // 36 doubles: 16-byte aligned rows
 
 struct GridDesc {
     double lat0, lon0, dlat, dlon;
@@ -354,9 +376,11 @@ __device__ __forceinline__ GridDesc read_desc(const double *g)
     return d;
 }
 
+template <bool kMasked>
 __global__ void __launch_bounds__(kGridThreads) k_grid_cost(const double *llh, int n_st, const double *gdesc,
                                                            const double *rd_all, int n_sets, int rd_stride,
-                                                           double *cta_cost, i64 *cta_idx)
+                                                           double *cta_cost, i64 *cta_idx, const uint8_t *used_all,
+                                                           const double *tab)
 {
     extern __shared__ double sm[];  // [n_st*3] station ECEF, then [kGridThreads] cost + idx scratch
     double *s_st = sm;
@@ -386,16 +410,20 @@ __global__ void __launch_bounds__(kGridThreads) k_grid_cost(const double *llh, i
     }
     for (int set = 0; set < n_sets; set++) {
         const double *rd = rd_all + (size_t)set * rd_stride;
+        const uint8_t *used = kMasked ? used_all + (size_t)set * rd_stride : nullptr;
+        const bool searched = !kMasked || tab[(size_t)set * kRankTabMasked + 19] != 0.0;
         double cost = 0.0;
-        if (live) {
+        if (live && searched) {
             int p = 0;
 #pragma unroll
             for (int i = 0; i < kMaxStations; i++) {
 #pragma unroll
                 for (int j = i + 1; j < kMaxStations; j++) {
                     if (j < n_st) {
-                        const double e = (r[j] - r[i]) - rd[p];
-                        cost = __dadd_rn(cost, __dmul_rn(e, e));
+                        if (!kMasked || used[p]) {
+                            const double e = (r[j] - r[i]) - rd[p];
+                            cost = __dadd_rn(cost, __dmul_rn(e, e));
+                        }
                         p++;
                     }
                 }
@@ -403,7 +431,7 @@ __global__ void __launch_bounds__(kGridThreads) k_grid_cost(const double *llh, i
         }
         // block arg-min (lowest index wins ties)
         s_cost[threadIdx.x] = cost;
-        s_idx[threadIdx.x] = live ? cell : (i64)-1;
+        s_idx[threadIdx.x] = live && searched ? cell : (i64)-1;
         __syncthreads();
         for (int o = kGridThreads / 2; o > 0; o >>= 1) {
             if (threadIdx.x < o) {
@@ -449,7 +477,7 @@ __global__ void __launch_bounds__(256) k_grid_reduce(const double *gdesc, const 
     if (threadIdx.x == 0) {
         const GridDesc G = read_desc(gdesc);
         const i64 bi = s_idx[0];
-        best_cost[set] = s_cost[0];
+        best_cost[set] = bi >= 0 ? s_cost[0] : __longlong_as_double(0x7ff8000000000000ll);   // no arg-min: NaN
         best_idx[set] = bi;
         if (bi >= 0) {
             out_llh[3 * set] = G.lat0 + (double)(bi / G.nlon) * G.dlat;
@@ -532,7 +560,6 @@ void launch_solve_ls(const double *d_llh, int n_st, const double *d_rd, int n_se
 constexpr int kRankThreads = 128;
 constexpr int kRankCells = 2;                    // cells per thread
 constexpr int kRankSpan = kRankThreads * kRankCells;
-constexpr int kRankTab = 20;                     // doubles per set: c[16], sum rd^2, 2 sum |rd|, pad
 constexpr double kGridKappa = 4e-13;             // ~3600 ulp of the largest partial result: far above the ~200 roundings
 constexpr int kRankMaxSets = 512;                // per launch (shared memory: 64 B per set)
 
@@ -584,7 +611,10 @@ __device__ __forceinline__ void rank_cell(const GridDesc &G, const double *s_st,
     }
 }
 
-// f and tol of one cell for one set; tab = the set's row (c[16], B, C1)
+// f and tol of one cell for one set; tab = the set's row (c[16], B, C1; masked: m, searched, the unused pairs).
+// Masked, the bracket loses the unused pairs' terms: a - sum_unused (q_j - q_i)^2 (m FMA more per cell and set);
+// a set that is not searched gives NaN, which no bound comparison lets through.
+template <bool kMasked>
 __device__ __forceinline__ void rank_eval(const RankCell &c, const double2 *__restrict__ tab, double &lo, double &hi)
 {
     double mid = 0.0;
@@ -595,7 +625,23 @@ __device__ __forceinline__ void rank_eval(const RankCell &c, const double2 *__re
         mid = __fma_rn(c.q[2 * m + 1], cc.y, mid);
     }
     const double2 bc = __ldg(tab + kMaxStations / 2);   // (sum rd^2, 2 sum |rd|)
-    const double f = __fma_rn(-2.0, mid, c.a + bc.x);
+    double a = c.a;
+    if (kMasked) {
+        const double2 ms = __ldg(tab + kMaxStations / 2 + 1);   // (unused pairs, searched)
+        if (ms.y == 0.0) {
+            lo = hi = __longlong_as_double(0x7ff8000000000000ll);
+            return;
+        }
+        const uint8_t *code = reinterpret_cast<const uint8_t *>(tab + kRankTab / 2);
+        double su = 0.0;
+        for (int m = 0; m < (int)ms.x; m++) {
+            const int k = __ldg(code + m);
+            const double d = c.q[k & 15] - c.q[k >> 4];
+            su = __fma_rn(d, d, su);
+        }
+        a = a - su;
+    }
+    const double f = __fma_rn(-2.0, mid, a + bc.x);
     const double tol = kGridKappa * (c.t0 + __fma_rn(2.0 * c.qmax, bc.y, bc.x));
     lo = f - tol;
     hi = f + tol;
@@ -608,9 +654,11 @@ __device__ __forceinline__ double warp_min(double v)
     return v;
 }
 
+template <bool kMasked>
 __global__ void __launch_bounds__(kRankThreads) k_grid_rank(const double *llh, int n_st, const double *gdesc,
                                                             const double *tab, int n_sets, double *cta_lo, double *cta_hi)
 {
+    constexpr int kTab = kMasked ? kRankTabMasked : kRankTab;
     extern __shared__ double sm[];   // [3 * 16] station ECEF, then [n_sets][4 warps] lo, [n_sets][4 warps] hi
     double *s_st = sm;
     double *s_lo = sm + 3 * kMaxStations;
@@ -627,10 +675,10 @@ __global__ void __launch_bounds__(kRankThreads) k_grid_rank(const double *llh, i
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const double inf = __longlong_as_double(0x7ff0000000000000ll);
     for (int set = 0; set < n_sets; set++) {
-        const double2 *row = reinterpret_cast<const double2 *>(tab + (size_t)set * kRankTab);
+        const double2 *row = reinterpret_cast<const double2 *>(tab + (size_t)set * kTab);
         double lo0, hi0, lo1, hi1;
-        rank_eval(c0, row, lo0, hi0);
-        rank_eval(c1, row, lo1, hi1);
+        rank_eval<kMasked>(c0, row, lo0, hi0);
+        rank_eval<kMasked>(c1, row, lo1, hi1);
         double lo = fmin(c0.live ? lo0 : inf, c1.live ? lo1 : inf);
         double hi = fmin(c0.live ? hi0 : inf, c1.live ? hi1 : inf);
         lo = warp_min(lo);
@@ -668,18 +716,21 @@ __global__ void __launch_bounds__(256) k_grid_bound(const double *cta_hi, int n_
 
 struct GridCand { i64 cell; double cost; int set; int pad; };
 
+template <bool kMasked>
 __global__ void __launch_bounds__(kRankThreads) k_grid_refine(const double *llh, int n_st, const double *gdesc,
                                                               const double *tab, const double *rd_all, int n_sets,
                                                               int rd_stride, const double *cta_lo, const double *bound,
                                                               GridCand *cands, int cap, int *n_cand)
 {
+    constexpr int kTab = kMasked ? kRankTabMasked : kRankTab;
     __shared__ double s_st[3 * kMaxStations];
     __shared__ int s_sets[kRankMaxSets];
     __shared__ int s_n;
     if (threadIdx.x == 0) s_n = 0;
     __syncthreads();
     for (int set = threadIdx.x; set < n_sets; set += kRankThreads)
-        if (cta_lo[(size_t)set * gridDim.x + blockIdx.x] <= bound[set]) s_sets[atomicAdd(&s_n, 1)] = set;
+        if (cta_lo[(size_t)set * gridDim.x + blockIdx.x] <= bound[set] && (!kMasked || tab[(size_t)set * kTab + 19] != 0.0))
+            s_sets[atomicAdd(&s_n, 1)] = set;
     __syncthreads();
     const int ns = s_n;
     if (ns == 0) return;   // nearly every CTA
@@ -696,7 +747,7 @@ __global__ void __launch_bounds__(kRankThreads) k_grid_refine(const double *llh,
         for (int u = 0; u < ns; u++) {
             const int set = s_sets[u];
             double lo, hi;
-            rank_eval(c, reinterpret_cast<const double2 *>(tab + (size_t)set * kRankTab), lo, hi);
+            rank_eval<kMasked>(c, reinterpret_cast<const double2 *>(tab + (size_t)set * kTab), lo, hi);
             if (!(lo <= bound[set])) continue;
             const int slot = atomicAdd(n_cand, 1);
             if (slot < cap) cands[slot] = GridCand{cell, 0.0, set, 0};
@@ -707,9 +758,10 @@ __global__ void __launch_bounds__(kRankThreads) k_grid_refine(const double *llh,
 // The statement itself (k_grid_cost / orc_grid_solve) on the surviving (cell, set) pairs, one thread each: pair by
 // pair, in order, no contraction.  (Inside k_grid_refine the survivors of all sets sit in two or three
 // neighbouring cells, i.e. in one warp, and their 120-term chains ran one after the other: 0.41 ms of 0.75.)
+template <bool kMasked>
 __global__ void __launch_bounds__(kRankThreads) k_grid_exact(const double *llh, int n_st, const double *gdesc,
                                                              const double *rd_all, int rd_stride, GridCand *cands, int cap,
-                                                             const int *n_cand)
+                                                             const int *n_cand, const uint8_t *used_all)
 {
     __shared__ double s_st[3 * kMaxStations];
     const int n = min(*n_cand, cap);
@@ -725,6 +777,7 @@ __global__ void __launch_bounds__(kRankThreads) k_grid_exact(const double *llh, 
     double r[kMaxStations];
     rank_cell(G, s_st, n_st, g.cell, (i64)G.nlat * G.nlon, c, r);
     const double *rd = rd_all + (size_t)g.set * rd_stride;
+    const uint8_t *used = kMasked ? used_all + (size_t)g.set * rd_stride : nullptr;
     double cost = 0.0;
     int p = 0;
 #pragma unroll
@@ -732,8 +785,10 @@ __global__ void __launch_bounds__(kRankThreads) k_grid_exact(const double *llh, 
 #pragma unroll
         for (int b = a + 1; b < kMaxStations; b++) {
             if (b < n_st) {
-                const double e = (r[b] - r[a]) - rd[p];
-                cost = __dadd_rn(cost, __dmul_rn(e, e));
+                if (!kMasked || used[p]) {
+                    const double e = (r[b] - r[a]) - rd[p];
+                    cost = __dadd_rn(cost, __dmul_rn(e, e));
+                }
                 p++;
             }
         }
@@ -768,7 +823,7 @@ __global__ void __launch_bounds__(128) k_grid_pick(const double *gdesc, const Gr
     if (threadIdx.x == 0) {
         const GridDesc G = read_desc(gdesc);
         const i64 bi = s_idx[0];
-        best_cost[set] = s_cost[0];
+        best_cost[set] = bi >= 0 ? s_cost[0] : __longlong_as_double(0x7ff8000000000000ll);   // no arg-min: NaN
         best_idx[set] = bi;
         if (bi >= 0) {
             out_llh[3 * set] = G.lat0 + (double)(bi / G.nlon) * G.dlat;
@@ -778,7 +833,51 @@ __global__ void __launch_bounds__(128) k_grid_pick(const double *gdesc, const Gr
     }
 }
 
-int grid_rank_tab_doubles() { return kRankTab; }
+// One set's row of the ranked table from its range differences (c_k, sum rd^2 and 2 sum |rd| over the used pairs,
+// the unused pairs), on the host for tdoa_grid / tdoa_grid_masked and in k_grid_rows for the windowed seed.  Products
+// and sums are separate roundings on both sides (solve.cu is compiled without contraction).
+__host__ __device__ inline void grid_row_fill(const double *rd, const uint8_t *used, int n_st, bool searched, double *row)
+{
+    double c[kMaxStations];
+    for (int k = 0; k < kMaxStations; k++) c[k] = 0.0;
+    double b = 0.0;
+    int p = 0, m = 0;
+    uint8_t *code = reinterpret_cast<uint8_t *>(row + kRankTab);
+    for (int i = 0; i < n_st; i++)
+        for (int j = i + 1; j < n_st; j++, p++) {
+            if (used && !used[p]) {
+                code[m++] = (uint8_t)(i * 16 + j);
+                continue;
+            }
+            c[j] += rd[p];
+            c[i] -= rd[p];
+            b += rd[p] * rd[p];
+        }
+    // the bound takes sum |rd| over the terms of every c_k (not sum |c_k|: a c_k that cancels keeps its rounding)
+    double c1 = 0.0;
+    p = 0;
+    for (int i = 0; i < n_st; i++)
+        for (int j = i + 1; j < n_st; j++, p++)
+            if (!used || used[p]) c1 += 2.0 * (rd[p] < 0 ? -rd[p] : rd[p]);
+    for (int k = 0; k < kMaxStations; k++) row[k] = c[k];
+    row[16] = b;
+    row[17] = c1;
+    row[18] = (double)m;
+    row[19] = searched ? 1.0 : 0.0;
+}
+
+// the windowed seed's rows, one thread per set: searched unless the least-squares step would refuse the set (status 2)
+__global__ void k_grid_rows(const double *rd_all, const uint8_t *used_all, int n_sets, int rd_stride, int n_st, int dims,
+                            double *tab)
+{
+    const int set = blockIdx.x * blockDim.x + threadIdx.x;
+    if (set >= n_sets) return;
+    const uint8_t *used = used_all + (size_t)set * rd_stride;
+    grid_row_fill(rd_all + (size_t)set * rd_stride, used, n_st, ls_used_pairs(used, n_st, dims) >= 0,
+                  tab + (size_t)set * kRankTabMasked);
+}
+
+int grid_rank_tab_doubles(bool masked) { return masked ? kRankTabMasked : kRankTab; }
 int grid_rank_max_sets() { return kRankMaxSets; }
 int grid_rank_cand_cap(int n_sets) { return 64 * n_sets + 1024; }
 
@@ -796,34 +895,27 @@ size_t grid_rank_scratch_bytes(int nlat, int nlon, int n_sets)
            (size_t)grid_rank_cand_cap(n_sets) * sizeof(GridCand) + 64;
 }
 
-// Host part of the expansion: the set's row of the table (c_k, sum rd^2, sum |c_k|) from its range differences.
-void grid_rank_row(const double *rd, int n_st, double *row)
+// Host rows (tdoa_grid, tdoa_grid_masked): the range differences are on the host already, and building the rows there
+// keeps the ranked arg-min at five launches per 512 sets.  used == nullptr: the unmasked row; masked, a set without a
+// used pair is not searched.  Returns whether the set is searched.
+bool grid_rank_row(const double *rd, const uint8_t *used, int n_st, double *row)
 {
-    double c[kMaxStations] = {0.0};
-    double b = 0.0;
-    int p = 0;
-    for (int i = 0; i < n_st; i++)
-        for (int j = i + 1; j < n_st; j++, p++) {
-            c[j] += rd[p];
-            c[i] -= rd[p];
-            b += rd[p] * rd[p];
-        }
-    // the bound takes sum |rd| over the terms of every c_k (not sum |c_k|: a c_k that cancels keeps its rounding)
-    double c1 = 0.0;
-    p = 0;
-    for (int i = 0; i < n_st; i++)
-        for (int j = i + 1; j < n_st; j++, p++) c1 += 2.0 * (rd[p] < 0 ? -rd[p] : rd[p]);
-    for (int k = 0; k < kMaxStations; k++) row[k] = c[k];
-    row[16] = b;
-    row[17] = c1;
-    row[18] = row[19] = 0.0;
+    const bool searched = !used || ls_used_pairs(used, n_st, 0) >= 0;
+    grid_row_fill(rd, used, n_st, searched, row);
+    return searched;
+}
+
+void launch_grid_rows(const double *d_rd, const uint8_t *d_used, int n_sets, int rd_stride, int n_st, int dims, double *d_tab,
+                      cudaStream_t st)
+{
+    if (n_sets > 0) k_grid_rows<<<(n_sets + 63) / 64, 64, 0, st>>>(d_rd, d_used, n_sets, rd_stride, n_st, dims, d_tab);
 }
 
 // n_sets <= grid_rank_max_sets().  d_count: one int, read back by the caller after the stream has drained --
 // more than grid_rank_cand_cap(n_sets) candidates means the table is incomplete (launch_grid_cells then).
 void launch_grid_ranked(const double *d_llh, int n_st, const double *d_grid_desc, int nlat, int nlon, const double *d_tab,
                         const double *d_rd, int n_sets, int rd_stride, double *d_best_cost, i64 *d_best_idx,
-                        double *d_out_llh, void *d_scratch, int *d_count, cudaStream_t st)
+                        double *d_out_llh, void *d_scratch, int *d_count, cudaStream_t st, const uint8_t *d_used)
 {
     const int n_cta = rank_n_cta(nlat, nlon);
     if (n_cta <= 0 || n_sets <= 0) return;
@@ -834,12 +926,22 @@ void launch_grid_ranked(const double *d_llh, int n_st, const double *d_grid_desc
     const int cap = grid_rank_cand_cap(n_sets);
     cudaMemsetAsync(d_count, 0, sizeof(int), st);
     const size_t smem = (3 * kMaxStations + 2 * (size_t)n_sets * (kRankThreads / 32)) * sizeof(double);
-    k_grid_rank<<<n_cta, kRankThreads, smem, st>>>(d_llh, n_st, d_grid_desc, d_tab, n_sets, cta_lo, cta_hi);
-    k_grid_bound<<<n_sets, 256, 0, st>>>(cta_hi, n_cta, bound);
-    k_grid_refine<<<n_cta, kRankThreads, 0, st>>>(d_llh, n_st, d_grid_desc, d_tab, d_rd, n_sets, rd_stride, cta_lo, bound, cands,
-                                                cap, d_count);
-    k_grid_exact<<<(cap + kRankThreads - 1) / kRankThreads, kRankThreads, 0, st>>>(d_llh, n_st, d_grid_desc, d_rd, rd_stride, cands,
-                                                                                   cap, d_count);
+    const int n_exact = (cap + kRankThreads - 1) / kRankThreads;
+    if (d_used) {
+        k_grid_rank<true><<<n_cta, kRankThreads, smem, st>>>(d_llh, n_st, d_grid_desc, d_tab, n_sets, cta_lo, cta_hi);
+        k_grid_bound<<<n_sets, 256, 0, st>>>(cta_hi, n_cta, bound);
+        k_grid_refine<true><<<n_cta, kRankThreads, 0, st>>>(d_llh, n_st, d_grid_desc, d_tab, d_rd, n_sets, rd_stride, cta_lo,
+                                                          bound, cands, cap, d_count);
+        k_grid_exact<true><<<n_exact, kRankThreads, 0, st>>>(d_llh, n_st, d_grid_desc, d_rd, rd_stride, cands, cap, d_count,
+                                                             d_used);
+    } else {
+        k_grid_rank<false><<<n_cta, kRankThreads, smem, st>>>(d_llh, n_st, d_grid_desc, d_tab, n_sets, cta_lo, cta_hi);
+        k_grid_bound<<<n_sets, 256, 0, st>>>(cta_hi, n_cta, bound);
+        k_grid_refine<false><<<n_cta, kRankThreads, 0, st>>>(d_llh, n_st, d_grid_desc, d_tab, d_rd, n_sets, rd_stride, cta_lo,
+                                                           bound, cands, cap, d_count);
+        k_grid_exact<false><<<n_exact, kRankThreads, 0, st>>>(d_llh, n_st, d_grid_desc, d_rd, rd_stride, cands, cap, d_count,
+                                                              nullptr);
+    }
     k_grid_pick<<<n_sets, 128, 0, st>>>(d_grid_desc, cands, cap, d_count, d_best_cost, d_best_idx, d_out_llh);
 }
 
@@ -857,14 +959,19 @@ size_t grid_scratch_bytes(int n_st, int nlat, int nlon, int n_sets)
 
 void launch_grid_cells(const double *d_llh, int n_st, const double *d_grid_desc, int nlat, int nlon,
                        const double *d_rd, int n_sets, int rd_stride, double *d_best_cost, i64 *d_best_idx,
-                       double *d_out_llh, void *d_scratch, cudaStream_t st)
+                       double *d_out_llh, void *d_scratch, cudaStream_t st, const uint8_t *d_used, const double *d_tab)
 {
     const int n_cta = grid_n_cta(nlat, nlon);
     if (n_cta <= 0 || n_sets <= 0) return;
     double *cta_cost = reinterpret_cast<double *>(d_scratch);
     i64 *cta_idx = reinterpret_cast<i64 *>(cta_cost + (size_t)n_cta * n_sets);
     const size_t smem = (3 * kMaxStations + kGridThreads) * sizeof(double) + kGridThreads * sizeof(i64);
-    k_grid_cost<<<n_cta, kGridThreads, smem, st>>>(d_llh, n_st, d_grid_desc, d_rd, n_sets, rd_stride, cta_cost, cta_idx);
+    if (d_used)
+        k_grid_cost<true><<<n_cta, kGridThreads, smem, st>>>(d_llh, n_st, d_grid_desc, d_rd, n_sets, rd_stride, cta_cost, cta_idx,
+                                                             d_used, d_tab);
+    else
+        k_grid_cost<false><<<n_cta, kGridThreads, smem, st>>>(d_llh, n_st, d_grid_desc, d_rd, n_sets, rd_stride, cta_cost, cta_idx,
+                                                              nullptr, nullptr);
     k_grid_reduce<<<n_sets, 256, 0, st>>>(d_grid_desc, cta_cost, cta_idx, n_cta, d_best_cost, d_best_idx, d_out_llh);
 }
 

@@ -1,5 +1,6 @@
 // window_fix.cu -- from window tables to range differences, one fix per TGT window
-// (tdoa_process_windows, tdoa_window_fixes; no reference equivalent; restated in tests/window_oracle.py).
+// (tdoa_process_windows, tdoa_window_fixes; no reference equivalent; restated in tests/window_oracle.py;
+// the grid seed of the _grid calls in tests/window_grid_oracle.py).
 //
 // An RTL-SDR's sample clock is off by ppm, so the lag between two collectors drifts linearly over
 // the capture (1 ppm of relative rate = 2 samples per second at 2 Msps).  The reference correlates
@@ -12,6 +13,12 @@
 //                     windows whose residual exceeds max_resid, the REF transmitter's geometric term
 //   k_window_rd       one thread per (TGT window, pair): rd = (y_tgt / fs - y_ref(t_w) / fs) * c
 //                     (+ the geometric term) and the used mask that k_solve_ls reads.
+// The _grid calls then seed each window's fix from the masked grid arg-min of its own used pairs (solve.cu):
+//   k_grid_rows       the window's row of the ranked table (not searched: the least-squares step's status 2)
+//   k_grid_rank ... k_grid_pick   write the arg-min cell into the window's start point, which holds the start
+//                     the window has without a grid; k_solve_ls starts there.
+// The ranked pass is optimistic: after the call's one synchronisation an overflowing candidate table or a searched
+// window without a survivor reruns the grid on every cell (k_grid_cost) and the fixes, before the call returns.
 // Window times and the usable test are stated in include/tdoa_b200.h (tdoa_process_windows).
 #include <cuda_runtime.h>
 
@@ -212,12 +219,21 @@ int window_check(tdoa_engine *e, const char *fn, const double *stations_llh, con
     return TDOA_OK;
 }
 
+// the grid seed of the _grid calls: descriptor and optional outputs
+struct GridSeed {
+    const double *desc = nullptr;   // nullptr: no grid
+    double *llh = nullptr, *cost = nullptr;
+    int64_t *index = nullptr;
+};
+
 // the fix stage on device tables, queued on the engine's stream inside the caller's begin_call / end_call;
-// the station table, times and options ride in the descriptor frame
+// the station table, times and options ride in the descriptor frame.  *synced: the stream was drained (the grid
+// seed's check) and holds nothing more
 int fix_stage(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts *o, const WinTimes &T, const PeakRec *d_ref,
               const PeakRec *d_tgt, double *ref_fit, double *range_diffs, uint8_t *pair_used, double *fix_llh, double *fix_rms,
-              int32_t *fix_status, int32_t *fix_iters)
+              int32_t *fix_status, int32_t *fix_iters, const GridSeed &G, bool *synced)
 {
+    *synced = false;
     const int S = e->cfg.n_stations, P = S * (S - 1) / 2, nt = T.n_tgt;
     int rc;
     const double *d_llh = nullptr, *d_t_ref = nullptr, *d_t_tgt = nullptr, *d_t_mid = nullptr, *d_ref_tx = nullptr,
@@ -226,10 +242,19 @@ int fix_stage(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts
         (rc = upload(e, T.t_ref, &d_t_ref)) || (rc = upload(e, T.t_tgt, &d_t_tgt)) || (rc = upload(e, T.t_mid, &d_t_mid)))
         return rc;
     if (o->has_ref_tx && (rc = upload(e, std::vector<double>(o->ref_tx_llh, o->ref_tx_llh + 3), &d_ref_tx))) return rc;
-    if (o->has_init) {
+    if (o->has_init || G.desc) {
+        // the start of every window: init_llh, or (grid seed) the mean of the stations as k_solve_ls takes it
+        double p0[3] = {0.0, 0.0, 0.0};
+        if (o->has_init) {
+            for (int k = 0; k < 3; k++) p0[k] = o->init_llh[k];
+        } else {
+            for (int s = 0; s < S; s++)
+                for (int k = 0; k < 3; k++) p0[k] += stations_llh[3 * s + k];
+            for (int k = 0; k < 3; k++) p0[k] /= S;
+        }
         std::vector<double> init((size_t)3 * nt);
         for (int w = 0; w < nt; w++)
-            for (int k = 0; k < 3; k++) init[(size_t)3 * w + k] = o->init_llh[k];
+            for (int k = 0; k < 3; k++) init[(size_t)3 * w + k] = p0[k];
         if ((rc = upload(e, init, &d_init))) return rc;
     }
     double *d_fit = nullptr, *d_ref_fit = nullptr, *d_rd = nullptr, *d_fix = nullptr, *d_rms = nullptr;
@@ -240,30 +265,110 @@ int fix_stage(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts
         (rc = alloc_t(e, &d_fix, (size_t)3 * nt)) || (rc = alloc_t(e, &d_rms, (size_t)nt)) ||
         (rc = alloc_t(e, &d_status, (size_t)nt)) || (rc = alloc_t(e, &d_iters, (size_t)nt)))
         return rc;
-    CU(cudaEventRecord(e->ev[1], e->stream));
-    launch_window_ref_fit(d_ref, T.n_ref, S, d_t_ref, d_t_mid, d_llh, d_ref_tx, o->min_margin, o->ref_max_residual, d_fit,
-                          d_ref_fit, e->stream);
-    launch_window_rd(d_tgt, nt, S, d_t_tgt, d_fit, o->min_margin, e->cfg.sample_rate, d_rd, d_used, e->stream);
-    launch_solve_ls(d_llh, S, d_rd, nt, P, d_init, o->dims, d_fix, d_rms, d_status, d_iters, e->stream, d_used);
-    count_launch(e, 3);
-    CU(cudaEventRecord(e->ev[2], e->stream));
-    CU(cudaGetLastError());
+    // the grid seed: the windows' start points (written by the grid where it finds a cell), the masked rows, the
+    // ranked arg-min per chunk of sets
+    const int chunk = grid_rank_max_sets(), n_chunks = (nt + chunk - 1) / chunk, TW = grid_rank_tab_doubles(true);
+    int nlat = 0, nlon = 0;
+    const double *d_desc = nullptr;
+    double *d_start = nullptr, *d_tab = nullptr, *d_cost = nullptr;
+    i64 *d_idx = nullptr;
+    int *d_count = nullptr;
+    void *d_rscratch = nullptr;
+    if (G.desc) {
+        nlat = (int)G.desc[4];
+        nlon = (int)G.desc[5];
+        if ((rc = upload(e, std::vector<double>(G.desc, G.desc + 7), &d_desc)) || (rc = alloc_t(e, &d_start, (size_t)3 * nt)) ||
+            (rc = alloc_t(e, &d_tab, (size_t)nt * TW)) || (rc = alloc_t(e, &d_cost, (size_t)nt)) ||
+            (rc = alloc_t(e, &d_idx, (size_t)nt)) || (rc = alloc_t(e, &d_count, (size_t)n_chunks)) ||
+            (rc = alloc(e, &d_rscratch, grid_rank_scratch_bytes(nlat, nlon, std::min(nt, chunk)))))
+            return rc;
+    }
+    // the grid (ranked, or every cell) between the range differences and the fixes
+    auto seed_and_fix = [&](bool exhaustive) -> int {
+        if (G.desc) {
+            CU(cudaMemcpyAsync(d_start, d_init, (size_t)3 * nt * sizeof(double), cudaMemcpyDeviceToDevice, e->stream));
+            if (exhaustive) {
+                void *d_scratch = nullptr;
+                int rc2 = alloc(e, &d_scratch, grid_scratch_bytes(S, nlat, nlon, nt));
+                if (rc2) return rc2;
+                launch_grid_cells(d_llh, S, d_desc, nlat, nlon, d_rd, nt, P, d_cost, d_idx, d_start, d_scratch, e->stream, d_used,
+                                  d_tab);
+                count_launch(e, 2);
+            } else {
+                for (int c = 0; c < n_chunks; c++) {
+                    const int s0 = c * chunk, ns = std::min(chunk, nt - s0);
+                    launch_grid_ranked(d_llh, S, d_desc, nlat, nlon, d_tab + (size_t)s0 * TW, d_rd + (size_t)s0 * P, ns, P,
+                                       d_cost + s0, d_idx + s0, d_start + 3 * s0, d_rscratch, d_count + c, e->stream,
+                                       d_used + (size_t)s0 * P);
+                    count_launch(e, 5);
+                }
+            }
+        }
+        launch_solve_ls(d_llh, S, d_rd, nt, P, G.desc ? d_start : d_init, o->dims, d_fix, d_rms, d_status, d_iters, e->stream,
+                        d_used);
+        count_launch(e);
+        CU(cudaEventRecord(e->ev[2], e->stream));
+        CU(cudaGetLastError());
+        return TDOA_OK;
+    };
     auto back = [&](void *dst, const void *src, size_t bytes) -> int {
         if (dst) CU(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, e->stream));
         return TDOA_OK;
     };
+    auto results = [&]() -> int {
+        int rc2;
+        if ((rc2 = back(fix_llh, d_fix, (size_t)3 * nt * sizeof(double))) || (rc2 = back(fix_rms, d_rms, (size_t)nt * sizeof(double))) ||
+            (rc2 = back(fix_status, d_status, (size_t)nt * sizeof(int32_t))) ||
+            (rc2 = back(fix_iters, d_iters, (size_t)nt * sizeof(int32_t))))
+            return rc2;
+        if (G.desc &&
+            ((rc2 = back(G.llh, d_start, (size_t)3 * nt * sizeof(double))) || (rc2 = back(G.cost, d_cost, (size_t)nt * sizeof(double))) ||
+             (rc2 = back(G.index, d_idx, (size_t)nt * sizeof(int64_t)))))
+            return rc2;
+        return TDOA_OK;
+    };
+    CU(cudaEventRecord(e->ev[1], e->stream));
+    launch_window_ref_fit(d_ref, T.n_ref, S, d_t_ref, d_t_mid, d_llh, d_ref_tx, o->min_margin, o->ref_max_residual, d_fit,
+                          d_ref_fit, e->stream);
+    launch_window_rd(d_tgt, nt, S, d_t_tgt, d_fit, o->min_margin, e->cfg.sample_rate, d_rd, d_used, e->stream);
+    count_launch(e, 2);
+    if (G.desc) {
+        launch_grid_rows(d_rd, d_used, nt, P, S, o->dims, d_tab, e->stream);
+        count_launch(e);
+    }
+    // use_fft = 0 evaluates every cell, as tdoa_grid does
+    if ((rc = seed_and_fix(e->cfg.use_fft == 0))) return rc;
     if ((rc = back(ref_fit, d_ref_fit, (size_t)3 * P * sizeof(double))) ||
         (rc = back(range_diffs, d_rd, (size_t)nt * P * sizeof(double))) || (rc = back(pair_used, d_used, (size_t)nt * P)) ||
-        (rc = back(fix_llh, d_fix, (size_t)3 * nt * sizeof(double))) || (rc = back(fix_rms, d_rms, (size_t)nt * sizeof(double))) ||
-        (rc = back(fix_status, d_status, (size_t)nt * sizeof(int32_t))) ||
-        (rc = back(fix_iters, d_iters, (size_t)nt * sizeof(int32_t))))
+        (rc = results()))
         return rc;
+    if (G.desc && e->cfg.use_fft != 0) {
+        // the optimistic ranked pass, checked after the call's one synchronisation
+        std::vector<int> h_count((size_t)n_chunks);
+        std::vector<i64> h_idx((size_t)nt);
+        std::vector<int> h_status((size_t)nt);
+        CU(cudaMemcpyAsync(h_count.data(), d_count, (size_t)n_chunks * sizeof(int), cudaMemcpyDeviceToHost, e->stream));
+        CU(cudaMemcpyAsync(h_idx.data(), d_idx, (size_t)nt * sizeof(i64), cudaMemcpyDeviceToHost, e->stream));
+        CU(cudaMemcpyAsync(h_status.data(), d_status, (size_t)nt * sizeof(int), cudaMemcpyDeviceToHost, e->stream));
+        CU(cudaStreamSynchronize(e->stream));
+        *synced = true;
+        bool again = false;
+        for (int c = 0; c < n_chunks; c++)
+            if (h_count[c] > grid_rank_cand_cap(std::min(chunk, nt - c * chunk))) again = true;   // a plateau of ties
+        for (int w = 0; w < nt; w++)
+            if (h_idx[w] < 0 && h_status[w] != 2) again = true;   // a searched window without a survivor
+        if (again) {
+            if ((rc = seed_and_fix(true)) || (rc = results())) return rc;
+            *synced = false;
+        }
+    }
     return TDOA_OK;
 }
 
-int finish_fix_stage(tdoa_engine *e)
+// synced: fix_stage drained the stream and queued nothing after (the frees and the frame's event need no wait)
+int finish_fix_stage(tdoa_engine *e, bool synced)
 {
-    const int rc = end_call(e, true);
+    const int rc = end_call(e, !synced);
     if (rc) return rc;
     float t = 0.f;
     cudaEventElapsedTime(&t, e->ev[1], e->ev[2]);
@@ -286,44 +391,56 @@ struct Tables {
 
 }  // namespace tdoa
 
-extern "C" {
+namespace tdoa {
+namespace {
 
-int tdoa_window_fixes(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts *o, int64_t win_start, int64_t win_len,
-                      int32_t n_ref_windows, int32_t n_tgt_windows, int64_t hop, const tdoa_peak *ref_in, const tdoa_peak *tgt_in,
-                      double *ref_fit, double *range_diffs, uint8_t *pair_used, double *fix_llh, double *fix_rms,
-                      int32_t *fix_status, int32_t *fix_iters)
+// the grid's refusals on top of window_check's
+int grid_seed_check(tdoa_engine *e, const char *fn, const GridSeed &G)
+{
+    if (!G.desc) return fail(e, TDOA_E_INVALID, "%s: grid_desc is NULL", fn);
+    if (e->cfg.n_stations > 16) return fail(e, TDOA_E_INVALID, "%s: the grid takes 2..16 stations, got %d", fn, e->cfg.n_stations);
+    return grid_check(e, fn, e->cfg.n_stations, G.desc);
+}
+
+int window_fixes_impl(tdoa_engine *e, const char *fn, const double *stations_llh, const tdoa_window_opts *o, int64_t win_start,
+                      int64_t win_len, int32_t n_ref_windows, int32_t n_tgt_windows, int64_t hop, const tdoa_peak *ref_in,
+                      const tdoa_peak *tgt_in, double *ref_fit, double *range_diffs, uint8_t *pair_used, double *fix_llh,
+                      double *fix_rms, int32_t *fix_status, int32_t *fix_iters, const GridSeed *grid)
 {
     if (!e) return TDOA_E_INVALID;
     int rc = begin_call(e);
     if (rc) return rc;
     WinTimes T;
-    if ((rc = window_check(e, "tdoa_window_fixes", stations_llh, o, win_start, win_len, n_ref_windows, n_tgt_windows, hop,
-                           fix_llh, fix_status, T)))
+    if ((rc = window_check(e, fn, stations_llh, o, win_start, win_len, n_ref_windows, n_tgt_windows, hop, fix_llh, fix_status, T)))
         return rc;
-    if (!ref_in || !tgt_in) return fail(e, TDOA_E_INVALID, "tdoa_window_fixes: a table is NULL");
+    if (grid && (rc = grid_seed_check(e, fn, *grid))) return rc;
+    const GridSeed G = grid ? *grid : GridSeed{};
+    if (!ref_in || !tgt_in) return fail(e, TDOA_E_INVALID, "%s: a table is NULL", fn);
     const int S = e->cfg.n_stations, P = S * (S - 1) / 2;
     PeakRec *d_ref = nullptr, *d_tgt = nullptr;
     if ((rc = alloc_t(e, &d_ref, (size_t)n_ref_windows * P)) || (rc = alloc_t(e, &d_tgt, (size_t)n_tgt_windows * P))) return rc;
     CU(cudaMemcpyAsync(d_ref, ref_in, (size_t)n_ref_windows * P * sizeof(PeakRec), cudaMemcpyHostToDevice, e->stream));
     CU(cudaMemcpyAsync(d_tgt, tgt_in, (size_t)n_tgt_windows * P * sizeof(PeakRec), cudaMemcpyHostToDevice, e->stream));
+    bool synced = false;
     if ((rc = fix_stage(e, stations_llh, o, T, d_ref, d_tgt, ref_fit, range_diffs, pair_used, fix_llh, fix_rms, fix_status,
-                        fix_iters)))
+                        fix_iters, G, &synced)))
         return rc;
-    return finish_fix_stage(e);
+    return finish_fix_stage(e, synced);
 }
 
-int tdoa_process_windows(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts *o, int64_t win_start,
-                         int64_t win_len, int32_t n_ref_windows, int32_t n_tgt_windows, int64_t hop, tdoa_peak *ref_out,
-                         tdoa_peak *tgt_out, double *ref_fit, double *range_diffs, uint8_t *pair_used, double *fix_llh,
-                         double *fix_rms, int32_t *fix_status, int32_t *fix_iters)
+int process_windows_impl(tdoa_engine *e, const char *fn, const double *stations_llh, const tdoa_window_opts *o,
+                         int64_t win_start, int64_t win_len, int32_t n_ref_windows, int32_t n_tgt_windows, int64_t hop,
+                         tdoa_peak *ref_out, tdoa_peak *tgt_out, double *ref_fit, double *range_diffs, uint8_t *pair_used,
+                         double *fix_llh, double *fix_rms, int32_t *fix_status, int32_t *fix_iters, const GridSeed *grid)
 {
     if (!e) return TDOA_E_INVALID;
     int rc = begin_call(e);
     if (rc) return rc;
     WinTimes T;
-    if ((rc = window_check(e, "tdoa_process_windows", stations_llh, o, win_start, win_len, n_ref_windows, n_tgt_windows, hop,
-                           fix_llh, fix_status, T)))
+    if ((rc = window_check(e, fn, stations_llh, o, win_start, win_len, n_ref_windows, n_tgt_windows, hop, fix_llh, fix_status, T)))
         return rc;
+    if (grid && (rc = grid_seed_check(e, fn, *grid))) return rc;
+    const GridSeed G = grid ? *grid : GridSeed{};
     const int S = e->cfg.n_stations, P = S * (S - 1) / 2;
     Tables tab{e->stream};
     CU(cudaMallocAsync(reinterpret_cast<void **>(&tab.ref), (size_t)n_ref_windows * P * sizeof(PeakRec), e->stream));
@@ -346,10 +463,58 @@ int tdoa_process_windows(tdoa_engine *e, const double *stations_llh, const tdoa_
         if (tgt_out)
             CU(cudaMemcpyAsync(tgt_out, tab.tgt, (size_t)n_tgt_windows * P * sizeof(PeakRec), cudaMemcpyDeviceToHost, e->stream));
     }
+    bool synced = false;
     if ((rc = fix_stage(e, stations_llh, o, T, tab.ref, tab.tgt, ref_fit, range_diffs, pair_used, fix_llh, fix_rms, fix_status,
-                        fix_iters)))
+                        fix_iters, G, &synced)))
         return rc;
-    return finish_fix_stage(e);
+    return finish_fix_stage(e, synced);
+}
+
+}  // namespace
+}  // namespace tdoa
+
+extern "C" {
+
+int tdoa_window_fixes(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts *o, int64_t win_start, int64_t win_len,
+                      int32_t n_ref_windows, int32_t n_tgt_windows, int64_t hop, const tdoa_peak *ref_in, const tdoa_peak *tgt_in,
+                      double *ref_fit, double *range_diffs, uint8_t *pair_used, double *fix_llh, double *fix_rms,
+                      int32_t *fix_status, int32_t *fix_iters)
+{
+    return window_fixes_impl(e, "tdoa_window_fixes", stations_llh, o, win_start, win_len, n_ref_windows, n_tgt_windows, hop,
+                             ref_in, tgt_in, ref_fit, range_diffs, pair_used, fix_llh, fix_rms, fix_status, fix_iters, nullptr);
+}
+
+int tdoa_window_fixes_grid(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts *o, int64_t win_start,
+                           int64_t win_len, int32_t n_ref_windows, int32_t n_tgt_windows, int64_t hop, const double *grid_desc,
+                           const tdoa_peak *ref_in, const tdoa_peak *tgt_in, double *ref_fit, double *range_diffs,
+                           uint8_t *pair_used, double *fix_llh, double *fix_rms, int32_t *fix_status, int32_t *fix_iters,
+                           double *seed_llh, double *seed_cost, int64_t *seed_index)
+{
+    const GridSeed G{grid_desc, seed_llh, seed_cost, seed_index};
+    return window_fixes_impl(e, "tdoa_window_fixes_grid", stations_llh, o, win_start, win_len, n_ref_windows, n_tgt_windows,
+                             hop, ref_in, tgt_in, ref_fit, range_diffs, pair_used, fix_llh, fix_rms, fix_status, fix_iters, &G);
+}
+
+int tdoa_process_windows(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts *o, int64_t win_start,
+                         int64_t win_len, int32_t n_ref_windows, int32_t n_tgt_windows, int64_t hop, tdoa_peak *ref_out,
+                         tdoa_peak *tgt_out, double *ref_fit, double *range_diffs, uint8_t *pair_used, double *fix_llh,
+                         double *fix_rms, int32_t *fix_status, int32_t *fix_iters)
+{
+    return process_windows_impl(e, "tdoa_process_windows", stations_llh, o, win_start, win_len, n_ref_windows, n_tgt_windows,
+                                hop, ref_out, tgt_out, ref_fit, range_diffs, pair_used, fix_llh, fix_rms, fix_status, fix_iters,
+                                nullptr);
+}
+
+int tdoa_process_windows_grid(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts *o, int64_t win_start,
+                              int64_t win_len, int32_t n_ref_windows, int32_t n_tgt_windows, int64_t hop, const double *grid_desc,
+                              tdoa_peak *ref_out, tdoa_peak *tgt_out, double *ref_fit, double *range_diffs, uint8_t *pair_used,
+                              double *fix_llh, double *fix_rms, int32_t *fix_status, int32_t *fix_iters, double *seed_llh,
+                              double *seed_cost, int64_t *seed_index)
+{
+    const GridSeed G{grid_desc, seed_llh, seed_cost, seed_index};
+    return process_windows_impl(e, "tdoa_process_windows_grid", stations_llh, o, win_start, win_len, n_ref_windows,
+                                n_tgt_windows, hop, ref_out, tgt_out, ref_fit, range_diffs, pair_used, fix_llh, fix_rms,
+                                fix_status, fix_iters, &G);
 }
 
 }  // extern "C"
