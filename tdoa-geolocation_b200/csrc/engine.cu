@@ -146,6 +146,51 @@ int grid_check(tdoa_engine *e, const char *fn, int n_stations, const double *gri
     return TDOA_OK;
 }
 
+int grid_search_queue(tdoa_engine *e, GridSearch &g, bool every_cell)
+{
+    int rc;
+    void *d_scratch = nullptr;
+    // use_fft = 0 evaluates every cell by the statement (SOURCE mode's default)
+    g.ranked = !every_cell && e->cfg.use_fft != 0;
+    if (!g.ranked) {
+        if ((rc = alloc(e, &d_scratch, grid_scratch_bytes(g.nlat, g.nlon, g.n_sets)))) return rc;
+        launch_grid_cells(g.d_llh, g.n_st, g.d_desc, g.nlat, g.nlon, g.d_rd, g.n_sets, g.rd_stride, g.d_cost, g.d_idx, g.d_out,
+                          d_scratch, e->stream, g.d_used, g.d_tab);
+        count_launch(e, 2);
+        return TDOA_OK;
+    }
+    // ranked: the expanded cost (16 FMA per cell and set) finds the cells that can hold the minimum, the statement
+    // settles them (solve.cu)
+    if ((rc = alloc_t(e, &g.d_count, (size_t)grid_rank_chunks(g.n_sets))) ||
+        (rc = alloc(e, &d_scratch, grid_rank_scratch_bytes(g.nlat, g.nlon, g.n_sets))))
+        return rc;
+    launch_grid_ranked(g.d_llh, g.n_st, g.d_desc, g.nlat, g.nlon, g.d_tab, g.d_rd, g.n_sets, g.rd_stride, g.d_cost, g.d_idx,
+                       g.d_out, d_scratch, g.d_count, e->stream, g.d_used);
+    count_launch(e, 5 * grid_rank_chunks(g.n_sets));
+    return TDOA_OK;
+}
+
+int grid_search_fetch(tdoa_engine *e, GridSearch &g)
+{
+    if (!g.ranked) return TDOA_OK;
+    g.h_count.resize((size_t)grid_rank_chunks(g.n_sets));
+    g.h_idx.resize((size_t)g.n_sets);
+    CU(cudaMemcpyAsync(g.h_count.data(), g.d_count, g.h_count.size() * sizeof(int), cudaMemcpyDeviceToHost, e->stream));
+    CU(cudaMemcpyAsync(g.h_idx.data(), g.d_idx, g.h_idx.size() * sizeof(i64), cudaMemcpyDeviceToHost, e->stream));
+    return TDOA_OK;
+}
+
+bool grid_search_complete(const GridSearch &g, const std::vector<char> &searched)
+{
+    if (!g.ranked) return true;
+    if (grid_rank_overflowed(g.h_count.data(), g.n_sets)) return false;   // a plateau of ties
+    // a searched set without a survivor (range differences that are not numbers: every comparison of the bound
+    // fails): the statement decides such sets too
+    for (int s = 0; s < g.n_sets; s++)
+        if (g.h_idx[s] < 0 && searched[s]) return false;
+    return true;
+}
+
 // tdoa_grid (used == nullptr) and tdoa_grid_masked
 int grid_impl(tdoa_engine *e, const char *fn, const double *stations_llh, int32_t n_stations, const double *grid_desc,
               const double *range_diffs, const uint8_t *used, int32_t n_sets, int32_t rd_stride, double *out_llh,
@@ -158,76 +203,39 @@ int grid_impl(tdoa_engine *e, const char *fn, const double *stations_llh, int32_
     if (!stations_llh || !range_diffs || !out_llh || n_sets < 0 || rd_stride < P)
         return fail(e, TDOA_E_INVALID, "%s: bad arguments (2..16 stations, rd_stride >= pairs)", fn);
     if ((rc = grid_check(e, fn, n_stations, grid_desc))) return rc;
-    const int nlat = (int)grid_desc[4], nlon = (int)grid_desc[5];
     if (n_sets == 0) return end_call(e, true);
-    double *d_llh = nullptr, *d_desc = nullptr, *d_rd = nullptr, *d_cost = nullptr, *d_out = nullptr;
-    i64 *d_idx = nullptr;
+    GridSearch g;
+    g.n_sets = n_sets; g.rd_stride = rd_stride; g.n_st = n_stations; g.nlat = (int)grid_desc[4]; g.nlon = (int)grid_desc[5];
+    double *d_llh = nullptr, *d_desc = nullptr, *d_rd = nullptr, *d_tab = nullptr;
     uint8_t *d_used = nullptr;
-    void *d_scratch = nullptr;
+    // the host's share: the table of c_k per set (masked: also which sets are searched, which every cell reads)
+    const int T = grid_rank_tab_doubles(used != nullptr);
+    std::vector<double> tab((size_t)n_sets * T, 0.0);
+    std::vector<char> searched((size_t)n_sets);
+    for (int s = 0; s < n_sets; s++)
+        searched[s] = grid_rank_row(range_diffs + (size_t)s * rd_stride, used ? used + (size_t)s * rd_stride : nullptr,
+                                    n_stations, tab.data() + (size_t)s * T);
     if ((rc = alloc_t(e, &d_llh, (size_t)3 * n_stations)) || (rc = alloc_t(e, &d_desc, 8)) ||
-        (rc = alloc_t(e, &d_rd, (size_t)n_sets * rd_stride)) || (rc = alloc_t(e, &d_cost, (size_t)n_sets)) ||
-        (rc = alloc_t(e, &d_idx, (size_t)n_sets)) || (rc = alloc_t(e, &d_out, (size_t)3 * n_sets)) ||
-        (rc = alloc(e, &d_scratch, grid_scratch_bytes(n_stations, nlat, nlon, n_sets))))
+        (rc = alloc_t(e, &d_rd, (size_t)n_sets * rd_stride)) || (rc = alloc_t(e, &d_tab, tab.size())) ||
+        (rc = alloc_t(e, &g.d_cost, (size_t)n_sets)) || (rc = alloc_t(e, &g.d_idx, (size_t)n_sets)) ||
+        (rc = alloc_t(e, &g.d_out, (size_t)3 * n_sets)))
         return rc;
     CU(cudaMemcpyAsync(d_llh, stations_llh, (size_t)3 * n_stations * sizeof(double), cudaMemcpyHostToDevice, e->stream));
     CU(cudaMemcpyAsync(d_desc, grid_desc, 7 * sizeof(double), cudaMemcpyHostToDevice, e->stream));
     CU(cudaMemcpyAsync(d_rd, range_diffs, (size_t)n_sets * rd_stride * sizeof(double), cudaMemcpyHostToDevice, e->stream));
+    CU(cudaMemcpyAsync(d_tab, tab.data(), tab.size() * sizeof(double), cudaMemcpyHostToDevice, e->stream));
     if (used) {
         if ((rc = alloc_t(e, &d_used, (size_t)n_sets * rd_stride))) return rc;
         CU(cudaMemcpyAsync(d_used, used, (size_t)n_sets * rd_stride, cudaMemcpyHostToDevice, e->stream));
-        CU(cudaMemsetAsync(d_out, 0xff, (size_t)3 * n_sets * sizeof(double), e->stream));   // NaN where no arg-min
+        CU(cudaMemsetAsync(g.d_out, 0xff, (size_t)3 * n_sets * sizeof(double), e->stream));   // NaN where no arg-min
     }
-    bool exhaustive = e->cfg.use_fft == 0;   // every cell by the statement (SOURCE mode's default; the fall-back below)
-    // the host's share: the table of c_k per set (masked: also which sets are searched, which the exhaustive kernel reads)
-    const int T = grid_rank_tab_doubles(used != nullptr);
-    std::vector<double> tab;
-    std::vector<char> searched((size_t)n_sets, 1);
-    double *d_tab = nullptr;
-    if (!exhaustive || used) {
-        tab.assign((size_t)n_sets * T, 0.0);
-        for (int s = 0; s < n_sets; s++)
-            searched[s] = grid_rank_row(range_diffs + (size_t)s * rd_stride, used ? used + (size_t)s * rd_stride : nullptr,
-                                        n_stations, tab.data() + (size_t)s * T);
-        if ((rc = alloc_t(e, &d_tab, tab.size()))) return rc;
-        CU(cudaMemcpyAsync(d_tab, tab.data(), tab.size() * sizeof(double), cudaMemcpyHostToDevice, e->stream));
-    }
-    if (!exhaustive) {
-        // ranked: the expanded cost (16 FMA per cell and set) finds the cells that can hold the minimum, the
-        // statement settles them (solve.cu)
-        int *d_count = nullptr;
-        const int chunk = grid_rank_max_sets();
-        const int n_chunks = (n_sets + chunk - 1) / chunk;
-        void *d_rscratch = nullptr;
-        if ((rc = alloc_t(e, &d_count, (size_t)n_chunks)) ||
-            (rc = alloc(e, &d_rscratch, grid_rank_scratch_bytes(nlat, nlon, std::min(n_sets, chunk)))))
-            return rc;
-        std::vector<int> h_count((size_t)n_chunks, 0);
-        for (int c = 0; c < n_chunks; c++) {
-            const int s0 = c * chunk, ns = std::min(chunk, n_sets - s0);
-            launch_grid_ranked(d_llh, n_stations, d_desc, nlat, nlon, d_tab + (size_t)s0 * T, d_rd + (size_t)s0 * rd_stride, ns,
-                               rd_stride, d_cost + s0, d_idx + s0, d_out + 3 * s0, d_rscratch, d_count + c, e->stream,
-                               used ? d_used + (size_t)s0 * rd_stride : nullptr);
-            count_launch(e, 5);
-        }
-        std::vector<i64> h_idx((size_t)n_sets, 0);
-        CU(cudaMemcpyAsync(h_count.data(), d_count, (size_t)n_chunks * sizeof(int), cudaMemcpyDeviceToHost, e->stream));
-        CU(cudaMemcpyAsync(h_idx.data(), d_idx, (size_t)n_sets * sizeof(i64), cudaMemcpyDeviceToHost, e->stream));
-        CU(cudaStreamSynchronize(e->stream));   // tab, h_count and h_idx are this frame's
-        for (int c = 0; c < n_chunks; c++)
-            if (h_count[c] > grid_rank_cand_cap(std::min(chunk, n_sets - c * chunk))) exhaustive = true;   // a plateau of ties
-        // a searched set without a survivor (range differences that are not numbers: every comparison of the bound
-        // fails): the statement decides such sets too
-        for (int s = 0; s < n_sets; s++)
-            if (h_idx[s] < 0 && searched[s]) exhaustive = true;
-    }
-    if (exhaustive) {
-        launch_grid_cells(d_llh, n_stations, d_desc, nlat, nlon, d_rd, n_sets, rd_stride, d_cost, d_idx, d_out, d_scratch,
-                          e->stream, d_used, d_tab);
-        count_launch(e, 2);
-    }
-    CU(cudaMemcpyAsync(out_llh, d_out, (size_t)3 * n_sets * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
-    if (out_cost) CU(cudaMemcpyAsync(out_cost, d_cost, (size_t)n_sets * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
-    if (out_index) CU(cudaMemcpyAsync(out_index, d_idx, (size_t)n_sets * sizeof(i64), cudaMemcpyDeviceToHost, e->stream));
+    g.d_llh = d_llh; g.d_desc = d_desc; g.d_rd = d_rd; g.d_tab = d_tab; g.d_used = d_used;
+    if ((rc = grid_search_queue(e, g, false)) || (rc = grid_search_fetch(e, g))) return rc;
+    CU(cudaStreamSynchronize(e->stream));   // tab and the read-back are this frame's
+    if (!grid_search_complete(g, searched) && (rc = grid_search_queue(e, g, true))) return rc;
+    CU(cudaMemcpyAsync(out_llh, g.d_out, (size_t)3 * n_sets * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
+    if (out_cost) CU(cudaMemcpyAsync(out_cost, g.d_cost, (size_t)n_sets * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
+    if (out_index) CU(cudaMemcpyAsync(out_index, g.d_idx, (size_t)n_sets * sizeof(i64), cudaMemcpyDeviceToHost, e->stream));
     return end_call(e, true);
 }
 

@@ -166,6 +166,22 @@ void spans_collect(tdoa_engine *e);   // the stream must be idle
 
 // ---- grid multilateration (engine.cu): the argument checks every grid entry point shares
 int grid_check(tdoa_engine *e, const char *fn, int n_stations, const double *grid_desc);
+// The arg-min search of the grid entry points: the ranked pass and, where it is incomplete or use_fft = 0, every cell
+struct GridSearch {
+    const double *d_llh = nullptr, *d_desc = nullptr, *d_tab = nullptr, *d_rd = nullptr;   // d_tab: the ranked rows
+    const uint8_t *d_used = nullptr;   // nullptr: unmasked
+    int n_sets = 0, rd_stride = 0, n_st = 0, nlat = 0, nlon = 0;
+    double *d_cost = nullptr, *d_out = nullptr;
+    i64 *d_idx = nullptr;
+    bool ranked = false;   // the last queued pass was the ranked one
+    int *d_count = nullptr;
+    std::vector<int> h_count;
+    std::vector<i64> h_idx;
+};
+int grid_search_queue(tdoa_engine *e, GridSearch &g, bool every_cell);
+int grid_search_fetch(tdoa_engine *e, GridSearch &g);   // the ranked pass's read-back, before the caller's sync
+// after the sync: false if the ranked pass overflowed or a searched set found no cell
+bool grid_search_complete(const GridSearch &g, const std::vector<char> &searched);
 
 // ---- signal views and lazy loads (engine_pipeline.cu)
 i64 signal_length(const Station &s, int kind, i64 guard);

@@ -188,18 +188,21 @@ void launch_window_rd(const PeakRec *d_tgt, int n_tgt, int n_st, const double *d
 constexpr int kWindowFitDoubles = 5;   // per pair: a, beta, t_mean, windows used, geometric term
 void launch_range_diffs(const PeakRec *d_ref, const PeakRec *d_tgt, int n_pairs, double fs, int mode, double *d_td,
                         double *d_rd, cudaStream_t st);
+// the grid arg-min; its one caller, grid_search_queue (engine.cu), chooses the form and checks the ranked one
 // d_used (may be nullptr): the masked statement, d_used[set * rd_stride + p]; d_tab then holds the masked rows (their
 // "searched" flags); a set without an arg-min gets index -1, cost NaN and leaves d_out_llh as it was
 void launch_grid_cells(const double *d_llh, int n_st, const double *d_grid_desc, int nlat, int nlon,
                        const double *d_rd, int n_sets, int rd_stride, double *d_best_cost, i64 *d_best_idx,
-                       double *d_out_llh, void *d_scratch, cudaStream_t st, const uint8_t *d_used = nullptr,
-                       const double *d_tab = nullptr);
-size_t grid_scratch_bytes(int n_st, int nlat, int nlon, int n_sets);
-// the same arg-min, ranked by the expanded cost (16 FMA per cell and set) and settled by the statement on the survivors
+                       double *d_out_llh, void *d_scratch, cudaStream_t st, const uint8_t *d_used, const double *d_tab);
+size_t grid_scratch_bytes(int nlat, int nlon, int n_sets);
+// the same arg-min, ranked by the expanded cost (16 FMA per cell and set) and settled by the statement on the survivors;
+// d_count: grid_rank_chunks(n_sets) ints, and grid_rank_overflowed on their host copy means the ranked pass is incomplete
 void launch_grid_ranked(const double *d_llh, int n_st, const double *d_grid_desc, int nlat, int nlon, const double *d_tab,
                         const double *d_rd, int n_sets, int rd_stride, double *d_best_cost, i64 *d_best_idx,
-                        double *d_out_llh, void *d_scratch, int *d_count, cudaStream_t st, const uint8_t *d_used = nullptr);
+                        double *d_out_llh, void *d_scratch, int *d_count, cudaStream_t st, const uint8_t *d_used);
 size_t grid_rank_scratch_bytes(int nlat, int nlon, int n_sets);
+int grid_rank_chunks(int n_sets);
+bool grid_rank_overflowed(const int *h_count, int n_sets);
 // one set's row of d_tab on the host (masked when used != nullptr); false: a masked set with no used pair
 bool grid_rank_row(const double *rd, const uint8_t *used, int n_st, double *row);
 // the masked rows on the device (the windowed seed): a set the least-squares step would refuse (status 2 with dims) is
@@ -207,7 +210,5 @@ bool grid_rank_row(const double *rd, const uint8_t *used, int n_st, double *row)
 void launch_grid_rows(const double *d_rd, const uint8_t *d_used, int n_sets, int rd_stride, int n_st, int dims, double *d_tab,
                       cudaStream_t st);
 int grid_rank_tab_doubles(bool masked = false);
-int grid_rank_max_sets();
-int grid_rank_cand_cap(int n_sets);
 
 }  // namespace tdoa

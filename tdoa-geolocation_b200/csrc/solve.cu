@@ -5,6 +5,9 @@
 // (:151-163), solveTDOA (:932-1020) and ecefToLatLon (:1023-1045).  All f64, written
 // in the reference's operation order.  The grid solve has no reference equivalent
 // (oracle: orc_grid_solve).
+#include <algorithm>
+#include <type_traits>
+
 #include "geodesy.cuh"
 #include "kernels.h"
 
@@ -878,8 +881,17 @@ __global__ void k_grid_rows(const double *rd_all, const uint8_t *used_all, int n
 }
 
 int grid_rank_tab_doubles(bool masked) { return masked ? kRankTabMasked : kRankTab; }
-int grid_rank_max_sets() { return kRankMaxSets; }
-int grid_rank_cand_cap(int n_sets) { return 64 * n_sets + 1024; }
+int grid_rank_chunks(int n_sets) { return (n_sets + kRankMaxSets - 1) / kRankMaxSets; }
+
+// the candidate table of a chunk of n_sets sets
+static int rank_cand_cap(int n_sets) { return 64 * n_sets + 1024; }
+
+bool grid_rank_overflowed(const int *h_count, int n_sets)
+{
+    for (int c = 0; c < grid_rank_chunks(n_sets); c++)
+        if (h_count[c] > rank_cand_cap(std::min(kRankMaxSets, n_sets - c * kRankMaxSets))) return true;
+    return false;
+}
 
 static int rank_n_cta(int nlat, int nlon)
 {
@@ -887,12 +899,13 @@ static int rank_n_cta(int nlat, int nlon)
     return (int)((cells + kRankSpan - 1) / kRankSpan);
 }
 
-// scratch: [n_sets][n_cta] lo, [n_sets][n_cta] hi, [n_sets] bound, candidates, counter
+// one chunk's scratch, which every chunk reuses: [n_sets][n_cta] lo, [n_sets][n_cta] hi, [n_sets] bound, candidates, counter
 size_t grid_rank_scratch_bytes(int nlat, int nlon, int n_sets)
 {
+    n_sets = std::min(n_sets, kRankMaxSets);
     const size_t n_cta = (size_t)rank_n_cta(nlat, nlon);
     return (2 * n_cta * (size_t)n_sets + (size_t)n_sets) * sizeof(double) +
-           (size_t)grid_rank_cand_cap(n_sets) * sizeof(GridCand) + 64;
+           (size_t)rank_cand_cap(n_sets) * sizeof(GridCand) + 64;
 }
 
 // Host rows (tdoa_grid, tdoa_grid_masked): the range differences are on the host already, and building the rows there
@@ -911,38 +924,39 @@ void launch_grid_rows(const double *d_rd, const uint8_t *d_used, int n_sets, int
     if (n_sets > 0) k_grid_rows<<<(n_sets + 63) / 64, 64, 0, st>>>(d_rd, d_used, n_sets, rd_stride, n_st, dims, d_tab);
 }
 
-// n_sets <= grid_rank_max_sets().  d_count: one int, read back by the caller after the stream has drained --
-// more than grid_rank_cand_cap(n_sets) candidates means the table is incomplete (launch_grid_cells then).
+// five launches per chunk of kRankMaxSets sets.  d_count: grid_rank_chunks(n_sets) ints, read back by the caller after
+// the stream has drained -- grid_rank_overflowed means the table is incomplete (launch_grid_cells then).
 void launch_grid_ranked(const double *d_llh, int n_st, const double *d_grid_desc, int nlat, int nlon, const double *d_tab,
                         const double *d_rd, int n_sets, int rd_stride, double *d_best_cost, i64 *d_best_idx,
                         double *d_out_llh, void *d_scratch, int *d_count, cudaStream_t st, const uint8_t *d_used)
 {
     const int n_cta = rank_n_cta(nlat, nlon);
     if (n_cta <= 0 || n_sets <= 0) return;
-    double *cta_lo = reinterpret_cast<double *>(d_scratch);
-    double *cta_hi = cta_lo + (size_t)n_cta * n_sets;
-    double *bound = cta_hi + (size_t)n_cta * n_sets;
-    GridCand *cands = reinterpret_cast<GridCand *>(bound + n_sets);
-    const int cap = grid_rank_cand_cap(n_sets);
-    cudaMemsetAsync(d_count, 0, sizeof(int), st);
-    const size_t smem = (3 * kMaxStations + 2 * (size_t)n_sets * (kRankThreads / 32)) * sizeof(double);
-    const int n_exact = (cap + kRankThreads - 1) / kRankThreads;
-    if (d_used) {
-        k_grid_rank<true><<<n_cta, kRankThreads, smem, st>>>(d_llh, n_st, d_grid_desc, d_tab, n_sets, cta_lo, cta_hi);
-        k_grid_bound<<<n_sets, 256, 0, st>>>(cta_hi, n_cta, bound);
-        k_grid_refine<true><<<n_cta, kRankThreads, 0, st>>>(d_llh, n_st, d_grid_desc, d_tab, d_rd, n_sets, rd_stride, cta_lo,
-                                                          bound, cands, cap, d_count);
-        k_grid_exact<true><<<n_exact, kRankThreads, 0, st>>>(d_llh, n_st, d_grid_desc, d_rd, rd_stride, cands, cap, d_count,
-                                                             d_used);
-    } else {
-        k_grid_rank<false><<<n_cta, kRankThreads, smem, st>>>(d_llh, n_st, d_grid_desc, d_tab, n_sets, cta_lo, cta_hi);
-        k_grid_bound<<<n_sets, 256, 0, st>>>(cta_hi, n_cta, bound);
-        k_grid_refine<false><<<n_cta, kRankThreads, 0, st>>>(d_llh, n_st, d_grid_desc, d_tab, d_rd, n_sets, rd_stride, cta_lo,
-                                                           bound, cands, cap, d_count);
-        k_grid_exact<false><<<n_exact, kRankThreads, 0, st>>>(d_llh, n_st, d_grid_desc, d_rd, rd_stride, cands, cap, d_count,
-                                                              nullptr);
-    }
-    k_grid_pick<<<n_sets, 128, 0, st>>>(d_grid_desc, cands, cap, d_count, d_best_cost, d_best_idx, d_out_llh);
+    cudaMemsetAsync(d_count, 0, (size_t)grid_rank_chunks(n_sets) * sizeof(int), st);
+    auto chunks = [&](auto masked) {
+        constexpr bool kMasked = decltype(masked)::value;
+        constexpr int kTab = kMasked ? kRankTabMasked : kRankTab;
+        for (int c = 0, s0 = 0; s0 < n_sets; c++, s0 += kRankMaxSets) {
+            const int ns = std::min(kRankMaxSets, n_sets - s0), cap = rank_cand_cap(ns);
+            const double *tab = d_tab + (size_t)s0 * kTab, *rd = d_rd + (size_t)s0 * rd_stride;
+            double *cta_lo = reinterpret_cast<double *>(d_scratch);
+            double *cta_hi = cta_lo + (size_t)n_cta * ns;
+            double *bound = cta_hi + (size_t)n_cta * ns;
+            GridCand *cands = reinterpret_cast<GridCand *>(bound + ns);
+            const size_t smem = (3 * kMaxStations + 2 * (size_t)ns * (kRankThreads / 32)) * sizeof(double);
+            const int n_exact = (cap + kRankThreads - 1) / kRankThreads;
+            k_grid_rank<kMasked><<<n_cta, kRankThreads, smem, st>>>(d_llh, n_st, d_grid_desc, tab, ns, cta_lo, cta_hi);
+            k_grid_bound<<<ns, 256, 0, st>>>(cta_hi, n_cta, bound);
+            k_grid_refine<kMasked><<<n_cta, kRankThreads, 0, st>>>(d_llh, n_st, d_grid_desc, tab, rd, ns, rd_stride, cta_lo,
+                                                                   bound, cands, cap, d_count + c);
+            k_grid_exact<kMasked><<<n_exact, kRankThreads, 0, st>>>(d_llh, n_st, d_grid_desc, rd, rd_stride, cands, cap,
+                                                                    d_count + c,
+                                                                    kMasked ? d_used + (size_t)s0 * rd_stride : nullptr);
+            k_grid_pick<<<ns, 128, 0, st>>>(d_grid_desc, cands, cap, d_count + c, d_best_cost + s0, d_best_idx + s0,
+                                            d_out_llh + 3 * s0);
+        }
+    };
+    if (d_used) chunks(std::true_type{}); else chunks(std::false_type{});
 }
 
 static int grid_n_cta(int nlat, int nlon)
@@ -951,9 +965,8 @@ static int grid_n_cta(int nlat, int nlon)
     return (int)((cells + kGridThreads - 1) / kGridThreads);
 }
 
-size_t grid_scratch_bytes(int n_st, int nlat, int nlon, int n_sets)
+size_t grid_scratch_bytes(int nlat, int nlon, int n_sets)
 {
-    (void)n_st;
     return (size_t)grid_n_cta(nlat, nlon) * (size_t)n_sets * (sizeof(double) + sizeof(i64));
 }
 
@@ -966,12 +979,11 @@ void launch_grid_cells(const double *d_llh, int n_st, const double *d_grid_desc,
     double *cta_cost = reinterpret_cast<double *>(d_scratch);
     i64 *cta_idx = reinterpret_cast<i64 *>(cta_cost + (size_t)n_cta * n_sets);
     const size_t smem = (3 * kMaxStations + kGridThreads) * sizeof(double) + kGridThreads * sizeof(i64);
-    if (d_used)
-        k_grid_cost<true><<<n_cta, kGridThreads, smem, st>>>(d_llh, n_st, d_grid_desc, d_rd, n_sets, rd_stride, cta_cost, cta_idx,
-                                                             d_used, d_tab);
-    else
-        k_grid_cost<false><<<n_cta, kGridThreads, smem, st>>>(d_llh, n_st, d_grid_desc, d_rd, n_sets, rd_stride, cta_cost, cta_idx,
-                                                              nullptr, nullptr);
+    auto cells = [&](auto masked) {
+        k_grid_cost<decltype(masked)::value><<<n_cta, kGridThreads, smem, st>>>(d_llh, n_st, d_grid_desc, d_rd, n_sets, rd_stride,
+                                                                                cta_cost, cta_idx, d_used, d_tab);
+    };
+    if (d_used) cells(std::true_type{}); else cells(std::false_type{});
     k_grid_reduce<<<n_sets, 256, 0, st>>>(d_grid_desc, cta_cost, cta_idx, n_cta, d_best_cost, d_best_idx, d_out_llh);
 }
 

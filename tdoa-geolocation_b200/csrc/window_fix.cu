@@ -15,10 +15,10 @@
 //                     (+ the geometric term) and the used mask that k_solve_ls reads.
 // The _grid calls then seed each window's fix from the masked grid arg-min of its own used pairs (solve.cu):
 //   k_grid_rows       the window's row of the ranked table (not searched: the least-squares step's status 2)
-//   k_grid_rank ... k_grid_pick   write the arg-min cell into the window's start point, which holds the start
-//                     the window has without a grid; k_solve_ls starts there.
-// The ranked pass is optimistic: after the call's one synchronisation an overflowing candidate table or a searched
-// window without a survivor reruns the grid on every cell (k_grid_cost) and the fixes, before the call returns.
+//   k_grid_rank ... k_grid_pick   (engine.cu's grid search, as in tdoa_grid) write the arg-min cell into the window's
+//                     start point, which holds the start the window has without a grid; k_solve_ls starts there.
+// The ranked pass is optimistic: when the grid search finds it incomplete after the call's one synchronisation, the
+// call reruns the grid on every cell (k_grid_cost) and the fixes before it returns.
 // Window times and the usable test are stated in include/tdoa_b200.h (tdoa_process_windows).
 #include <cuda_runtime.h>
 
@@ -183,9 +183,17 @@ double window_time(const Station &s, int kind, i64 start, i64 len, i64 guard)
     return (double)v.run0_start + 0.5 * (double)(len - 1);
 }
 
+// the grid seed of the _grid calls: descriptor and optional outputs
+struct GridSeed {
+    const double *desc = nullptr;   // nullptr: no grid
+    double *llh = nullptr, *cost = nullptr;
+    int64_t *index = nullptr;
+};
+
+// grid: the seed of the _grid calls, nullptr without
 int window_check(tdoa_engine *e, const char *fn, const double *stations_llh, const tdoa_window_opts *o, int64_t win_start,
                  int64_t win_len, int32_t n_ref, int32_t n_tgt, int64_t hop, const double *fix_llh, const int32_t *fix_status,
-                 WinTimes &T)
+                 const GridSeed *grid, WinTimes &T)
 {
     const int S = e->cfg.n_stations;
     if (!stations_llh || !o || !fix_llh || !fix_status) return fail(e, TDOA_E_INVALID, "%s: NULL argument", fn);
@@ -216,24 +224,21 @@ int window_check(tdoa_engine *e, const char *fn, const double *stations_llh, con
         const i64 b = e->stations[st].nsamp / 3;
         T.t_mid[st] = (double)b + 0.5 * (double)(b - 1);
     }
-    return TDOA_OK;
+    if (!grid) return TDOA_OK;
+    if (!grid->desc) return fail(e, TDOA_E_INVALID, "%s: grid_desc is NULL", fn);
+    if (S > 16) return fail(e, TDOA_E_INVALID, "%s: the grid takes 2..16 stations, got %d", fn, S);
+    return grid_check(e, fn, S, grid->desc);
 }
-
-// the grid seed of the _grid calls: descriptor and optional outputs
-struct GridSeed {
-    const double *desc = nullptr;   // nullptr: no grid
-    double *llh = nullptr, *cost = nullptr;
-    int64_t *index = nullptr;
-};
 
 // the fix stage on device tables, queued on the engine's stream inside the caller's begin_call / end_call;
 // the station table, times and options ride in the descriptor frame.  *synced: the stream was drained (the grid
 // seed's check) and holds nothing more
 int fix_stage(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts *o, const WinTimes &T, const PeakRec *d_ref,
               const PeakRec *d_tgt, double *ref_fit, double *range_diffs, uint8_t *pair_used, double *fix_llh, double *fix_rms,
-              int32_t *fix_status, int32_t *fix_iters, const GridSeed &G, bool *synced)
+              int32_t *fix_status, int32_t *fix_iters, const GridSeed *grid, bool *synced)
 {
     *synced = false;
+    const GridSeed G = grid ? *grid : GridSeed{};
     const int S = e->cfg.n_stations, P = S * (S - 1) / 2, nt = T.n_tgt;
     int rc;
     const double *d_llh = nullptr, *d_t_ref = nullptr, *d_t_tgt = nullptr, *d_t_mid = nullptr, *d_ref_tx = nullptr,
@@ -265,44 +270,23 @@ int fix_stage(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts
         (rc = alloc_t(e, &d_fix, (size_t)3 * nt)) || (rc = alloc_t(e, &d_rms, (size_t)nt)) ||
         (rc = alloc_t(e, &d_status, (size_t)nt)) || (rc = alloc_t(e, &d_iters, (size_t)nt)))
         return rc;
-    // the grid seed: the windows' start points (written by the grid where it finds a cell), the masked rows, the
-    // ranked arg-min per chunk of sets
-    const int chunk = grid_rank_max_sets(), n_chunks = (nt + chunk - 1) / chunk, TW = grid_rank_tab_doubles(true);
-    int nlat = 0, nlon = 0;
-    const double *d_desc = nullptr;
-    double *d_start = nullptr, *d_tab = nullptr, *d_cost = nullptr;
-    i64 *d_idx = nullptr;
-    int *d_count = nullptr;
-    void *d_rscratch = nullptr;
+    // the grid seed: the windows' start points (written by the grid where it finds a cell), the masked rows
+    GridSearch g;
+    double *d_start = nullptr, *d_tab = nullptr;
     if (G.desc) {
-        nlat = (int)G.desc[4];
-        nlon = (int)G.desc[5];
+        const double *d_desc = nullptr;
         if ((rc = upload(e, std::vector<double>(G.desc, G.desc + 7), &d_desc)) || (rc = alloc_t(e, &d_start, (size_t)3 * nt)) ||
-            (rc = alloc_t(e, &d_tab, (size_t)nt * TW)) || (rc = alloc_t(e, &d_cost, (size_t)nt)) ||
-            (rc = alloc_t(e, &d_idx, (size_t)nt)) || (rc = alloc_t(e, &d_count, (size_t)n_chunks)) ||
-            (rc = alloc(e, &d_rscratch, grid_rank_scratch_bytes(nlat, nlon, std::min(nt, chunk)))))
+            (rc = alloc_t(e, &d_tab, (size_t)nt * grid_rank_tab_doubles(true))) || (rc = alloc_t(e, &g.d_cost, (size_t)nt)) ||
+            (rc = alloc_t(e, &g.d_idx, (size_t)nt)))
             return rc;
+        g.d_llh = d_llh; g.d_desc = d_desc; g.d_tab = d_tab; g.d_rd = d_rd; g.d_used = d_used; g.d_out = d_start;
+        g.n_sets = nt; g.rd_stride = P; g.n_st = S; g.nlat = (int)G.desc[4]; g.nlon = (int)G.desc[5];
     }
     // the grid (ranked, or every cell) between the range differences and the fixes
-    auto seed_and_fix = [&](bool exhaustive) -> int {
+    auto seed_and_fix = [&](bool every_cell) -> int {
         if (G.desc) {
             CU(cudaMemcpyAsync(d_start, d_init, (size_t)3 * nt * sizeof(double), cudaMemcpyDeviceToDevice, e->stream));
-            if (exhaustive) {
-                void *d_scratch = nullptr;
-                int rc2 = alloc(e, &d_scratch, grid_scratch_bytes(S, nlat, nlon, nt));
-                if (rc2) return rc2;
-                launch_grid_cells(d_llh, S, d_desc, nlat, nlon, d_rd, nt, P, d_cost, d_idx, d_start, d_scratch, e->stream, d_used,
-                                  d_tab);
-                count_launch(e, 2);
-            } else {
-                for (int c = 0; c < n_chunks; c++) {
-                    const int s0 = c * chunk, ns = std::min(chunk, nt - s0);
-                    launch_grid_ranked(d_llh, S, d_desc, nlat, nlon, d_tab + (size_t)s0 * TW, d_rd + (size_t)s0 * P, ns, P,
-                                       d_cost + s0, d_idx + s0, d_start + 3 * s0, d_rscratch, d_count + c, e->stream,
-                                       d_used + (size_t)s0 * P);
-                    count_launch(e, 5);
-                }
-            }
+            if (const int rc2 = grid_search_queue(e, g, every_cell)) return rc2;
         }
         launch_solve_ls(d_llh, S, d_rd, nt, P, G.desc ? d_start : d_init, o->dims, d_fix, d_rms, d_status, d_iters, e->stream,
                         d_used);
@@ -322,8 +306,8 @@ int fix_stage(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts
             (rc2 = back(fix_iters, d_iters, (size_t)nt * sizeof(int32_t))))
             return rc2;
         if (G.desc &&
-            ((rc2 = back(G.llh, d_start, (size_t)3 * nt * sizeof(double))) || (rc2 = back(G.cost, d_cost, (size_t)nt * sizeof(double))) ||
-             (rc2 = back(G.index, d_idx, (size_t)nt * sizeof(int64_t)))))
+            ((rc2 = back(G.llh, d_start, (size_t)3 * nt * sizeof(double))) || (rc2 = back(G.cost, g.d_cost, (size_t)nt * sizeof(double))) ||
+             (rc2 = back(G.index, g.d_idx, (size_t)nt * sizeof(int64_t)))))
             return rc2;
         return TDOA_OK;
     };
@@ -336,28 +320,22 @@ int fix_stage(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts
         launch_grid_rows(d_rd, d_used, nt, P, S, o->dims, d_tab, e->stream);
         count_launch(e);
     }
-    // use_fft = 0 evaluates every cell, as tdoa_grid does
-    if ((rc = seed_and_fix(e->cfg.use_fft == 0))) return rc;
+    if ((rc = seed_and_fix(false))) return rc;
     if ((rc = back(ref_fit, d_ref_fit, (size_t)3 * P * sizeof(double))) ||
         (rc = back(range_diffs, d_rd, (size_t)nt * P * sizeof(double))) || (rc = back(pair_used, d_used, (size_t)nt * P)) ||
         (rc = results()))
         return rc;
-    if (G.desc && e->cfg.use_fft != 0) {
-        // the optimistic ranked pass, checked after the call's one synchronisation
-        std::vector<int> h_count((size_t)n_chunks);
-        std::vector<i64> h_idx((size_t)nt);
+    if (G.desc) {
+        // the grid's check after the call's one synchronisation; its pageable read-back returns only when done, so
+        // it is queued behind the fixes
         std::vector<int> h_status((size_t)nt);
-        CU(cudaMemcpyAsync(h_count.data(), d_count, (size_t)n_chunks * sizeof(int), cudaMemcpyDeviceToHost, e->stream));
-        CU(cudaMemcpyAsync(h_idx.data(), d_idx, (size_t)nt * sizeof(i64), cudaMemcpyDeviceToHost, e->stream));
+        if ((rc = grid_search_fetch(e, g))) return rc;
         CU(cudaMemcpyAsync(h_status.data(), d_status, (size_t)nt * sizeof(int), cudaMemcpyDeviceToHost, e->stream));
         CU(cudaStreamSynchronize(e->stream));
         *synced = true;
-        bool again = false;
-        for (int c = 0; c < n_chunks; c++)
-            if (h_count[c] > grid_rank_cand_cap(std::min(chunk, nt - c * chunk))) again = true;   // a plateau of ties
-        for (int w = 0; w < nt; w++)
-            if (h_idx[w] < 0 && h_status[w] != 2) again = true;   // a searched window without a survivor
-        if (again) {
+        std::vector<char> searched((size_t)nt);
+        for (int w = 0; w < nt; w++) searched[w] = h_status[w] != 2;
+        if (!grid_search_complete(g, searched)) {
             if ((rc = seed_and_fix(true)) || (rc = results())) return rc;
             *synced = false;
         }
@@ -387,21 +365,6 @@ struct Tables {
     }
 };
 
-}  // namespace
-
-}  // namespace tdoa
-
-namespace tdoa {
-namespace {
-
-// the grid's refusals on top of window_check's
-int grid_seed_check(tdoa_engine *e, const char *fn, const GridSeed &G)
-{
-    if (!G.desc) return fail(e, TDOA_E_INVALID, "%s: grid_desc is NULL", fn);
-    if (e->cfg.n_stations > 16) return fail(e, TDOA_E_INVALID, "%s: the grid takes 2..16 stations, got %d", fn, e->cfg.n_stations);
-    return grid_check(e, fn, e->cfg.n_stations, G.desc);
-}
-
 int window_fixes_impl(tdoa_engine *e, const char *fn, const double *stations_llh, const tdoa_window_opts *o, int64_t win_start,
                       int64_t win_len, int32_t n_ref_windows, int32_t n_tgt_windows, int64_t hop, const tdoa_peak *ref_in,
                       const tdoa_peak *tgt_in, double *ref_fit, double *range_diffs, uint8_t *pair_used, double *fix_llh,
@@ -411,10 +374,9 @@ int window_fixes_impl(tdoa_engine *e, const char *fn, const double *stations_llh
     int rc = begin_call(e);
     if (rc) return rc;
     WinTimes T;
-    if ((rc = window_check(e, fn, stations_llh, o, win_start, win_len, n_ref_windows, n_tgt_windows, hop, fix_llh, fix_status, T)))
+    if ((rc = window_check(e, fn, stations_llh, o, win_start, win_len, n_ref_windows, n_tgt_windows, hop, fix_llh, fix_status, grid,
+                          T)))
         return rc;
-    if (grid && (rc = grid_seed_check(e, fn, *grid))) return rc;
-    const GridSeed G = grid ? *grid : GridSeed{};
     if (!ref_in || !tgt_in) return fail(e, TDOA_E_INVALID, "%s: a table is NULL", fn);
     const int S = e->cfg.n_stations, P = S * (S - 1) / 2;
     PeakRec *d_ref = nullptr, *d_tgt = nullptr;
@@ -423,7 +385,7 @@ int window_fixes_impl(tdoa_engine *e, const char *fn, const double *stations_llh
     CU(cudaMemcpyAsync(d_tgt, tgt_in, (size_t)n_tgt_windows * P * sizeof(PeakRec), cudaMemcpyHostToDevice, e->stream));
     bool synced = false;
     if ((rc = fix_stage(e, stations_llh, o, T, d_ref, d_tgt, ref_fit, range_diffs, pair_used, fix_llh, fix_rms, fix_status,
-                        fix_iters, G, &synced)))
+                        fix_iters, grid, &synced)))
         return rc;
     return finish_fix_stage(e, synced);
 }
@@ -437,10 +399,9 @@ int process_windows_impl(tdoa_engine *e, const char *fn, const double *stations_
     int rc = begin_call(e);
     if (rc) return rc;
     WinTimes T;
-    if ((rc = window_check(e, fn, stations_llh, o, win_start, win_len, n_ref_windows, n_tgt_windows, hop, fix_llh, fix_status, T)))
+    if ((rc = window_check(e, fn, stations_llh, o, win_start, win_len, n_ref_windows, n_tgt_windows, hop, fix_llh, fix_status, grid,
+                          T)))
         return rc;
-    if (grid && (rc = grid_seed_check(e, fn, *grid))) return rc;
-    const GridSeed G = grid ? *grid : GridSeed{};
     const int S = e->cfg.n_stations, P = S * (S - 1) / 2;
     Tables tab{e->stream};
     CU(cudaMallocAsync(reinterpret_cast<void **>(&tab.ref), (size_t)n_ref_windows * P * sizeof(PeakRec), e->stream));
@@ -465,7 +426,7 @@ int process_windows_impl(tdoa_engine *e, const char *fn, const double *stations_
     }
     bool synced = false;
     if ((rc = fix_stage(e, stations_llh, o, T, tab.ref, tab.tgt, ref_fit, range_diffs, pair_used, fix_llh, fix_rms, fix_status,
-                        fix_iters, G, &synced)))
+                        fix_iters, grid, &synced)))
         return rc;
     return finish_fix_stage(e, synced);
 }

@@ -1,8 +1,9 @@
 #!/usr/bin/env python
 """Times grid-seeded windowed fixes (tdoa_process_windows_grid) against tdoa_process_windows on the two windowed
 workloads of tools/windows_bench.py (same run, alternating), with the fix stage's device time of both and an oracle
-verdict on one window; and times BASELINE config 5 (tdoa_grid, 1000 x 1000 cells, 16 stations, 64 sets) with this
-tree's library and with a second library (e.g. built from the parent commit), alternating in one process.
+verdict on one window.  With --parent-lib it also times BASELINE config 5 (tdoa_grid, 1000 x 1000 cells, 16 stations,
+64 sets) and tdoa_process_windows_grid on both workloads with this tree's library and with a second library (e.g. built
+from the parent commit), alternating in one process, and checks that both give the same bits.
 
     python tools/window_grid_bench.py [--reps K] [--parent-lib PATH] [--out profiles/r4_window_grid.jsonl]
 
@@ -112,7 +113,8 @@ def run_case(name, e, stations, caps, grid, reps, tx):
 def engine_on(lib_path, *args, **kw):
     """an Engine bound to another build of the library (which may lack this build's newer symbols)"""
     other, cur = ctypes.CDLL(str(lib_path)), _N.load_library()
-    for name in ("tdoa_default_config", "tdoa_create", "tdoa_destroy", "tdoa_last_error", "tdoa_grid", "tdoa_get_stats"):
+    for name in ("tdoa_default_config", "tdoa_create", "tdoa_destroy", "tdoa_last_error", "tdoa_grid", "tdoa_get_stats",
+                 "tdoa_load_u8_device", "tdoa_process_windows_grid"):
         getattr(other, name).argtypes = getattr(cur, name).argtypes
         getattr(other, name).restype = getattr(cur, name).restype
     saved = _N._lib
@@ -149,10 +151,36 @@ def cfg5_ab(parent_lib, reps):
             "same_index_and_cost": bool(same)}
 
 
+def windows_ab(name, engines, stations, grid, reps):
+    """tdoa_process_windows_grid with this tree's library and the other (engines: {"branch", "parent"}, both loaded
+    with the same captures), alternating; every returned array must be the same bits"""
+    nw_t, nw_r = BLOCK // W, 2 * BLOCK // W
+    times = {k: [] for k in engines}
+    fix = {k: [] for k in engines}
+    outs = {}
+    for _ in range(2):   # warm every shape
+        for e in engines.values():
+            e.process_windows(stations, 0, W, nw_r, nw_t, W, grid=grid)
+    for _ in range(reps):
+        for k, e in engines.items():
+            torch.cuda.synchronize(); t0 = time.perf_counter()
+            outs[k] = e.process_windows(stations, 0, W, nw_r, nw_t, W, grid=grid)
+            times[k].append(time.perf_counter() - t0)
+            fix[k].append(e.stats()["ms_fix"])
+    same = all(np.asarray(outs["branch"][k]).tobytes() == np.asarray(outs["parent"][k]).tobytes() for k in outs["branch"])
+    med = lambda v: 1e3 * float(np.median(v))   # noqa: E731
+    return {"case": name + ": tdoa_process_windows_grid, branch vs parent build", "grid": grid, "reps": reps,
+            "branch_ms": med(times["branch"]), "parent_ms": med(times["parent"]),
+            "branch_ms_all": [1e3 * t for t in times["branch"]], "parent_ms_all": [1e3 * t for t in times["parent"]],
+            "branch_ms_fix": float(np.median(fix["branch"])), "parent_ms_fix": float(np.median(fix["parent"])),
+            "branch_ms_fix_all": fix["branch"], "parent_ms_fix_all": fix["parent"], "same_outputs": bool(same)}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--reps", type=int, default=5)
-    ap.add_argument("--parent-lib", default="", help="libtdoa_b200.so of another build for the config 5 comparison")
+    ap.add_argument("--parent-lib", default="",
+                    help="libtdoa_b200.so of another build for the config 5 and windowed comparisons")
     ap.add_argument("--cfg5-reps", type=int, default=21)
     ap.add_argument("--out", default=str(ROOT / "profiles" / "r4_window_grid.jsonl"))
     args = ap.parse_args()
@@ -163,20 +191,25 @@ def main():
         lines.append(cfg5_ab(args.parent_lib, args.cfg5_reps))
     delays, _ = configs_bench.delays_for(bench.STATION_LLH)
     caps = configs_bench.synth(dev, 3, BLOCK, delays)
-    with T.Engine(T.MODE_EXTENDED, max_lag=50_000) as e:
-        for k in range(3):
-            e.load_u8_device(k, caps[k].data_ptr(), caps[k].numel(), keep=caps[k])
-        lines.append(run_case("config 3: 3 stations, Mode B FM, EXTENDED, +-50000 lags", e, bench.STATION_LLH, caps,
-                              around(bench.STATION_LLH, 400), args.reps, bench.TX_LLH))
+    def case(name, stations, caps, grid, **kw):
+        with T.Engine(T.MODE_EXTENDED, **kw) as e:
+            for k, c in enumerate(caps):
+                e.load_u8_device(k, c.data_ptr(), c.numel(), keep=c)
+            lines.append(run_case(name, e, stations, caps, grid, args.reps, bench.TX_LLH))
+            if args.parent_lib:
+                with engine_on(args.parent_lib, T.MODE_EXTENDED, **kw) as p:
+                    for k, c in enumerate(caps):
+                        p.load_u8_device(k, c.data_ptr(), c.numel(), keep=c)
+                    lines.append(windows_ab(name, {"branch": e, "parent": p}, stations, grid, args.reps))
+
+    case("config 3: 3 stations, Mode B FM, EXTENDED, +-50000 lags", bench.STATION_LLH, caps, around(bench.STATION_LLH, 400),
+         max_lag=50_000)
     del caps
     torch.cuda.empty_cache()
     stations = S.ring_stations(16)
     caps, _ = S.simulate_weak(stations, tuple(bench.TX_LLH), 92300000.0, 10.0, 1000.0, BLOCK, seed=4242, device=dev)
-    with T.Engine(T.MODE_EXTENDED, n_stations=16, max_lag=2000) as e:
-        for k in range(16):
-            e.load_u8_device(k, caps[k].data_ptr(), caps[k].numel(), keep=caps[k])
-        lines.append(run_case("configs[3]: 16 stations, weak_signal_simulator.go content, EXTENDED, +-2000 lags", e,
-                              np.asarray(stations), caps, around(stations, 1000), args.reps, bench.TX_LLH))
+    case("configs[3]: 16 stations, weak_signal_simulator.go content, EXTENDED, +-2000 lags", np.asarray(stations), caps,
+         around(stations, 1000), n_stations=16, max_lag=2000)
     out = Path(args.out)
     out.parent.mkdir(parents=True, exist_ok=True)
     with out.open("a") as f:
