@@ -223,5 +223,12 @@ TDOA_HD2 void cross_accumulate(float2 a, float2 c, float2 b, float2 d, float *ac
     acc[7] = fmaf(t1x, s1y, fmaf(-t1y, s1x, acc[7]));
 }
 
+// Bins k < N/2 of a tile, one per register slot c = 0..7: thread t of transform g takes k = 2t + q + 512 c, whose
+// X_g[k] it holds after pass 3 (u0[c] for q = 0, u1[c] for q = 1), and loads only A or B at k, A[N-k] and B[N-k].
+// The two transforms' threads t split the pair {2t, 2t + 1} + 512 c between them.  Lanes 8..15 and 24..31 of a warp
+// take the other parity than lanes 0..7 and 16..23, so the 16 lanes of each half warp hit 16 distinct 64-bit bank
+// pairs at k and at N - k: one wavefront each, where all-even bins (a 16-byte stride) would be two-way conflicted.
+TDOA_HD2 int tile_bin_parity(int g, int t) { return ((t >> 3) & 1) ^ g; }
+
 }  // namespace fft2
 }  // namespace tdoa

@@ -140,13 +140,16 @@ __global__ void __launch_bounds__(kTileThreads, 1) k_fft_tiles(const TileJob *jo
         }
     };
 
+    const int n_seg = J.n_seg, stride = J.n_cta;
     float2 v[32];
-    int seg = cta;
-    load_segment(seg, v);
+    load_segment(cta, v);
     const float2 *ZA = sm, *ZB = sm + kBuf;
-    for (; seg < J.n_seg; seg += J.n_cta) {
+    const float2 *ZO = g ? ZA : ZB;   // the other transform's spectrum
+    const int q = tile_bin_parity(g, t);
+    for (int seg = cta; seg < n_seg; seg += stride) {
         pass1_store(v, t, buf);
         bar_transform(g);
+        float2 own[8];   // X_g[2t + q + 512 c], c = 0..7: this thread's own operand of its bins
         {
             float2 u0[16], u1[16];
             pass_load(buf, t, u0, u1);
@@ -159,20 +162,29 @@ __global__ void __launch_bounds__(kTileThreads, 1) k_fft_tiles(const TileJob *jo
             pass3_compute(u0, w1a);
             pass3_compute(u1, w1b);
             spectrum_store(u0, u1, t, buf);  // natural order, into the (free again) buffer
+#pragma unroll
+            for (int c = 0; c < 8; c++) own[c] = q ? u1[c] : u0[c];
         }
         // the next segment's samples travel while the cross-spectra are formed (the fence
         // keeps the loads from being hoisted into the transform, where registers are full)
         asm volatile("" ::: "memory");
-        if (seg + J.n_cta < J.n_seg) load_segment(seg + J.n_cta, v);
+        // pass 1 transformed v in place: without the else, the last segment's spectrum (64 registers) would stay
+        // live through passes 2 and 3 for an iteration the compiler cannot rule out, and the transform would spill
+        if (seg + stride < n_seg) load_segment(seg + stride, v);
+        else
+#pragma unroll
+            for (int r = 0; r < 32; r++) v[r] = make_float2(0.f, 0.f);
         __syncthreads();
-        // bins k = t + 256 w, w = 8 g .. 8 g + 7: four products per 8-column chunk
+        // bins k = 2t + q + 512 c, c = 0..7: X_g[k] is in a register, three operands come from shared memory
 #pragma unroll
         for (int c = 0; c < 8; c++) {
             float acc[8];
             tmem_ld8(tmem + 8 * c, acc);
-            const int k = t + 256 * (8 * g + c);
+            const int k = 2 * t + q + 512 * c;
             const int nk = (kN - k) & (kN - 1);
-            cross_accumulate(ZA[k], ZA[nk], ZB[k], ZB[nk], acc);
+            const float2 o = ZO[k];
+            if (g == 0) cross_accumulate(own[c], ZA[nk], o, ZB[nk], acc);
+            else cross_accumulate(o, ZA[nk], own[c], ZB[nk], acc);
             tmem_st8(tmem + 8 * c, acc);
         }
         if (warp == 8) {  // Nyquist bin: thread 0 of transform B; the whole warp moves its columns
@@ -189,7 +201,7 @@ __global__ void __launch_bounds__(kTileThreads, 1) k_fft_tiles(const TileJob *jo
     for (int c = 0; c < 8; c++) {
         float acc[8];
         tmem_ld8(tmem + 8 * c, acc);
-        const int k = t + 256 * (8 * g + c);
+        const int k = 2 * t + q + 512 * c;
 #pragma unroll
         for (int p = 0; p < 4; p++)
             if (J.partials[p]) J.partials[p][(size_t)cta * kBins + k] = make_float2(0.5f * acc[2 * p], acc[2 * p + 1]);
