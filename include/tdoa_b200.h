@@ -275,6 +275,44 @@ TDOA_API int tdoa_window_fixes(tdoa_engine *e, const double *stations_llh, const
                                int64_t hop, const tdoa_peak *ref_in, const tdoa_peak *tgt_in, double *ref_fit,
                                double *range_diffs, uint8_t *pair_used, double *fix_llh, double *fix_rms,
                                int32_t *fix_status, int32_t *fix_iters);
+/* ---- re-timed target correlation (no reference equivalent; engine-defined): tdoa_process_windows with every
+ * station's TGT planes re-timed by that station's clock rate, so that a TGT window may be as long as block 2.
+ * 1 ppm of relative rate moves the lag 2 samples per second; tdoa_process_windows corrects the OFFSET of each TGT
+ * lag but not the drift inside a window, which smears a long window's peak.  Clock error belongs to a station:
+ * the REF fit's slopes satisfy beta_ij = c_j - c_i.
+ *  - Station rates: the pairs whose REF fit used at least 2 windows (ref_fit[p][2] >= 2) enter the fit.  c[S]
+ *    minimises the sum over those pairs of (c_j - c_i - beta_ij)^2, and sums to zero within each connected
+ *    component of those pairs.  Computed in f64, every operation rounded to nearest (no fused multiply-add), in
+ *    this order: A = the normal matrix of the pairs plus, for each component, 1 at every (i, j) of its stations;
+ *    b[i] -= beta and b[j] += beta pair by pair in pair order; A = L L^T by Cholesky, right-looking (L_kk =
+ *    sqrt(A_kk), L_ik = A_ik / L_kk, then A_ij -= L_ik L_jk for k < j <= i, k ascending); L y = b and L^T c = y
+ *    column by column (y_k = b_k / L_kk, then b_i -= L_ik y_k for i > k; c_k = y_k / L_kk, then y_i -= L_ki c_k
+ *    for i < k, k descending).  A station with no fitted pair gets rate 0 (it re-times nothing) and NaN in
+ *    clock_rate; its pairs are used in no TGT window anyway.
+ *  - Re-timing: x[0..len) is station k's preprocessed plane of one TGT window, the plane the correlator reads, in
+ *    that plane's own samples (n / decimate with the decimator).  Its re-timed plane is x~[n] = x[n + delta(n)]
+ *    where 0 <= n + delta(n) < len, and 0 elsewhere; delta(n) = floor(c_k * (n - n_c) + 0.5), n_c = (len - 1) / 2,
+ *    in f64 rounded to nearest with no fused multiply-add.  Length, statistics and normalisation scale stay
+ *    those of x.  delta(n_c) = 0, so a record's lag + frac is the lag at the window's centre: the time the range
+ *    differences already take.
+ *  - The call: the REF pair loop over the REF windows (records as tdoa_xcorr gives them), the REF fit, the
+ *    station rates, the TGT pair loop over the TGT windows on re-timed planes, then the range differences and
+ *    fixes of tdoa_process_windows.  REF and TGT windows have separate geometry (e.g. short REF windows and one
+ *    TGT window of the whole block); tgt_win_len = 0 follows tdoa_xcorr's rule.  Outputs are those of
+ *    tdoa_process_windows plus clock_rate[S] (samples per sample), which may be NULL.  With rates so small that
+ *    |c| (len - 1) / 2 < 0.5 for every station, delta is 0 everywhere and the results are tdoa_process_windows'.
+ *  - On a multi-GPU engine the call is collective.  The REF windows are dealt and gathered as tdoa_xcorr deals
+ *    them, every rank fits the rates from its gathered table (the fit is deterministic: the same bits on every
+ *    rank), then the TGT windows are dealt and gathered the same way.  The TGT pass depends on the fit, so the
+ *    ranks meet twice per call instead of once.
+ * Refused (TDOA_E_INVALID): what tdoa_process_windows refuses, for either geometry. */
+TDOA_API int tdoa_process_windows_retimed(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts *o,
+                                          int64_t ref_win_start, int64_t ref_win_len, int32_t n_ref_windows,
+                                          int64_t ref_hop, int64_t tgt_win_start, int64_t tgt_win_len,
+                                          int32_t n_tgt_windows, int64_t tgt_hop, tdoa_peak *ref_out, tdoa_peak *tgt_out,
+                                          double *ref_fit, double *range_diffs, uint8_t *pair_used, double *fix_llh,
+                                          double *fix_rms, int32_t *fix_status, int32_t *fix_iters, double *clock_rate);
+
 /* Grid-seeded windowed fixes: as tdoa_process_windows / tdoa_window_fixes, with each TGT window's
  * least-squares fix started from the arg-min of tdoa_grid_masked over grid_desc (7 doubles, as
  * tdoa_grid) with that window's range differences and used pairs -- computed on the device between the

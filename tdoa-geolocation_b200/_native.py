@@ -23,7 +23,7 @@ ERRORS = {-1: "TDOA_E_INVALID", -2: "TDOA_E_NODEVICE", -3: "TDOA_E_CUDA", -4: "T
 # every symbol include/tdoa_b200.h declares (tests check the library exports them all)
 ABI_SYMBOLS = [
     "tdoa_default_config", "tdoa_create", "tdoa_destroy", "tdoa_last_error", "tdoa_host_alloc", "tdoa_host_free",
-    "tdoa_load_u8", "tdoa_load_file", "tdoa_load_u8_pinned", "tdoa_load_u8_device", "tdoa_unpack", "tdoa_preprocess", "tdoa_xcorr", "tdoa_xcorr_device", "tdoa_xcorr_windows", "tdoa_process", "tdoa_process_windows", "tdoa_window_fixes", "tdoa_process_windows_grid", "tdoa_window_fixes_grid", "tdoa_xcorr_info", "tdoa_analyze",
+    "tdoa_load_u8", "tdoa_load_file", "tdoa_load_u8_pinned", "tdoa_load_u8_device", "tdoa_unpack", "tdoa_preprocess", "tdoa_xcorr", "tdoa_xcorr_device", "tdoa_xcorr_windows", "tdoa_process", "tdoa_process_windows", "tdoa_window_fixes", "tdoa_process_windows_grid", "tdoa_window_fixes_grid", "tdoa_process_windows_retimed", "tdoa_xcorr_info", "tdoa_analyze",
     "tdoa_cross_correlate", "tdoa_baselines", "tdoa_solve", "tdoa_solve_binary", "tdoa_solve_ls", "tdoa_grid", "tdoa_grid_masked", "tdoa_get_stats", "tdoa_stream",
     "tdoa_set_stream", "tdoa_synchronize", "tdoa_selftest",
     "tdoa_comm_unique_id", "tdoa_comm_init", "tdoa_comm_rank", "tdoa_shard_windows",
@@ -154,6 +154,7 @@ def load_library():
     L.tdoa_window_fixes.argtypes = [vp, vp, C.POINTER(WindowOpts), i64, i64, i32, i32, i64] + [vp] * 9
     L.tdoa_process_windows_grid.argtypes = [vp, vp, C.POINTER(WindowOpts), i64, i64, i32, i32, i64] + [vp] * 13
     L.tdoa_window_fixes_grid.argtypes = [vp, vp, C.POINTER(WindowOpts), i64, i64, i32, i32, i64] + [vp] * 13
+    L.tdoa_process_windows_retimed.argtypes = [vp, vp, C.POINTER(WindowOpts), i64, i64, i32, i64, i64, i64, i32, i64] + [vp] * 10
     L.tdoa_cross_correlate.argtypes = [vp, vp, i64, vp, i64, C.POINTER(PeakStruct)]
     L.tdoa_baselines.argtypes = [vp, vp, i32, vp]
     L.tdoa_solve.argtypes = [vp, vp, i32, vp, i32, i32, vp, vp, vp]
@@ -454,8 +455,7 @@ class Engine:
         return {"ref": ref, "tgt": tgt, "time_differences": td, "range_differences": rd, "position": fix,
                 "status": int(status.value), "iters": int(iters.value)}
 
-    def _windows(self, fn, stations_llh, win_start, win_len, n_ref_windows, n_tgt_windows, hop, tables, dims,
-                 min_margin, ref_max_residual, ref_tx_llh, init_llh, grid=None) -> dict:
+    def _window_opts(self, stations_llh, dims, min_margin, ref_max_residual, ref_tx_llh, init_llh):
         st = np.ascontiguousarray(stations_llh, dtype=np.float64).reshape(-1, 3)
         if st.shape[0] != self.n_stations:
             raise ValueError(f"stations_llh has {st.shape[0]} rows, the engine holds {self.n_stations} stations")
@@ -465,6 +465,11 @@ class Engine:
             o.ref_tx_llh[:] = [float(v) for v in ref_tx_llh]
         if init_llh is not None:
             o.init_llh[:] = [float(v) for v in init_llh]
+        return st, o
+
+    def _windows(self, fn, stations_llh, win_start, win_len, n_ref_windows, n_tgt_windows, hop, tables, dims,
+                 min_margin, ref_max_residual, ref_tx_llh, init_llh, grid=None) -> dict:
+        st, o = self._window_opts(stations_llh, dims, min_margin, ref_max_residual, ref_tx_llh, init_llh)
         P, nt = self.n_pairs, max(n_tgt_windows, 0)
         ref_fit, rd = np.zeros((P, 3), np.float64), np.zeros((nt, P), np.float64)
         used = np.zeros((nt, P), np.uint8)
@@ -504,6 +509,28 @@ class Engine:
                             min_margin, ref_max_residual, ref_tx_llh, init_llh, grid)
         out["ref"], out["tgt"] = ref, tgt
         return out
+
+    def process_windows_retimed(self, stations_llh, ref, tgt, dims: int = 2, min_margin: float = 0.0,
+                                ref_max_residual: float = 0.0, ref_tx_llh=None, init_llh=None) -> dict:
+        """Re-timed target correlation (tdoa_process_windows_retimed): ref = (start, len, n, hop) and tgt = (start,
+        len, n, hop) are the two kinds' window geometries.  The REF windows give each pair's drift line as in
+        process_windows; the station clock rates fitted from those slopes re-time every TGT plane, so a TGT window
+        may span the whole block without smearing its peak.  Returns process_windows' dict plus clock_rate[S]
+        (samples per sample; NaN for a station without a fitted pair)."""
+        (r0, rl, nr, rh), (t0, tl, nt, th) = (tuple(int(v) for v in g) for g in (ref, tgt))
+        st, o = self._window_opts(stations_llh, dims, min_margin, ref_max_residual, ref_tx_llh, init_llh)
+        P, nt_ = self.n_pairs, max(nt, 0)
+        ref_t, tgt_t = np.zeros((max(nr, 0), P), PEAK_DTYPE), np.zeros((nt_, P), PEAK_DTYPE)
+        ref_fit, rd = np.zeros((P, 3), np.float64), np.zeros((nt_, P), np.float64)
+        used = np.zeros((nt_, P), np.uint8)
+        fix, rms = np.zeros((nt_, 3), np.float64), np.zeros(nt_, np.float64)
+        status, iters = np.zeros(nt_, np.int32), np.zeros(nt_, np.int32)
+        rate = np.zeros(self.n_stations, np.float64)
+        self._check(self._lib.tdoa_process_windows_retimed(
+            self._h, _ptr(st), C.byref(o), r0, rl, nr, rh, t0, tl, nt, th, _ptr(ref_t), _ptr(tgt_t), _ptr(ref_fit),
+            _ptr(rd), _ptr(used), _ptr(fix), _ptr(rms), _ptr(status), _ptr(iters), _ptr(rate)))
+        return {"ref_fit": ref_fit, "range_differences": rd, "pair_used": used.astype(bool), "position": fix,
+                "rms": rms, "status": status, "iters": iters, "ref": ref_t, "tgt": tgt_t, "clock_rate": rate}
 
     def window_fixes(self, stations_llh, win_start: int, win_len: int, ref, tgt, hop: int, dims: int = 2,
                      min_margin: float = 0.0, ref_max_residual: float = 0.0, ref_tx_llh=None, init_llh=None,

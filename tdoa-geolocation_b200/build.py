@@ -29,6 +29,7 @@ UNITS = [
     ("xcorr_exact.cu", ["-fmad=false"]),
     ("solve.cu", ["-fmad=false"]),
     ("window_fix.cu", ["-fmad=false"]),
+    ("retime.cu", ["-fmad=false"]),
     ("analyze.cu", ["-fmad=false"]),
     ("xcorr_fft.cu", []),
     ("xcorr_tile.cu", []),

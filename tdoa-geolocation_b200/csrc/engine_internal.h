@@ -195,12 +195,13 @@ int capture_ready(tdoa_engine *e, Station &s);
 void stats_reset(tdoa_engine *e);
 int window_lengths(tdoa_engine *e, int32_t kind, int64_t win_start, int64_t win_len, int32_t n_windows, int64_t hop,
                    std::vector<i64> &len);
+// d_rates (device, S doubles, may be nullptr): every plane re-timed by its station's rate (tdoa_process_windows_retimed)
 int xcorr_core(tdoa_engine *e, int32_t kind, int64_t win_start, const std::vector<i64> &len, int32_t n_windows,
-               int64_t hop, PeakRec *d_out, Pending *pend);
+               int64_t hop, PeakRec *d_out, Pending *pend, const double *d_rates = nullptr);
 // tdoa_xcorr / tdoa_xcorr_device as one call; d_table (device, n_windows * P, out may then be nullptr): the
-// records are also left there, past the call's end (tdoa_process_windows)
+// records are also left there, past the call's end (tdoa_process_windows); d_rates as xcorr_core
 int xcorr_impl(tdoa_engine *e, int32_t kind, int64_t win_start, int64_t win_len, int32_t n_windows, int64_t hop,
-               tdoa_peak *out, bool out_is_device, PeakRec *d_table = nullptr);
+               tdoa_peak *out, bool out_is_device, PeakRec *d_table = nullptr, const double *d_rates = nullptr);
 
 // ---- more than one GPU (engine_multi.cu)
 // windows dealt over the ranks of the engine's communicator, records gathered: true if it took the call
@@ -216,6 +217,7 @@ struct ShardPart {
     int64_t hop = 0;
     tdoa_peak *out = nullptr;   // host or device table of n_windows * P records, or nullptr
     bool out_is_device = false;
+    const double *rates = nullptr;   // station rates on the calling rank's device: the planes are re-timed (xcorr_core)
 };
 int xcorr_sharded(tdoa_engine *e, const std::vector<ShardPart> &parts);
 void multi_destroy(tdoa_engine *e);

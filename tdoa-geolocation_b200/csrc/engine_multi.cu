@@ -140,7 +140,8 @@ int sharded_rank(tdoa_engine *e, const std::vector<ShardPart> &parts)
             else if ((rc = alloc_t(e, &W.d_table, (size_t)Q.n_windows * P))) return rc;
             W.mine = W.d_gather + (size_t)M.rank * W.n_max * P;
             CU(cudaMemsetAsync(W.mine, 0, (size_t)W.n_max * P * sizeof(PeakRec), e->stream));
-            if (count > 0 && (rc = xcorr_core(e, Q.kind, Q.win_start + (i64)first * Q.hop, Q.len, count, Q.hop * world, W.mine, nullptr)))
+            if (count > 0 && (rc = xcorr_core(e, Q.kind, Q.win_start + (i64)first * Q.hop, Q.len, count, Q.hop * world, W.mine, nullptr,
+                                              Q.rates)))
                 return rc;
         }
         return TDOA_OK;
@@ -188,6 +189,16 @@ int xcorr_sharded(tdoa_engine *e, const std::vector<ShardPart> &parts)
     // one process, several devices: one host thread per peer (each queues on its own device and
     // joins the gather); this thread is rank 0
     const int n = (int)M.peers.size();
+    // station rates (tdoa_process_windows_retimed) live on this device: each peer gets the same S doubles in its own
+    std::vector<std::vector<double>> h_rates(parts.size());
+    bool any_rates = false;
+    for (size_t k = 0; k < parts.size(); k++) {
+        if (!parts[k].rates) continue;
+        h_rates[k].resize(e->cfg.n_stations);
+        CU(cudaMemcpyAsync(h_rates[k].data(), parts[k].rates, h_rates[k].size() * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
+        any_rates = true;
+    }
+    if (any_rates) CU(cudaStreamSynchronize(e->stream));
     std::vector<int> rcs(n, TDOA_OK);
     std::vector<std::thread> threads;
     Rendezvous rdv;
@@ -198,10 +209,12 @@ int xcorr_sharded(tdoa_engine *e, const std::vector<ShardPart> &parts)
             tdoa_engine *p = M.peers[r];
             int rc = begin_call(p);
             std::vector<ShardPart> mine = parts;   // the peer's own window lengths; its tables stay on its device
-            for (ShardPart &Q : mine) {
+            for (size_t k = 0; k < mine.size(); k++) {
+                ShardPart &Q = mine[k];
                 const i64 wl = Q.len.empty() ? 0 : Q.len[0];
                 Q.out = nullptr; Q.out_is_device = false;
                 if (!rc) rc = window_lengths(p, Q.kind, Q.win_start, wl, Q.n_windows, Q.hop, Q.len);
+                if (!rc && Q.rates) rc = upload(p, h_rates[k], &Q.rates);
             }
             if (rc) rdv.arrive(false);
             else rc = sharded_rank(p, mine);

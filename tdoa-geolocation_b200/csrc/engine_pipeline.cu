@@ -1241,28 +1241,54 @@ int window_lengths(tdoa_engine *e, int32_t kind, int64_t win_start, int64_t win_
     return TDOA_OK;
 }
 
-// windows per group: the planes of a group stay under 24 GiB
-int window_group(const tdoa_engine *e, const std::vector<i64> &len, int n_windows)
+// windows per group: the planes of a group stay under 24 GiB (retimed: one more plane per signal)
+int window_group(const tdoa_engine *e, const std::vector<i64> &len, int n_windows, bool retimed)
 {
     i64 per_window_bytes = 0;
-    for (int s = 0; s < e->cfg.n_stations; s++) per_window_bytes += len[s] * 4 * 4;
+    for (int s = 0; s < e->cfg.n_stations; s++) per_window_bytes += len[s] * 4 * (retimed ? 5 : 4);
     const i64 budget = (i64)24 << 30;
     const int group = (int)std::max<i64>(1, std::min<i64>(n_windows, budget / std::max<i64>(per_window_bytes, 1)));
     return std::min(group, 64);
+}
+
+// Every preprocessed plane re-timed by its station's rate (k_retime): the correlators read the re-timed plane with
+// the statistics block (normalisation scale) of the original.  The imaginary plane is dropped: the BINARY and
+// EXTENDED correlators read real parts only, and SOURCE mode has no re-timed call.
+int retime(tdoa_engine *e, std::vector<Sig> &sigs, const double *d_rates)
+{
+    std::vector<RetimeJob> jobs;
+    i64 max_n = 0;
+    for (Sig &sg : sigs) {
+        const i64 n = sg.n_out >= 0 ? sg.n_out : sg.n;
+        if (n == 0) continue;
+        RetimeJob j{sg.out_re, nullptr, n, sg.station};
+        if (const int rc = alloc_t(e, &j.y, (size_t)n)) return rc;
+        sg.out_re = j.y;
+        sg.out_im = nullptr;
+        jobs.push_back(j);
+        max_n = std::max(max_n, n);
+    }
+    if (jobs.empty()) return TDOA_OK;
+    const RetimeJob *d_jobs = nullptr;
+    if (const int rc = upload(e, jobs, &d_jobs)) return rc;
+    launch_retime(d_jobs, (int)jobs.size(), max_n, d_rates, e->stream);
+    count_launch(e);
+    return TDOA_OK;
 }
 
 // The pair loops of one signal kind over the windows, records to d_out (device).
 // pend == nullptr: every check is made here (the stream is synchronised as needed).
 // pend != nullptr: one window, everything only QUEUED -- branch guesses and candidate
 // overflow are the caller's to check after its synchronisation (tdoa_process).
+// d_rates != nullptr: station rates on the device; every plane is re-timed between preprocessing and correlation.
 int xcorr_core(tdoa_engine *e, int32_t kind, int64_t win_start, const std::vector<i64> &len, int32_t n_windows,
-               int64_t hop, PeakRec *d_out, Pending *pend)
+               int64_t hop, PeakRec *d_out, Pending *pend, const double *d_rates)
 {
     int rc;
     const int S = e->cfg.n_stations, P = S * (S - 1) / 2;
     if ((rc = queue_lazy_copies(e, kind))) return rc;
     // windows are processed in groups that keep the working set bounded
-    const int group = window_group(e, len, n_windows);
+    const int group = window_group(e, len, n_windows, d_rates != nullptr);
     for (int w0 = 0; w0 < n_windows; w0 += group) {
         const int gw = std::min(group, n_windows - w0);
         std::vector<Sig> sigs((size_t)gw * S);
@@ -1291,6 +1317,7 @@ int xcorr_core(tdoa_engine *e, int32_t kind, int64_t win_start, const std::vecto
         for (int attempt = 0; attempt < 2; attempt++) {
             const int sp_pre = span_begin(e, SPAN_STAGE_PRE);
             if ((rc = preprocess(e, sigs, attempt == 0))) return rc;
+            if (d_rates && (rc = retime(e, sigs, d_rates))) return rc;
             span_end(e, sp_pre);
             const int sp_corr = span_begin(e, SPAN_STAGE_CORR);
             d_first = nullptr;
@@ -1344,7 +1371,7 @@ int xcorr_core(tdoa_engine *e, int32_t kind, int64_t win_start, const std::vecto
 }
 
 int xcorr_impl(tdoa_engine *e, int32_t kind, int64_t win_start, int64_t win_len, int32_t n_windows, int64_t hop,
-               tdoa_peak *out, bool out_is_device, PeakRec *d_table)
+               tdoa_peak *out, bool out_is_device, PeakRec *d_table, const double *d_rates)
 {
     if (!e) return TDOA_E_INVALID;
     int rc = begin_call(e);
@@ -1367,14 +1394,14 @@ int xcorr_impl(tdoa_engine *e, int32_t kind, int64_t win_start, int64_t win_len,
     // checked after the one synchronisation, and any failure falls back to the checked pass.
     const int nA = (n_windows + 1) / 2, nB = n_windows - nA;
     bool done = false;
-    if (!e->cfg.serial_kinds && !out_is_device && nB >= 1 && window_group(e, len, nA) >= nA) {
+    if (!e->cfg.serial_kinds && !out_is_device && nB >= 1 && window_group(e, len, nA, d_rates != nullptr) >= nA) {
         Pending pend[2];
         cudaStream_t main_stream = e->stream;
         CU(cudaEventRecord(e->ev_fork, main_stream));
         CU(cudaStreamWaitEvent(e->side_stream, e->ev_fork, 0));
-        if ((rc = xcorr_core(e, kind, win_start, len, nA, hop, d_out, &pend[0]))) return rc;
+        if ((rc = xcorr_core(e, kind, win_start, len, nA, hop, d_out, &pend[0], d_rates))) return rc;
         e->stream = e->side_stream;
-        rc = xcorr_core(e, kind, win_start + (i64)nA * hop, len, nB, hop, d_out + (size_t)nA * P, &pend[1]);
+        rc = xcorr_core(e, kind, win_start + (i64)nA * hop, len, nB, hop, d_out + (size_t)nA * P, &pend[1], d_rates);
         e->stream = main_stream;
         CU(cudaEventRecord(e->ev_join, e->side_stream));
         CU(cudaStreamWaitEvent(main_stream, e->ev_join, 0));
@@ -1405,7 +1432,7 @@ int xcorr_impl(tdoa_engine *e, int32_t kind, int64_t win_start, int64_t win_len,
         }
     }
     if (!done) {
-        if ((rc = xcorr_core(e, kind, win_start, len, n_windows, hop, d_out, nullptr))) return rc;
+        if ((rc = xcorr_core(e, kind, win_start, len, n_windows, hop, d_out, nullptr, d_rates))) return rc;
         cudaEventRecord(e->ev[4], e->stream);
         if (!out_is_device && out)
             CU(cudaMemcpyAsync(out, d_out, (size_t)n_windows * P * sizeof(tdoa_peak), cudaMemcpyDeviceToHost, e->stream));

@@ -186,6 +186,17 @@ void launch_window_ref_fit(const PeakRec *d_ref, int n_ref, int n_st, const doub
 void launch_window_rd(const PeakRec *d_tgt, int n_tgt, int n_st, const double *d_t_tgt, const double *d_fit, float min_margin,
                       double fs, double *d_rd, uint8_t *d_used, cudaStream_t st);
 constexpr int kWindowFitDoubles = 5;   // per pair: a, beta, t_mean, windows used, geometric term
+// ---- retime.cu (tdoa_process_windows_retimed): station clock rates from the REF fits, and the re-timing gather
+// rate[S] (0 for a station without a fitted pair) re-times the planes, clock[S] (NaN there) is what the call returns;
+// n_st <= 64 (solve_ls_max_stations)
+void launch_station_rates(const double *d_fit, int n_st, double *d_rate, double *d_clock, cudaStream_t st);
+struct RetimeJob {
+    const float *x;   // one preprocessed plane, n samples
+    float *y;         // its re-timed plane (16-byte aligned)
+    i64 n;
+    int station;      // index into the rates
+};
+void launch_retime(const RetimeJob *d_jobs, int n_jobs, i64 max_n, const double *d_rates, cudaStream_t st);
 void launch_range_diffs(const PeakRec *d_ref, const PeakRec *d_tgt, int n_pairs, double fs, int mode, double *d_td,
                         double *d_rd, cudaStream_t st);
 // the grid arg-min; its one caller, grid_search_queue (engine.cu), chooses the form and checks the ranked one

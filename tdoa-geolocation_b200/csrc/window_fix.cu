@@ -19,6 +19,8 @@
 //                     start point, which holds the start the window has without a grid; k_solve_ls starts there.
 // The ranked pass is optimistic: when the grid search finds it incomplete after the call's one synchronisation, the
 // call reruns the grid on every cell (k_grid_cost) and the fixes before it returns.
+// tdoa_process_windows_retimed runs the REF pair loop, k_window_ref_fit and k_station_rates (retime.cu) before the TGT
+// pair loop, which re-times every plane by its station's rate; the fix stage is the same.
 // Window times and the usable test are stated in include/tdoa_b200.h (tdoa_process_windows).
 #include <cuda_runtime.h>
 
@@ -168,6 +170,13 @@ void launch_window_rd(const PeakRec *d_tgt, int n_tgt, int n_st, const double *d
 
 namespace {
 
+// the windows of one signal kind, as tdoa_xcorr takes them
+struct WinGeom {
+    int64_t start, len;
+    int32_t n;
+    int64_t hop;
+};
+
 // what the fix stage needs besides the tables: window times per (window, station), block-2 centres
 struct WinTimes {
     int n_ref = 0, n_tgt = 0;
@@ -191,10 +200,10 @@ struct GridSeed {
 };
 
 // grid: the seed of the _grid calls, nullptr without
-int window_check(tdoa_engine *e, const char *fn, const double *stations_llh, const tdoa_window_opts *o, int64_t win_start,
-                 int64_t win_len, int32_t n_ref, int32_t n_tgt, int64_t hop, const double *fix_llh, const int32_t *fix_status,
-                 const GridSeed *grid, WinTimes &T)
+int window_check(tdoa_engine *e, const char *fn, const double *stations_llh, const tdoa_window_opts *o, const WinGeom &ref,
+                 const WinGeom &tgt, const double *fix_llh, const int32_t *fix_status, const GridSeed *grid, WinTimes &T)
 {
+    const int32_t n_ref = ref.n, n_tgt = tgt.n;
     const int S = e->cfg.n_stations;
     if (!stations_llh || !o || !fix_llh || !fix_status) return fail(e, TDOA_E_INVALID, "%s: NULL argument", fn);
     if (e->cfg.mode == TDOA_MODE_SOURCE)
@@ -209,15 +218,15 @@ int window_check(tdoa_engine *e, const char *fn, const double *stations_llh, con
     T.parts.assign(2, ShardPart{});
     int rc;
     for (int kind = 0; kind < 2; kind++) {
+        const WinGeom &G = kind == TDOA_KIND_REF ? ref : tgt;
         ShardPart &Q = T.parts[kind];
-        Q.kind = kind; Q.win_start = win_start; Q.hop = hop;
-        Q.n_windows = kind == TDOA_KIND_REF ? n_ref : n_tgt;
-        if ((rc = window_lengths(e, kind, win_start, win_len, Q.n_windows, hop, Q.len))) return rc;
+        Q.kind = kind; Q.win_start = G.start; Q.hop = G.hop; Q.n_windows = G.n;
+        if ((rc = window_lengths(e, kind, G.start, G.len, G.n, G.hop, Q.len))) return rc;
         std::vector<double> &t = kind == TDOA_KIND_REF ? T.t_ref : T.t_tgt;
         t.resize((size_t)Q.n_windows * S);
         for (int w = 0; w < Q.n_windows; w++)
             for (int st = 0; st < S; st++)
-                t[(size_t)w * S + st] = window_time(e->stations[st], kind, win_start + (i64)w * hop, Q.len[st], e->cfg.guard_samples);
+                t[(size_t)w * S + st] = window_time(e->stations[st], kind, G.start + (i64)w * G.hop, Q.len[st], e->cfg.guard_samples);
     }
     T.t_mid.resize(S);
     for (int st = 0; st < S; st++) {
@@ -354,16 +363,36 @@ int finish_fix_stage(tdoa_engine *e, bool synced)
     return TDOA_OK;
 }
 
-// the two device tables of tdoa_process_windows: they outlive the pair loops' calls
+// the two device tables of tdoa_process_windows, and the station rates of the retimed call (re-timing rates, then
+// the returned clock_rate): they outlive the pair loops' calls
 struct Tables {
     cudaStream_t st;
     PeakRec *ref = nullptr, *tgt = nullptr;
+    double *rates = nullptr;
     ~Tables()
     {
         if (ref) cudaFreeAsync(ref, st);
         if (tgt) cudaFreeAsync(tgt, st);
+        if (rates) cudaFreeAsync(rates, st);
     }
 };
+
+// the station rates from the REF table, as one call of their own: k_window_ref_fit (the slopes only), k_station_rates
+int station_rates(tdoa_engine *e, const tdoa_window_opts *o, const WinTimes &T, const PeakRec *d_ref, double *d_rates)
+{
+    int rc = begin_call(e);
+    if (rc) return rc;
+    const int S = e->cfg.n_stations, P = S * (S - 1) / 2;
+    const double *d_t_ref = nullptr;
+    double *d_fit = nullptr;
+    if ((rc = upload(e, T.t_ref, &d_t_ref)) || (rc = alloc_t(e, &d_fit, (size_t)kWindowFitDoubles * P))) return rc;
+    launch_window_ref_fit(d_ref, T.n_ref, S, d_t_ref, nullptr, nullptr, nullptr, o->min_margin, o->ref_max_residual, d_fit,
+                          nullptr, e->stream);
+    launch_station_rates(d_fit, S, d_rates, d_rates + S, e->stream);
+    count_launch(e, 2);
+    CU(cudaGetLastError());
+    return end_call(e, false);
+}
 
 int window_fixes_impl(tdoa_engine *e, const char *fn, const double *stations_llh, const tdoa_window_opts *o, int64_t win_start,
                       int64_t win_len, int32_t n_ref_windows, int32_t n_tgt_windows, int64_t hop, const tdoa_peak *ref_in,
@@ -374,8 +403,8 @@ int window_fixes_impl(tdoa_engine *e, const char *fn, const double *stations_llh
     int rc = begin_call(e);
     if (rc) return rc;
     WinTimes T;
-    if ((rc = window_check(e, fn, stations_llh, o, win_start, win_len, n_ref_windows, n_tgt_windows, hop, fix_llh, fix_status, grid,
-                          T)))
+    if ((rc = window_check(e, fn, stations_llh, o, WinGeom{win_start, win_len, n_ref_windows, hop},
+                          WinGeom{win_start, win_len, n_tgt_windows, hop}, fix_llh, fix_status, grid, T)))
         return rc;
     if (!ref_in || !tgt_in) return fail(e, TDOA_E_INVALID, "%s: a table is NULL", fn);
     const int S = e->cfg.n_stations, P = S * (S - 1) / 2;
@@ -390,40 +419,57 @@ int window_fixes_impl(tdoa_engine *e, const char *fn, const double *stations_llh
     return finish_fix_stage(e, synced);
 }
 
+// retimed: tdoa_process_windows_retimed -- the TGT planes re-timed by the station rates fitted from the REF table;
+// clock_rate (may be NULL) receives those rates
 int process_windows_impl(tdoa_engine *e, const char *fn, const double *stations_llh, const tdoa_window_opts *o,
-                         int64_t win_start, int64_t win_len, int32_t n_ref_windows, int32_t n_tgt_windows, int64_t hop,
-                         tdoa_peak *ref_out, tdoa_peak *tgt_out, double *ref_fit, double *range_diffs, uint8_t *pair_used,
-                         double *fix_llh, double *fix_rms, int32_t *fix_status, int32_t *fix_iters, const GridSeed *grid)
+                         const WinGeom &ref, const WinGeom &tgt, tdoa_peak *ref_out, tdoa_peak *tgt_out, double *ref_fit,
+                         double *range_diffs, uint8_t *pair_used, double *fix_llh, double *fix_rms, int32_t *fix_status,
+                         int32_t *fix_iters, const GridSeed *grid, bool retimed, double *clock_rate)
 {
     if (!e) return TDOA_E_INVALID;
     int rc = begin_call(e);
     if (rc) return rc;
     WinTimes T;
-    if ((rc = window_check(e, fn, stations_llh, o, win_start, win_len, n_ref_windows, n_tgt_windows, hop, fix_llh, fix_status, grid,
-                          T)))
-        return rc;
+    if ((rc = window_check(e, fn, stations_llh, o, ref, tgt, fix_llh, fix_status, grid, T))) return rc;
     const int S = e->cfg.n_stations, P = S * (S - 1) / 2;
     Tables tab{e->stream};
-    CU(cudaMallocAsync(reinterpret_cast<void **>(&tab.ref), (size_t)n_ref_windows * P * sizeof(PeakRec), e->stream));
-    CU(cudaMallocAsync(reinterpret_cast<void **>(&tab.tgt), (size_t)n_tgt_windows * P * sizeof(PeakRec), e->stream));
-    const bool sharded = multi_wants(e, n_ref_windows + n_tgt_windows);
-    if (sharded) {   // the tables tdoa_xcorr_windows gathers, left on this rank's device
+    CU(cudaMallocAsync(reinterpret_cast<void **>(&tab.ref), (size_t)ref.n * P * sizeof(PeakRec), e->stream));
+    CU(cudaMallocAsync(reinterpret_cast<void **>(&tab.tgt), (size_t)tgt.n * P * sizeof(PeakRec), e->stream));
+    // the pair loop of one kind into its device table: dealt and gathered as tdoa_xcorr deals them, or on this GPU
+    bool sharded[2] = {false, false};
+    auto pass = [&](int kind, const double *d_rates) -> int {
+        const WinGeom &G = kind == TDOA_KIND_REF ? ref : tgt;
+        PeakRec *table = kind == TDOA_KIND_REF ? tab.ref : tab.tgt;
+        if ((sharded[kind] = multi_wants(e, G.n))) {
+            if (const int rc2 = begin_call(e)) return rc2;
+            ShardPart Q = T.parts[kind];
+            Q.out = reinterpret_cast<tdoa_peak *>(table); Q.out_is_device = true; Q.rates = d_rates;
+            return xcorr_sharded(e, std::vector<ShardPart>{Q});
+        }
+        return xcorr_impl(e, kind, G.start, G.len, G.n, G.hop, kind == TDOA_KIND_REF ? ref_out : tgt_out, false, table, d_rates);
+    };
+    if (retimed) {
+        // the TGT pass needs the rates, the rates need the gathered REF table: two meetings of the ranks
+        CU(cudaMallocAsync(reinterpret_cast<void **>(&tab.rates), (size_t)2 * S * sizeof(double), e->stream));
+        if ((rc = pass(TDOA_KIND_REF, nullptr)) || (rc = station_rates(e, o, T, tab.ref, tab.rates)) ||
+            (rc = pass(TDOA_KIND_TGT, tab.rates)))
+            return rc;
+    } else if (multi_wants(e, ref.n + tgt.n)) {   // the tables tdoa_xcorr_windows gathers, left on this rank's device
         T.parts[TDOA_KIND_REF].out = reinterpret_cast<tdoa_peak *>(tab.ref);
         T.parts[TDOA_KIND_TGT].out = reinterpret_cast<tdoa_peak *>(tab.tgt);
         for (ShardPart &Q : T.parts) Q.out_is_device = true;
         if ((rc = xcorr_sharded(e, T.parts))) return rc;
+        sharded[0] = sharded[1] = true;
     } else {         // tdoa_xcorr_windows on one GPU: the REF pair loop, then the TGT pair loop
-        if ((rc = xcorr_impl(e, TDOA_KIND_REF, win_start, win_len, n_ref_windows, hop, ref_out, false, tab.ref)) ||
-            (rc = xcorr_impl(e, TDOA_KIND_TGT, win_start, win_len, n_tgt_windows, hop, tgt_out, false, tab.tgt)))
-            return rc;
+        if ((rc = pass(TDOA_KIND_REF, nullptr)) || (rc = pass(TDOA_KIND_TGT, nullptr))) return rc;
     }
     if ((rc = begin_call(e))) return rc;
-    if (sharded) {
-        if (ref_out)
-            CU(cudaMemcpyAsync(ref_out, tab.ref, (size_t)n_ref_windows * P * sizeof(PeakRec), cudaMemcpyDeviceToHost, e->stream));
-        if (tgt_out)
-            CU(cudaMemcpyAsync(tgt_out, tab.tgt, (size_t)n_tgt_windows * P * sizeof(PeakRec), cudaMemcpyDeviceToHost, e->stream));
-    }
+    if (sharded[TDOA_KIND_REF] && ref_out)
+        CU(cudaMemcpyAsync(ref_out, tab.ref, (size_t)ref.n * P * sizeof(PeakRec), cudaMemcpyDeviceToHost, e->stream));
+    if (sharded[TDOA_KIND_TGT] && tgt_out)
+        CU(cudaMemcpyAsync(tgt_out, tab.tgt, (size_t)tgt.n * P * sizeof(PeakRec), cudaMemcpyDeviceToHost, e->stream));
+    if (retimed && clock_rate)
+        CU(cudaMemcpyAsync(clock_rate, tab.rates + S, (size_t)S * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
     bool synced = false;
     if ((rc = fix_stage(e, stations_llh, o, T, tab.ref, tab.tgt, ref_fit, range_diffs, pair_used, fix_llh, fix_rms, fix_status,
                         fix_iters, grid, &synced)))
@@ -461,9 +507,21 @@ int tdoa_process_windows(tdoa_engine *e, const double *stations_llh, const tdoa_
                          tdoa_peak *tgt_out, double *ref_fit, double *range_diffs, uint8_t *pair_used, double *fix_llh,
                          double *fix_rms, int32_t *fix_status, int32_t *fix_iters)
 {
-    return process_windows_impl(e, "tdoa_process_windows", stations_llh, o, win_start, win_len, n_ref_windows, n_tgt_windows,
-                                hop, ref_out, tgt_out, ref_fit, range_diffs, pair_used, fix_llh, fix_rms, fix_status, fix_iters,
-                                nullptr);
+    return process_windows_impl(e, "tdoa_process_windows", stations_llh, o, WinGeom{win_start, win_len, n_ref_windows, hop},
+                                WinGeom{win_start, win_len, n_tgt_windows, hop}, ref_out, tgt_out, ref_fit, range_diffs, pair_used,
+                                fix_llh, fix_rms, fix_status, fix_iters, nullptr, false, nullptr);
+}
+
+int tdoa_process_windows_retimed(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts *o, int64_t ref_win_start,
+                                 int64_t ref_win_len, int32_t n_ref_windows, int64_t ref_hop, int64_t tgt_win_start,
+                                 int64_t tgt_win_len, int32_t n_tgt_windows, int64_t tgt_hop, tdoa_peak *ref_out,
+                                 tdoa_peak *tgt_out, double *ref_fit, double *range_diffs, uint8_t *pair_used, double *fix_llh,
+                                 double *fix_rms, int32_t *fix_status, int32_t *fix_iters, double *clock_rate)
+{
+    return process_windows_impl(e, "tdoa_process_windows_retimed", stations_llh, o,
+                                WinGeom{ref_win_start, ref_win_len, n_ref_windows, ref_hop},
+                                WinGeom{tgt_win_start, tgt_win_len, n_tgt_windows, tgt_hop}, ref_out, tgt_out, ref_fit,
+                                range_diffs, pair_used, fix_llh, fix_rms, fix_status, fix_iters, nullptr, true, clock_rate);
 }
 
 int tdoa_process_windows_grid(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts *o, int64_t win_start,
@@ -473,9 +531,9 @@ int tdoa_process_windows_grid(tdoa_engine *e, const double *stations_llh, const 
                               double *seed_cost, int64_t *seed_index)
 {
     const GridSeed G{grid_desc, seed_llh, seed_cost, seed_index};
-    return process_windows_impl(e, "tdoa_process_windows_grid", stations_llh, o, win_start, win_len, n_ref_windows,
-                                n_tgt_windows, hop, ref_out, tgt_out, ref_fit, range_diffs, pair_used, fix_llh, fix_rms,
-                                fix_status, fix_iters, &G);
+    return process_windows_impl(e, "tdoa_process_windows_grid", stations_llh, o, WinGeom{win_start, win_len, n_ref_windows, hop},
+                                WinGeom{win_start, win_len, n_tgt_windows, hop}, ref_out, tgt_out, ref_fit, range_diffs, pair_used,
+                                fix_llh, fix_rms, fix_status, fix_iters, &G, false, nullptr);
 }
 
 }  // extern "C"
