@@ -4,8 +4,9 @@
                     (Python floats are IEEE doubles rounded to nearest, with no fused multiply-add);
   - delta, retime:  the re-timing index delta(n) = floor(c (n - n_c) + 0.5) and the gather of one plane (numpy
                     evaluates multiply and add as separate roundings, as k_retime does);
-  - window_record:  one TGT window of one pair as the engine computes it in EXTENDED mode: oracle.preprocess_binary,
-                    re-time, oracle.xcorr_two_sided, oracle.peak_parabolic.
+  - window_record:  one TGT window of one pair as the engine computes it: in EXTENDED mode (decimated or not)
+                    oracle.preprocess_binary_dec, re-time, oracle.xcorr_two_sided, oracle.peak_parabolic; in BINARY
+                    mode oracle.preprocess_binary, re-time, oracle.tdcorr_binary.
 The range differences and fixes are tests/window_oracle.py's, unchanged.  The product never imports this module."""
 from __future__ import annotations
 
@@ -73,23 +74,40 @@ def delta(c, length):
 
 
 def retime(x, c):
-    """x~[n] = x[n + delta(n)] where that index is on the plane, 0 elsewhere"""
+    """x~[n] = x[n + delta(n)] where that index is on the plane, 0 elsewhere.  The source index is formed in doubles,
+    as k_retime forms it, so a rate far beyond any clock's (|delta| past 2^63) still reads 0 rather than a wrapped
+    integer."""
     x = np.asarray(x)
-    s = np.arange(x.size, dtype=np.int64) + delta(c, x.size)
-    ok = (s >= 0) & (s < x.size)
+    n = np.arange(x.size, dtype=np.float64)
+    nc = float(x.size - 1) * 0.5
+    s = n + np.floor(np.float64(c) * (n - nc) + 0.5)
+    ok = (s >= 0.0) & (s < float(x.size))
     out = np.zeros_like(x)
-    out[ok] = x[s[ok]]
+    out[ok] = x[s[ok].astype(np.int64)]
     return out
 
 
-def window_record(sig_i, sig_j, c_i, c_j, max_lag, shift=0):
-    """(lag, frac, corr) of one TGT window of pair (i, j) in EXTENDED mode on re-timed planes.  sig_*: the two
-    stations' TGT samples of the window (complex, as oracle.extract_target gives them).  shift: an integer the
-    lag is known to be near -- plane j is moved by it before correlating over +-max_lag, so that a far lag needs
-    few lags (the engine's records always come from the full lag range; this is the same value when the peak
-    lies well inside both ranges)."""
-    yi = retime(oracle.preprocess_binary(sig_i)[0], c_i)
-    yj = retime(oracle.preprocess_binary(sig_j)[0], c_j)
+def window_record(sig_i, sig_j, c_i, c_j, max_lag, shift=0, mode="extended", D=1, block=10000, sanity=120):
+    """(lag, frac, corr) of one TGT window of pair (i, j) on re-timed planes.  sig_*: the two stations' TGT samples
+    of the window (complex, as oracle.extract_target gives them).
+
+    mode "extended", decimate D: oracle.preprocess_binary_dec, re-time in the decimated plane's own samples (its
+    centre is (n / D - 1) / 2), oracle.xcorr_two_sided over +-(max_lag // D) and oracle.peak_parabolic.  lag and
+    frac are in decimated samples (the engine reports D (lag + frac), rounded, in capture samples).  shift: an
+    integer the lag is known to be near -- plane j is moved by it before correlating, so that a far lag needs few
+    lags (the engine's records always come from the full lag range; this is the same value when the peak lies well
+    inside both ranges).
+    mode "binary": oracle.preprocess_binary, re-time the complex plane (both parts), oracle.tdcorr_binary with the
+    engine's max_lag, block and sanity; frac is 0."""
+    if mode == "binary":
+        yi = retime(oracle.preprocess_binary(sig_i)[0], c_i)
+        yj = retime(oracle.preprocess_binary(sig_j)[0], c_j)
+        lag, val, _ = oracle.tdcorr_binary(yi, yj, max_lag, block, sanity)
+        return lag, 0.0, val
+    assert mode == "extended", mode
+    yi = retime(oracle.preprocess_binary_dec(sig_i, D)[0], c_i)
+    yj = retime(oracle.preprocess_binary_dec(sig_j, D)[0], c_j)
+    max_lag //= D
     if shift:
         z = np.zeros_like(yj)
         if shift > 0:

@@ -31,11 +31,17 @@ def tgt_planes(raws):
     return [oracle.extract_target(oracle.unpack_u8(r)) for r in raws]
 
 
+def check_clock(out, S):
+    """clock_rate is the restatement's fit of the returned REF fits, bit for bit (NaN at the same stations)"""
+    _, clock = RO.station_rates(out["ref_fit"][:, 1], out["ref_fit"][:, 2], S)
+    got = np.asarray(out["clock_rate"], np.float64)
+    assert got.view(np.uint64).tolist() == clock.view(np.uint64).tolist(), (got, clock)
+
+
 def check_parity(out, raws, L, pair_ids):
     """TGT window 0 (the whole block) of the given pairs against the restatement re-timed by the returned rates"""
     S = len(raws)
-    rate, clock = RO.station_rates(out["ref_fit"][:, 1], out["ref_fit"][:, 2], S)
-    assert np.all(np.abs(out["clock_rate"] - clock) <= 1e-12 * np.abs(clock).max())
+    check_clock(out, S)
     tg = tgt_planes(raws)
     pp = RO.pairs(S)
     oracle.set_seq_dc_limit(0)
@@ -100,6 +106,7 @@ def test_without_drift_it_is_process_windows():
         want = e.process_windows(ST4, 0, W, nr, nt, W)
         got = e.process_windows_retimed(ST4, ref=(0, W, nr, W), tgt=(0, W, nt, W))
     assert got["ref"].tobytes() == ref_alone.tobytes()
+    check_clock(got, 4)
     # rates this small shift no sample of a W-sample plane: delta is 0 everywhere
     assert (np.abs(got["clock_rate"]) * W / 2 < 0.5).all()
     for k in want:
@@ -167,6 +174,8 @@ def test_whole_block_tgt_window_with_drift():
                                         init_llh=[ST4[:, 0].mean(), ST4[:, 1].mean(), TX[2]])
         plain = e.process_windows(ST4, 0, B4, 2, 1, B4)
     assert out["pair_used"].all()
+    check_clock(out, 4)
+    check_clock(geo, 4)
     td = out["range_differences"][0] * FS / C
     assert np.abs(td - truth).max() <= 1.0, td - truth
     c = out["clock_rate"] - out["clock_rate"].mean()
@@ -187,6 +196,8 @@ def test_weak_target_needs_the_long_window():
         load_all(e, raws)
         short = e.process_windows_retimed(ST4, ref=ref_geo, tgt=(0, W4, B4 // W4, W4))
         whole = e.process_windows_retimed(ST4, ref=ref_geo, tgt=(0, B4, 1, B4))
+    check_clock(short, 4)
+    check_clock(whole, 4)
     es = short["range_differences"] * FS / C - truth        # 8 windows x 6 pairs
     ew = whole["range_differences"][0] * FS / C - truth
     # every pair from the whole block within 1 sample
@@ -206,6 +217,7 @@ def multi_args():
 def same_results(want, got):
     """Everything bit for bit, but the tables' margin, which a dealt call may move by ~1e-7 (the runner-up lags are
     evaluated in other batches; see tests/test_gpu_window_grid.py)"""
+    check_clock(want, 4)
     for k in want:
         if k in ("ref", "tgt"):
             for f in want[k].dtype.names:

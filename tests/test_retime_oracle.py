@@ -67,6 +67,38 @@ def test_delta_at_change_points(c, length):
     assert (not ok[0] and not ok[-1]) == (c >= 1e-4)
 
 
+def test_extended_window_record_without_decimation_is_the_undecimated_chain():
+    """window_record in EXTENDED mode with D = 1 (preprocess_binary_dec) gives the bits of the chain without the
+    decimator: preprocess_binary, re-time, two-sided correlation, parabolic peak -- on odd and even lengths, both
+    signs of drift, with and without a shift"""
+    B = 200_000
+    eps = np.array([0.0, 40.0, -40.0, 25.0])
+    raws, _, _ = drift_captures(ST4, eps, block=B, seed=12)
+    tgt = [oracle.extract_target(oracle.unpack_u8(r)) for r in raws]
+    oracle.set_seq_dc_limit(0)
+    try:
+        for (i, j), (a, z), shift in (((0, 1), (0, B), 0), ((1, 2), (137, 100_138), 0), ((2, 3), (3, 150_002), 5)):
+            si, sj = tgt[i][a:z], tgt[j][a:z]
+            ci, cj = eps[i] * 1e-6, eps[j] * 1e-6
+            yi = RO.retime(oracle.preprocess_binary(si)[0], ci)
+            yj = RO.retime(oracle.preprocess_binary(sj)[0], cj)
+            if shift:
+                yj = np.concatenate([yj[shift:], np.zeros(shift, yj.dtype)])
+            idx, frac, val = oracle.peak_parabolic(oracle.xcorr_two_sided(yi, yj, 300))
+            assert RO.window_record(si, sj, ci, cj, 300, shift=shift) == (idx - 300 + shift, frac, val)
+            assert RO.window_record(si, sj, ci, cj, 300, shift=shift, mode="extended", D=1) == (idx - 300 + shift, frac, val)
+    finally:
+        oracle.set_seq_dc_limit(-1)
+
+
+def test_retime_forms_far_indices_in_doubles():
+    """a rate far beyond any clock's moves every sample off the plane but the centre one (odd lengths)"""
+    x = np.arange(1, 10, dtype=np.float32)
+    for c in (1e20, -1e20):
+        y = RO.retime(x, c)
+        assert y[4] == x[4] and (np.delete(y, 4) == 0).all()
+
+
 def test_retiming_whole_block_with_true_rates_puts_peaks_on_the_centre_lag():
     B = 4_000_000
     eps = np.array([0.0, 40.0, -40.0, 25.0])
