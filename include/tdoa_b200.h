@@ -338,6 +338,78 @@ TDOA_API int tdoa_window_fixes_grid(tdoa_engine *e, const double *stations_llh, 
                                     double *fix_llh, double *fix_rms, int32_t *fix_status, int32_t *fix_iters,
                                     double *seed_llh, double *seed_cost, int64_t *seed_index);
 
+/* ---- closure-checked windowed fixes (no reference equivalent; engine-defined).  A range difference is a
+ * difference of two station ranges, rd_ij = r_j - r_i, so the P pairs of a window hold only S - 1 independent
+ * numbers and every cycle of pairs closes (rd_ij + rd_jk - rd_ik = 0; the REF correction keeps this, clock offsets
+ * belong to stations).  One wrong TGT lag (a noise peak, an interferer, one of several equal peaks of periodic
+ * content) enters the fix at full weight; the check drops the pairs the rest of the window contradicts.
+ * Per set (one TGT window): rd[P] in metres, the usable mask u[P] in {0, 1} (pair_used of tdoa_process_windows),
+ * dims, max_residual (metres, > 0, may be +inf) and max_drop (>= 0, 0 = no limit).  m = u, 0 drops; then repeat:
+ *  1. Station values: on the graph of the pairs with m = 1, components labelled with their smallest station
+ *     index, tau[S] (metres) minimises sum (tau_j - tau_i - rd_ij)^2 over those pairs and sums to zero in each
+ *     component; a station with no pair is its own component and gets tau = 0.  Solved exactly as the station
+ *     rates of tdoa_process_windows_retimed, with rd in place of beta (b[i] -= rd, b[j] += rd in pair order; the
+ *     same Cholesky and solves, every f64 operation rounded to nearest, no contraction).
+ *  2. Residuals: e_p = rd_p - (tau_j - tau_i) (that rounding order) for every pair with u = 1, dropped ones
+ *     included; NaN for the others.
+ *  3. Stop if the redundancy of m (used pairs - stations they touch + components among those stations) is below
+ *     2 (a single cycle shows an inconsistency but cannot say which pair caused it), or max_drop > 0 and the
+ *     drops have reached max_drop, or q = the m-pair with the largest |e_p| (ties: the lowest p) has
+ *     |e_q| <= max_residual.
+ *  4. Tentative drop: m' = m without q; then, repeatedly, a station that lost a pair in this step and has exactly
+ *     one m'-pair left loses that pair too (a station seen through one pair cannot be checked).
+ *  5. If m' fails the least-squares step's status-2 rule (fewer than dims pairs, or pairs touching fewer than
+ *     dims + 1 stations), stop and keep m; else m = m', add the pairs removed to the drops and go to 1.
+ * Outputs: the final m (which the grid seed and the fix read in place of u), e from the last solve (the one on
+ * the final m) and the number of drops.  When nothing exceeds max_residual in the first pass, m = u and every
+ * output of the fix stage is, bit for bit, that of the call without the check: max_residual = INFINITY turns it
+ * off.  The check sees errors of single pairs only: an error common to all of one station's pairs is a station
+ * value, which tau absorbs.  A station that hears another programme, or only its own noise, in block 2 gives such
+ * an error (the peak of pair (i, s) moves with station i's own delay), so the check does not find that station.
+ * In BINARY mode lags are integers, so consistent pairs can already disagree by about 1 sample (150 m at
+ * 2 Msps); set max_residual above that. */
+typedef struct {
+    double max_residual;   /* metres; > 0, may be INFINITY                                     */
+    int32_t max_drop;      /* pairs per set; 0 = no limit                                      */
+    int32_t reserved;
+} tdoa_closure_opts;
+
+/* The check alone over host sets: range_diffs[set * rd_stride + p], used[...] in {0, 1} (an unused slot is never
+ * read); out_used[...] in {0, 1, 2} (2: usable but dropped), out_resid[...] (may be NULL), out_dropped[n_sets]
+ * (may be NULL).  Only the first P slots of each set are read or written.  Refused (TDOA_E_INVALID): a NULL
+ * range_diffs, used, out_used or c, S outside 3..64, dims not 2 or 3, n_sets < 0, rd_stride < P, max_residual
+ * NaN or <= 0, max_drop < 0. */
+TDOA_API int tdoa_closure(tdoa_engine *e, int32_t n_stations, const double *range_diffs, const uint8_t *used,
+                          int32_t n_sets, int32_t rd_stride, int32_t dims, const tdoa_closure_opts *c,
+                          uint8_t *out_used, double *out_resid, int32_t *out_dropped);
+/* One process call for every combination: REF and TGT window geometry as tdoa_process_windows_retimed; retimed 1
+ * re-times the TGT planes as that call does, 0 correlates them as tdoa_process_windows does (with two different
+ * geometries the tables are those tdoa_xcorr gives for each kind's geometry); grid_desc (may be NULL) seeds the
+ * fixes as tdoa_process_windows_grid.  The check runs on the device between the range differences and the grid
+ * seed / fix, in the same stream, with no other host synchronisation; on a multi-GPU engine every rank runs it on
+ * its own gathered tables and returns the same bits.  pair_used[n_tgt][P]: 0 not usable, 1 used by the fix, 2
+ * usable but dropped by the check.  closure_resid[n_tgt][P], n_dropped[n_tgt], clock_rate[S] (retimed 1 only),
+ * seed_llh, seed_cost and seed_index may be NULL.  ms_fix covers the check.  Refused (TDOA_E_INVALID): what the
+ * base calls refuse, a NULL c, max_residual NaN or <= 0, max_drop < 0, retimed not 0 or 1. */
+TDOA_API int tdoa_process_windows_closure(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts *o,
+                                          const tdoa_closure_opts *c, int64_t ref_win_start, int64_t ref_win_len,
+                                          int32_t n_ref_windows, int64_t ref_hop, int64_t tgt_win_start,
+                                          int64_t tgt_win_len, int32_t n_tgt_windows, int64_t tgt_hop, int32_t retimed,
+                                          const double *grid_desc, tdoa_peak *ref_out, tdoa_peak *tgt_out,
+                                          double *ref_fit, double *range_diffs, uint8_t *pair_used,
+                                          double *closure_resid, int32_t *n_dropped, double *fix_llh, double *fix_rms,
+                                          int32_t *fix_status, int32_t *fix_iters, double *clock_rate,
+                                          double *seed_llh, double *seed_cost, int64_t *seed_index);
+/* The same on host tables, as tdoa_window_fixes_grid (grid_desc may be NULL). */
+TDOA_API int tdoa_window_fixes_closure(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts *o,
+                                       const tdoa_closure_opts *c, int64_t win_start, int64_t win_len,
+                                       int32_t n_ref_windows, int32_t n_tgt_windows, int64_t hop,
+                                       const double *grid_desc, const tdoa_peak *ref_in, const tdoa_peak *tgt_in,
+                                       double *ref_fit, double *range_diffs, uint8_t *pair_used,
+                                       double *closure_resid, int32_t *n_dropped, double *fix_llh, double *fix_rms,
+                                       int32_t *fix_status, int32_t *fix_iters, double *seed_llh, double *seed_cost,
+                                       int64_t *seed_index);
+
 /* crossCorrelate seam (processor.go:619-643): two host complex64 slices
  * (interleaved re,im), returns (delay, correlation).  Empty input -> (0, 0.0). */
 TDOA_API int tdoa_cross_correlate(tdoa_engine *e, const float *sig1_c64, int64_t n1,

@@ -23,7 +23,7 @@ ERRORS = {-1: "TDOA_E_INVALID", -2: "TDOA_E_NODEVICE", -3: "TDOA_E_CUDA", -4: "T
 # every symbol include/tdoa_b200.h declares (tests check the library exports them all)
 ABI_SYMBOLS = [
     "tdoa_default_config", "tdoa_create", "tdoa_destroy", "tdoa_last_error", "tdoa_host_alloc", "tdoa_host_free",
-    "tdoa_load_u8", "tdoa_load_file", "tdoa_load_u8_pinned", "tdoa_load_u8_device", "tdoa_unpack", "tdoa_preprocess", "tdoa_xcorr", "tdoa_xcorr_device", "tdoa_xcorr_windows", "tdoa_process", "tdoa_process_windows", "tdoa_window_fixes", "tdoa_process_windows_grid", "tdoa_window_fixes_grid", "tdoa_process_windows_retimed", "tdoa_xcorr_info", "tdoa_analyze",
+    "tdoa_load_u8", "tdoa_load_file", "tdoa_load_u8_pinned", "tdoa_load_u8_device", "tdoa_unpack", "tdoa_preprocess", "tdoa_xcorr", "tdoa_xcorr_device", "tdoa_xcorr_windows", "tdoa_process", "tdoa_process_windows", "tdoa_window_fixes", "tdoa_process_windows_grid", "tdoa_window_fixes_grid", "tdoa_process_windows_retimed", "tdoa_closure", "tdoa_process_windows_closure", "tdoa_window_fixes_closure", "tdoa_xcorr_info", "tdoa_analyze",
     "tdoa_cross_correlate", "tdoa_baselines", "tdoa_solve", "tdoa_solve_binary", "tdoa_solve_ls", "tdoa_grid", "tdoa_grid_masked", "tdoa_get_stats", "tdoa_stream",
     "tdoa_set_stream", "tdoa_synchronize", "tdoa_selftest",
     "tdoa_comm_unique_id", "tdoa_comm_init", "tdoa_comm_rank", "tdoa_shard_windows",
@@ -78,6 +78,19 @@ class WindowOpts(C.Structure):
     _fields_ = [("dims", C.c_int32), ("min_margin", C.c_float), ("ref_max_residual", C.c_double),
                 ("has_ref_tx", C.c_int32), ("has_init", C.c_int32), ("ref_tx_llh", C.c_double * 3),
                 ("init_llh", C.c_double * 3)]
+
+
+class ClosureOpts(C.Structure):
+    _fields_ = [("max_residual", C.c_double), ("max_drop", C.c_int32), ("reserved", C.c_int32)]
+
+
+def _closure_opts(closure) -> ClosureOpts:
+    """closure = dict(max_residual=metres, max_drop=0); None: the inert check (max_residual = inf)"""
+    c = dict(closure or {"max_residual": float("inf")})
+    unknown = set(c) - {"max_residual", "max_drop"}
+    if unknown or "max_residual" not in c:
+        raise ValueError(f"closure takes max_residual and max_drop, got {sorted(c)}")
+    return ClosureOpts(max_residual=float(c["max_residual"]), max_drop=int(c.get("max_drop", 0)))
 
 
 class Stats(C.Structure):
@@ -155,6 +168,10 @@ def load_library():
     L.tdoa_process_windows_grid.argtypes = [vp, vp, C.POINTER(WindowOpts), i64, i64, i32, i32, i64] + [vp] * 13
     L.tdoa_window_fixes_grid.argtypes = [vp, vp, C.POINTER(WindowOpts), i64, i64, i32, i32, i64] + [vp] * 13
     L.tdoa_process_windows_retimed.argtypes = [vp, vp, C.POINTER(WindowOpts), i64, i64, i32, i64, i64, i64, i32, i64] + [vp] * 10
+    L.tdoa_closure.argtypes = [vp, i32, vp, vp, i32, i32, i32, C.POINTER(ClosureOpts), vp, vp, vp]
+    L.tdoa_process_windows_closure.argtypes = ([vp, vp, C.POINTER(WindowOpts), C.POINTER(ClosureOpts), i64, i64, i32, i64, i64,
+                                                i64, i32, i64, i32] + [vp] * 16)
+    L.tdoa_window_fixes_closure.argtypes = [vp, vp, C.POINTER(WindowOpts), C.POINTER(ClosureOpts), i64, i64, i32, i32, i64] + [vp] * 15
     L.tdoa_cross_correlate.argtypes = [vp, vp, i64, vp, i64, C.POINTER(PeakStruct)]
     L.tdoa_baselines.argtypes = [vp, vp, i32, vp]
     L.tdoa_solve.argtypes = [vp, vp, i32, vp, i32, i32, vp, vp, vp]
@@ -492,16 +509,66 @@ class Engine:
                 "rms": rms, "status": status, "iters": iters, "seed": seed, "seed_cost": seed_cost,
                 "seed_index": seed_index}
 
+    def _closure_windows(self, fn, stations_llh, geometry, tables, retimed, dims, min_margin, ref_max_residual,
+                         ref_tx_llh, init_llh, grid, closure) -> dict:
+        """tdoa_process_windows_closure (tables None: the call fills them) or tdoa_window_fixes_closure (tables =
+        (ref, tgt) host inputs)"""
+        st, o = self._window_opts(stations_llh, dims, min_margin, ref_max_residual, ref_tx_llh, init_llh)
+        c = _closure_opts(closure)
+        P = self.n_pairs
+        (r0, rl, nr, rh), (t0, tl, nt, th) = geometry
+        nt_ = max(nt, 0)
+        ref_fit, rd = np.zeros((P, 3), np.float64), np.zeros((nt_, P), np.float64)
+        used, resid, dropped = np.zeros((nt_, P), np.uint8), np.zeros((nt_, P), np.float64), np.zeros(nt_, np.int32)
+        fix, rms = np.zeros((nt_, 3), np.float64), np.zeros(nt_, np.float64)
+        status, iters = np.zeros(nt_, np.int32), np.zeros(nt_, np.int32)
+        gd = None
+        if grid is not None:
+            gd = np.ascontiguousarray(grid, dtype=np.float64).reshape(-1)
+            if gd.size != 7:
+                raise ValueError(f"grid must be 7 numbers (lat0, lon0, dlat, dlon, nlat, nlon, elev), got {gd.size}")
+        seed, seed_cost, seed_index = np.zeros((nt_, 3), np.float64), np.zeros(nt_, np.float64), np.zeros(nt_, np.int64)
+        outs = [_ptr(ref_fit), _ptr(rd), _ptr(used), _ptr(resid), _ptr(dropped), _ptr(fix), _ptr(rms), _ptr(status),
+                _ptr(iters)]
+        seeds = [_ptr(seed), _ptr(seed_cost), _ptr(seed_index)]
+        out = {}
+        if tables is None:
+            ref_t, tgt_t = np.zeros((max(nr, 0), P), PEAK_DTYPE), np.zeros((nt_, P), PEAK_DTYPE)
+            rate = np.zeros(self.n_stations, np.float64)
+            self._check(fn(self._h, _ptr(st), C.byref(o), C.byref(c), r0, rl, nr, rh, t0, tl, nt, th, int(retimed),
+                           None if gd is None else _ptr(gd), _ptr(ref_t), _ptr(tgt_t), *outs, _ptr(rate), *seeds))
+            out.update(ref=ref_t, tgt=tgt_t)
+            if retimed:
+                out["clock_rate"] = rate
+        else:
+            self._check(fn(self._h, _ptr(st), C.byref(o), C.byref(c), r0, rl, nr, nt, rh, None if gd is None else _ptr(gd),
+                           *[_ptr(t) for t in tables], *outs, *seeds))
+        out.update({"ref_fit": ref_fit, "range_differences": rd, "pair_used": used == 1, "pair_dropped": used == 2,
+                    "closure_residual": resid, "dropped": dropped, "position": fix, "rms": rms, "status": status,
+                    "iters": iters})
+        if gd is not None:
+            out.update(seed=seed, seed_cost=seed_cost, seed_index=seed_index)
+        return out
+
     def process_windows(self, stations_llh, win_start: int, win_len: int, n_ref_windows: int, n_tgt_windows: int,
                         hop: int, dims: int = 2, min_margin: float = 0.0, ref_max_residual: float = 0.0,
-                        ref_tx_llh=None, init_llh=None, grid=None) -> dict:
+                        ref_tx_llh=None, init_llh=None, grid=None, closure=None) -> dict:
         """Windowed ProcessTDOA (tdoa_process_windows): REF and TGT tables as xcorr_windows gives them, the REF
         lag's linear track per pair (ref_fit: lag at block 2's centre, drift in samples per sample, windows
         used), range differences and the used mask per (TGT window, pair), one least-squares fix per TGT window
         (status 0 ok, 1 degenerate, 2 too few measurements).  ref_tx_llh: the REF transmitter's position, whose
         geometric range difference is added back.  grid = (lat0, lon0, dlat, dlon, nlat, nlon, elev): each window's
         fix starts from the masked grid arg-min of its used pairs (tdoa_process_windows_grid); the result gains
-        seed (the start cell), seed_cost and seed_index (-1 and NaN for a window with status 2)."""
+        seed (the start cell), seed_cost and seed_index (-1 and NaN for a window with status 2).
+        closure = dict(max_residual=metres, max_drop=0): each window's usable pairs are checked against each other
+        first and the pairs the rest contradict are dropped (tdoa_process_windows_closure, statement in
+        include/tdoa_b200.h); the result gains pair_dropped (usable but dropped), closure_residual (NaN where not
+        usable) and dropped (pairs per window), and pair_used is the mask the fix read."""
+        if closure is not None:
+            g = (int(win_start), int(win_len), int(n_ref_windows), int(hop))
+            return self._closure_windows(self._lib.tdoa_process_windows_closure, stations_llh,
+                                         (g, (g[0], g[1], int(n_tgt_windows), g[3])), None, 0, dims, min_margin,
+                                         ref_max_residual, ref_tx_llh, init_llh, grid, closure)
         ref = np.zeros((max(n_ref_windows, 0), self.n_pairs), PEAK_DTYPE)
         tgt = np.zeros((max(n_tgt_windows, 0), self.n_pairs), PEAK_DTYPE)
         fn = self._lib.tdoa_process_windows if grid is None else self._lib.tdoa_process_windows_grid
@@ -511,13 +578,19 @@ class Engine:
         return out
 
     def process_windows_retimed(self, stations_llh, ref, tgt, dims: int = 2, min_margin: float = 0.0,
-                                ref_max_residual: float = 0.0, ref_tx_llh=None, init_llh=None) -> dict:
+                                ref_max_residual: float = 0.0, ref_tx_llh=None, init_llh=None, grid=None,
+                                closure=None) -> dict:
         """Re-timed target correlation (tdoa_process_windows_retimed): ref = (start, len, n, hop) and tgt = (start,
         len, n, hop) are the two kinds' window geometries.  The REF windows give each pair's drift line as in
         process_windows; the station clock rates fitted from those slopes re-time every TGT plane, so a TGT window
         may span the whole block without smearing its peak.  Returns process_windows' dict plus clock_rate[S]
-        (samples per sample; NaN for a station without a fitted pair)."""
+        (samples per sample; NaN for a station without a fitted pair).  grid and closure as process_windows (through
+        tdoa_process_windows_closure; without closure the check is inert)."""
         (r0, rl, nr, rh), (t0, tl, nt, th) = (tuple(int(v) for v in g) for g in (ref, tgt))
+        if grid is not None or closure is not None:
+            return self._closure_windows(self._lib.tdoa_process_windows_closure, stations_llh,
+                                         ((r0, rl, nr, rh), (t0, tl, nt, th)), None, 1, dims, min_margin,
+                                         ref_max_residual, ref_tx_llh, init_llh, grid, closure)
         st, o = self._window_opts(stations_llh, dims, min_margin, ref_max_residual, ref_tx_llh, init_llh)
         P, nt_ = self.n_pairs, max(nt, 0)
         ref_t, tgt_t = np.zeros((max(nr, 0), P), PEAK_DTYPE), np.zeros((nt_, P), PEAK_DTYPE)
@@ -534,15 +607,37 @@ class Engine:
 
     def window_fixes(self, stations_llh, win_start: int, win_len: int, ref, tgt, hop: int, dims: int = 2,
                      min_margin: float = 0.0, ref_max_residual: float = 0.0, ref_tx_llh=None, init_llh=None,
-                     grid=None) -> dict:
+                     grid=None, closure=None) -> dict:
         """The fix stage of process_windows on given tables (tdoa_window_fixes): ref[n_ref][P], tgt[n_tgt][P] of
         PEAK_DTYPE, e.g. kept from xcorr_windows; window times come from the captures the engine holds.  grid: as
-        process_windows (tdoa_window_fixes_grid)."""
+        process_windows (tdoa_window_fixes_grid); closure: as process_windows (tdoa_window_fixes_closure)."""
         ref = np.ascontiguousarray(ref, PEAK_DTYPE).reshape(-1, self.n_pairs)
         tgt = np.ascontiguousarray(tgt, PEAK_DTYPE).reshape(-1, self.n_pairs)
+        if closure is not None:
+            g = (int(win_start), int(win_len), ref.shape[0], int(hop))
+            return self._closure_windows(self._lib.tdoa_window_fixes_closure, stations_llh,
+                                         (g, (g[0], g[1], tgt.shape[0], g[3])), (ref, tgt), 0, dims, min_margin,
+                                         ref_max_residual, ref_tx_llh, init_llh, grid, closure)
         fn = self._lib.tdoa_window_fixes if grid is None else self._lib.tdoa_window_fixes_grid
         return self._windows(fn, stations_llh, win_start, win_len, ref.shape[0], tgt.shape[0], hop, (ref, tgt), dims,
                              min_margin, ref_max_residual, ref_tx_llh, init_llh, grid)
+
+    def closure(self, n_stations: int, range_diffs, used, dims: int = 2, *, max_residual: float, max_drop: int = 0):
+        """The closure check alone (tdoa_closure) over sets range_diffs[n_sets][>= P], used[n_sets][>= P] (an unused
+        slot is never read).  Returns (used in {0, 1, 2} with 2 = dropped, residuals (NaN where not usable), dropped
+        pairs per set); one set when range_diffs is 1-D."""
+        rd = np.ascontiguousarray(range_diffs, dtype=np.float64)
+        single = rd.ndim == 1
+        rd = rd.reshape(1, -1) if single else rd
+        n, stride = rd.shape
+        u = np.ascontiguousarray(np.asarray(used).astype(np.uint8).reshape(n, stride))
+        c = _closure_opts({"max_residual": max_residual, "max_drop": max_drop})
+        out, resid, dropped = np.zeros((n, stride), np.uint8), np.full((n, stride), np.nan), np.zeros(n, np.int32)
+        self._check(self._lib.tdoa_closure(self._h, n_stations, _ptr(rd), _ptr(u), n, stride, dims, C.byref(c), _ptr(out),
+                                           _ptr(resid), _ptr(dropped)))
+        if single:
+            return out[0], resid[0], int(dropped[0])
+        return out, resid, dropped
 
     def solve_ls(self, stations_llh, range_diffs, init_llh=None, dims: int = 2):
         """Levenberg-Marquardt fix over all pair range differences (engine-defined, SURVEY 8f-4).

@@ -190,6 +190,11 @@ constexpr int kWindowFitDoubles = 5;   // per pair: a, beta, t_mean, windows use
 // rate[S] (0 for a station without a fitted pair) re-times the planes, clock[S] (NaN there) is what the call returns;
 // n_st <= 64 (solve_ls_max_stations)
 void launch_station_rates(const double *d_fit, int n_st, double *d_rate, double *d_clock, cudaStream_t st);
+// the closure check of the windowed fixes (tdoa_closure), one CTA per set, n_st <= 64: d_used[set * stride + p] in u
+// (0 / 1), out 0 / 1 / 2 (2: dropped); d_mask (may be nullptr) the final 0 / 1 mask; d_resid (may be nullptr) the
+// residuals, NaN where u = 0; d_dropped (may be nullptr) the pairs dropped per set
+void launch_window_closure(const double *d_rd, uint8_t *d_used, uint8_t *d_mask, int n_sets, int stride, int n_st, int dims,
+                           double max_resid, int max_drop, double *d_resid, int *d_dropped, cudaStream_t st);
 struct RetimeJob {
     const float *x;   // one preprocessed plane, n samples
     float *y;         // its re-timed plane (16-byte aligned)

@@ -10,19 +10,25 @@
 //                    function that changes at most once per 1/|c| samples, so a tile evaluates the f64 formula at
 //                    its two ends and at its few change points only (a binary search each), stages the source run
 //                    it needs in shared memory with 16-byte loads and writes 16-byte stores.
-// Both follow the statement operation for operation (__dmul_rn / __dadd_rn / __dsub_rn / __ddiv_rn / __dsqrt_rn:
+//   k_window_closure one CTA per TGT window (the _closure windowed calls, tdoa_closure): the same solve with the
+//                    window's range differences in place of the slopes, and the drop of the pairs the rest of the
+//                    window contradicts (statement in include/tdoa_b200.h, tdoa_closure; tests/closure_oracle.py)
+// All three follow the statement operation for operation (__dmul_rn / __dadd_rn / __dsub_rn / __ddiv_rn / __dsqrt_rn:
 // no contraction), so the restatement reproduces the bits.
 #include <cuda_runtime.h>
 
 #include <cstdint>
 
+#include "graph_ls.cuh"
 #include "kernels.h"
 
 namespace tdoa {
 
 namespace {
 
-constexpr int kRatesMaxStations = 64;
+constexpr int kRatesMaxStations = kGraphLsMaxStations;
+constexpr int kClosureThreads = 64;
+constexpr int kClosureMaxPairs = kGraphLsMaxStations * (kGraphLsMaxStations - 1) / 2;
 constexpr int kRetimeTile = 4096;      // output samples per CTA
 constexpr int kRetimeThreads = 256;
 constexpr int kRetimeMaxSteps = 32;    // change points a tile takes on the staged path
@@ -31,65 +37,120 @@ constexpr int kRetimeLoads = (kRetimeTile + kRetimeMaxSteps + 8) / 4 / kRetimeTh
 __global__ void __launch_bounds__(kRatesMaxStations) k_station_rates(const double *__restrict__ fit, int n_st,
                                                                      double *__restrict__ rate, double *__restrict__ clock)
 {
-    __shared__ double A[kRatesMaxStations][kRatesMaxStations + 1];
+    __shared__ GraphLsMatrix A[kRatesMaxStations];
     __shared__ double b[kRatesMaxStations];
-    __shared__ int comp[kRatesMaxStations], fitted[kRatesMaxStations];
+    __shared__ int comp[kRatesMaxStations], deg[kRatesMaxStations];
     const int t = threadIdx.x, S = n_st;
-    if (t == 0) {
-        // components of the fitted-pair graph: every station ends labelled with the smallest index of its component
-        for (int k = 0; k < S; k++) { comp[k] = k; fitted[k] = 0; }
-        for (bool changed = true; changed;) {
-            changed = false;
-            for (int i = 0, p = 0; i < S; i++)
-                for (int j = i + 1; j < S; j++, p++) {
-                    if (!(fit[(size_t)kWindowFitDoubles * p + 3] >= 2.0)) continue;
-                    const int m = min(comp[i], comp[j]);
-                    if (comp[i] != m || comp[j] != m) { comp[i] = comp[j] = m; changed = true; }
-                }
-        }
-        // normal equations of the fitted pairs, plus one all-ones block per component (the zero-sum gauge)
-        for (int i = 0; i < S; i++) {
-            b[i] = 0.0;
-            for (int j = 0; j < S; j++) A[i][j] = comp[i] == comp[j] ? 1.0 : 0.0;
-        }
-        for (int i = 0, p = 0; i < S; i++)
-            for (int j = i + 1; j < S; j++, p++) {
-                const double *f = fit + (size_t)kWindowFitDoubles * p;
-                if (!(f[3] >= 2.0)) continue;
-                A[i][i] += 1.0; A[j][j] += 1.0; A[i][j] -= 1.0; A[j][i] -= 1.0;
-                b[i] = __dsub_rn(b[i], f[1]);
-                b[j] = __dadd_rn(b[j], f[1]);
-                fitted[i] = fitted[j] = 1;
-            }
-    }
-    __syncthreads();
-    // Cholesky, right-looking, row t on thread t: A[i][j] -= L[i][k] L[j][k] in k order
-    for (int k = 0; k < S; k++) {
-        if (t == k) A[k][k] = __dsqrt_rn(A[k][k]);
-        __syncthreads();
-        if (t > k && t < S) A[t][k] = __ddiv_rn(A[t][k], A[k][k]);
-        __syncthreads();
-        if (t > k && t < S)
-            for (int j = k + 1; j <= t; j++) A[t][j] = __dsub_rn(A[t][j], __dmul_rn(A[t][k], A[j][k]));
-        __syncthreads();
-    }
-    // L y = b, then L^T c = y, both column by column (b holds y, then c)
-    for (int k = 0; k < S; k++) {
-        if (t == k) b[k] = __ddiv_rn(b[k], A[k][k]);
-        __syncthreads();
-        if (t > k && t < S) b[t] = __dsub_rn(b[t], __dmul_rn(A[t][k], b[k]));
-        __syncthreads();
-    }
-    for (int k = S - 1; k >= 0; k--) {
-        if (t == k) b[k] = __ddiv_rn(b[k], A[k][k]);
-        __syncthreads();
-        if (t < k) b[t] = __dsub_rn(b[t], __dmul_rn(A[k][t], b[k]));
-        __syncthreads();
-    }
+    auto fitted = [&](int p) { return fit[(size_t)kWindowFitDoubles * p + 3] >= 2.0; };
+    auto slope = [&](int p) { return fit[(size_t)kWindowFitDoubles * p + 1]; };
+    graph_components(S, t, comp, fitted);
+    graph_normal(S, t, comp, A, b, deg, fitted, slope);
+    graph_ls_solve(S, t, A, b);
     if (t < S) {
         rate[t] = b[t];   // exactly 0 for a station without a fitted pair
-        clock[t] = fitted[t] ? b[t] : __longlong_as_double(0x7ff8000000000000ll);
+        clock[t] = deg[t] ? b[t] : __longlong_as_double(0x7ff8000000000000ll);
     }
+}
+
+// One TGT window per CTA (include/tdoa_b200.h, tdoa_closure): station ranges tau from the window's used range
+// differences, the residual of every usable pair, and the drop of the pair with the largest |residual| (with the
+// pairs the degree rule takes after it) while that residual exceeds max_resid.  Each drop solves again from scratch,
+// so every solve is the stated one.  used[P] in: the usable mask u (0 / 1); out: 0, 1 used, 2 dropped.  mask[P]
+// (may be nullptr): the final 0 / 1 mask the fix reads.  resid[P] (may be nullptr): NaN where u = 0.
+__global__ void __launch_bounds__(kClosureThreads) k_window_closure(const double *__restrict__ rd_all, uint8_t *used_all,
+                                                                    uint8_t *mask_all, int n_st, int stride, int dims,
+                                                                    double max_resid, int max_drop, double *resid_all,
+                                                                    int *dropped)
+{
+    __shared__ GraphLsMatrix A[kGraphLsMaxStations];
+    __shared__ double b[kGraphLsMaxStations];
+    __shared__ int comp[kGraphLsMaxStations], deg[kGraphLsMaxStations];
+    __shared__ uint8_t u[kClosureMaxPairs], m[kClosureMaxPairs], cut[kClosureMaxPairs];
+    __shared__ uint8_t pi[kClosureMaxPairs], pj[kClosureMaxPairs];
+    __shared__ double best_v[kClosureThreads / 32];
+    __shared__ int best_p[kClosureThreads / 32];
+    __shared__ int s_drops, s_go, s_keep;
+    const int t = threadIdx.x, S = n_st, P = S * (S - 1) / 2;
+    const double *rd = rd_all + (size_t)blockIdx.x * stride;
+    uint8_t *used = used_all + (size_t)blockIdx.x * stride;
+    double *resid = resid_all ? resid_all + (size_t)blockIdx.x * stride : nullptr;
+    for (int i = 0, p = 0; i < S; i++)
+        for (int j = i + 1; j < S; j++, p++)
+            if (p % kClosureThreads == t) { pi[p] = (uint8_t)i; pj[p] = (uint8_t)j; }
+    for (int p = t; p < P; p += kClosureThreads) { u[p] = m[p] = used[p] != 0; cut[p] = 0; }
+    if (t == 0) s_drops = 0;
+    __syncthreads();
+    auto in_m = [&](int p) { return m[p] != 0; };
+    auto rd_of = [&](int p) { return rd[p]; };
+    for (;;) {
+        graph_components(S, t, comp, in_m);
+        graph_normal(S, t, comp, A, b, deg, in_m, rd_of);
+        graph_ls_solve(S, t, A, b);
+        // residuals of the usable pairs; the m-pair with the largest |e| (ties: the lowest p)
+        double bv = -1.0;
+        int bp = -1;
+        for (int p = t; p < P; p += kClosureThreads) {
+            double e = __longlong_as_double(0x7ff8000000000000ll);
+            if (u[p]) {
+                e = __dsub_rn(rd[p], __dsub_rn(b[pj[p]], b[pi[p]]));
+                if (m[p] && fabs(e) > bv) { bv = fabs(e); bp = p; }
+            }
+            if (resid) resid[p] = e;
+        }
+        for (int off = 16; off > 0; off >>= 1) {
+            const double ov = __shfl_down_sync(0xffffffffu, bv, off);
+            const int op = __shfl_down_sync(0xffffffffu, bp, off);
+            if (op >= 0 && (ov > bv || (ov == bv && op < bp))) { bv = ov; bp = op; }
+        }
+        if ((t & 31) == 0) { best_v[t >> 5] = bv; best_p[t >> 5] = bp; }
+        __syncthreads();
+        if (t == 0) {
+            for (int w = 1; w < kClosureThreads / 32; w++)
+                if (best_p[w] >= 0 && (best_v[w] > bv || (best_v[w] == bv && best_p[w] < bp))) { bv = best_v[w]; bp = best_p[w]; }
+            // redundancy = used pairs - stations they touch + components among those stations
+            int n2 = 0, touched = 0, comps = 0;
+            for (int s = 0; s < S; s++) {
+                n2 += deg[s];
+                touched += deg[s] > 0;
+                comps += deg[s] > 0 && comp[s] == s;
+            }
+            bool go = n2 / 2 - touched + comps >= 2 && !(max_drop > 0 && s_drops >= max_drop) && bp >= 0 && bv > max_resid;
+            s_keep = 1;
+            if (go) {
+                // the tentative drop: q, then every station that lost a pair here and has one pair left loses it too
+                unsigned long long lost = 0ull;
+                int n_cut = 0;
+                for (int q = bp; q >= 0;) {
+                    const int i = pi[q], j = pj[q];
+                    m[q] = 0; cut[q] = 1; n_cut++;
+                    deg[i]--; deg[j]--;
+                    lost |= (1ull << i) | (1ull << j);
+                    q = -1;
+                    for (int s = 0; s < S && q < 0; s++) {
+                        if (!((lost >> s) & 1ull) || deg[s] != 1) continue;
+                        for (int k = 0; k < S && q < 0; k++)
+                            if (k != s && m[graph_pair(min(s, k), max(s, k), S)]) q = graph_pair(min(s, k), max(s, k), S);
+                    }
+                }
+                if (ls_used_pairs(m, S, dims) < 0) { go = false; s_keep = 0; }
+                else s_drops += n_cut;
+            }
+            s_go = go;
+        }
+        __syncthreads();
+        const bool go = s_go, keep = s_keep;
+        for (int p = t; p < P; p += kClosureThreads) {
+            if (cut[p] && !keep) m[p] = 1;
+            cut[p] = 0;
+        }
+        __syncthreads();
+        if (!go) break;
+    }
+    for (int p = t; p < P; p += kClosureThreads) {
+        if (mask_all) mask_all[(size_t)blockIdx.x * stride + p] = m[p];
+        used[p] = u[p] ? (m[p] ? 1 : 2) : 0;
+    }
+    if (t == 0 && dropped) dropped[blockIdx.x] = s_drops;
 }
 
 // delta(n) = floor(c (n - n_c) + 0.5); n - n_c is exact (n < 2^52, n_c a multiple of 1/2)
@@ -181,6 +242,14 @@ __global__ void __launch_bounds__(kRetimeThreads) k_retime(const RetimeJob *__re
 void launch_station_rates(const double *d_fit, int n_st, double *d_rate, double *d_clock, cudaStream_t st)
 {
     k_station_rates<<<1, kRatesMaxStations, 0, st>>>(d_fit, n_st, d_rate, d_clock);
+}
+
+void launch_window_closure(const double *d_rd, uint8_t *d_used, uint8_t *d_mask, int n_sets, int stride, int n_st, int dims,
+                           double max_resid, int max_drop, double *d_resid, int *d_dropped, cudaStream_t st)
+{
+    if (n_sets > 0)
+        k_window_closure<<<n_sets, kClosureThreads, 0, st>>>(d_rd, d_used, d_mask, n_st, stride, dims, max_resid, max_drop,
+                                                           d_resid, d_dropped);
 }
 
 void launch_retime(const RetimeJob *d_jobs, int n_jobs, i64 max_n, const double *d_rates, cudaStream_t st)

@@ -9,6 +9,7 @@
 #include <type_traits>
 
 #include "geodesy.cuh"
+#include "graph_ls.cuh"
 #include "kernels.h"
 
 namespace tdoa {
@@ -237,23 +238,6 @@ __device__ bool ls_step(const double (&A)[3][3], const double (&b)[3], double la
 }
 
 constexpr int kLsMaxStations = 64;
-
-// The status-2 rule of a masked fix (k_solve_ls) and of the grid seed (k_grid_rows): the number of used pairs, or -1
-// when there are fewer than `dims` of them or they touch fewer than dims + 1 stations (dims = 0: no used pair).
-__host__ __device__ __forceinline__ int ls_used_pairs(const uint8_t *used, int n_st, int dims)
-{
-    int n_used = 0, q = 0;
-    unsigned long long touched = 0ull;
-    for (int i = 0; i < n_st; i++)
-        for (int j = i + 1; j < n_st; j++, q++)
-            if (used[q]) { n_used++; touched |= (1ull << i) | (1ull << j); }
-#ifdef __CUDA_ARCH__
-    const int n_touched = __popcll(touched);
-#else
-    const int n_touched = __builtin_popcountll(touched);
-#endif
-    return (n_used < dims || n_touched < dims + 1) ? -1 : n_used;
-}
 
 __global__ void k_solve_ls(const double *llh, int n_st, const double *rd_all, int n_sets, int rd_stride,
                            const double *init_llh, int dims, double *out_llh, double *out_rms, int *status, int *iters,

@@ -19,6 +19,9 @@
 //                     start point, which holds the start the window has without a grid; k_solve_ls starts there.
 // The ranked pass is optimistic: when the grid search finds it incomplete after the call's one synchronisation, the
 // call reruns the grid on every cell (k_grid_cost) and the fixes before it returns.
+// The _closure calls check each window's range differences against each other first (retime.cu):
+//   k_window_closure  one CTA per TGT window: drops the pairs the window's other pairs contradict, into a separate
+//                     0 / 1 mask that k_grid_rows and k_solve_ls read in place of the used mask.
 // tdoa_process_windows_retimed runs the REF pair loop, k_window_ref_fit and k_station_rates (retime.cu) before the TGT
 // pair loop, which re-times every plane by its station's rate; the fix stage is the same.
 // Window times and the usable test are stated in include/tdoa_b200.h (tdoa_process_windows).
@@ -29,6 +32,7 @@
 
 #include "engine_internal.h"
 #include "geodesy.cuh"
+#include "graph_ls.cuh"
 
 using namespace tdoa;
 
@@ -199,9 +203,25 @@ struct GridSeed {
     int64_t *index = nullptr;
 };
 
+// the closure check of the _closure calls: options and optional outputs
+struct Closure {
+    const tdoa_closure_opts *opts = nullptr;   // nullptr: no check
+    double *resid = nullptr;
+    int32_t *dropped = nullptr;
+};
+
+int closure_opts_check(tdoa_engine *e, const char *fn, const tdoa_closure_opts *c)
+{
+    if (!c) return fail(e, TDOA_E_INVALID, "%s: closure options are NULL", fn);
+    if (!(c->max_residual > 0.0)) return fail(e, TDOA_E_INVALID, "%s: max_residual must be > 0, got %g", fn, c->max_residual);
+    if (c->max_drop < 0) return fail(e, TDOA_E_INVALID, "%s: max_drop must be >= 0, got %d", fn, c->max_drop);
+    return TDOA_OK;
+}
+
 // grid: the seed of the _grid calls, nullptr without
 int window_check(tdoa_engine *e, const char *fn, const double *stations_llh, const tdoa_window_opts *o, const WinGeom &ref,
-                 const WinGeom &tgt, const double *fix_llh, const int32_t *fix_status, const GridSeed *grid, WinTimes &T)
+                 const WinGeom &tgt, const double *fix_llh, const int32_t *fix_status, const GridSeed *grid, WinTimes &T,
+                 const Closure &closure)
 {
     const int32_t n_ref = ref.n, n_tgt = tgt.n;
     const int S = e->cfg.n_stations;
@@ -214,9 +234,10 @@ int window_check(tdoa_engine *e, const char *fn, const double *stations_llh, con
     if (o->dims == 3 && S < 4) return fail(e, TDOA_E_INVALID, "%s: dims 3 needs at least 4 stations", fn);
     if (n_ref < 1 || n_tgt < 1)
         return fail(e, TDOA_E_INVALID, "%s: need >= 1 REF and >= 1 TGT window, got %d and %d", fn, n_ref, n_tgt);
+    int rc;
+    if (closure.opts && (rc = closure_opts_check(e, fn, closure.opts))) return rc;
     T.n_ref = n_ref; T.n_tgt = n_tgt;
     T.parts.assign(2, ShardPart{});
-    int rc;
     for (int kind = 0; kind < 2; kind++) {
         const WinGeom &G = kind == TDOA_KIND_REF ? ref : tgt;
         ShardPart &Q = T.parts[kind];
@@ -244,7 +265,7 @@ int window_check(tdoa_engine *e, const char *fn, const double *stations_llh, con
 // seed's check) and holds nothing more
 int fix_stage(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts *o, const WinTimes &T, const PeakRec *d_ref,
               const PeakRec *d_tgt, double *ref_fit, double *range_diffs, uint8_t *pair_used, double *fix_llh, double *fix_rms,
-              int32_t *fix_status, int32_t *fix_iters, const GridSeed *grid, bool *synced)
+              int32_t *fix_status, int32_t *fix_iters, const GridSeed *grid, const Closure &closure, bool *synced)
 {
     *synced = false;
     const GridSeed G = grid ? *grid : GridSeed{};
@@ -279,6 +300,14 @@ int fix_stage(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts
         (rc = alloc_t(e, &d_fix, (size_t)3 * nt)) || (rc = alloc_t(e, &d_rms, (size_t)nt)) ||
         (rc = alloc_t(e, &d_status, (size_t)nt)) || (rc = alloc_t(e, &d_iters, (size_t)nt)))
         return rc;
+    // the closure check: the mask the grid rows and the fixes read (the used mask without a check)
+    uint8_t *d_fix_used = d_used;
+    double *d_cresid = nullptr;
+    int *d_dropped = nullptr;
+    if (closure.opts &&
+        ((rc = alloc_t(e, &d_fix_used, (size_t)nt * P)) || (rc = alloc_t(e, &d_cresid, (size_t)nt * P)) ||
+         (rc = alloc_t(e, &d_dropped, (size_t)nt))))
+        return rc;
     // the grid seed: the windows' start points (written by the grid where it finds a cell), the masked rows
     GridSearch g;
     double *d_start = nullptr, *d_tab = nullptr;
@@ -288,7 +317,7 @@ int fix_stage(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts
             (rc = alloc_t(e, &d_tab, (size_t)nt * grid_rank_tab_doubles(true))) || (rc = alloc_t(e, &g.d_cost, (size_t)nt)) ||
             (rc = alloc_t(e, &g.d_idx, (size_t)nt)))
             return rc;
-        g.d_llh = d_llh; g.d_desc = d_desc; g.d_tab = d_tab; g.d_rd = d_rd; g.d_used = d_used; g.d_out = d_start;
+        g.d_llh = d_llh; g.d_desc = d_desc; g.d_tab = d_tab; g.d_rd = d_rd; g.d_used = d_fix_used; g.d_out = d_start;
         g.n_sets = nt; g.rd_stride = P; g.n_st = S; g.nlat = (int)G.desc[4]; g.nlon = (int)G.desc[5];
     }
     // the grid (ranked, or every cell) between the range differences and the fixes
@@ -298,7 +327,7 @@ int fix_stage(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts
             if (const int rc2 = grid_search_queue(e, g, every_cell)) return rc2;
         }
         launch_solve_ls(d_llh, S, d_rd, nt, P, G.desc ? d_start : d_init, o->dims, d_fix, d_rms, d_status, d_iters, e->stream,
-                        d_used);
+                        d_fix_used);
         count_launch(e);
         CU(cudaEventRecord(e->ev[2], e->stream));
         CU(cudaGetLastError());
@@ -325,13 +354,20 @@ int fix_stage(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts
                           d_ref_fit, e->stream);
     launch_window_rd(d_tgt, nt, S, d_t_tgt, d_fit, o->min_margin, e->cfg.sample_rate, d_rd, d_used, e->stream);
     count_launch(e, 2);
+    if (closure.opts) {
+        launch_window_closure(d_rd, d_used, d_fix_used, nt, P, S, o->dims, closure.opts->max_residual, closure.opts->max_drop,
+                              d_cresid, d_dropped, e->stream);
+        count_launch(e);
+    }
     if (G.desc) {
-        launch_grid_rows(d_rd, d_used, nt, P, S, o->dims, d_tab, e->stream);
+        launch_grid_rows(d_rd, d_fix_used, nt, P, S, o->dims, d_tab, e->stream);
         count_launch(e);
     }
     if ((rc = seed_and_fix(false))) return rc;
     if ((rc = back(ref_fit, d_ref_fit, (size_t)3 * P * sizeof(double))) ||
         (rc = back(range_diffs, d_rd, (size_t)nt * P * sizeof(double))) || (rc = back(pair_used, d_used, (size_t)nt * P)) ||
+        (closure.opts && ((rc = back(closure.resid, d_cresid, (size_t)nt * P * sizeof(double))) ||
+                          (rc = back(closure.dropped, d_dropped, (size_t)nt * sizeof(int32_t))))) ||
         (rc = results()))
         return rc;
     if (G.desc) {
@@ -397,14 +433,15 @@ int station_rates(tdoa_engine *e, const tdoa_window_opts *o, const WinTimes &T, 
 int window_fixes_impl(tdoa_engine *e, const char *fn, const double *stations_llh, const tdoa_window_opts *o, int64_t win_start,
                       int64_t win_len, int32_t n_ref_windows, int32_t n_tgt_windows, int64_t hop, const tdoa_peak *ref_in,
                       const tdoa_peak *tgt_in, double *ref_fit, double *range_diffs, uint8_t *pair_used, double *fix_llh,
-                      double *fix_rms, int32_t *fix_status, int32_t *fix_iters, const GridSeed *grid)
+                      double *fix_rms, int32_t *fix_status, int32_t *fix_iters, const GridSeed *grid,
+                      const Closure &closure = Closure{})
 {
     if (!e) return TDOA_E_INVALID;
     int rc = begin_call(e);
     if (rc) return rc;
     WinTimes T;
     if ((rc = window_check(e, fn, stations_llh, o, WinGeom{win_start, win_len, n_ref_windows, hop},
-                          WinGeom{win_start, win_len, n_tgt_windows, hop}, fix_llh, fix_status, grid, T)))
+                          WinGeom{win_start, win_len, n_tgt_windows, hop}, fix_llh, fix_status, grid, T, closure)))
         return rc;
     if (!ref_in || !tgt_in) return fail(e, TDOA_E_INVALID, "%s: a table is NULL", fn);
     const int S = e->cfg.n_stations, P = S * (S - 1) / 2;
@@ -414,7 +451,7 @@ int window_fixes_impl(tdoa_engine *e, const char *fn, const double *stations_llh
     CU(cudaMemcpyAsync(d_tgt, tgt_in, (size_t)n_tgt_windows * P * sizeof(PeakRec), cudaMemcpyHostToDevice, e->stream));
     bool synced = false;
     if ((rc = fix_stage(e, stations_llh, o, T, d_ref, d_tgt, ref_fit, range_diffs, pair_used, fix_llh, fix_rms, fix_status,
-                        fix_iters, grid, &synced)))
+                        fix_iters, grid, closure, &synced)))
         return rc;
     return finish_fix_stage(e, synced);
 }
@@ -424,13 +461,14 @@ int window_fixes_impl(tdoa_engine *e, const char *fn, const double *stations_llh
 int process_windows_impl(tdoa_engine *e, const char *fn, const double *stations_llh, const tdoa_window_opts *o,
                          const WinGeom &ref, const WinGeom &tgt, tdoa_peak *ref_out, tdoa_peak *tgt_out, double *ref_fit,
                          double *range_diffs, uint8_t *pair_used, double *fix_llh, double *fix_rms, int32_t *fix_status,
-                         int32_t *fix_iters, const GridSeed *grid, bool retimed, double *clock_rate)
+                         int32_t *fix_iters, const GridSeed *grid, bool retimed, double *clock_rate,
+                         const Closure &closure = Closure{})
 {
     if (!e) return TDOA_E_INVALID;
     int rc = begin_call(e);
     if (rc) return rc;
     WinTimes T;
-    if ((rc = window_check(e, fn, stations_llh, o, ref, tgt, fix_llh, fix_status, grid, T))) return rc;
+    if ((rc = window_check(e, fn, stations_llh, o, ref, tgt, fix_llh, fix_status, grid, T, closure))) return rc;
     const int S = e->cfg.n_stations, P = S * (S - 1) / 2;
     Tables tab{e->stream};
     CU(cudaMallocAsync(reinterpret_cast<void **>(&tab.ref), (size_t)ref.n * P * sizeof(PeakRec), e->stream));
@@ -472,7 +510,7 @@ int process_windows_impl(tdoa_engine *e, const char *fn, const double *stations_
         CU(cudaMemcpyAsync(clock_rate, tab.rates + S, (size_t)S * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
     bool synced = false;
     if ((rc = fix_stage(e, stations_llh, o, T, tab.ref, tab.tgt, ref_fit, range_diffs, pair_used, fix_llh, fix_rms, fix_status,
-                        fix_iters, grid, &synced)))
+                        fix_iters, grid, closure, &synced)))
         return rc;
     return finish_fix_stage(e, synced);
 }
@@ -534,6 +572,81 @@ int tdoa_process_windows_grid(tdoa_engine *e, const double *stations_llh, const 
     return process_windows_impl(e, "tdoa_process_windows_grid", stations_llh, o, WinGeom{win_start, win_len, n_ref_windows, hop},
                                 WinGeom{win_start, win_len, n_tgt_windows, hop}, ref_out, tgt_out, ref_fit, range_diffs, pair_used,
                                 fix_llh, fix_rms, fix_status, fix_iters, &G, false, nullptr);
+}
+
+int tdoa_process_windows_closure(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts *o,
+                                 const tdoa_closure_opts *c, int64_t ref_win_start, int64_t ref_win_len, int32_t n_ref_windows,
+                                 int64_t ref_hop, int64_t tgt_win_start, int64_t tgt_win_len, int32_t n_tgt_windows,
+                                 int64_t tgt_hop, int32_t retimed, const double *grid_desc, tdoa_peak *ref_out,
+                                 tdoa_peak *tgt_out, double *ref_fit, double *range_diffs, uint8_t *pair_used,
+                                 double *closure_resid, int32_t *n_dropped, double *fix_llh, double *fix_rms,
+                                 int32_t *fix_status, int32_t *fix_iters, double *clock_rate, double *seed_llh,
+                                 double *seed_cost, int64_t *seed_index)
+{
+    static const char *fn = "tdoa_process_windows_closure";
+    if (!e) return TDOA_E_INVALID;
+    if (!c) return fail(e, TDOA_E_INVALID, "%s: closure options are NULL", fn);
+    if (retimed != 0 && retimed != 1) return fail(e, TDOA_E_INVALID, "%s: retimed must be 0 or 1, got %d", fn, retimed);
+    const GridSeed G{grid_desc, seed_llh, seed_cost, seed_index};
+    return process_windows_impl(e, fn, stations_llh, o, WinGeom{ref_win_start, ref_win_len, n_ref_windows, ref_hop},
+                                WinGeom{tgt_win_start, tgt_win_len, n_tgt_windows, tgt_hop}, ref_out, tgt_out, ref_fit,
+                                range_diffs, pair_used, fix_llh, fix_rms, fix_status, fix_iters, grid_desc ? &G : nullptr,
+                                retimed == 1, clock_rate, Closure{c, closure_resid, n_dropped});
+}
+
+int tdoa_window_fixes_closure(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts *o,
+                              const tdoa_closure_opts *c, int64_t win_start, int64_t win_len, int32_t n_ref_windows,
+                              int32_t n_tgt_windows, int64_t hop, const double *grid_desc, const tdoa_peak *ref_in,
+                              const tdoa_peak *tgt_in, double *ref_fit, double *range_diffs, uint8_t *pair_used,
+                              double *closure_resid, int32_t *n_dropped, double *fix_llh, double *fix_rms,
+                              int32_t *fix_status, int32_t *fix_iters, double *seed_llh, double *seed_cost,
+                              int64_t *seed_index)
+{
+    static const char *fn = "tdoa_window_fixes_closure";
+    if (!e) return TDOA_E_INVALID;
+    if (!c) return fail(e, TDOA_E_INVALID, "%s: closure options are NULL", fn);
+    const GridSeed G{grid_desc, seed_llh, seed_cost, seed_index};
+    return window_fixes_impl(e, fn, stations_llh, o, win_start, win_len, n_ref_windows, n_tgt_windows, hop, ref_in, tgt_in,
+                             ref_fit, range_diffs, pair_used, fix_llh, fix_rms, fix_status, fix_iters,
+                             grid_desc ? &G : nullptr, Closure{c, closure_resid, n_dropped});
+}
+
+int tdoa_closure(tdoa_engine *e, int32_t n_stations, const double *range_diffs, const uint8_t *used, int32_t n_sets,
+                 int32_t rd_stride, int32_t dims, const tdoa_closure_opts *c, uint8_t *out_used, double *out_resid,
+                 int32_t *out_dropped)
+{
+    static const char *fn = "tdoa_closure";
+    if (!e) return TDOA_E_INVALID;
+    int rc = begin_call(e);
+    if (rc) return rc;
+    const int S = n_stations, P = S * (S - 1) / 2;
+    if (!range_diffs || !used || !out_used) return fail(e, TDOA_E_INVALID, "%s: NULL argument", fn);
+    if (S < 3 || S > kGraphLsMaxStations) return fail(e, TDOA_E_INVALID, "%s: 3..%d stations, got %d", fn, kGraphLsMaxStations, S);
+    if (dims != 2 && dims != 3) return fail(e, TDOA_E_INVALID, "%s: dims must be 2 or 3, got %d", fn, dims);
+    if (n_sets < 0 || rd_stride < P)
+        return fail(e, TDOA_E_INVALID, "%s: n_sets >= 0 and rd_stride >= %d, got %d and %d", fn, P, n_sets, rd_stride);
+    if ((rc = closure_opts_check(e, fn, c))) return rc;
+    if (n_sets == 0) return end_call(e, true);
+    const size_t n = (size_t)n_sets * rd_stride;
+    double *d_rd = nullptr, *d_resid = nullptr;
+    uint8_t *d_used = nullptr;
+    int *d_dropped = nullptr;
+    if ((rc = alloc_t(e, &d_rd, n)) || (rc = alloc_t(e, &d_used, n)) || (rc = alloc_t(e, &d_resid, n)) ||
+        (rc = alloc_t(e, &d_dropped, (size_t)n_sets)))
+        return rc;
+    CU(cudaMemcpyAsync(d_rd, range_diffs, n * sizeof(double), cudaMemcpyHostToDevice, e->stream));
+    CU(cudaMemcpyAsync(d_used, used, n, cudaMemcpyHostToDevice, e->stream));
+    launch_window_closure(d_rd, d_used, nullptr, n_sets, rd_stride, S, dims, c->max_residual, c->max_drop, d_resid, d_dropped,
+                          e->stream);
+    count_launch(e);
+    CU(cudaGetLastError());
+    // the first P slots of each set only: the rest of the caller's rows are left as they are
+    CU(cudaMemcpy2DAsync(out_used, rd_stride, d_used, rd_stride, P, n_sets, cudaMemcpyDeviceToHost, e->stream));
+    if (out_resid)
+        CU(cudaMemcpy2DAsync(out_resid, rd_stride * sizeof(double), d_resid, rd_stride * sizeof(double), P * sizeof(double),
+                             n_sets, cudaMemcpyDeviceToHost, e->stream));
+    if (out_dropped) CU(cudaMemcpyAsync(out_dropped, d_dropped, (size_t)n_sets * sizeof(int32_t), cudaMemcpyDeviceToHost, e->stream));
+    return end_call(e, true);
 }
 
 }  // extern "C"
