@@ -410,6 +410,83 @@ TDOA_API int tdoa_window_fixes_closure(tdoa_engine *e, const double *stations_ll
                                        int32_t *fix_status, int32_t *fix_iters, double *seed_llh, double *seed_cost,
                                        int64_t *seed_index);
 
+/* ---- station-checked windowed fixes (no reference equivalent; engine-defined).  An error common to all of one
+ * station's pairs (a collector tuned to another programme, overloaded by one, or with its antenna down) is a
+ * station value: the closure check cannot see it.  The range differences must also agree with ONE position: with
+ * S stations the used pairs carry S - 1 independent numbers and the position takes dims of them, so S - 1 - dims
+ * are left to check with.  As a GNSS receiver's fault detection and exclusion does, the check detects the fault
+ * from the fix's rms, identifies the station by solving again without each station in turn, and keeps the solve
+ * that fits.  Per set (one TGT window): rd[P] in metres; the fix mask m[P] in {0, 1} (the used mask, or the
+ * closure check's output when both checks run); the start x0 (init_llh, the station mean, or with a grid the grid
+ * arg-min over m); dims; max_rms (metres, > 0, may be +inf) and max_exclude (>= 0, 0 = no limit).  LS(mask, x) is
+ * exactly what tdoa_solve_ls's least-squares step returns for that mask from start x (position, rms, status,
+ * iterations).
+ *  1. F = LS(m, x0) (the fix without the check); E = {}.
+ *  2. Stop if F.status != 0, or F.rms <= max_rms, or max_exclude > 0 and |E| = max_exclude.
+ *  3. Station k is a candidate if it touches an m-pair, m_k (m without every pair that touches k) passes the
+ *     status-2 rule, and m_k has redundancy >= 1: (stations m_k touches) - (components of m_k's pair graph) - dims.
+ *     (Without that rule an exclusion that leaves an exactly determined fix would win with rms 0; one exclusion
+ *     needs dims + 3 stations: 5 for dims 2, 6 for dims 3.)  No candidate: stop.
+ *  4. F_k = LS(m_k, x0) for every candidate; a candidate with F_k.status != 0 is not eligible.
+ *  5. k* = the eligible candidate with the least F_k.rms (ties: the lowest k).  Stop if there is none or
+ *     F_k*.rms >= F.rms; else m = m_k*, E = E + {k*}, F = F_k*, go to 2.
+ * With a grid and E not empty, the window is seeded again from the grid arg-min over the final m (a wrong station
+ * can have pulled the first arg-min into a trap) and F = LS(m, that seed); the seed outputs report that seed.
+ * Outputs per set: the final m; station_round[S] (0: not excluded, else the round, from 1, that excluded it);
+ * station_rms[S] (F_k.rms of the FIRST round for every candidate, NaN for the others or when no round ran: how far
+ * the bad station stands apart); the number excluded; F.  When the first F.rms <= max_rms every output of the fix
+ * stage is, bit for bit, that of the call without the check: max_rms = INFINITY turns it off.  Decisions rest on
+ * the unweighted rms, as the fix does.  The check does not see an error that a shift of the position can absorb
+ * (near-collinear stations, a station whose error moves the fix along its own gradient).  In BINARY mode integer
+ * lags already give rms of order 100 m; set max_rms above that. */
+typedef struct {
+    double max_rms;        /* metres; > 0, may be INFINITY                                     */
+    int32_t max_exclude;   /* stations per set; 0 = no limit                                   */
+    int32_t reserved;
+} tdoa_exclusion_opts;
+
+/* The check alone over host sets (no grid): range_diffs[set * rd_stride + p], used[...] in {0, 1} (an unused slot is
+ * never read), init_llh[n_sets][3] (NULL: the station mean).  out_used[...] in {0, 1, 3} (3: used, excluded with
+ * its station); station_round[n_sets][S], station_rms[n_sets][S], n_excluded[n_sets], out_llh[n_sets][3],
+ * out_rms[n_sets], status[n_sets] and iters[n_sets] (F, as tdoa_solve_ls gives it).  Only the first P slots of each
+ * set are read or written.  Every output but out_used, out_llh and status may be NULL.  Refused (TDOA_E_INVALID): a
+ * NULL stations_llh, range_diffs, used, out_used, out_llh, status or x, S outside 3..64, dims not 2 or 3,
+ * n_sets < 0, rd_stride < P, max_rms NaN or <= 0, max_exclude < 0. */
+TDOA_API int tdoa_exclude_stations(tdoa_engine *e, const double *stations_llh, int32_t n_stations,
+                                   const double *range_diffs, const uint8_t *used, int32_t n_sets, int32_t rd_stride,
+                                   const double *init_llh, int32_t dims, const tdoa_exclusion_opts *x,
+                                   uint8_t *out_used, uint8_t *station_round, double *station_rms,
+                                   int32_t *n_excluded, double *out_llh, double *out_rms, int32_t *status,
+                                   int32_t *iters);
+/* tdoa_process_windows_closure with the station check after the first fix: c may be NULL (no closure check); with
+ * both, the closure check runs first, so pair outliers are dropped before a station outlier is looked for.  The
+ * check runs on the device after the first grid seed and fix, on the same stream, with no other host
+ * synchronisation; on a multi-GPU engine every rank runs it on its own gathered tables.  pair_used[n_tgt][P]: 0
+ * not usable, 1 used by the fix, 2 dropped by the closure check, 3 excluded with its station.  station_round,
+ * station_rms and n_excluded may be NULL; ms_fix covers the check.  Refused (TDOA_E_INVALID): what
+ * tdoa_process_windows_closure refuses (but c may be NULL), a NULL x, max_rms NaN or <= 0, max_exclude < 0. */
+TDOA_API int tdoa_process_windows_exclude(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts *o,
+                                          const tdoa_closure_opts *c, const tdoa_exclusion_opts *x,
+                                          int64_t ref_win_start, int64_t ref_win_len, int32_t n_ref_windows,
+                                          int64_t ref_hop, int64_t tgt_win_start, int64_t tgt_win_len,
+                                          int32_t n_tgt_windows, int64_t tgt_hop, int32_t retimed,
+                                          const double *grid_desc, tdoa_peak *ref_out, tdoa_peak *tgt_out,
+                                          double *ref_fit, double *range_diffs, uint8_t *pair_used,
+                                          double *closure_resid, int32_t *n_dropped, uint8_t *station_round,
+                                          double *station_rms, int32_t *n_excluded, double *fix_llh, double *fix_rms,
+                                          int32_t *fix_status, int32_t *fix_iters, double *clock_rate,
+                                          double *seed_llh, double *seed_cost, int64_t *seed_index);
+/* The same on host tables, as tdoa_window_fixes_closure (c and grid_desc may be NULL). */
+TDOA_API int tdoa_window_fixes_exclude(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts *o,
+                                       const tdoa_closure_opts *c, const tdoa_exclusion_opts *x, int64_t win_start,
+                                       int64_t win_len, int32_t n_ref_windows, int32_t n_tgt_windows, int64_t hop,
+                                       const double *grid_desc, const tdoa_peak *ref_in, const tdoa_peak *tgt_in,
+                                       double *ref_fit, double *range_diffs, uint8_t *pair_used,
+                                       double *closure_resid, int32_t *n_dropped, uint8_t *station_round,
+                                       double *station_rms, int32_t *n_excluded, double *fix_llh, double *fix_rms,
+                                       int32_t *fix_status, int32_t *fix_iters, double *seed_llh, double *seed_cost,
+                                       int64_t *seed_index);
+
 /* crossCorrelate seam (processor.go:619-643): two host complex64 slices
  * (interleaved re,im), returns (delay, correlation).  Empty input -> (0, 0.0). */
 TDOA_API int tdoa_cross_correlate(tdoa_engine *e, const float *sig1_c64, int64_t n1,

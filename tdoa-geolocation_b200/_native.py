@@ -23,7 +23,7 @@ ERRORS = {-1: "TDOA_E_INVALID", -2: "TDOA_E_NODEVICE", -3: "TDOA_E_CUDA", -4: "T
 # every symbol include/tdoa_b200.h declares (tests check the library exports them all)
 ABI_SYMBOLS = [
     "tdoa_default_config", "tdoa_create", "tdoa_destroy", "tdoa_last_error", "tdoa_host_alloc", "tdoa_host_free",
-    "tdoa_load_u8", "tdoa_load_file", "tdoa_load_u8_pinned", "tdoa_load_u8_device", "tdoa_unpack", "tdoa_preprocess", "tdoa_xcorr", "tdoa_xcorr_device", "tdoa_xcorr_windows", "tdoa_process", "tdoa_process_windows", "tdoa_window_fixes", "tdoa_process_windows_grid", "tdoa_window_fixes_grid", "tdoa_process_windows_retimed", "tdoa_closure", "tdoa_process_windows_closure", "tdoa_window_fixes_closure", "tdoa_xcorr_info", "tdoa_analyze",
+    "tdoa_load_u8", "tdoa_load_file", "tdoa_load_u8_pinned", "tdoa_load_u8_device", "tdoa_unpack", "tdoa_preprocess", "tdoa_xcorr", "tdoa_xcorr_device", "tdoa_xcorr_windows", "tdoa_process", "tdoa_process_windows", "tdoa_window_fixes", "tdoa_process_windows_grid", "tdoa_window_fixes_grid", "tdoa_process_windows_retimed", "tdoa_closure", "tdoa_process_windows_closure", "tdoa_window_fixes_closure", "tdoa_exclude_stations", "tdoa_process_windows_exclude", "tdoa_window_fixes_exclude", "tdoa_xcorr_info", "tdoa_analyze",
     "tdoa_cross_correlate", "tdoa_baselines", "tdoa_solve", "tdoa_solve_binary", "tdoa_solve_ls", "tdoa_grid", "tdoa_grid_masked", "tdoa_get_stats", "tdoa_stream",
     "tdoa_set_stream", "tdoa_synchronize", "tdoa_selftest",
     "tdoa_comm_unique_id", "tdoa_comm_init", "tdoa_comm_rank", "tdoa_shard_windows",
@@ -91,6 +91,19 @@ def _closure_opts(closure) -> ClosureOpts:
     if unknown or "max_residual" not in c:
         raise ValueError(f"closure takes max_residual and max_drop, got {sorted(c)}")
     return ClosureOpts(max_residual=float(c["max_residual"]), max_drop=int(c.get("max_drop", 0)))
+
+
+class ExclusionOpts(C.Structure):
+    _fields_ = [("max_rms", C.c_double), ("max_exclude", C.c_int32), ("reserved", C.c_int32)]
+
+
+def _exclusion_opts(exclusion) -> ExclusionOpts:
+    """exclusion = dict(max_rms=metres, max_exclude=1)"""
+    x = dict(exclusion)
+    unknown = set(x) - {"max_rms", "max_exclude"}
+    if unknown or "max_rms" not in x:
+        raise ValueError(f"exclusion takes max_rms and max_exclude, got {sorted(x)}")
+    return ExclusionOpts(max_rms=float(x["max_rms"]), max_exclude=int(x.get("max_exclude", 1)))
 
 
 class Stats(C.Structure):
@@ -172,6 +185,11 @@ def load_library():
     L.tdoa_process_windows_closure.argtypes = ([vp, vp, C.POINTER(WindowOpts), C.POINTER(ClosureOpts), i64, i64, i32, i64, i64,
                                                 i64, i32, i64, i32] + [vp] * 16)
     L.tdoa_window_fixes_closure.argtypes = [vp, vp, C.POINTER(WindowOpts), C.POINTER(ClosureOpts), i64, i64, i32, i32, i64] + [vp] * 15
+    L.tdoa_exclude_stations.argtypes = [vp, vp, i32, vp, vp, i32, i32, vp, i32, C.POINTER(ExclusionOpts)] + [vp] * 8
+    L.tdoa_process_windows_exclude.argtypes = ([vp, vp, C.POINTER(WindowOpts), C.POINTER(ClosureOpts), C.POINTER(ExclusionOpts),
+                                                i64, i64, i32, i64, i64, i64, i32, i64, i32] + [vp] * 19)
+    L.tdoa_window_fixes_exclude.argtypes = ([vp, vp, C.POINTER(WindowOpts), C.POINTER(ClosureOpts), C.POINTER(ExclusionOpts),
+                                             i64, i64, i32, i32, i64] + [vp] * 18)
     L.tdoa_cross_correlate.argtypes = [vp, vp, i64, vp, i64, C.POINTER(PeakStruct)]
     L.tdoa_baselines.argtypes = [vp, vp, i32, vp]
     L.tdoa_solve.argtypes = [vp, vp, i32, vp, i32, i32, vp, vp, vp]
@@ -510,11 +528,12 @@ class Engine:
                 "seed_index": seed_index}
 
     def _closure_windows(self, fn, stations_llh, geometry, tables, retimed, dims, min_margin, ref_max_residual,
-                         ref_tx_llh, init_llh, grid, closure) -> dict:
+                         ref_tx_llh, init_llh, grid, closure, exclusion=None) -> dict:
         """tdoa_process_windows_closure (tables None: the call fills them) or tdoa_window_fixes_closure (tables =
-        (ref, tgt) host inputs)"""
+        (ref, tgt) host inputs); with exclusion, fn is the matching _exclude call and closure may be None"""
         st, o = self._window_opts(stations_llh, dims, min_margin, ref_max_residual, ref_tx_llh, init_llh)
-        c = _closure_opts(closure)
+        S = self.n_stations
+        c = _closure_opts(closure) if closure is not None or exclusion is None else None
         P = self.n_pairs
         (r0, rl, nr, rh), (t0, tl, nt, th) = geometry
         nt_ = max(nt, 0)
@@ -528,31 +547,39 @@ class Engine:
             if gd.size != 7:
                 raise ValueError(f"grid must be 7 numbers (lat0, lon0, dlat, dlon, nlat, nlon, elev), got {gd.size}")
         seed, seed_cost, seed_index = np.zeros((nt_, 3), np.float64), np.zeros(nt_, np.float64), np.zeros(nt_, np.int64)
-        outs = [_ptr(ref_fit), _ptr(rd), _ptr(used), _ptr(resid), _ptr(dropped), _ptr(fix), _ptr(rms), _ptr(status),
-                _ptr(iters)]
+        rounds, srms, excluded = np.zeros((nt_, S), np.uint8), np.full((nt_, S), np.nan), np.zeros(nt_, np.int32)
+        checks = [_ptr(resid), _ptr(dropped)]
+        opts = [None if c is None else C.byref(c)]
+        if exclusion is not None:
+            checks += [_ptr(rounds), _ptr(srms), _ptr(excluded)]
+            opts.append(C.byref(_exclusion_opts(exclusion)))
+        outs = [_ptr(ref_fit), _ptr(rd), _ptr(used), *checks, _ptr(fix), _ptr(rms), _ptr(status), _ptr(iters)]
         seeds = [_ptr(seed), _ptr(seed_cost), _ptr(seed_index)]
         out = {}
         if tables is None:
             ref_t, tgt_t = np.zeros((max(nr, 0), P), PEAK_DTYPE), np.zeros((nt_, P), PEAK_DTYPE)
             rate = np.zeros(self.n_stations, np.float64)
-            self._check(fn(self._h, _ptr(st), C.byref(o), C.byref(c), r0, rl, nr, rh, t0, tl, nt, th, int(retimed),
+            self._check(fn(self._h, _ptr(st), C.byref(o), *opts, r0, rl, nr, rh, t0, tl, nt, th, int(retimed),
                            None if gd is None else _ptr(gd), _ptr(ref_t), _ptr(tgt_t), *outs, _ptr(rate), *seeds))
             out.update(ref=ref_t, tgt=tgt_t)
             if retimed:
                 out["clock_rate"] = rate
         else:
-            self._check(fn(self._h, _ptr(st), C.byref(o), C.byref(c), r0, rl, nr, nt, rh, None if gd is None else _ptr(gd),
+            self._check(fn(self._h, _ptr(st), C.byref(o), *opts, r0, rl, nr, nt, rh, None if gd is None else _ptr(gd),
                            *[_ptr(t) for t in tables], *outs, *seeds))
         out.update({"ref_fit": ref_fit, "range_differences": rd, "pair_used": used == 1, "pair_dropped": used == 2,
-                    "closure_residual": resid, "dropped": dropped, "position": fix, "rms": rms, "status": status,
-                    "iters": iters})
+                    "position": fix, "rms": rms, "status": status, "iters": iters})
+        if c is not None:
+            out.update(closure_residual=resid, dropped=dropped)
+        if exclusion is not None:
+            out.update(pair_excluded=used == 3, station_excluded=rounds, station_rms=srms, excluded=excluded)
         if gd is not None:
             out.update(seed=seed, seed_cost=seed_cost, seed_index=seed_index)
         return out
 
     def process_windows(self, stations_llh, win_start: int, win_len: int, n_ref_windows: int, n_tgt_windows: int,
                         hop: int, dims: int = 2, min_margin: float = 0.0, ref_max_residual: float = 0.0,
-                        ref_tx_llh=None, init_llh=None, grid=None, closure=None) -> dict:
+                        ref_tx_llh=None, init_llh=None, grid=None, closure=None, exclusion=None) -> dict:
         """Windowed ProcessTDOA (tdoa_process_windows): REF and TGT tables as xcorr_windows gives them, the REF
         lag's linear track per pair (ref_fit: lag at block 2's centre, drift in samples per sample, windows
         used), range differences and the used mask per (TGT window, pair), one least-squares fix per TGT window
@@ -563,12 +590,18 @@ class Engine:
         closure = dict(max_residual=metres, max_drop=0): each window's usable pairs are checked against each other
         first and the pairs the rest contradict are dropped (tdoa_process_windows_closure, statement in
         include/tdoa_b200.h); the result gains pair_dropped (usable but dropped), closure_residual (NaN where not
-        usable) and dropped (pairs per window), and pair_used is the mask the fix read."""
-        if closure is not None:
+        usable) and dropped (pairs per window), and pair_used is the mask the fix read.
+        exclusion = dict(max_rms=metres, max_exclude=1): after the first fix, each window whose rms exceeds max_rms
+        is solved again without each station in turn and the station whose solve fits best is excluded
+        (tdoa_process_windows_exclude, statement in include/tdoa_b200.h; combines with closure, which runs first, and
+        grid, which seeds again); the result gains station_excluded[n_tgt][S] (0, or the round that excluded the
+        station), station_rms[n_tgt][S] (first-round rms without each candidate station, NaN for the others),
+        excluded (stations per window) and pair_excluded, and pair_used is the mask the fix read."""
+        if closure is not None or exclusion is not None:
             g = (int(win_start), int(win_len), int(n_ref_windows), int(hop))
-            return self._closure_windows(self._lib.tdoa_process_windows_closure, stations_llh,
-                                         (g, (g[0], g[1], int(n_tgt_windows), g[3])), None, 0, dims, min_margin,
-                                         ref_max_residual, ref_tx_llh, init_llh, grid, closure)
+            fn = self._lib.tdoa_process_windows_closure if exclusion is None else self._lib.tdoa_process_windows_exclude
+            return self._closure_windows(fn, stations_llh, (g, (g[0], g[1], int(n_tgt_windows), g[3])), None, 0, dims,
+                                         min_margin, ref_max_residual, ref_tx_llh, init_llh, grid, closure, exclusion)
         ref = np.zeros((max(n_ref_windows, 0), self.n_pairs), PEAK_DTYPE)
         tgt = np.zeros((max(n_tgt_windows, 0), self.n_pairs), PEAK_DTYPE)
         fn = self._lib.tdoa_process_windows if grid is None else self._lib.tdoa_process_windows_grid
@@ -579,14 +612,19 @@ class Engine:
 
     def process_windows_retimed(self, stations_llh, ref, tgt, dims: int = 2, min_margin: float = 0.0,
                                 ref_max_residual: float = 0.0, ref_tx_llh=None, init_llh=None, grid=None,
-                                closure=None) -> dict:
+                                closure=None, exclusion=None) -> dict:
         """Re-timed target correlation (tdoa_process_windows_retimed): ref = (start, len, n, hop) and tgt = (start,
         len, n, hop) are the two kinds' window geometries.  The REF windows give each pair's drift line as in
         process_windows; the station clock rates fitted from those slopes re-time every TGT plane, so a TGT window
         may span the whole block without smearing its peak.  Returns process_windows' dict plus clock_rate[S]
-        (samples per sample; NaN for a station without a fitted pair).  grid and closure as process_windows (through
-        tdoa_process_windows_closure; without closure the check is inert)."""
+        (samples per sample; NaN for a station without a fitted pair).  grid, closure and exclusion as process_windows
+        (through tdoa_process_windows_closure, or _exclude with exclusion; without closure the closure check is
+        inert)."""
         (r0, rl, nr, rh), (t0, tl, nt, th) = (tuple(int(v) for v in g) for g in (ref, tgt))
+        if exclusion is not None:
+            return self._closure_windows(self._lib.tdoa_process_windows_exclude, stations_llh,
+                                         ((r0, rl, nr, rh), (t0, tl, nt, th)), None, 1, dims, min_margin,
+                                         ref_max_residual, ref_tx_llh, init_llh, grid, closure, exclusion)
         if grid is not None or closure is not None:
             return self._closure_windows(self._lib.tdoa_process_windows_closure, stations_llh,
                                          ((r0, rl, nr, rh), (t0, tl, nt, th)), None, 1, dims, min_margin,
@@ -607,17 +645,18 @@ class Engine:
 
     def window_fixes(self, stations_llh, win_start: int, win_len: int, ref, tgt, hop: int, dims: int = 2,
                      min_margin: float = 0.0, ref_max_residual: float = 0.0, ref_tx_llh=None, init_llh=None,
-                     grid=None, closure=None) -> dict:
+                     grid=None, closure=None, exclusion=None) -> dict:
         """The fix stage of process_windows on given tables (tdoa_window_fixes): ref[n_ref][P], tgt[n_tgt][P] of
         PEAK_DTYPE, e.g. kept from xcorr_windows; window times come from the captures the engine holds.  grid: as
-        process_windows (tdoa_window_fixes_grid); closure: as process_windows (tdoa_window_fixes_closure)."""
+        process_windows (tdoa_window_fixes_grid); closure and exclusion: as process_windows
+        (tdoa_window_fixes_closure, tdoa_window_fixes_exclude)."""
         ref = np.ascontiguousarray(ref, PEAK_DTYPE).reshape(-1, self.n_pairs)
         tgt = np.ascontiguousarray(tgt, PEAK_DTYPE).reshape(-1, self.n_pairs)
-        if closure is not None:
+        if closure is not None or exclusion is not None:
             g = (int(win_start), int(win_len), ref.shape[0], int(hop))
-            return self._closure_windows(self._lib.tdoa_window_fixes_closure, stations_llh,
-                                         (g, (g[0], g[1], tgt.shape[0], g[3])), (ref, tgt), 0, dims, min_margin,
-                                         ref_max_residual, ref_tx_llh, init_llh, grid, closure)
+            fn = self._lib.tdoa_window_fixes_closure if exclusion is None else self._lib.tdoa_window_fixes_exclude
+            return self._closure_windows(fn, stations_llh, (g, (g[0], g[1], tgt.shape[0], g[3])), (ref, tgt), 0, dims,
+                                         min_margin, ref_max_residual, ref_tx_llh, init_llh, grid, closure, exclusion)
         fn = self._lib.tdoa_window_fixes if grid is None else self._lib.tdoa_window_fixes_grid
         return self._windows(fn, stations_llh, win_start, win_len, ref.shape[0], tgt.shape[0], hop, (ref, tgt), dims,
                              min_margin, ref_max_residual, ref_tx_llh, init_llh, grid)
@@ -638,6 +677,34 @@ class Engine:
         if single:
             return out[0], resid[0], int(dropped[0])
         return out, resid, dropped
+
+    def exclude_stations(self, stations_llh, range_diffs, used, init_llh=None, dims: int = 2, *, max_rms: float,
+                         max_exclude: int = 1) -> dict:
+        """The station check alone (tdoa_exclude_stations) over sets range_diffs[n_sets][>= P], used[n_sets][>= P]
+        (an unused slot is never read), from init_llh (one point, or one per set; None: the station mean).  Returns
+        used (0, 1, or 3 = excluded with its station), station_excluded[n_sets][S] (0 or the round), station_rms,
+        excluded (stations per set), position, rms, status and iters of the final fix; one set when range_diffs is
+        1-D."""
+        st = np.ascontiguousarray(stations_llh, dtype=np.float64).reshape(-1, 3)
+        S = st.shape[0]
+        rd = np.ascontiguousarray(range_diffs, dtype=np.float64)
+        single = rd.ndim == 1
+        rd = rd.reshape(1, -1) if single else rd
+        n, stride = rd.shape
+        u = np.ascontiguousarray(np.asarray(used).astype(np.uint8).reshape(n, stride))
+        init = None
+        if init_llh is not None:
+            init = np.ascontiguousarray(np.broadcast_to(np.asarray(init_llh, np.float64).reshape(-1, 3), (n, 3)))
+        x = _exclusion_opts({"max_rms": max_rms, "max_exclude": max_exclude})
+        out = {"used": np.zeros((n, stride), np.uint8), "station_excluded": np.zeros((n, S), np.uint8),
+               "station_rms": np.full((n, S), np.nan), "excluded": np.zeros(n, np.int32),
+               "position": np.zeros((n, 3), np.float64), "rms": np.zeros(n, np.float64),
+               "status": np.zeros(n, np.int32), "iters": np.zeros(n, np.int32)}
+        self._check(self._lib.tdoa_exclude_stations(
+            self._h, _ptr(st), S, _ptr(rd), _ptr(u), n, stride, None if init is None else _ptr(init), dims, C.byref(x),
+            *[_ptr(out[k]) for k in ("used", "station_excluded", "station_rms", "excluded", "position", "rms", "status",
+                                     "iters")]))
+        return {k: v[0] for k, v in out.items()} if single else out
 
     def solve_ls(self, stations_llh, range_diffs, init_llh=None, dims: int = 2):
         """Levenberg-Marquardt fix over all pair range differences (engine-defined, SURVEY 8f-4).

@@ -30,6 +30,7 @@ UNITS = [
     ("solve.cu", ["-fmad=false"]),
     ("window_fix.cu", ["-fmad=false"]),
     ("retime.cu", ["-fmad=false"]),
+    ("exclude.cu", ["-fmad=false"]),
     ("analyze.cu", ["-fmad=false"]),
     ("xcorr_fft.cu", []),
     ("xcorr_tile.cu", []),

@@ -19,16 +19,17 @@ typedef double GraphLsMatrix[kGraphLsMaxStations + 1];   // a row of A (padded a
 // pair p = (i, j), i < j, in lexicographic order
 __host__ __device__ __forceinline__ int graph_pair(int i, int j, int S) { return i * (2 * S - i - 1) / 2 + (j - i - 1); }
 
-// The status-2 rule of a masked fix (k_solve_ls), of the grid seed (k_grid_rows) and of a closure drop
-// (k_window_closure): the number of used pairs, or -1 when there are fewer than `dims` of them or they touch fewer
-// than dims + 1 stations (dims = 0: no used pair).
-__host__ __device__ __forceinline__ int ls_used_pairs(const uint8_t *used, int n_st, int dims)
+// The status-2 rule of a masked fix (k_solve_ls), of the grid seed (k_grid_rows), of a closure drop
+// (k_window_closure) and of a station exclusion (k_window_exclude): the number of used pairs, or -1 when there are
+// fewer than `dims` of them or they touch fewer than dims + 1 stations (dims = 0: no used pair).  skip: stations
+// whose pairs count as unused.
+__host__ __device__ __forceinline__ int ls_used_pairs(const uint8_t *used, int n_st, int dims, unsigned long long skip = 0ull)
 {
     int n_used = 0, q = 0;
     unsigned long long touched = 0ull;
     for (int i = 0; i < n_st; i++)
         for (int j = i + 1; j < n_st; j++, q++)
-            if (used[q]) { n_used++; touched |= (1ull << i) | (1ull << j); }
+            if (used[q] && !((skip >> i | skip >> j) & 1ull)) { n_used++; touched |= (1ull << i) | (1ull << j); }
 #ifdef __CUDA_ARCH__
     const int n_touched = __popcll(touched);
 #else

@@ -195,6 +195,15 @@ void launch_station_rates(const double *d_fit, int n_st, double *d_rate, double 
 // residuals, NaN where u = 0; d_dropped (may be nullptr) the pairs dropped per set
 void launch_window_closure(const double *d_rd, uint8_t *d_used, uint8_t *d_mask, int n_sets, int stride, int n_st, int dims,
                            double max_resid, int max_drop, double *d_resid, int *d_dropped, cudaStream_t st);
+// the station check of the windowed fixes (tdoa_exclude_stations; exclude.cu), one CTA per set, n_st <= 64, after
+// launch_solve_ls with the same mask and start (d_init may be nullptr: the station mean): d_mask the fix mask (0 /
+// nonzero); d_used (may be nullptr, may be d_mask) gets 3 on the pairs of excluded stations; d_final (may be nullptr)
+// the final 0 / 1 mask; the fix arrays are overwritten where a station is excluded; d_round[set * n_st + k] (uint8)
+// and d_srms[set * n_st + k] (NaN: not a candidate) and d_n_excl may be nullptr
+void launch_window_exclude(const double *d_llh, int n_st, const double *d_rd, const uint8_t *d_mask, uint8_t *d_used,
+                           uint8_t *d_final, int n_sets, int stride, const double *d_init, int dims, double max_rms,
+                           int max_exclude, double *d_out_llh, double *d_rms, int *d_status, int *d_iters, uint8_t *d_round,
+                           double *d_srms, int *d_n_excl, cudaStream_t st);
 struct RetimeJob {
     const float *x;   // one preprocessed plane, n samples
     float *y;         // its re-timed plane (16-byte aligned)

@@ -22,6 +22,10 @@
 // The _closure calls check each window's range differences against each other first (retime.cu):
 //   k_window_closure  one CTA per TGT window: drops the pairs the window's other pairs contradict, into a separate
 //                     0 / 1 mask that k_grid_rows and k_solve_ls read in place of the used mask.
+// The _exclude calls check each window's fix for one wrong station after it (exclude.cu):
+//   k_window_exclude  one CTA per TGT window: solves again without each station in turn and excludes the station
+//                     whose solve fits best, while the fix's rms exceeds max_rms; with a grid, k_grid_rows and the
+//                     grid search run again on the final mask and k_solve_ls fixes every window from that seed.
 // tdoa_process_windows_retimed runs the REF pair loop, k_window_ref_fit and k_station_rates (retime.cu) before the TGT
 // pair loop, which re-times every plane by its station's rate; the fix stage is the same.
 // Window times and the usable test are stated in include/tdoa_b200.h (tdoa_process_windows).
@@ -210,6 +214,22 @@ struct Closure {
     int32_t *dropped = nullptr;
 };
 
+// the station check of the _exclude calls: options and optional outputs
+struct Exclusion {
+    const tdoa_exclusion_opts *opts = nullptr;   // nullptr: no check
+    uint8_t *round = nullptr;
+    double *rms = nullptr;
+    int32_t *excluded = nullptr;
+};
+
+int exclusion_opts_check(tdoa_engine *e, const char *fn, const tdoa_exclusion_opts *x)
+{
+    if (!x) return fail(e, TDOA_E_INVALID, "%s: exclusion options are NULL", fn);
+    if (!(x->max_rms > 0.0)) return fail(e, TDOA_E_INVALID, "%s: max_rms must be > 0, got %g", fn, x->max_rms);
+    if (x->max_exclude < 0) return fail(e, TDOA_E_INVALID, "%s: max_exclude must be >= 0, got %d", fn, x->max_exclude);
+    return TDOA_OK;
+}
+
 int closure_opts_check(tdoa_engine *e, const char *fn, const tdoa_closure_opts *c)
 {
     if (!c) return fail(e, TDOA_E_INVALID, "%s: closure options are NULL", fn);
@@ -221,7 +241,7 @@ int closure_opts_check(tdoa_engine *e, const char *fn, const tdoa_closure_opts *
 // grid: the seed of the _grid calls, nullptr without
 int window_check(tdoa_engine *e, const char *fn, const double *stations_llh, const tdoa_window_opts *o, const WinGeom &ref,
                  const WinGeom &tgt, const double *fix_llh, const int32_t *fix_status, const GridSeed *grid, WinTimes &T,
-                 const Closure &closure)
+                 const Closure &closure, const Exclusion &exclusion)
 {
     const int32_t n_ref = ref.n, n_tgt = tgt.n;
     const int S = e->cfg.n_stations;
@@ -236,6 +256,7 @@ int window_check(tdoa_engine *e, const char *fn, const double *stations_llh, con
         return fail(e, TDOA_E_INVALID, "%s: need >= 1 REF and >= 1 TGT window, got %d and %d", fn, n_ref, n_tgt);
     int rc;
     if (closure.opts && (rc = closure_opts_check(e, fn, closure.opts))) return rc;
+    if (exclusion.opts && (rc = exclusion_opts_check(e, fn, exclusion.opts))) return rc;
     T.n_ref = n_ref; T.n_tgt = n_tgt;
     T.parts.assign(2, ShardPart{});
     for (int kind = 0; kind < 2; kind++) {
@@ -265,8 +286,10 @@ int window_check(tdoa_engine *e, const char *fn, const double *stations_llh, con
 // seed's check) and holds nothing more
 int fix_stage(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts *o, const WinTimes &T, const PeakRec *d_ref,
               const PeakRec *d_tgt, double *ref_fit, double *range_diffs, uint8_t *pair_used, double *fix_llh, double *fix_rms,
-              int32_t *fix_status, int32_t *fix_iters, const GridSeed *grid, const Closure &closure, bool *synced)
+              int32_t *fix_status, int32_t *fix_iters, const GridSeed *grid, const Closure &closure,
+              const Exclusion &exclusion, bool *synced)
 {
+    const tdoa_exclusion_opts *X = exclusion.opts;
     *synced = false;
     const GridSeed G = grid ? *grid : GridSeed{};
     const int S = e->cfg.n_stations, P = S * (S - 1) / 2, nt = T.n_tgt;
@@ -308,9 +331,18 @@ int fix_stage(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts
         ((rc = alloc_t(e, &d_fix_used, (size_t)nt * P)) || (rc = alloc_t(e, &d_cresid, (size_t)nt * P)) ||
          (rc = alloc_t(e, &d_dropped, (size_t)nt))))
         return rc;
-    // the grid seed: the windows' start points (written by the grid where it finds a cell), the masked rows
-    GridSearch g;
-    double *d_start = nullptr, *d_tab = nullptr;
+    // the station check: rounds and rms per (window, station), stations excluded per window
+    uint8_t *d_round = nullptr;
+    double *d_srms = nullptr;
+    int *d_n_excl = nullptr;
+    if (X && ((rc = alloc_t(e, &d_round, (size_t)nt * S)) || (rc = alloc_t(e, &d_srms, (size_t)nt * S)) ||
+              (rc = alloc_t(e, &d_n_excl, (size_t)nt))))
+        return rc;
+    // the grid seed: the windows' start points (written by the grid where it finds a cell), the masked rows; with the
+    // station check, a second search (g2) on the check's final mask, into the same start points
+    GridSearch g, g2;
+    double *d_start = nullptr, *d_tab = nullptr, *d_tab2 = nullptr;
+    uint8_t *d_final = nullptr;
     if (G.desc) {
         const double *d_desc = nullptr;
         if ((rc = upload(e, std::vector<double>(G.desc, G.desc + 7), &d_desc)) || (rc = alloc_t(e, &d_start, (size_t)3 * nt)) ||
@@ -319,7 +351,16 @@ int fix_stage(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts
             return rc;
         g.d_llh = d_llh; g.d_desc = d_desc; g.d_tab = d_tab; g.d_rd = d_rd; g.d_used = d_fix_used; g.d_out = d_start;
         g.n_sets = nt; g.rd_stride = P; g.n_st = S; g.nlat = (int)G.desc[4]; g.nlon = (int)G.desc[5];
+        if (X) {
+            g2 = g;
+            if ((rc = alloc_t(e, &d_final, (size_t)nt * P)) ||
+                (rc = alloc_t(e, &d_tab2, (size_t)nt * grid_rank_tab_doubles(true))) || (rc = alloc_t(e, &g2.d_cost, (size_t)nt)) ||
+                (rc = alloc_t(e, &g2.d_idx, (size_t)nt)))
+                return rc;
+            g2.d_tab = d_tab2; g2.d_used = d_final;
+        }
     }
+    const GridSearch &g_seed = G.desc && X ? g2 : g;   // the search whose arg-min the seed outputs report
     // the grid (ranked, or every cell) between the range differences and the fixes
     auto seed_and_fix = [&](bool every_cell) -> int {
         if (G.desc) {
@@ -329,6 +370,22 @@ int fix_stage(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts
         launch_solve_ls(d_llh, S, d_rd, nt, P, G.desc ? d_start : d_init, o->dims, d_fix, d_rms, d_status, d_iters, e->stream,
                         d_fix_used);
         count_launch(e);
+        if (X) {
+            // d_used gets 3 on the excluded stations' pairs; without the closure check it is the fix mask itself,
+            // which a rerun then reads as before (3 is in the mask as 1 is)
+            launch_window_exclude(d_llh, S, d_rd, d_fix_used, d_used, d_final, nt, P, G.desc ? d_start : d_init, o->dims,
+                                  X->max_rms, X->max_exclude, d_fix, d_rms, d_status, d_iters, d_round, d_srms, d_n_excl,
+                                  e->stream);
+            count_launch(e);
+            if (G.desc) {   // seeded again from the grid arg-min over the final mask (the same seed where none is excluded)
+                CU(cudaMemcpyAsync(d_start, d_init, (size_t)3 * nt * sizeof(double), cudaMemcpyDeviceToDevice, e->stream));
+                launch_grid_rows(d_rd, d_final, nt, P, S, o->dims, d_tab2, e->stream);
+                count_launch(e);
+                if (const int rc2 = grid_search_queue(e, g2, every_cell)) return rc2;
+                launch_solve_ls(d_llh, S, d_rd, nt, P, d_start, o->dims, d_fix, d_rms, d_status, d_iters, e->stream, d_final);
+                count_launch(e);
+            }
+        }
         CU(cudaEventRecord(e->ev[2], e->stream));
         CU(cudaGetLastError());
         return TDOA_OK;
@@ -344,8 +401,14 @@ int fix_stage(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts
             (rc2 = back(fix_iters, d_iters, (size_t)nt * sizeof(int32_t))))
             return rc2;
         if (G.desc &&
-            ((rc2 = back(G.llh, d_start, (size_t)3 * nt * sizeof(double))) || (rc2 = back(G.cost, g.d_cost, (size_t)nt * sizeof(double))) ||
-             (rc2 = back(G.index, g.d_idx, (size_t)nt * sizeof(int64_t)))))
+            ((rc2 = back(G.llh, d_start, (size_t)3 * nt * sizeof(double))) ||
+             (rc2 = back(G.cost, g_seed.d_cost, (size_t)nt * sizeof(double))) ||
+             (rc2 = back(G.index, g_seed.d_idx, (size_t)nt * sizeof(int64_t)))))
+            return rc2;
+        if (X && ((rc2 = back(pair_used, d_used, (size_t)nt * P)) ||
+                  (rc2 = back(exclusion.round, d_round, (size_t)nt * S)) ||
+                  (rc2 = back(exclusion.rms, d_srms, (size_t)nt * S * sizeof(double))) ||
+                  (rc2 = back(exclusion.excluded, d_n_excl, (size_t)nt * sizeof(int32_t)))))
             return rc2;
         return TDOA_OK;
     };
@@ -365,7 +428,7 @@ int fix_stage(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts
     }
     if ((rc = seed_and_fix(false))) return rc;
     if ((rc = back(ref_fit, d_ref_fit, (size_t)3 * P * sizeof(double))) ||
-        (rc = back(range_diffs, d_rd, (size_t)nt * P * sizeof(double))) || (rc = back(pair_used, d_used, (size_t)nt * P)) ||
+        (rc = back(range_diffs, d_rd, (size_t)nt * P * sizeof(double))) || (!X && (rc = back(pair_used, d_used, (size_t)nt * P))) ||
         (closure.opts && ((rc = back(closure.resid, d_cresid, (size_t)nt * P * sizeof(double))) ||
                           (rc = back(closure.dropped, d_dropped, (size_t)nt * sizeof(int32_t))))) ||
         (rc = results()))
@@ -374,13 +437,14 @@ int fix_stage(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts
         // the grid's check after the call's one synchronisation; its pageable read-back returns only when done, so
         // it is queued behind the fixes
         std::vector<int> h_status((size_t)nt);
-        if ((rc = grid_search_fetch(e, g))) return rc;
+        if ((rc = grid_search_fetch(e, g)) || (X && (rc = grid_search_fetch(e, g2)))) return rc;
         CU(cudaMemcpyAsync(h_status.data(), d_status, (size_t)nt * sizeof(int), cudaMemcpyDeviceToHost, e->stream));
         CU(cudaStreamSynchronize(e->stream));
         *synced = true;
+        // an exclusion keeps the status-2 rule, so both searches searched the same windows
         std::vector<char> searched((size_t)nt);
         for (int w = 0; w < nt; w++) searched[w] = h_status[w] != 2;
-        if (!grid_search_complete(g, searched)) {
+        if (!grid_search_complete(g, searched) || (X && !grid_search_complete(g2, searched))) {
             if ((rc = seed_and_fix(true)) || (rc = results())) return rc;
             *synced = false;
         }
@@ -434,14 +498,14 @@ int window_fixes_impl(tdoa_engine *e, const char *fn, const double *stations_llh
                       int64_t win_len, int32_t n_ref_windows, int32_t n_tgt_windows, int64_t hop, const tdoa_peak *ref_in,
                       const tdoa_peak *tgt_in, double *ref_fit, double *range_diffs, uint8_t *pair_used, double *fix_llh,
                       double *fix_rms, int32_t *fix_status, int32_t *fix_iters, const GridSeed *grid,
-                      const Closure &closure = Closure{})
+                      const Closure &closure = Closure{}, const Exclusion &exclusion = Exclusion{})
 {
     if (!e) return TDOA_E_INVALID;
     int rc = begin_call(e);
     if (rc) return rc;
     WinTimes T;
     if ((rc = window_check(e, fn, stations_llh, o, WinGeom{win_start, win_len, n_ref_windows, hop},
-                          WinGeom{win_start, win_len, n_tgt_windows, hop}, fix_llh, fix_status, grid, T, closure)))
+                          WinGeom{win_start, win_len, n_tgt_windows, hop}, fix_llh, fix_status, grid, T, closure, exclusion)))
         return rc;
     if (!ref_in || !tgt_in) return fail(e, TDOA_E_INVALID, "%s: a table is NULL", fn);
     const int S = e->cfg.n_stations, P = S * (S - 1) / 2;
@@ -451,7 +515,7 @@ int window_fixes_impl(tdoa_engine *e, const char *fn, const double *stations_llh
     CU(cudaMemcpyAsync(d_tgt, tgt_in, (size_t)n_tgt_windows * P * sizeof(PeakRec), cudaMemcpyHostToDevice, e->stream));
     bool synced = false;
     if ((rc = fix_stage(e, stations_llh, o, T, d_ref, d_tgt, ref_fit, range_diffs, pair_used, fix_llh, fix_rms, fix_status,
-                        fix_iters, grid, closure, &synced)))
+                        fix_iters, grid, closure, exclusion, &synced)))
         return rc;
     return finish_fix_stage(e, synced);
 }
@@ -462,13 +526,13 @@ int process_windows_impl(tdoa_engine *e, const char *fn, const double *stations_
                          const WinGeom &ref, const WinGeom &tgt, tdoa_peak *ref_out, tdoa_peak *tgt_out, double *ref_fit,
                          double *range_diffs, uint8_t *pair_used, double *fix_llh, double *fix_rms, int32_t *fix_status,
                          int32_t *fix_iters, const GridSeed *grid, bool retimed, double *clock_rate,
-                         const Closure &closure = Closure{})
+                         const Closure &closure = Closure{}, const Exclusion &exclusion = Exclusion{})
 {
     if (!e) return TDOA_E_INVALID;
     int rc = begin_call(e);
     if (rc) return rc;
     WinTimes T;
-    if ((rc = window_check(e, fn, stations_llh, o, ref, tgt, fix_llh, fix_status, grid, T, closure))) return rc;
+    if ((rc = window_check(e, fn, stations_llh, o, ref, tgt, fix_llh, fix_status, grid, T, closure, exclusion))) return rc;
     const int S = e->cfg.n_stations, P = S * (S - 1) / 2;
     Tables tab{e->stream};
     CU(cudaMallocAsync(reinterpret_cast<void **>(&tab.ref), (size_t)ref.n * P * sizeof(PeakRec), e->stream));
@@ -510,7 +574,7 @@ int process_windows_impl(tdoa_engine *e, const char *fn, const double *stations_
         CU(cudaMemcpyAsync(clock_rate, tab.rates + S, (size_t)S * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
     bool synced = false;
     if ((rc = fix_stage(e, stations_llh, o, T, tab.ref, tab.tgt, ref_fit, range_diffs, pair_used, fix_llh, fix_rms, fix_status,
-                        fix_iters, grid, closure, &synced)))
+                        fix_iters, grid, closure, exclusion, &synced)))
         return rc;
     return finish_fix_stage(e, synced);
 }
@@ -609,6 +673,100 @@ int tdoa_window_fixes_closure(tdoa_engine *e, const double *stations_llh, const 
     return window_fixes_impl(e, fn, stations_llh, o, win_start, win_len, n_ref_windows, n_tgt_windows, hop, ref_in, tgt_in,
                              ref_fit, range_diffs, pair_used, fix_llh, fix_rms, fix_status, fix_iters,
                              grid_desc ? &G : nullptr, Closure{c, closure_resid, n_dropped});
+}
+
+int tdoa_process_windows_exclude(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts *o,
+                                 const tdoa_closure_opts *c, const tdoa_exclusion_opts *x, int64_t ref_win_start,
+                                 int64_t ref_win_len, int32_t n_ref_windows, int64_t ref_hop, int64_t tgt_win_start,
+                                 int64_t tgt_win_len, int32_t n_tgt_windows, int64_t tgt_hop, int32_t retimed,
+                                 const double *grid_desc, tdoa_peak *ref_out, tdoa_peak *tgt_out, double *ref_fit,
+                                 double *range_diffs, uint8_t *pair_used, double *closure_resid, int32_t *n_dropped,
+                                 uint8_t *station_round, double *station_rms, int32_t *n_excluded, double *fix_llh,
+                                 double *fix_rms, int32_t *fix_status, int32_t *fix_iters, double *clock_rate,
+                                 double *seed_llh, double *seed_cost, int64_t *seed_index)
+{
+    static const char *fn = "tdoa_process_windows_exclude";
+    if (!e) return TDOA_E_INVALID;
+    if (!x) return fail(e, TDOA_E_INVALID, "%s: exclusion options are NULL", fn);
+    if (retimed != 0 && retimed != 1) return fail(e, TDOA_E_INVALID, "%s: retimed must be 0 or 1, got %d", fn, retimed);
+    const GridSeed G{grid_desc, seed_llh, seed_cost, seed_index};
+    return process_windows_impl(e, fn, stations_llh, o, WinGeom{ref_win_start, ref_win_len, n_ref_windows, ref_hop},
+                                WinGeom{tgt_win_start, tgt_win_len, n_tgt_windows, tgt_hop}, ref_out, tgt_out, ref_fit,
+                                range_diffs, pair_used, fix_llh, fix_rms, fix_status, fix_iters, grid_desc ? &G : nullptr,
+                                retimed == 1, clock_rate, Closure{c, closure_resid, n_dropped},
+                                Exclusion{x, station_round, station_rms, n_excluded});
+}
+
+int tdoa_window_fixes_exclude(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts *o,
+                              const tdoa_closure_opts *c, const tdoa_exclusion_opts *x, int64_t win_start, int64_t win_len,
+                              int32_t n_ref_windows, int32_t n_tgt_windows, int64_t hop, const double *grid_desc,
+                              const tdoa_peak *ref_in, const tdoa_peak *tgt_in, double *ref_fit, double *range_diffs,
+                              uint8_t *pair_used, double *closure_resid, int32_t *n_dropped, uint8_t *station_round,
+                              double *station_rms, int32_t *n_excluded, double *fix_llh, double *fix_rms,
+                              int32_t *fix_status, int32_t *fix_iters, double *seed_llh, double *seed_cost,
+                              int64_t *seed_index)
+{
+    static const char *fn = "tdoa_window_fixes_exclude";
+    if (!e) return TDOA_E_INVALID;
+    if (!x) return fail(e, TDOA_E_INVALID, "%s: exclusion options are NULL", fn);
+    const GridSeed G{grid_desc, seed_llh, seed_cost, seed_index};
+    return window_fixes_impl(e, fn, stations_llh, o, win_start, win_len, n_ref_windows, n_tgt_windows, hop, ref_in, tgt_in,
+                             ref_fit, range_diffs, pair_used, fix_llh, fix_rms, fix_status, fix_iters,
+                             grid_desc ? &G : nullptr, Closure{c, closure_resid, n_dropped},
+                             Exclusion{x, station_round, station_rms, n_excluded});
+}
+
+int tdoa_exclude_stations(tdoa_engine *e, const double *stations_llh, int32_t n_stations, const double *range_diffs,
+                          const uint8_t *used, int32_t n_sets, int32_t rd_stride, const double *init_llh, int32_t dims,
+                          const tdoa_exclusion_opts *x, uint8_t *out_used, uint8_t *station_round, double *station_rms,
+                          int32_t *n_excluded, double *out_llh, double *out_rms, int32_t *status, int32_t *iters)
+{
+    static const char *fn = "tdoa_exclude_stations";
+    if (!e) return TDOA_E_INVALID;
+    int rc = begin_call(e);
+    if (rc) return rc;
+    const int S = n_stations, P = S * (S - 1) / 2;
+    if (!stations_llh || !range_diffs || !used || !out_used || !out_llh || !status)
+        return fail(e, TDOA_E_INVALID, "%s: NULL argument", fn);
+    if (S < 3 || S > solve_ls_max_stations())
+        return fail(e, TDOA_E_INVALID, "%s: 3..%d stations, got %d", fn, solve_ls_max_stations(), S);
+    if (dims != 2 && dims != 3) return fail(e, TDOA_E_INVALID, "%s: dims must be 2 or 3, got %d", fn, dims);
+    if (n_sets < 0 || rd_stride < P)
+        return fail(e, TDOA_E_INVALID, "%s: n_sets >= 0 and rd_stride >= %d, got %d and %d", fn, P, n_sets, rd_stride);
+    if ((rc = exclusion_opts_check(e, fn, x))) return rc;
+    if (n_sets == 0) return end_call(e, true);
+    const size_t n = (size_t)n_sets * rd_stride, ns = (size_t)n_sets;
+    double *d_rd = nullptr, *d_init = nullptr, *d_fix = nullptr, *d_rms = nullptr, *d_srms = nullptr;
+    const double *d_llh = nullptr;
+    uint8_t *d_used = nullptr, *d_round = nullptr;
+    int *d_status = nullptr, *d_iters = nullptr, *d_n_excl = nullptr;
+    if ((rc = upload(e, std::vector<double>(stations_llh, stations_llh + (size_t)3 * S), &d_llh)) ||
+        (rc = alloc_t(e, &d_rd, n)) || (rc = alloc_t(e, &d_used, n)) || (rc = alloc_t(e, &d_fix, 3 * ns)) ||
+        (rc = alloc_t(e, &d_rms, ns)) || (rc = alloc_t(e, &d_status, ns)) || (rc = alloc_t(e, &d_iters, ns)) ||
+        (rc = alloc_t(e, &d_round, ns * S)) || (rc = alloc_t(e, &d_srms, ns * S)) || (rc = alloc_t(e, &d_n_excl, ns)))
+        return rc;
+    CU(cudaMemcpyAsync(d_rd, range_diffs, n * sizeof(double), cudaMemcpyHostToDevice, e->stream));
+    CU(cudaMemcpyAsync(d_used, used, n, cudaMemcpyHostToDevice, e->stream));
+    if (init_llh) {
+        if ((rc = alloc_t(e, &d_init, 3 * ns))) return rc;
+        CU(cudaMemcpyAsync(d_init, init_llh, 3 * ns * sizeof(double), cudaMemcpyHostToDevice, e->stream));
+    }
+    // F: the fix without the check; then the check, which marks d_used (the mask it reads) in place
+    launch_solve_ls(d_llh, S, d_rd, n_sets, rd_stride, d_init, dims, d_fix, d_rms, d_status, d_iters, e->stream, d_used);
+    launch_window_exclude(d_llh, S, d_rd, d_used, d_used, nullptr, n_sets, rd_stride, d_init, dims, x->max_rms, x->max_exclude,
+                          d_fix, d_rms, d_status, d_iters, d_round, d_srms, d_n_excl, e->stream);
+    count_launch(e, 2);
+    CU(cudaGetLastError());
+    // the first P slots of each set only: the rest of the caller's rows are left as they are
+    CU(cudaMemcpy2DAsync(out_used, rd_stride, d_used, rd_stride, P, n_sets, cudaMemcpyDeviceToHost, e->stream));
+    CU(cudaMemcpyAsync(out_llh, d_fix, 3 * ns * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
+    CU(cudaMemcpyAsync(status, d_status, ns * sizeof(int32_t), cudaMemcpyDeviceToHost, e->stream));
+    if (out_rms) CU(cudaMemcpyAsync(out_rms, d_rms, ns * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
+    if (iters) CU(cudaMemcpyAsync(iters, d_iters, ns * sizeof(int32_t), cudaMemcpyDeviceToHost, e->stream));
+    if (station_round) CU(cudaMemcpyAsync(station_round, d_round, ns * S, cudaMemcpyDeviceToHost, e->stream));
+    if (station_rms) CU(cudaMemcpyAsync(station_rms, d_srms, ns * S * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
+    if (n_excluded) CU(cudaMemcpyAsync(n_excluded, d_n_excl, ns * sizeof(int32_t), cudaMemcpyDeviceToHost, e->stream));
+    return end_call(e, true);
 }
 
 int tdoa_closure(tdoa_engine *e, int32_t n_stations, const double *range_diffs, const uint8_t *used, int32_t n_sets,
