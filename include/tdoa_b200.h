@@ -170,6 +170,38 @@ TDOA_API int tdoa_unpack(tdoa_engine *e, int32_t station, int64_t first, int64_t
 TDOA_API int tdoa_preprocess(tdoa_engine *e, int32_t station, int32_t kind, int64_t start, int64_t len,
                              float *out_c64, double *power, int32_t *branch);
 
+/* Channel filter (EXTENDED mode, engine-defined; the reference has none): a complex FIR with the caller's taps,
+ * per signal kind, applied to a signal's unpacked samples before preprocessSignal.  An RTL-SDR capture is 2 MHz
+ * wide and the discriminator follows the strongest carrier in it, so a stronger station in an adjacent channel
+ * (or the wanted one tuned off-centre, away from the DC spike) gives the other programme's lags.  A band-pass
+ * around the wanted station recovers it, as any FM receiver does.
+ *
+ * For one signal -- a REF or TGT view or window, after guard_samples, in view order (a REF view filters across
+ * the block 1 | block 3 joint, as the box-car does) -- with x[0..n) its unpacked samples (as loadIQData), the
+ * kind's taps h[0..T) (f32 re / im, T odd, 1 <= T <= 127) and c = (T - 1) / 2:
+ *   for every i in [0, n): acc_r = acc_i = +0; for k = 0 .. T-1 ascending, v = x[i + c - k] (+0 + 0j outside
+ *   [0, n)):  acc_r = fmaf(hr[k], vr, acc_r); acc_r = fmaf(-hi[k], vi, acc_r);
+ *             acc_i = fmaf(hr[k], vi, acc_i); acc_i = fmaf(hi[k], vr, acc_i);
+ *   y[i] = acc.
+ * The signal IS y from then on: BINARY preprocessing runs on it exactly as on unpacked samples, its power picks
+ * the branch, and tdoa_xcorr_info reports y's power and DC.  Every other stage (DC, box-car, normalisation,
+ * decimator, correlators, fits, re-timing, checks) is unchanged.
+ * - The taps are the same for every station of a kind: their delay is common to both stations of every pair and
+ *   cancels in every lag; window times are unchanged.
+ * - A band-pass centred at f0 adds the constant 2 pi f0 / fs to the discriminator output; the strong branch's DC
+ *   removal takes it out.
+ * - Co-channel interference (another programme on the same frequency) is not helped; that is the station check's
+ *   job (tdoa_exclude_stations).
+ * It applies to every signal the engine cuts from its captures: tdoa_xcorr*, tdoa_process, every
+ * tdoa_process_windows* (including _retimed, which re-times the filtered chain's plane) and tdoa_preprocess; not to
+ * tdoa_cross_correlate or tdoa_analyze.  With no channel set every call runs as before.  taps_im may be NULL (real
+ * taps); n_taps = 0 clears the kind's channel.  Setting or clearing resets the kind's remembered branches.  A
+ * capture still arriving (tdoa_load_u8_pinned) is waited for as a whole before it is filtered.  An n_devices > 1
+ * engine sets every device; with tdoa_comm_init each rank sets its own.  Refused (TDOA_E_INVALID): a mode other
+ * than EXTENDED, a kind other than 0 or 1, n_taps < 0, even or > 127, a NULL taps_re with n_taps > 0, a NaN,
+ * infinite or subnormal tap. */
+TDOA_API int tdoa_set_channel(tdoa_engine *e, int32_t kind, const float *taps_re, const float *taps_im, int32_t n_taps);
+
 /* ProcessTDOA pair loops (processor.go:816-850): correlates every station pair i<j
  * (lexicographic, = argv order) of `kind` over n_windows windows
  * [win_start + w*hop, +win_len).  win_len = 0 means the config's chunk (0 = whole

@@ -17,6 +17,7 @@ from ._native import (  # noqa: F401
     KIND_REF,
     KIND_TGT,
     default_config,
+    channel_taps,
     library_path,
     load_library,
     host_alloc,
@@ -31,5 +32,5 @@ from . import analyzer  # noqa: F401
 
 __all__ = [
     "Engine", "TdoaError", "Peak", "MODE_SOURCE", "MODE_BINARY", "MODE_EXTENDED", "KIND_REF", "KIND_TGT",
-    "default_config", "library_path", "load_library", "host_alloc", "comm_unique_id", "PEAK_DTYPE", "PEAK_EDGE", "PEAK_EMPTY", "Station", "TDOAProcessor", "sharding", "analyzer",
+    "default_config", "channel_taps", "library_path", "load_library", "host_alloc", "comm_unique_id", "PEAK_DTYPE", "PEAK_EDGE", "PEAK_EMPTY", "Station", "TDOAProcessor", "sharding", "analyzer",
 ]

@@ -23,7 +23,7 @@ ERRORS = {-1: "TDOA_E_INVALID", -2: "TDOA_E_NODEVICE", -3: "TDOA_E_CUDA", -4: "T
 # every symbol include/tdoa_b200.h declares (tests check the library exports them all)
 ABI_SYMBOLS = [
     "tdoa_default_config", "tdoa_create", "tdoa_destroy", "tdoa_last_error", "tdoa_host_alloc", "tdoa_host_free",
-    "tdoa_load_u8", "tdoa_load_file", "tdoa_load_u8_pinned", "tdoa_load_u8_device", "tdoa_unpack", "tdoa_preprocess", "tdoa_xcorr", "tdoa_xcorr_device", "tdoa_xcorr_windows", "tdoa_process", "tdoa_process_windows", "tdoa_window_fixes", "tdoa_process_windows_grid", "tdoa_window_fixes_grid", "tdoa_process_windows_retimed", "tdoa_closure", "tdoa_process_windows_closure", "tdoa_window_fixes_closure", "tdoa_exclude_stations", "tdoa_process_windows_exclude", "tdoa_window_fixes_exclude", "tdoa_xcorr_info", "tdoa_analyze",
+    "tdoa_load_u8", "tdoa_load_file", "tdoa_load_u8_pinned", "tdoa_load_u8_device", "tdoa_unpack", "tdoa_preprocess", "tdoa_set_channel", "tdoa_xcorr", "tdoa_xcorr_device", "tdoa_xcorr_windows", "tdoa_process", "tdoa_process_windows", "tdoa_window_fixes", "tdoa_process_windows_grid", "tdoa_window_fixes_grid", "tdoa_process_windows_retimed", "tdoa_closure", "tdoa_process_windows_closure", "tdoa_window_fixes_closure", "tdoa_exclude_stations", "tdoa_process_windows_exclude", "tdoa_window_fixes_exclude", "tdoa_xcorr_info", "tdoa_analyze",
     "tdoa_cross_correlate", "tdoa_baselines", "tdoa_solve", "tdoa_solve_binary", "tdoa_solve_ls", "tdoa_grid", "tdoa_grid_masked", "tdoa_get_stats", "tdoa_stream",
     "tdoa_set_stream", "tdoa_synchronize", "tdoa_selftest",
     "tdoa_comm_unique_id", "tdoa_comm_init", "tdoa_comm_rank", "tdoa_shard_windows",
@@ -170,6 +170,7 @@ def load_library():
     L.tdoa_load_u8_device.argtypes = [vp, i32, vp, C.c_size_t]
     L.tdoa_unpack.argtypes = [vp, i32, i64, i64, vp]
     L.tdoa_preprocess.argtypes = [vp, i32, i32, i64, i64, vp, f64p, C.POINTER(i32)]
+    L.tdoa_set_channel.argtypes = [vp, i32, vp, vp, i32]
     L.tdoa_xcorr.argtypes = [vp, i32, i64, i64, i32, i64, vp]
     L.tdoa_xcorr_info.argtypes = [vp, i32, vp, vp]
     L.tdoa_process.argtypes = [vp, vp, vp, vp, vp, vp, vp, C.POINTER(i32), C.POINTER(i32)]
@@ -209,6 +210,23 @@ def load_library():
     L.tdoa_shard_windows.argtypes = [i32, i32, i32, i32, C.POINTER(i32), C.POINTER(i32)]
     _lib = L
     return L
+
+
+def channel_taps(offset_hz: float, half_width_hz: float, n_taps: int = 63, fs: float = 2e6) -> np.ndarray:
+    """Taps for Engine.set_channel: a Blackman-windowed sinc low-pass with unit DC gain whose -6 dB point is
+    half_width_hz (the window's transition is symmetric about the sinc's cut-off), modulated to offset_hz about
+    the centre tap, so the pass band is offset_hz +- half_width_hz with zero phase at its centre.  Designed in f64
+    and rounded to complex64.  The transition is about +-2.75 fs / n_taps wide; the stop band lies below -60 dB."""
+    if n_taps < 1 or n_taps % 2 == 0 or n_taps > 127:
+        raise ValueError("n_taps must be odd, 1..127")
+    c = (n_taps - 1) // 2
+    k = np.arange(n_taps, dtype=np.float64) - c
+    g = np.sinc(2.0 * half_width_hz / fs * k)
+    if n_taps > 1:
+        a = 2.0 * np.pi * np.arange(n_taps) / (n_taps - 1)
+        g = g * (0.42 - 0.5 * np.cos(a) + 0.08 * np.cos(2.0 * a))
+    g = g / g.sum()
+    return (g * np.exp(2j * np.pi * offset_hz / fs * k)).astype(np.complex64)
 
 
 def default_config(mode: int, **overrides) -> Config:
@@ -395,6 +413,20 @@ class Engine:
         if self.cfg.mode == MODE_EXTENDED and self.cfg.decimate > 1:
             out = out[:length // self.cfg.decimate]
         return out, power.value, branch.value
+
+    def set_channel(self, kind: int, taps) -> None:
+        """Channel filter of `kind` (EXTENDED mode, tdoa_set_channel): a complex FIR over every signal's unpacked
+        samples ahead of preprocessing.  taps: a real or complex 1-D array of odd length <= 127 (rounded to f32,
+        e.g. channel_taps(...)), or None to clear."""
+        if taps is None:
+            self._check(self._lib.tdoa_set_channel(self._h, kind, None, None, 0))
+            return
+        t = np.asarray(taps)
+        if t.ndim != 1:
+            raise ValueError("taps must be a 1-D array")
+        re = np.ascontiguousarray(t.real, np.float32)
+        im = np.ascontiguousarray(t.imag, np.float32) if np.iscomplexobj(t) else None
+        self._check(self._lib.tdoa_set_channel(self._h, kind, _ptr(re), _ptr(im) if im is not None else None, t.size))
 
     # -- ProcessTDOA pair loops (processor.go:816-850)
     def xcorr(self, kind: int, win_start: int = 0, win_len: int = 0, n_windows: int = 1, hop: int = 0) -> np.ndarray:

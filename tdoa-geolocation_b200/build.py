@@ -25,6 +25,7 @@ UNITS = [
     ("preprocess.cu", ["-fmad=false"]),
     ("preprocess_fast.cu", []),
     ("preprocess_weak.cu", ["-fmad=false"]),
+    ("channel.cu", ["-fmad=false"]),
     ("seqsum.cu", ["-fmad=false"]),
     ("xcorr_exact.cu", ["-fmad=false"]),
     ("solve.cu", ["-fmad=false"]),

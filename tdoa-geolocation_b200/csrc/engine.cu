@@ -614,6 +614,38 @@ int tdoa_load_u8_device(tdoa_engine *e, int32_t station, const uint8_t *d_iq, si
     return TDOA_OK;
 }
 
+int tdoa_set_channel(tdoa_engine *e, int32_t kind, const float *taps_re, const float *taps_im, int32_t n_taps)
+{
+    if (!e) return TDOA_E_INVALID;
+    int rc = begin_call(e);
+    if (rc) return rc;
+    if (e->cfg.mode != TDOA_MODE_EXTENDED)
+        return fail(e, TDOA_E_INVALID, "tdoa_set_channel: the channel filter is an EXTENDED-mode option");
+    if (kind != TDOA_KIND_REF && kind != TDOA_KIND_TGT) return fail(e, TDOA_E_INVALID, "tdoa_set_channel: bad kind %d", kind);
+    if (n_taps < 0 || n_taps > kChannelMaxTaps || (n_taps > 0 && n_taps % 2 == 0))
+        return fail(e, TDOA_E_INVALID, "tdoa_set_channel: n_taps must be 0 or odd and at most %d, got %d", kChannelMaxTaps, n_taps);
+    if (n_taps > 0 && !taps_re) return fail(e, TDOA_E_INVALID, "tdoa_set_channel: taps_re is NULL");
+    ChannelTaps t{};
+    bool cplx = false;
+    for (int k = 0; k < n_taps; k++) {
+        const float hr = taps_re[k], hi = taps_im ? taps_im[k] : 0.f;
+        for (const float h : {hr, hi}) {
+            const int c = std::fpclassify(h);
+            if (c != FP_NORMAL && c != FP_ZERO)
+                return fail(e, TDOA_E_INVALID, "tdoa_set_channel: tap %d is NaN, infinite or subnormal", k);
+        }
+        t.re[k] = hr;
+        t.im[k] = hi;
+        cplx |= hi != 0.f;
+    }
+    t.n = n_taps;
+    e->channel[kind] = t;
+    e->channel_cplx[kind] = cplx;
+    // the filter changes the signal's power: the branch seen before is no longer a guess worth making
+    for (int s = 0; s < e->cfg.n_stations; s++) e->branch_memo[(size_t)s * 2 + kind] = -1;
+    return multi_forward_channel(e, kind, taps_re, taps_im, n_taps);
+}
+
 int tdoa_baselines(tdoa_engine *e, const double *stations_llh, int32_t n_stations, double *baselines)
 {
     if (!e) return TDOA_E_INVALID;

@@ -61,6 +61,8 @@ struct Sig {
     bool deferred = false;  // branch 0 was assumed without reading the power back; the caller verifies
     bool raw_sums = false;  // the power pass was k_raw_stats: ST_SUM_* / ST_DC_* of the raw signal are in place
     bool need_im = false;   // a consumer reads out_im of a BINARY / EXTENDED signal (the tdoa_preprocess probe)
+    bool filtered = false;  // the kind's channel filter wrote the signal to planes: ysrc is its source from then on
+    SigSrc ysrc{};
 };
 
 struct Pair {
@@ -104,6 +106,8 @@ struct tdoa_engine {
     float2 *d_tw = nullptr;  // FFT twiddle table
     float2 *d_tw_fine = nullptr;  // W_N^k, k < 2048, of the 2^21-point transform
     std::vector<int8_t> branch_memo;  // last preprocess branch per (station, kind); -1 unknown
+    tdoa::ChannelTaps channel[2] = {};   // per kind (tdoa_set_channel); n = 0: no channel filter
+    bool channel_cplx[2] = {false, false};
     std::vector<tdoa_signal_info> info_sig[2];  // window 0 of the last xcorr per kind
     std::vector<double> info_first[2];
     int sm_count = 148;
@@ -224,5 +228,6 @@ void multi_destroy(tdoa_engine *e);
 int multi_create_peers(tdoa_engine *e, const tdoa_config *cfg);   // tdoa_create with n_devices > 1
 // which: 0 tdoa_load_u8, 1 tdoa_load_u8_pinned, 2 tdoa_load_file (p = path)
 int multi_forward_load(tdoa_engine *e, int which, int32_t station, const void *p, size_t nbytes, int64_t *n_samples);
+int multi_forward_channel(tdoa_engine *e, int32_t kind, const float *taps_re, const float *taps_im, int32_t n_taps);
 
 }  // namespace tdoa

@@ -301,6 +301,19 @@ int multi_forward_load(tdoa_engine *e, int which, int32_t station, const void *p
     return TDOA_OK;
 }
 
+// the same channel filter on every peer of a multi-device engine (a communicator's ranks each set their own)
+int multi_forward_channel(tdoa_engine *e, int32_t kind, const float *taps_re, const float *taps_im, int32_t n_taps)
+{
+    if (!e->multi || e->multi->peers.size() <= 1) return TDOA_OK;
+    for (size_t r = 1; r < e->multi->peers.size(); r++) {
+        tdoa_engine *q = e->multi->peers[r];
+        const int rc = tdoa_set_channel(q, kind, taps_re, taps_im, n_taps);
+        if (rc) { cudaSetDevice(e->device); return fail(e, rc, "device %d: %s", q->device, q->error.c_str()); }
+    }
+    CU(cudaSetDevice(e->device));
+    return TDOA_OK;
+}
+
 }  // namespace tdoa
 
 extern "C" {

@@ -160,7 +160,7 @@ struct Step {  // one batched kernel over a set of signals
 SigJob base_job(const Sig &s)
 {
     SigJob j{};
-    j.src = s.src;
+    j.src = s.filtered ? s.ysrc : s.src;
     j.n = s.n;
     j.stats = s.stats;
     j.partials = s.partials;
@@ -302,6 +302,52 @@ inline int decimation(const tdoa_engine *e) { return e->cfg.mode == TDOA_MODE_EX
 // shipped binary (ELF 0x49cd40): > 0.01 strong, > 0.001 moderate, else weak
 inline int binary_branch(double power0) { return power0 > 0.01 ? 0 : (power0 > 0.001 ? 1 : 2); }
 
+// the channel filter of the signal's kind (tdoa_set_channel; EXTENDED mode only), nullptr: none.  It applies to
+// every capture view; an empty one has nothing to filter.
+inline const ChannelTaps *channel_of(const tdoa_engine *e, const Sig &s)
+{
+    return s.station >= 0 && s.n > 0 && e->channel[s.kind].n > 0 ? &e->channel[s.kind] : nullptr;
+}
+
+// the filtered signal as planes (k_channel): queued per kind in jobs, the signal reads them from then on
+int channel_planes(tdoa_engine *e, Sig &s, std::vector<SigJob> (&jobs)[2])
+{
+    float *yr = nullptr, *yi = nullptr;
+    int rc;
+    if ((rc = alloc_t(e, &yr, (size_t)s.n)) || (rc = alloc_t(e, &yi, (size_t)s.n))) return rc;
+    SigJob j = base_job(s);
+    j.p_re = yr; j.p_im = yi;
+    jobs[s.kind].push_back(j);
+    s.ysrc = SigSrc{};
+    s.ysrc.re = yr; s.ysrc.im = yi;
+    s.filtered = true;
+    return TDOA_OK;
+}
+
+// demod = false: k_channel (planes); true: k_channel_demod, a discriminator launch
+int launch_channels(tdoa_engine *e, const std::vector<SigJob> (&jobs)[2], bool demod)
+{
+    for (int kind = 0; kind < 2; kind++) {
+        if (jobs[kind].empty()) continue;
+        const SigJob *d_jobs = nullptr;
+        if (int rc = upload(e, jobs[kind], &d_jobs)) return rc;
+        i64 max_n = 0;
+        for (const SigJob &j : jobs[kind]) max_n = std::max(max_n, j.n);
+        const ChannelTaps &t = e->channel[kind];
+        if (demod) {
+            const int sp = span_begin(e, SPAN_DEMOD);
+            launch_channel_demod(d_jobs, (int)jobs[kind].size(), max_n, t, e->channel_cplx[kind], e->stream);
+            span_end(e, sp);
+            for (const SigJob &j : jobs[kind]) e->st.demod_samples += j.n;
+        } else {
+            launch_channel(d_jobs, (int)jobs[kind].size(), max_n, t, e->channel_cplx[kind], e->stream);
+        }
+        CU(cudaGetLastError());
+        count_launch(e);
+    }
+    return TDOA_OK;
+}
+
 // Preprocess every signal (preprocessSignal, processor.go:469-499 / ELF 0x49cd40).
 // On return out_re/out_im/stats of each signal are valid on the stream.
 // allow_defer: when every signal runs the speculative fused kernel, do not wait for the
@@ -342,6 +388,9 @@ int preprocess(tdoa_engine *e, std::vector<Sig> &sigs, bool allow_defer = false)
         // follows the copy chunk by chunk, every launch waiting for one chunk only
         struct Follow { SigJob job; cudaEvent_t wait; i64 len; int sig; bool last; int n_sub; double *sums; };
         std::vector<Follow> follow;
+        // channel-filtered signals: the fused filter + discriminator (cdjobs), or the filter to planes (cjobs) whose
+        // power k_power takes (ppjobs: k_raw_stats reads bytes)
+        std::vector<SigJob> cjobs[2], cdjobs[2], ppjobs;
         for (size_t si = 0; si < sigs.size(); si++) {
             Sig &s = sigs[si];
             const bool spec = e->cfg.mode != TDOA_MODE_SOURCE && s.src.raw && s.n >= 2 &&
@@ -349,6 +398,20 @@ int preprocess(tdoa_engine *e, std::vector<Sig> &sigs, bool allow_defer = false)
             s.fused = spec;
             Station *stn = s.station >= 0 ? &e->stations[s.station] : nullptr;
             const bool arriving = stn && !stn->chunks[s.kind].empty();
+            if (channel_of(e, s)) {
+                // every output reads samples on both sides: a capture still arriving is waited for as a whole
+                if (arriving && (rc = wait_kind(e, *stn, s.kind))) return rc;
+                if (spec) {
+                    if ((rc = ensure_plane(e, s, 0, false))) return rc;
+                    SigJob j = base_job(s);
+                    j.p_re = s.plane[0][0];
+                    cdjobs[s.kind].push_back(j);
+                } else {
+                    if ((rc = channel_planes(e, s, cjobs))) return rc;
+                    ppjobs.push_back(base_job(s));
+                }
+                continue;
+            }
             if (spec) {
                 if ((rc = ensure_plane(e, s, 0, false))) return rc;
                 SigJob j = base_job(s);
@@ -403,6 +466,13 @@ int preprocess(tdoa_engine *e, std::vector<Sig> &sigs, bool allow_defer = false)
                 }
             }
         }
+        if ((rc = launch_channels(e, cjobs, false)) || (rc = launch_channels(e, cdjobs, true))) return rc;
+        if (!ppjobs.empty()) {
+            const SigJob *d_jobs = nullptr;
+            if ((rc = upload(e, ppjobs, &d_jobs))) return rc;
+            launch_power(d_jobs, (int)ppjobs.size(), max_n, gx, e->stream);
+            count_launch(e);
+        }
         if (!pjobs.empty()) {
             const SigJob *d_jobs = nullptr;
             if ((rc = upload(e, pjobs, &d_jobs))) return rc;
@@ -421,7 +491,7 @@ int preprocess(tdoa_engine *e, std::vector<Sig> &sigs, bool allow_defer = false)
             for (const SigJob &j : fjobs) e->st.demod_samples += j.n;
             count_launch(e);
         }
-        const bool defer = allow_defer && pjobs.empty();
+        const bool defer = allow_defer && pjobs.empty() && ppjobs.empty();
         (void)follow;
         if (defer) {
             for (auto &s : sigs) s.deferred = true;
@@ -430,6 +500,11 @@ int preprocess(tdoa_engine *e, std::vector<Sig> &sigs, bool allow_defer = false)
             CU(cudaMemcpyAsync(h_stats.data(), d_stats, h_stats.size() * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
             CU(cudaStreamSynchronize(e->stream));
             for (int i = 0; i < ns; i++) sigs[i].power0 = h_stats[(size_t)i * ST_COUNT + ST_POWER0];
+            // a speculated filtered signal off the strong branch: its branch reads the filtered samples
+            for (auto &q : cjobs) q.clear();
+            for (auto &s : sigs)
+                if (s.fused && channel_of(e, s) && binary_branch(s.power0) != 0 && (rc = channel_planes(e, s, cjobs))) return rc;
+            if ((rc = launch_channels(e, cjobs, false))) return rc;
         }
     }
     // ---- per-branch pipelines
@@ -504,7 +579,7 @@ int preprocess(tdoa_engine *e, std::vector<Sig> &sigs, bool allow_defer = false)
                 s.out_re = s.plane[1][0]; s.out_im = nullptr;
             } else {
                 const int w_hp = cutoff_window(100.0), w_lp = cutoff_window(200000.0);
-                if (mode == TDOA_MODE_EXTENDED && s.raw_sums && s.src.raw && !wants_seq_dc(e, s.n) && w_hp >= 3 && w_lp >= 3 &&
+                if (mode == TDOA_MODE_EXTENDED && s.raw_sums && s.src.raw && !s.filtered && !wants_seq_dc(e, s.n) && w_hp >= 3 && w_lp >= 3 &&
                     w_hp / 2 <= weak_fused_max_half_wide() && w_lp / 2 <= weak_fused_max_half_small()) {
                     // the whole chain in one pass over the bytes (preprocess_weak.cu); the imaginary plane only
                     // where somebody reads it (the correlators of this revision take real parts only)

@@ -126,6 +126,20 @@ int boxcar_grid_x(i64 n);
 int stream_grid_x(i64 n);
 int unpack_selftest(cudaStream_t st);  // 0 ok: arithmetic unpack == host LUT for all 256 codes
 
+// ---- channel.cu (EXTENDED mode, tdoa_set_channel): the complex FIR ahead of preprocessSignal
+constexpr int kChannelMaxTaps = 127;
+struct ChannelTaps {   // h[k] = re[k] + i im[k], k < n; n odd, 1..kChannelMaxTaps
+    float re[kChannelMaxTaps + 1];
+    float im[kChannelMaxTaps + 1];
+    int n;
+};
+// capture bytes of jobs[j].src (n samples) -> the filtered signal as planes p_re / p_im; cplx = 0: every im[k] is
+// zero and its FMAs are skipped
+void launch_channel(const SigJob *d_jobs, int n_jobs, i64 max_n, const ChannelTaps &taps, bool cplx, cudaStream_t st);
+// the same filter fused with the discriminator (k_demod's bits on the filtered signal): p_re gets the discriminator
+// output, the statistics block ST_POWER0 (of the filtered signal), ST_SUM_* and ST_DC_* as k_demod leaves them; n >= 2
+void launch_channel_demod(const SigJob *d_jobs, int n_jobs, i64 max_n, const ChannelTaps &taps, bool cplx, cudaStream_t st);
+
 // ---- preprocess_weak.cu (EXTENDED mode, weak branch: two passes over the capture bytes)
 void launch_raw_stats(const SigJob *d_jobs, int n_jobs, i64 max_n, cudaStream_t st);    // ST_POWER0 + ST_SUM_* + ST_DC_*
 void launch_weak_fused(const SigJob *d_jobs, int n_jobs, i64 max_n, cudaStream_t st);   // bytes -> DC, HP(window), LP(window2), power
