@@ -63,13 +63,25 @@ extern "C" {
 
 typedef struct tdoa_engine tdoa_engine; /* opaque: device memory, streams, plans */
 
-/* One correlation peak; 32 bytes; also the record exchanged between GPUs. */
+/* One correlation peak; 32 bytes; also the record exchanged between GPUs.
+ * margin = (|peak| - |runner-up|) / |peak|, rounded to f32, the runner-up being the largest |corr| over every
+ * other lag of the first pass.  On the every-lag path (TDOA_PEAK_BRUTE: use_fft = 0, the candidate-overflow redo)
+ * every |corr| is exact.  On the FFT paths the runner-up is the largest |approximate value| of the f32 ranking
+ * (exact values exist only for the candidates), so the margin differs from the exact one by at most eps / |peak|
+ * plus its rounding, eps (~1e-6 in correlation units) being the ranking's error.  Two tied peaks: margin 0 exactly
+ * on the every-lag path, |margin| <= eps / |peak| on the FFT paths.
+ * Which signal is the template: BINARY and SOURCE make the shorter of the two signals the template
+ * (processor.go:653-661), so with signal 1 longer the lag is the delay of signal 1.  EXTENDED keeps signal 1 as
+ * the template whatever the lengths: with W = min(n1, n2) the search is over the first W samples of both
+ * preprocessed signals (each preprocessed over its own full length) and the lag is always the delay of signal 2,
+ * i.e. d_j - d_i for pair i < j. */
 typedef struct {
-    int32_t lag;       /* integer lag of the peak, samples (delay of signal 2)       */
+    int32_t lag;       /* integer lag of the peak, samples (delay of signal 2; see above) */
     uint32_t flags;    /* TDOA_PEAK_*                                                */
     double corr;       /* correlation at the peak, signed (the Go float64 return)    */
     float frac;        /* sub-sample offset in [-0.5,0.5]; 0 in SOURCE/BINARY modes  */
-    float margin;      /* (|peak|-|runner-up|)/|peak| among exactly evaluated lags   */
+    float margin;      /* (|peak|-|runner-up|)/|peak|; exact runner-up on BRUTE records,
+                          the f32 ranking's on FFT records (see above)                */
     int32_t first_lag; /* first-pass lag before the sanity re-search                 */
     int32_t n_blocks;  /* whole blocks that contributed (processor.go:691-712)       */
 } tdoa_peak;

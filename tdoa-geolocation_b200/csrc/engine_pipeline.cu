@@ -1158,13 +1158,15 @@ int correlate(tdoa_engine *e, const std::vector<Sig> &sigs, const std::vector<Pa
             brute.push_back(&pl);
             continue;
         }
-        // processor.go:653-661: the shorter input is the template
+        // processor.go:653-661: the shorter input is the template.  EXTENDED keeps signal 1 as the
+        // template whatever the lengths, so that the lag is always the delay of signal 2; its search
+        // reads both signals over [0, min(n1, n2)) only, and sl = n2 bounds the reads of signal 2
         const Sig *tp = &s1, *sg = &s2;
-        if (n1 > n2) { tp = &s2; sg = &s1; }
+        if (n1 > n2 && cfg.mode != TDOA_MODE_EXTENDED) { tp = &s2; sg = &s1; }
         const i64 tl = std::min(n1, n2), sl = std::max(n1, n2);
         J.t_re = tp->out_re; J.t_im = tp->out_im; J.t_stats = tp->stats;
         J.s_re = sg->out_re; J.s_im = sg->out_im; J.s_stats = sg->stats;
-        J.sl = sl;
+        J.sl = cfg.mode == TDOA_MODE_EXTENDED ? n2 : sl;
         J.lag0 = 0;
         J.t_off = 0;
         if (cfg.mode == TDOA_MODE_EXTENDED) {
