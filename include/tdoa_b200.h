@@ -57,6 +57,9 @@ extern "C" {
 #define TDOA_PEAK_EDGE 0x2u       /* peak on the edge of the lag range (frac = 0)    */
 #define TDOA_PEAK_BRUTE 0x4u      /* every lag was evaluated in the time domain      */
 #define TDOA_PEAK_EMPTY 0x8u      /* empty input: (0, 0.0) as processor.go:622-625   */
+#define TDOA_PEAK_BOUNDED 0x20u   /* lag searched within an interval (tdoa_xcorr_bounded,
+                                     tdoa_set_tgt_bounds); EMPTY too: the interval held
+                                     no lag of the range                               */
 #define TDOA_PEAK_NCAND(f) (((f) >> 16) & 0xffu)   /* lags re-evaluated exactly (FFT path)   */
 #define TDOA_PEAK_BRANCH1(f) (((f) >> 8) & 3u)  /* preprocess branch of signal 1      */
 #define TDOA_PEAK_BRANCH2(f) (((f) >> 10) & 3u) /* 0 strong/std, 1 moderate, 2 weak   */
@@ -223,6 +226,45 @@ TDOA_API int tdoa_xcorr(tdoa_engine *e, int32_t kind, int64_t win_start, int64_t
 /* Same, peaks left in device memory (e.g. an NCCL send buffer); d_out[n_windows*P]. */
 TDOA_API int tdoa_xcorr_device(tdoa_engine *e, int32_t kind, int64_t win_start, int64_t win_len,
                                int32_t n_windows, int64_t hop, tdoa_peak *d_out);
+
+/* ---- bounded lag search (EXTENDED mode; no reference equivalent; engine-defined): tdoa_xcorr with an interval
+ * [lag_lo[k], lag_hi[k]] (int32, capture samples: the units of the records) for each record k = w * P + p.  With
+ * D = decimate (1 without the decimator) the searched lags are the correlation's own lags k in -max_lag / D ..
+ * +max_lag / D with lo <= D k <= hi: one contiguous run.
+ *  - lag: the arg-max of |corr| over the run (ties: the lowest lag); corr its value.
+ *  - frac: the 3-point parabola when lags k - 1 and k + 1 are both in the run; otherwise TDOA_PEAK_EDGE and frac 0,
+ *    so a maximum pinned to the interval's boundary is unusable in the windowed fixes, as a maximum at +-max_lag is.
+ *  - margin: the runner-up over the run without the peak (exact on BRUTE records, the f32 ranking's on FFT records).
+ *  - flags: every record carries TDOA_PEAK_BOUNDED; a run without any lag gives EMPTY | BOUNDED, lag 0, corr 0.
+ *    The candidate cap's lag-by-lag redo keeps the interval.
+ * An interval that covers the whole range gives tdoa_xcorr's record bit for bit, apart from TDOA_PEAK_BOUNDED.
+ * It is the primitive for a caller with its own prior on the lags (e.g. a known search area).  On a multi-GPU engine
+ * the intervals are dealt with the windows.  Refused (TDOA_E_INVALID): a mode other than EXTENDED, a NULL bound
+ * array, lo > hi; and what tdoa_xcorr refuses. */
+TDOA_API int tdoa_xcorr_bounded(tdoa_engine *e, int32_t kind, int64_t win_start, int64_t win_len, int32_t n_windows,
+                                int64_t hop, const int32_t *lag_lo, const int32_t *lag_hi, tdoa_peak *out);
+
+/* Bounded TGT search in the windowed process calls (EXTENDED mode; engine setting; default off).  Once the REF line
+ * of pair p = (i, j) is fitted, physics limits where the target's peak can be: for any transmitter |r_j - r_i| <=
+ * d_ij, the baseline, and rd = (y_tgt - y_ref(t_w)) / fs * c + geo, so y_tgt lies within d_ij fs / c of
+ * y_ref(t_w) - geo fs / c when the REF transmitter is known (has_ref_tx), within 2 d_ij fs / c of y_ref(t_w)
+ * otherwise (|geo| <= d_ij too).  A peak outside is noise, another programme or a repeat of periodic content.
+ * While on, every tdoa_process_windows* call (plain, _grid, _retimed, _closure, _exclude) runs the REF pair loop, the
+ * REF fit (k_window_ref_fit) and k_tgt_bounds on the REF table, then the TGT pair loop as tdoa_xcorr_bounded with
+ * these intervals; the fix stage is unchanged and reads that TGT table.  On a multi-GPU engine the ranks meet twice
+ * per call (REF, then TGT), as in the re-timed call.  Per (TGT window w, pair p) with a REF fit (a, beta, t_mean,
+ * geo; geo = 0 without has_ref_tx), d = the baseline as tdoa_baselines gives it, t_w = the window time of station i,
+ * all in f64 rounded to nearest with no fused multiply-add, in this order:
+ *   y_ref  = a + beta * (t_w - t_mean)
+ *   centre = y_ref - geo / c * fs                          (c = 299792458, fs = sample_rate)
+ *   half   = (has_ref_tx ? d : 2 * d) / c * fs + guard_samples
+ *   lo = ceil(centre - half), hi = floor(centre + half), each clamped to [INT32_MIN, INT32_MAX].
+ * A pair without a REF fit keeps the unbounded search (no TDOA_PEAK_BOUNDED); it is used in no window anyway.
+ * Not affected: tdoa_window_fixes* (their tables are given), tdoa_xcorr* and tdoa_process.  on = 0 launches exactly
+ * what the calls launch without the setting.  An n_devices > 1 engine sets every device; with tdoa_comm_init each
+ * rank sets its own.  Refused (TDOA_E_INVALID): a mode other than EXTENDED, on not 0 or 1, guard_samples NaN,
+ * infinite or negative. */
+TDOA_API int tdoa_set_tgt_bounds(tdoa_engine *e, int32_t on, double guard_samples);
 
 /* Both pair loops of ProcessTDOA over windows in ONE call (processor.go:816-830 REF, then :836-850 TGT):
  * ref_out[n_ref_windows * P], tgt_out[n_tgt_windows * P] as tdoa_xcorr(TDOA_KIND_REF, ...) followed by

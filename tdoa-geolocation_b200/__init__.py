@@ -25,6 +25,7 @@ from ._native import (  # noqa: F401
     PEAK_DTYPE,
     PEAK_EDGE,
     PEAK_EMPTY,
+    PEAK_BOUNDED,
 )
 from .processor import Station, TDOAProcessor  # noqa: F401
 from . import sharding  # noqa: F401
@@ -32,5 +33,5 @@ from . import analyzer  # noqa: F401
 
 __all__ = [
     "Engine", "TdoaError", "Peak", "MODE_SOURCE", "MODE_BINARY", "MODE_EXTENDED", "KIND_REF", "KIND_TGT",
-    "default_config", "channel_taps", "library_path", "load_library", "host_alloc", "comm_unique_id", "PEAK_DTYPE", "PEAK_EDGE", "PEAK_EMPTY", "Station", "TDOAProcessor", "sharding", "analyzer",
+    "default_config", "channel_taps", "library_path", "load_library", "host_alloc", "comm_unique_id", "PEAK_DTYPE", "PEAK_EDGE", "PEAK_EMPTY", "PEAK_BOUNDED", "Station", "TDOAProcessor", "sharding", "analyzer",
 ]

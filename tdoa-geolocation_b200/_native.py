@@ -16,6 +16,7 @@ MODE_SOURCE, MODE_BINARY, MODE_EXTENDED = 0, 1, 2
 KIND_REF, KIND_TGT = 0, 1
 
 PEAK_RESEARCHED, PEAK_EDGE, PEAK_BRUTE, PEAK_EMPTY = 0x1, 0x2, 0x4, 0x8
+PEAK_BOUNDED = 0x20
 
 ERRORS = {-1: "TDOA_E_INVALID", -2: "TDOA_E_NODEVICE", -3: "TDOA_E_CUDA", -4: "TDOA_E_NOMEM",
           -5: "TDOA_E_STATE", -6: "TDOA_E_SINGULAR", -7: "TDOA_E_IO"}
@@ -23,7 +24,7 @@ ERRORS = {-1: "TDOA_E_INVALID", -2: "TDOA_E_NODEVICE", -3: "TDOA_E_CUDA", -4: "T
 # every symbol include/tdoa_b200.h declares (tests check the library exports them all)
 ABI_SYMBOLS = [
     "tdoa_default_config", "tdoa_create", "tdoa_destroy", "tdoa_last_error", "tdoa_host_alloc", "tdoa_host_free",
-    "tdoa_load_u8", "tdoa_load_file", "tdoa_load_u8_pinned", "tdoa_load_u8_device", "tdoa_unpack", "tdoa_preprocess", "tdoa_set_channel", "tdoa_xcorr", "tdoa_xcorr_device", "tdoa_xcorr_windows", "tdoa_process", "tdoa_process_windows", "tdoa_window_fixes", "tdoa_process_windows_grid", "tdoa_window_fixes_grid", "tdoa_process_windows_retimed", "tdoa_closure", "tdoa_process_windows_closure", "tdoa_window_fixes_closure", "tdoa_exclude_stations", "tdoa_process_windows_exclude", "tdoa_window_fixes_exclude", "tdoa_xcorr_info", "tdoa_analyze",
+    "tdoa_load_u8", "tdoa_load_file", "tdoa_load_u8_pinned", "tdoa_load_u8_device", "tdoa_unpack", "tdoa_preprocess", "tdoa_set_channel", "tdoa_set_tgt_bounds", "tdoa_xcorr", "tdoa_xcorr_bounded", "tdoa_xcorr_device", "tdoa_xcorr_windows", "tdoa_process", "tdoa_process_windows", "tdoa_window_fixes", "tdoa_process_windows_grid", "tdoa_window_fixes_grid", "tdoa_process_windows_retimed", "tdoa_closure", "tdoa_process_windows_closure", "tdoa_window_fixes_closure", "tdoa_exclude_stations", "tdoa_process_windows_exclude", "tdoa_window_fixes_exclude", "tdoa_xcorr_info", "tdoa_analyze",
     "tdoa_cross_correlate", "tdoa_baselines", "tdoa_solve", "tdoa_solve_binary", "tdoa_solve_ls", "tdoa_grid", "tdoa_grid_masked", "tdoa_get_stats", "tdoa_stream",
     "tdoa_set_stream", "tdoa_synchronize", "tdoa_selftest",
     "tdoa_comm_unique_id", "tdoa_comm_init", "tdoa_comm_rank", "tdoa_shard_windows",
@@ -172,6 +173,8 @@ def load_library():
     L.tdoa_preprocess.argtypes = [vp, i32, i32, i64, i64, vp, f64p, C.POINTER(i32)]
     L.tdoa_set_channel.argtypes = [vp, i32, vp, vp, i32]
     L.tdoa_xcorr.argtypes = [vp, i32, i64, i64, i32, i64, vp]
+    L.tdoa_xcorr_bounded.argtypes = [vp, i32, i64, i64, i32, i64, vp, vp, vp]
+    L.tdoa_set_tgt_bounds.argtypes = [vp, i32, C.c_double]
     L.tdoa_xcorr_info.argtypes = [vp, i32, vp, vp]
     L.tdoa_process.argtypes = [vp, vp, vp, vp, vp, vp, vp, C.POINTER(i32), C.POINTER(i32)]
     L.tdoa_analyze.argtypes = [vp, i32, i32, vp, vp]
@@ -433,6 +436,34 @@ class Engine:
         out = np.zeros((n_windows, self.n_pairs), PEAK_DTYPE)
         self._check(self._lib.tdoa_xcorr(self._h, kind, win_start, win_len, n_windows, hop, _ptr(out)))
         return out
+
+    def xcorr_bounded(self, kind: int, lo, hi, win_start: int = 0, win_len: int = 0, n_windows: int = 1,
+                      hop: int = 0) -> np.ndarray:
+        """xcorr with each record's lag searched within [lo, hi] (EXTENDED mode, tdoa_xcorr_bounded): lo, hi are
+        int32 capture samples, broadcast to (n_windows, n_pairs).  Every record carries PEAK_BOUNDED; a maximum on the
+        interval's boundary has PEAK_EDGE, an interval without a lag of the range gives PEAK_EMPTY."""
+        shape = (n_windows, self.n_pairs)
+
+        def i32(v, name):
+            a = np.asarray(v)
+            if a.dtype.kind not in "iu" or (a.size and (a.min() < -2 ** 31 or a.max() > 2 ** 31 - 1)):
+                raise ValueError(f"{name} must be integers within int32")
+            return np.ascontiguousarray(np.broadcast_to(a.astype(np.int32), shape))
+
+        lo, hi = i32(lo, "lo"), i32(hi, "hi")
+        out = np.zeros(shape, PEAK_DTYPE)
+        self._check(self._lib.tdoa_xcorr_bounded(self._h, kind, win_start, win_len, n_windows, hop, _ptr(lo), _ptr(hi),
+                                                 _ptr(out)))
+        return out
+
+    def set_tgt_bounds(self, guard) -> None:
+        """Bounded TGT search in every windowed process call (EXTENDED mode, tdoa_set_tgt_bounds): each TGT lag is
+        searched within the interval its pair's REF line and baseline allow, widened by `guard` samples on each side;
+        None turns it off (the default)."""
+        if guard is None:
+            self._check(self._lib.tdoa_set_tgt_bounds(self._h, 0, 0.0))
+        else:
+            self._check(self._lib.tdoa_set_tgt_bounds(self._h, 1, float(guard)))
 
     def xcorr_windows(self, win_start: int, win_len: int, n_ref_windows: int, n_tgt_windows: int, hop: int):
         """Both pair loops over windows in one call (tdoa_xcorr_windows): (ref, tgt) tables.  On a multi-GPU

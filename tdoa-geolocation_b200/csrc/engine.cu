@@ -646,6 +646,20 @@ int tdoa_set_channel(tdoa_engine *e, int32_t kind, const float *taps_re, const f
     return multi_forward_channel(e, kind, taps_re, taps_im, n_taps);
 }
 
+int tdoa_set_tgt_bounds(tdoa_engine *e, int32_t on, double guard_samples)
+{
+    static const char *fn = "tdoa_set_tgt_bounds";
+    if (!e) return TDOA_E_INVALID;
+    if (e->cfg.mode != TDOA_MODE_EXTENDED)
+        return fail(e, TDOA_E_INVALID, "%s: the bounded search is an EXTENDED-mode option", fn);
+    if (on != 0 && on != 1) return fail(e, TDOA_E_INVALID, "%s: on must be 0 or 1, got %d", fn, on);
+    if (!std::isfinite(guard_samples) || guard_samples < 0.0)
+        return fail(e, TDOA_E_INVALID, "%s: guard_samples must be finite and >= 0, got %g", fn, guard_samples);
+    e->tgt_bounds = on == 1;
+    e->tgt_guard = guard_samples;
+    return multi_forward_tgt_bounds(e, on, guard_samples);
+}
+
 int tdoa_baselines(tdoa_engine *e, const double *stations_llh, int32_t n_stations, double *baselines)
 {
     if (!e) return TDOA_E_INVALID;

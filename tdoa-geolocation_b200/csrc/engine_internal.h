@@ -117,6 +117,8 @@ struct tdoa_engine {
     size_t spans_used = 0;
     float ms_corr = 0.f;   // correlation stage of the current call (ms_exact = ms_corr - ms_fft)
     tdoa::MultiState *multi = nullptr;   // engine_multi.cu; nullptr: one process, one GPU
+    bool tgt_bounds = false;             // tdoa_set_tgt_bounds: the windowed calls bound their TGT lag search
+    double tgt_guard = 0.0;              // samples added to each side of those intervals
 };
 
 namespace tdoa {
@@ -200,18 +202,22 @@ void stats_reset(tdoa_engine *e);
 int window_lengths(tdoa_engine *e, int32_t kind, int64_t win_start, int64_t win_len, int32_t n_windows, int64_t hop,
                    std::vector<i64> &len);
 // d_rates (device, S doubles, may be nullptr): every plane re-timed by its station's rate (tdoa_process_windows_retimed)
+// d_bounds (device, n_windows * P intervals, may be nullptr): the bounded search of tdoa_xcorr_bounded, record by record
 int xcorr_core(tdoa_engine *e, int32_t kind, int64_t win_start, const std::vector<i64> &len, int32_t n_windows,
-               int64_t hop, PeakRec *d_out, Pending *pend, const double *d_rates = nullptr);
+               int64_t hop, PeakRec *d_out, Pending *pend, const double *d_rates = nullptr, const int2 *d_bounds = nullptr);
 // tdoa_xcorr / tdoa_xcorr_device as one call; d_table (device, n_windows * P, out may then be nullptr): the
-// records are also left there, past the call's end (tdoa_process_windows); d_rates as xcorr_core
+// records are also left there, past the call's end (tdoa_process_windows); d_rates, d_bounds as xcorr_core.
+// h_bounds: the same intervals on the host -- what a multi-GPU engine deals with the windows; on one GPU they are
+// copied to the device when d_bounds is nullptr
 int xcorr_impl(tdoa_engine *e, int32_t kind, int64_t win_start, int64_t win_len, int32_t n_windows, int64_t hop,
-               tdoa_peak *out, bool out_is_device, PeakRec *d_table = nullptr, const double *d_rates = nullptr);
+               tdoa_peak *out, bool out_is_device, PeakRec *d_table = nullptr, const double *d_rates = nullptr,
+               const int2 *d_bounds = nullptr, const int2 *h_bounds = nullptr);
 
 // ---- more than one GPU (engine_multi.cu)
 // windows dealt over the ranks of the engine's communicator, records gathered: true if it took the call
 bool multi_wants(const tdoa_engine *e, int32_t n_windows);
 int xcorr_sharded(tdoa_engine *e, int32_t kind, int64_t win_start, const std::vector<i64> &len, int32_t n_windows, int64_t hop,
-                  tdoa_peak *out, bool out_is_device);
+                  tdoa_peak *out, bool out_is_device, const int2 *h_bounds = nullptr);
 // several signal kinds' windows in one collective call (tdoa_xcorr_windows): one meeting of the ranks
 struct ShardPart {
     int32_t kind = 0;
@@ -222,6 +228,7 @@ struct ShardPart {
     tdoa_peak *out = nullptr;   // host or device table of n_windows * P records, or nullptr
     bool out_is_device = false;
     const double *rates = nullptr;   // station rates on the calling rank's device: the planes are re-timed (xcorr_core)
+    const int2 *bounds = nullptr;    // host intervals [n_windows * P] (tdoa_xcorr_bounded): each rank takes its windows'
 };
 int xcorr_sharded(tdoa_engine *e, const std::vector<ShardPart> &parts);
 void multi_destroy(tdoa_engine *e);
@@ -229,5 +236,6 @@ int multi_create_peers(tdoa_engine *e, const tdoa_config *cfg);   // tdoa_create
 // which: 0 tdoa_load_u8, 1 tdoa_load_u8_pinned, 2 tdoa_load_file (p = path)
 int multi_forward_load(tdoa_engine *e, int which, int32_t station, const void *p, size_t nbytes, int64_t *n_samples);
 int multi_forward_channel(tdoa_engine *e, int32_t kind, const float *taps_re, const float *taps_im, int32_t n_taps);
+int multi_forward_tgt_bounds(tdoa_engine *e, int32_t on, double guard_samples);
 
 }  // namespace tdoa

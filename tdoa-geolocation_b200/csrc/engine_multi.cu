@@ -140,8 +140,18 @@ int sharded_rank(tdoa_engine *e, const std::vector<ShardPart> &parts)
             else if ((rc = alloc_t(e, &W.d_table, (size_t)Q.n_windows * P))) return rc;
             W.mine = W.d_gather + (size_t)M.rank * W.n_max * P;
             CU(cudaMemsetAsync(W.mine, 0, (size_t)W.n_max * P * sizeof(PeakRec), e->stream));
+            // the intervals of this rank's windows first, first + world, ..., side by side as its records are
+            int2 *d_bounds = nullptr;
+            if (Q.bounds && count > 0) {
+                std::vector<int2> mine((size_t)count * P);
+                for (int k = 0; k < count; k++)
+                    std::memcpy(mine.data() + (size_t)k * P, Q.bounds + (size_t)(first + k * world) * P, (size_t)P * sizeof(int2));
+                if ((rc = alloc_t(e, &d_bounds, mine.size()))) return rc;
+                // pageable source: the copy has been staged when the call returns
+                CU(cudaMemcpyAsync(d_bounds, mine.data(), mine.size() * sizeof(int2), cudaMemcpyHostToDevice, e->stream));
+            }
             if (count > 0 && (rc = xcorr_core(e, Q.kind, Q.win_start + (i64)first * Q.hop, Q.len, count, Q.hop * world, W.mine, nullptr,
-                                              Q.rates)))
+                                              Q.rates, d_bounds)))
                 return rc;
         }
         return TDOA_OK;
@@ -230,11 +240,11 @@ int xcorr_sharded(tdoa_engine *e, const std::vector<ShardPart> &parts)
 }
 
 int xcorr_sharded(tdoa_engine *e, int32_t kind, int64_t win_start, const std::vector<i64> &len, int32_t n_windows, int64_t hop,
-                  tdoa_peak *out, bool out_is_device)
+                  tdoa_peak *out, bool out_is_device, const int2 *h_bounds)
 {
     std::vector<ShardPart> parts(1);
     parts[0].kind = kind; parts[0].win_start = win_start; parts[0].len = len; parts[0].n_windows = n_windows; parts[0].hop = hop;
-    parts[0].out = out; parts[0].out_is_device = out_is_device;
+    parts[0].out = out; parts[0].out_is_device = out_is_device; parts[0].bounds = h_bounds;
     return xcorr_sharded(e, parts);
 }
 
@@ -308,6 +318,19 @@ int multi_forward_channel(tdoa_engine *e, int32_t kind, const float *taps_re, co
     for (size_t r = 1; r < e->multi->peers.size(); r++) {
         tdoa_engine *q = e->multi->peers[r];
         const int rc = tdoa_set_channel(q, kind, taps_re, taps_im, n_taps);
+        if (rc) { cudaSetDevice(e->device); return fail(e, rc, "device %d: %s", q->device, q->error.c_str()); }
+    }
+    CU(cudaSetDevice(e->device));
+    return TDOA_OK;
+}
+
+// the same TGT bound setting on every peer of a multi-device engine (a communicator's ranks each set their own)
+int multi_forward_tgt_bounds(tdoa_engine *e, int32_t on, double guard_samples)
+{
+    if (!e->multi || e->multi->peers.size() <= 1) return TDOA_OK;
+    for (size_t r = 1; r < e->multi->peers.size(); r++) {
+        tdoa_engine *q = e->multi->peers[r];
+        const int rc = tdoa_set_tgt_bounds(q, on, guard_samples);
         if (rc) { cudaSetDevice(e->device); return fail(e, rc, "device %d: %s", q->device, q->error.c_str()); }
     }
     CU(cudaSetDevice(e->device));

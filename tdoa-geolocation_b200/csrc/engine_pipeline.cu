@@ -866,6 +866,7 @@ int run_fft(tdoa_engine *e, std::vector<CorrPlan *> &plans)
         S.tol = 2e-5f;
         S.cand = d_cand; S.n_cand = d_ncand; S.approx_max = d_amax;
         S.t_stats = J.t_stats; S.s_stats = J.s_stats;
+        S.bound = K.bound; S.lag_origin = K.lag_origin; S.decim = K.decim;
         CandJob &C = cjobs[p];
         C.cand = d_cand; C.n_cand = d_ncand; C.max_cand = kMaxCand; C.approx = d_approx; C.blocksums = J.blocksums;
         pjobs[p] = J;
@@ -1130,9 +1131,10 @@ int run_fft(tdoa_engine *e, std::vector<CorrPlan *> &plans)
 }
 
 // optimistic = true: queue only -- the candidate-overflow check (and the lag-by-lag redo it may
-// ask for) is left to the caller, who looks at the records' flags after its own synchronisation
+// ask for) is left to the caller, who looks at the records' flags after its own synchronisation.
+// d_bound (EXTENDED, device, may be nullptr): the interval of record p at d_bound[p] (tdoa_xcorr_bounded)
 int correlate(tdoa_engine *e, const std::vector<Sig> &sigs, const std::vector<Pair> &pairs, PeakRec *d_out,
-              double *d_first = nullptr, bool optimistic = false)
+              double *d_first = nullptr, bool optimistic = false, const int2 *d_bound = nullptr)
 {
     if (pairs.empty()) return TDOA_OK;
     const tdoa_config &cfg = e->cfg;
@@ -1150,6 +1152,8 @@ int correlate(tdoa_engine *e, const std::vector<Sig> &sigs, const std::vector<Pa
         K.flags = ((uint32_t)s1.branch << 8) | ((uint32_t)s2.branch << 10);
         K.sanity = 0;
         K.lag_origin = 0;
+        K.bound = d_bound ? d_bound + p : nullptr;
+        K.decim = decimation(e);
         const i64 n1 = s1.n_out >= 0 ? s1.n_out : s1.n, n2 = s2.n_out >= 0 ? s2.n_out : s2.n;
         if (n1 == 0 || n2 == 0) {  // processor.go:622-625
             K.flags |= TDOA_PEAK_EMPTY;
@@ -1359,7 +1363,7 @@ int retime(tdoa_engine *e, std::vector<Sig> &sigs, const double *d_rates)
 // overflow are the caller's to check after its synchronisation (tdoa_process).
 // d_rates != nullptr: station rates on the device; every plane is re-timed between preprocessing and correlation.
 int xcorr_core(tdoa_engine *e, int32_t kind, int64_t win_start, const std::vector<i64> &len, int32_t n_windows,
-               int64_t hop, PeakRec *d_out, Pending *pend, const double *d_rates)
+               int64_t hop, PeakRec *d_out, Pending *pend, const double *d_rates, const int2 *d_bounds)
 {
     int rc;
     const int S = e->cfg.n_stations, P = S * (S - 1) / 2;
@@ -1399,7 +1403,9 @@ int xcorr_core(tdoa_engine *e, int32_t kind, int64_t win_start, const std::vecto
             const int sp_corr = span_begin(e, SPAN_STAGE_CORR);
             d_first = nullptr;
             if (w0 == 0 && (rc = alloc_t(e, &d_first, pairs.size()))) return rc;
-            if ((rc = correlate(e, sigs, pairs, d_out + (size_t)w0 * P, d_first, pend != nullptr))) return rc;
+            if ((rc = correlate(e, sigs, pairs, d_out + (size_t)w0 * P, d_first, pend != nullptr,
+                                d_bounds ? d_bounds + (size_t)w0 * P : nullptr)))
+                return rc;
             if (decimation(e) > 1) {
                 launch_lag_units(d_out + (size_t)w0 * P, (int)pairs.size(), decimation(e), e->stream);
                 count_launch(e);
@@ -1448,7 +1454,8 @@ int xcorr_core(tdoa_engine *e, int32_t kind, int64_t win_start, const std::vecto
 }
 
 int xcorr_impl(tdoa_engine *e, int32_t kind, int64_t win_start, int64_t win_len, int32_t n_windows, int64_t hop,
-               tdoa_peak *out, bool out_is_device, PeakRec *d_table, const double *d_rates)
+               tdoa_peak *out, bool out_is_device, PeakRec *d_table, const double *d_rates, const int2 *d_bounds,
+               const int2 *h_bounds)
 {
     if (!e) return TDOA_E_INVALID;
     int rc = begin_call(e);
@@ -1457,8 +1464,14 @@ int xcorr_impl(tdoa_engine *e, int32_t kind, int64_t win_start, int64_t win_len,
     std::vector<i64> len;
     if ((rc = window_lengths(e, kind, win_start, win_len, n_windows, hop, len))) return rc;
     // more than one GPU: windows dealt over the ranks, records gathered (engine_multi.cu)
-    if (multi_wants(e, n_windows)) return xcorr_sharded(e, kind, win_start, len, n_windows, hop, out, out_is_device);
+    if (multi_wants(e, n_windows)) return xcorr_sharded(e, kind, win_start, len, n_windows, hop, out, out_is_device, h_bounds);
     const int S = e->cfg.n_stations, P = S * (S - 1) / 2;
+    if (h_bounds && !d_bounds) {
+        int2 *d = nullptr;
+        if ((rc = alloc_t(e, &d, (size_t)n_windows * P))) return rc;
+        CU(cudaMemcpyAsync(d, h_bounds, (size_t)n_windows * P * sizeof(int2), cudaMemcpyHostToDevice, e->stream));
+        d_bounds = d;
+    }
     PeakRec *d_out = nullptr;
     if (out_is_device) d_out = reinterpret_cast<PeakRec *>(out);
     else if (d_table) d_out = d_table;
@@ -1476,9 +1489,10 @@ int xcorr_impl(tdoa_engine *e, int32_t kind, int64_t win_start, int64_t win_len,
         cudaStream_t main_stream = e->stream;
         CU(cudaEventRecord(e->ev_fork, main_stream));
         CU(cudaStreamWaitEvent(e->side_stream, e->ev_fork, 0));
-        if ((rc = xcorr_core(e, kind, win_start, len, nA, hop, d_out, &pend[0], d_rates))) return rc;
+        if ((rc = xcorr_core(e, kind, win_start, len, nA, hop, d_out, &pend[0], d_rates, d_bounds))) return rc;
         e->stream = e->side_stream;
-        rc = xcorr_core(e, kind, win_start + (i64)nA * hop, len, nB, hop, d_out + (size_t)nA * P, &pend[1], d_rates);
+        rc = xcorr_core(e, kind, win_start + (i64)nA * hop, len, nB, hop, d_out + (size_t)nA * P, &pend[1], d_rates,
+                        d_bounds ? d_bounds + (size_t)nA * P : nullptr);
         e->stream = main_stream;
         CU(cudaEventRecord(e->ev_join, e->side_stream));
         CU(cudaStreamWaitEvent(main_stream, e->ev_join, 0));
@@ -1509,7 +1523,7 @@ int xcorr_impl(tdoa_engine *e, int32_t kind, int64_t win_start, int64_t win_len,
         }
     }
     if (!done) {
-        if ((rc = xcorr_core(e, kind, win_start, len, n_windows, hop, d_out, nullptr, d_rates))) return rc;
+        if ((rc = xcorr_core(e, kind, win_start, len, n_windows, hop, d_out, nullptr, d_rates, d_bounds))) return rc;
         cudaEventRecord(e->ev[4], e->stream);
         if (!out_is_device && out)
             CU(cudaMemcpyAsync(out, d_out, (size_t)n_windows * P * sizeof(tdoa_peak), cudaMemcpyDeviceToHost, e->stream));
@@ -1621,6 +1635,27 @@ int tdoa_xcorr_device(tdoa_engine *e, int32_t kind, int64_t win_start, int64_t w
                       int64_t hop, tdoa_peak *d_out)
 {
     return xcorr_impl(e, kind, win_start, win_len, n_windows, hop, d_out, true);
+}
+
+int tdoa_xcorr_bounded(tdoa_engine *e, int32_t kind, int64_t win_start, int64_t win_len, int32_t n_windows, int64_t hop,
+                       const int32_t *lag_lo, const int32_t *lag_hi, tdoa_peak *out)
+{
+    static const char *fn = "tdoa_xcorr_bounded";
+    if (!e) return TDOA_E_INVALID;
+    int rc = begin_call(e);
+    if (rc) return rc;
+    if (e->cfg.mode != TDOA_MODE_EXTENDED)
+        return fail(e, TDOA_E_INVALID, "%s: the bounded search is an EXTENDED-mode option (BINARY and SOURCE search one-sided)", fn);
+    if (!lag_lo || !lag_hi) return fail(e, TDOA_E_INVALID, "%s: a bound array is NULL", fn);
+    if (n_windows < 1) return fail(e, TDOA_E_INVALID, "tdoa_xcorr: bad window arguments");
+    const int S = e->cfg.n_stations, P = S * (S - 1) / 2;
+    std::vector<int2> bounds((size_t)n_windows * P);
+    for (size_t k = 0; k < bounds.size(); k++) {
+        if (lag_lo[k] > lag_hi[k])
+            return fail(e, TDOA_E_INVALID, "%s: record %zu has lo %d > hi %d", fn, k, lag_lo[k], lag_hi[k]);
+        bounds[k] = make_int2(lag_lo[k], lag_hi[k]);
+    }
+    return xcorr_impl(e, kind, win_start, win_len, n_windows, hop, out, false, nullptr, nullptr, nullptr, bounds.data());
 }
 
 int tdoa_xcorr_windows(tdoa_engine *e, int64_t win_start, int64_t win_len, int32_t n_ref_windows, int32_t n_tgt_windows,

@@ -95,7 +95,30 @@ struct PeakJob {
     uint32_t flags;       // flags or-ed into the record
     PeakRec *out;
     double *first_corr;   // optional: correlation of the first-pass peak (before the sanity re-search)
+    const int2 *bound;    // EXTENDED: this record's interval {lo, hi} in capture samples (nullptr: unbounded)
+    int decim;            // lag k of the correlation is decim * k capture samples
 };
+
+// The bounded search (tdoa_xcorr_bounded): an interval of kNoBound is no bound at all (k_tgt_bounds' pair without a
+// REF fit); any other interval [lo, hi] searches the lag indices i in [0, n_lags) with lo <= decim (i + lag_origin)
+// <= hi, one contiguous run [*i0, *i1] (empty when *i0 > *i1).  Without a bound the run is every index.
+constexpr int2 kNoBound = {0x7fffffff, (int)0x80000000};
+
+__device__ __forceinline__ bool bound_run(const int2 *bound, int lag_origin, int decim, int n_lags, int *i0, int *i1)
+{
+    *i0 = 0;
+    *i1 = n_lags - 1;
+    if (!bound) return false;
+    const int2 b = *bound;
+    if (b.x == kNoBound.x && b.y == kNoBound.y) return false;
+    const i64 D = decim, lo = b.x, hi = b.y;
+    const i64 k0 = lo >= 0 ? (lo + D - 1) / D : -((-lo) / D);   // ceil(lo / D)
+    const i64 k1 = hi >= 0 ? hi / D : -((-hi + D - 1) / D);     // floor(hi / D)
+    // clipped in i64 before the narrowing: an interval far beyond the range (lo or hi near +-2^31) is an empty run
+    *i0 = (int)min((i64)n_lags, max((i64)0, k0 - lag_origin));
+    *i1 = (int)max((i64)-1, min((i64)n_lags - 1, k1 - lag_origin));
+    return true;
+}
 
 // ---- preprocess.cu
 void launch_power(const SigJob *d_jobs, int n_jobs, i64 max_n, int grid_x, cudaStream_t st);
@@ -200,6 +223,10 @@ void launch_window_ref_fit(const PeakRec *d_ref, int n_ref, int n_st, const doub
 void launch_window_rd(const PeakRec *d_tgt, int n_tgt, int n_st, const double *d_t_tgt, const double *d_fit, float min_margin,
                       double fs, double *d_rd, uint8_t *d_used, cudaStream_t st);
 constexpr int kWindowFitDoubles = 5;   // per pair: a, beta, t_mean, windows used, geometric term
+// the TGT intervals of tdoa_set_tgt_bounds from the fit, the baselines (launch_baselines) and the TGT window times:
+// d_bounds[w * P + p], kNoBound for a pair without a REF fit
+void launch_tgt_bounds(const double *d_fit, const double *d_base, const double *d_t_tgt, int n_tgt, int n_st, int has_ref_tx,
+                       double guard, double fs, int2 *d_bounds, cudaStream_t st);
 // ---- retime.cu (tdoa_process_windows_retimed): station clock rates from the REF fits, and the re-timing gather
 // rate[S] (0 for a station without a fitted pair) re-times the planes, clock[S] (NaN there) is what the call returns;
 // n_st <= 64 (solve_ls_max_stations)

@@ -28,6 +28,9 @@
 //                     grid search run again on the final mask and k_solve_ls fixes every window from that seed.
 // tdoa_process_windows_retimed runs the REF pair loop, k_window_ref_fit and k_station_rates (retime.cu) before the TGT
 // pair loop, which re-times every plane by its station's rate; the fix stage is the same.
+// With tdoa_set_tgt_bounds on, every windowed process call runs the REF pair loop, k_window_ref_fit and
+//   k_tgt_bounds      one thread per (TGT window, pair): the interval of TGT lags the REF line and the baseline allow
+//                     (|r_j - r_i| <= d_ij for any transmitter), which the TGT pair loop's search is bounded to.
 // Window times and the usable test are stated in include/tdoa_b200.h (tdoa_process_windows).
 #include <cuda_runtime.h>
 
@@ -155,7 +158,43 @@ __global__ void k_window_rd(const PeakRec *tgt, int n_tgt, int n_st, const doubl
     used[k] = ok ? 1 : 0;
 }
 
+// include/tdoa_b200.h (tdoa_set_tgt_bounds) states the operation order; f64, rounded to nearest, no contraction
+// (this unit is compiled with -fmad=false)
+__device__ __forceinline__ int clamp_i32(double v)
+{
+    return v <= -2147483648.0 ? (int)0x80000000 : (v >= 2147483647.0 ? 0x7fffffff : (int)v);
+}
+
+__global__ void k_tgt_bounds(const double *fit, const double *base, const double *t_tgt, int n_tgt, int n_st, int has_ref_tx,
+                             double guard, double fs, int2 *bounds)
+{
+    const int P = n_st * (n_st - 1) / 2;
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n_tgt * P) return;
+    const int w = k / P, p = k - w * P;
+    int i, j;
+    pair_stations(p, n_st, i, j);
+    const double *f = fit + (size_t)kWindowFitDoubles * p;
+    int2 b = kNoBound;   // no REF fit: the pair is used in no window, its search stays unbounded
+    if (f[3] > 0.0) {
+        const double y_ref = f[0] + f[1] * (t_tgt[(size_t)w * n_st + i] - f[2]);   // k_window_rd's expression
+        const double centre = y_ref - f[4] / kC * fs;
+        const double half = (has_ref_tx ? base[p] : 2.0 * base[p]) / kC * fs + guard;
+        const double lo = ceil(centre - half), hi = floor(centre + half);
+        if (!isnan(lo) && !isnan(hi)) b = make_int2(clamp_i32(lo), clamp_i32(hi));
+    }
+    bounds[k] = b;
+}
+
 }  // namespace
+
+void launch_tgt_bounds(const double *d_fit, const double *d_base, const double *d_t_tgt, int n_tgt, int n_st, int has_ref_tx,
+                       double guard, double fs, int2 *d_bounds, cudaStream_t st)
+{
+    const int n = n_tgt * (n_st * (n_st - 1) / 2);
+    if (n > 0)
+        k_tgt_bounds<<<(n + 127) / 128, 128, 0, st>>>(d_fit, d_base, d_t_tgt, n_tgt, n_st, has_ref_tx, guard, fs, d_bounds);
+}
 
 void launch_window_ref_fit(const PeakRec *d_ref, int n_ref, int n_st, const double *d_t_ref, const double *d_t_mid,
                            const double *d_llh, const double *d_ref_tx, float min_margin, double max_resid, double *d_fit,
@@ -469,11 +508,13 @@ struct Tables {
     cudaStream_t st;
     PeakRec *ref = nullptr, *tgt = nullptr;
     double *rates = nullptr;
+    int2 *bounds = nullptr;   // tdoa_set_tgt_bounds: the TGT intervals, [n_tgt][P]
     ~Tables()
     {
         if (ref) cudaFreeAsync(ref, st);
         if (tgt) cudaFreeAsync(tgt, st);
         if (rates) cudaFreeAsync(rates, st);
+        if (bounds) cudaFreeAsync(bounds, st);
     }
 };
 
@@ -490,6 +531,31 @@ int station_rates(tdoa_engine *e, const tdoa_window_opts *o, const WinTimes &T, 
                           nullptr, e->stream);
     launch_station_rates(d_fit, S, d_rates, d_rates + S, e->stream);
     count_launch(e, 2);
+    CU(cudaGetLastError());
+    return end_call(e, false);
+}
+
+// the TGT intervals from the REF table, as one call of their own: k_window_ref_fit (with the REF transmitter's
+// geometric term), k_baselines, k_tgt_bounds
+int tgt_bounds(tdoa_engine *e, const double *stations_llh, const tdoa_window_opts *o, const WinTimes &T, const PeakRec *d_ref,
+               int2 *d_bounds)
+{
+    int rc = begin_call(e);
+    if (rc) return rc;
+    const int S = e->cfg.n_stations, P = S * (S - 1) / 2;
+    const double *d_llh = nullptr, *d_t_ref = nullptr, *d_t_tgt = nullptr, *d_ref_tx = nullptr;
+    double *d_fit = nullptr, *d_base = nullptr;
+    if ((rc = upload(e, std::vector<double>(stations_llh, stations_llh + (size_t)3 * S), &d_llh)) ||
+        (rc = upload(e, T.t_ref, &d_t_ref)) || (rc = upload(e, T.t_tgt, &d_t_tgt)) ||
+        (o->has_ref_tx && (rc = upload(e, std::vector<double>(o->ref_tx_llh, o->ref_tx_llh + 3), &d_ref_tx))) ||
+        (rc = alloc_t(e, &d_fit, (size_t)kWindowFitDoubles * P)) || (rc = alloc_t(e, &d_base, (size_t)P)))
+        return rc;
+    launch_window_ref_fit(d_ref, T.n_ref, S, d_t_ref, nullptr, d_llh, d_ref_tx, o->min_margin, o->ref_max_residual, d_fit,
+                          nullptr, e->stream);
+    launch_baselines(d_llh, S, d_base, e->stream);
+    launch_tgt_bounds(d_fit, d_base, d_t_tgt, T.n_tgt, S, o->has_ref_tx ? 1 : 0, e->tgt_guard, e->cfg.sample_rate, d_bounds,
+                      e->stream);
+    count_launch(e, 3);
     CU(cudaGetLastError());
     return end_call(e, false);
 }
@@ -537,33 +603,46 @@ int process_windows_impl(tdoa_engine *e, const char *fn, const double *stations_
     Tables tab{e->stream};
     CU(cudaMallocAsync(reinterpret_cast<void **>(&tab.ref), (size_t)ref.n * P * sizeof(PeakRec), e->stream));
     CU(cudaMallocAsync(reinterpret_cast<void **>(&tab.tgt), (size_t)tgt.n * P * sizeof(PeakRec), e->stream));
+    // the TGT intervals (tdoa_set_tgt_bounds), from the REF table of the same call
+    const bool bounded = e->tgt_bounds;
+    if (bounded) CU(cudaMallocAsync(reinterpret_cast<void **>(&tab.bounds), (size_t)tgt.n * P * sizeof(int2), e->stream));
     // the pair loop of one kind into its device table: dealt and gathered as tdoa_xcorr deals them, or on this GPU
     bool sharded[2] = {false, false};
-    auto pass = [&](int kind, const double *d_rates) -> int {
+    auto pass = [&](int kind, const double *d_rates, const int2 *d_bounds) -> int {
         const WinGeom &G = kind == TDOA_KIND_REF ? ref : tgt;
         PeakRec *table = kind == TDOA_KIND_REF ? tab.ref : tab.tgt;
         if ((sharded[kind] = multi_wants(e, G.n))) {
             if (const int rc2 = begin_call(e)) return rc2;
             ShardPart Q = T.parts[kind];
             Q.out = reinterpret_cast<tdoa_peak *>(table); Q.out_is_device = true; Q.rates = d_rates;
+            std::vector<int2> h_bounds;   // dealt with the windows: every rank takes its windows' intervals
+            if (d_bounds) {
+                h_bounds.resize((size_t)G.n * P);
+                CU(cudaMemcpyAsync(h_bounds.data(), d_bounds, h_bounds.size() * sizeof(int2), cudaMemcpyDeviceToHost, e->stream));
+                CU(cudaStreamSynchronize(e->stream));
+                Q.bounds = h_bounds.data();
+            }
             return xcorr_sharded(e, std::vector<ShardPart>{Q});
         }
-        return xcorr_impl(e, kind, G.start, G.len, G.n, G.hop, kind == TDOA_KIND_REF ? ref_out : tgt_out, false, table, d_rates);
+        return xcorr_impl(e, kind, G.start, G.len, G.n, G.hop, kind == TDOA_KIND_REF ? ref_out : tgt_out, false, table, d_rates,
+                          d_bounds);
     };
+    auto bounds = [&]() -> int { return bounded ? tgt_bounds(e, stations_llh, o, T, tab.ref, tab.bounds) : TDOA_OK; };
     if (retimed) {
         // the TGT pass needs the rates, the rates need the gathered REF table: two meetings of the ranks
         CU(cudaMallocAsync(reinterpret_cast<void **>(&tab.rates), (size_t)2 * S * sizeof(double), e->stream));
-        if ((rc = pass(TDOA_KIND_REF, nullptr)) || (rc = station_rates(e, o, T, tab.ref, tab.rates)) ||
-            (rc = pass(TDOA_KIND_TGT, tab.rates)))
+        if ((rc = pass(TDOA_KIND_REF, nullptr, nullptr)) || (rc = station_rates(e, o, T, tab.ref, tab.rates)) ||
+            (rc = bounds()) || (rc = pass(TDOA_KIND_TGT, tab.rates, tab.bounds)))
             return rc;
-    } else if (multi_wants(e, ref.n + tgt.n)) {   // the tables tdoa_xcorr_windows gathers, left on this rank's device
+    } else if (!bounded && multi_wants(e, ref.n + tgt.n)) {   // the tables tdoa_xcorr_windows gathers, left on this rank's device
         T.parts[TDOA_KIND_REF].out = reinterpret_cast<tdoa_peak *>(tab.ref);
         T.parts[TDOA_KIND_TGT].out = reinterpret_cast<tdoa_peak *>(tab.tgt);
         for (ShardPart &Q : T.parts) Q.out_is_device = true;
         if ((rc = xcorr_sharded(e, T.parts))) return rc;
         sharded[0] = sharded[1] = true;
-    } else {         // tdoa_xcorr_windows on one GPU: the REF pair loop, then the TGT pair loop
-        if ((rc = pass(TDOA_KIND_REF, nullptr)) || (rc = pass(TDOA_KIND_TGT, nullptr))) return rc;
+    } else {   // tdoa_xcorr_windows on one GPU (the REF pair loop, then the TGT pair loop), or bounded: the ranks meet twice
+        if ((rc = pass(TDOA_KIND_REF, nullptr, nullptr)) || (rc = bounds()) || (rc = pass(TDOA_KIND_TGT, nullptr, tab.bounds)))
+            return rc;
     }
     if ((rc = begin_call(e))) return rc;
     if (sharded[TDOA_KIND_REF] && ref_out)

@@ -167,16 +167,23 @@ __device__ double warp_second_abs(const double *c, int n, int skip)
     return m;
 }
 
+// A bounded record (EXTENDED) scans its run [i0, i1] only: arg-max, runner-up and the parabola's neighbours.
 __global__ void __launch_bounds__(32) k_peak(const PeakJob *jobs)
 {
     const PeakJob &J = jobs[blockIdx.x];
     PeakRec r;
     r.lag = 0; r.flags = J.flags; r.corr = 0.0; r.frac = 0.f; r.margin = 0.f; r.first_lag = 0; r.n_blocks = J.nb;
+    int i0, i1;
+    if (bound_run(J.bound, J.lag_origin, J.decim, J.n_lags, &i0, &i1))
+        r.flags |= i0 > i1 ? TDOA_PEAK_BOUNDED | TDOA_PEAK_EMPTY : TDOA_PEAK_BOUNDED;
     double first = 0.0;
-    if (J.nb > 0 && J.n_lags > 0) {
-        const Best b = warp_argmax_abs(J.corr, J.n_lags);
+    if (J.nb > 0 && i0 <= i1) {
+        const double *c = J.corr + i0;
+        const int n = i1 - i0 + 1;
+        Best b = warp_argmax_abs(c, n);
+        const double second = warp_second_abs(c, n, b.idx);
+        b.idx += i0;
         first = b.v;
-        const double second = warp_second_abs(J.corr, J.n_lags, b.idx);
         r.lag = b.idx + J.lag_origin;
         r.first_lag = r.lag;
         r.corr = b.v;
@@ -192,7 +199,7 @@ __global__ void __launch_bounds__(32) k_peak(const PeakJob *jobs)
         }
         if (J.variant == CORR_EXTENDED) {
             // 3-point parabolic vertex on |c| (engine-defined; oracle orc_peak_parabolic)
-            if (b.idx > 0 && b.idx < J.n_lags - 1) {
+            if (b.idx > i0 && b.idx < i1) {
                 const double a = fabs(J.corr[b.idx - 1]), m = fabs(J.corr[b.idx]), d = fabs(J.corr[b.idx + 1]);
                 const double den = a - 2.0 * m + d;
                 r.frac = den != 0.0 ? (float)(0.5 * (a - d) / den) : 0.f;

@@ -186,7 +186,8 @@ __global__ void __launch_bounds__(kThreads, 1) k_fft_finish(const FftJob *jobs, 
 // ---------------------------------------------------------------- candidate selection
 // One CTA per pair.  Candidates = lags whose approximate |corr| is within tol of the
 // maximum over the whole search, plus (sanity > 0) the same for the re-search range
-// [0, sanity), plus (neighbours) the lags either side for the parabolic vertex.
+// [0, sanity), plus (neighbours) the lags either side for the parabolic vertex.  A bounded
+// record (EXTENDED) takes all three from its run [i0, i1] only.
 __global__ void __launch_bounds__(256) k_select_candidates(const SelJob *jobs)
 {
     __shared__ float s_red[256];
@@ -194,12 +195,14 @@ __global__ void __launch_bounds__(256) k_select_candidates(const SelJob *jobs)
     const SelJob &J = jobs[blockIdx.x];
     const int tid = threadIdx.x;
     const int n = J.n_lags;
-    if (n <= 0) {
+    int i0, i1;
+    bound_run(J.bound, J.lag_origin, J.decim, n, &i0, &i1);
+    if (i0 > i1) {   // n <= 0, or an empty run: k_peak_candidates writes the record
         if (tid == 0) *J.n_cand = 0;
         return;
     }
     float m1 = 0.f, m2 = 0.f;
-    for (int i = tid; i < n; i += 256) {
+    for (int i = i0 + tid; i <= i1; i += 256) {
         const float a = fabsf(J.approx[i]);
         m1 = fmaxf(m1, a);
         if (i < J.sanity) m2 = fmaxf(m2, a);
@@ -219,7 +222,7 @@ __global__ void __launch_bounds__(256) k_select_candidates(const SelJob *jobs)
     // is exactly 0, and the reference's strict `>` keeps its initial (first lag, 0.0).  One
     // candidate says the same; without this the flat surface makes every lag a candidate.
     if (m1 == 0.f && ((J.t_stats && J.t_stats[ST_POWER1] == 0.0) || (J.s_stats && J.s_stats[ST_POWER1] == 0.0))) {
-        if (tid == 0) { J.cand[0] = 0; *J.n_cand = 1; *J.approx_max = 0.f; }
+        if (tid == 0) { J.cand[0] = i0; *J.n_cand = 1; *J.approx_max = 0.f; }
         return;
     }
     const float thr1 = m1 - J.tol, thr2 = m2 - J.tol;
@@ -228,12 +231,12 @@ __global__ void __launch_bounds__(256) k_select_candidates(const SelJob *jobs)
     __shared__ int s_list[256];
     if (tid == 0) s_base = 0;
     __syncthreads();
-    for (int i = tid; i < n; i += 256) {
+    for (int i = i0 + tid; i <= i1; i += 256) {
         const float a = fabsf(J.approx[i]);
         bool take = a >= thr1 || (i < J.sanity && a >= thr2);
         if (!take && J.neighbours) {
-            if (i > 0 && fabsf(J.approx[i - 1]) >= thr1) take = true;
-            if (i + 1 < n && fabsf(J.approx[i + 1]) >= thr1) take = true;
+            if (i > i0 && fabsf(J.approx[i - 1]) >= thr1) take = true;
+            if (i < i1 && fabsf(J.approx[i + 1]) >= thr1) take = true;
         }
         if (take) {
             const int pos = atomicAdd(&s_base, 1);
@@ -509,6 +512,8 @@ __global__ void __launch_bounds__(kCandThreads) k_corr_candidates(const PairJob 
 // ---------------------------------------------------------------- peak from the exact candidate values
 // One CTA (8 warps) per pair: warp w adds the blocks of candidates w, w+8, ...; then
 // thread 0 runs the reference's selection (strict >, ascending lag; sanity re-search).
+// A bounded record's candidates all lie in its run (k_select_candidates), so only the
+// runner-up, the BOUNDED flag and an empty run's EMPTY flag need the run here.
 __global__ void __launch_bounds__(256) k_peak_candidates(const PairJob *jobs, const CandJob *cjobs, const PeakJob *pjobs)
 {
     __shared__ double s_val[kMaxCand];
@@ -559,8 +564,10 @@ __global__ void __launch_bounds__(256) k_peak_candidates(const PairJob *jobs, co
     __shared__ int s_best_idx;
     if (tid == 0) s_best_idx = best >= 0 ? C.cand[best] : -1;
     __syncthreads();
+    int i0, i1;
+    const bool bounded = bound_run(K.bound, K.lag_origin, K.decim, K.n_lags, &i0, &i1);
     float ru = 0.f;
-    for (int i = tid; i < K.n_lags; i += 256)
+    for (int i = i0 + tid; i <= i1; i += 256)
         if (i != s_best_idx) ru = fmaxf(ru, fabsf(C.approx[i]));
     s_red[tid] = ru;
     __syncthreads();
@@ -570,6 +577,7 @@ __global__ void __launch_bounds__(256) k_peak_candidates(const PairJob *jobs, co
     r.lag = 0; r.flags = K.flags; r.corr = 0.0; r.frac = 0.f; r.margin = 0.f; r.first_lag = 0; r.n_blocks = K.nb;
     if (n_all > C.max_cand) r.flags |= 0x10u;  // TDOA_PEAK_OVERFLOW: the host re-runs this pair brute force
     r.flags |= (uint32_t)min(n_all, 255) << 16;  // TDOA_PEAK_NCAND: exactly evaluated lags
+    if (bounded) r.flags |= i0 > i1 ? TDOA_PEAK_BOUNDED | TDOA_PEAK_EMPTY : TDOA_PEAK_BOUNDED;
     if (K.nb > 0 && best >= 0) {
         const int bi = C.cand[best];
         r.lag = bi + K.lag_origin;

@@ -48,6 +48,8 @@ struct SelJob {
     int *n_cand;          // candidates found (may exceed max_cand: overflow)
     float *approx_max;
     const double *t_stats, *s_stats;   // per-signal statistics (ST_POWER1): a signal without power is identically zero
+    const int2 *bound;    // the record's interval (PeakJob::bound): maximum, candidates and neighbours from its run only
+    int lag_origin, decim;
 };
 
 struct CandJob {
