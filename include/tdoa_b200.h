@@ -71,7 +71,8 @@ typedef struct tdoa_engine tdoa_engine; /* opaque: device memory, streams, plans
  * other lag of the first pass.  On the every-lag path (TDOA_PEAK_BRUTE: use_fft = 0, the candidate-overflow redo)
  * every |corr| is exact.  On the FFT paths the runner-up is the largest |approximate value| of the f32 ranking
  * (exact values exist only for the candidates), so the margin differs from the exact one by at most eps / |peak|
- * plus its rounding, eps (~1e-6 in correlation units) being the ranking's error.  Two tied peaks: margin 0 exactly
+ * plus its rounding, eps (<= 1e-6 in correlation units, measured against an f64 correlation on every FFT path,
+ * weak-branch stations beside strong ones included) being the ranking's error.  Two tied peaks: margin 0 exactly
  * on the every-lag path, |margin| <= eps / |peak| on the FFT paths.
  * Which signal is the template: BINARY and SOURCE make the shorter of the two signals the template
  * (processor.go:653-661), so with signal 1 longer the lag is the delay of signal 1.  EXTENDED keeps signal 1 as
@@ -226,6 +227,17 @@ TDOA_API int tdoa_xcorr(tdoa_engine *e, int32_t kind, int64_t win_start, int64_t
 /* Same, peaks left in device memory (e.g. an NCCL send buffer); d_out[n_windows*P]. */
 TDOA_API int tdoa_xcorr_device(tdoa_engine *e, int32_t kind, int64_t win_start, int64_t win_len,
                                int32_t n_windows, int64_t hop, tdoa_peak *d_out);
+/* Ranking-plane probe (BINARY and EXTENDED): tdoa_xcorr, plus the f32 ranking each FFT record's candidates were
+ * chosen from.  out[n_windows * P] is bit for bit what tdoa_xcorr returns; ranking[(w * P + p) * M + d], with M =
+ * max_lag (BINARY) or 2 (max_lag / D) + 1 (EXTENDED, D = decimate), is the record's approx at lag index d (lag
+ * d in BINARY, d - max_lag / D in EXTENDED, correlation lags before the decimator's scaling).  NaN past the
+ * record's lag count and on records that had no ranking (BRUTE without the candidate overflow: use_fft = 0, <= 8
+ * lags, BINARY's second template; EMPTY); a record redone lag by lag after the overflow keeps its FFT plane.  The
+ * planes are copied out only in this call: tdoa_xcorr runs exactly as before.  Refused (TDOA_E_INVALID): SOURCE
+ * mode, an engine over several GPUs (n_devices > 1 or tdoa_comm_init), a NULL out or ranking, and what tdoa_xcorr
+ * refuses. */
+TDOA_API int tdoa_xcorr_ranking(tdoa_engine *e, int32_t kind, int64_t win_start, int64_t win_len, int32_t n_windows,
+                                int64_t hop, tdoa_peak *out, float *ranking);
 
 /* ---- bounded lag search (EXTENDED mode; no reference equivalent; engine-defined): tdoa_xcorr with an interval
  * [lag_lo[k], lag_hi[k]] (int32, capture samples: the units of the records) for each record k = w * P + p.  With

@@ -24,7 +24,7 @@ ERRORS = {-1: "TDOA_E_INVALID", -2: "TDOA_E_NODEVICE", -3: "TDOA_E_CUDA", -4: "T
 # every symbol include/tdoa_b200.h declares (tests check the library exports them all)
 ABI_SYMBOLS = [
     "tdoa_default_config", "tdoa_create", "tdoa_destroy", "tdoa_last_error", "tdoa_host_alloc", "tdoa_host_free",
-    "tdoa_load_u8", "tdoa_load_file", "tdoa_load_u8_pinned", "tdoa_load_u8_device", "tdoa_unpack", "tdoa_preprocess", "tdoa_set_channel", "tdoa_set_tgt_bounds", "tdoa_xcorr", "tdoa_xcorr_bounded", "tdoa_xcorr_device", "tdoa_xcorr_windows", "tdoa_process", "tdoa_process_windows", "tdoa_window_fixes", "tdoa_process_windows_grid", "tdoa_window_fixes_grid", "tdoa_process_windows_retimed", "tdoa_closure", "tdoa_process_windows_closure", "tdoa_window_fixes_closure", "tdoa_exclude_stations", "tdoa_process_windows_exclude", "tdoa_window_fixes_exclude", "tdoa_xcorr_info", "tdoa_analyze",
+    "tdoa_load_u8", "tdoa_load_file", "tdoa_load_u8_pinned", "tdoa_load_u8_device", "tdoa_unpack", "tdoa_preprocess", "tdoa_set_channel", "tdoa_set_tgt_bounds", "tdoa_xcorr", "tdoa_xcorr_bounded", "tdoa_xcorr_device", "tdoa_xcorr_ranking", "tdoa_xcorr_windows", "tdoa_process", "tdoa_process_windows", "tdoa_window_fixes", "tdoa_process_windows_grid", "tdoa_window_fixes_grid", "tdoa_process_windows_retimed", "tdoa_closure", "tdoa_process_windows_closure", "tdoa_window_fixes_closure", "tdoa_exclude_stations", "tdoa_process_windows_exclude", "tdoa_window_fixes_exclude", "tdoa_xcorr_info", "tdoa_analyze",
     "tdoa_cross_correlate", "tdoa_baselines", "tdoa_solve", "tdoa_solve_binary", "tdoa_solve_ls", "tdoa_grid", "tdoa_grid_masked", "tdoa_get_stats", "tdoa_stream",
     "tdoa_set_stream", "tdoa_synchronize", "tdoa_selftest",
     "tdoa_comm_unique_id", "tdoa_comm_init", "tdoa_comm_rank", "tdoa_shard_windows",
@@ -179,6 +179,7 @@ def load_library():
     L.tdoa_process.argtypes = [vp, vp, vp, vp, vp, vp, vp, C.POINTER(i32), C.POINTER(i32)]
     L.tdoa_analyze.argtypes = [vp, i32, i32, vp, vp]
     L.tdoa_xcorr_device.argtypes = [vp, i32, i64, i64, i32, i64, vp]
+    L.tdoa_xcorr_ranking.argtypes = [vp, i32, i64, i64, i32, i64, vp, vp]
     L.tdoa_xcorr_windows.argtypes = [vp, i64, i64, i32, i32, i64, vp, vp]
     L.tdoa_process_windows.argtypes = [vp, vp, C.POINTER(WindowOpts), i64, i64, i32, i32, i64] + [vp] * 9
     L.tdoa_window_fixes.argtypes = [vp, vp, C.POINTER(WindowOpts), i64, i64, i32, i32, i64] + [vp] * 9
@@ -436,6 +437,20 @@ class Engine:
         out = np.zeros((n_windows, self.n_pairs), PEAK_DTYPE)
         self._check(self._lib.tdoa_xcorr(self._h, kind, win_start, win_len, n_windows, hop, _ptr(out)))
         return out
+
+    def xcorr_ranking(self, kind: int, win_start: int = 0, win_len: int = 0, n_windows: int = 1, hop: int = 0):
+        """xcorr plus the f32 ranking plane each FFT record's candidates came from (tdoa_xcorr_ranking): (records,
+        ranking), ranking[w, p, d] the approximate correlation at lag index d (lag d in BINARY, d - max_lag / D in
+        EXTENDED); NaN past the record's lags and on records without a ranking.  One GPU only."""
+        if self.cfg.mode == MODE_EXTENDED:
+            m = 2 * (self.cfg.max_lag // max(1, self.cfg.decimate)) + 1
+        else:
+            m = self.cfg.max_lag
+        out = np.zeros((n_windows, self.n_pairs), PEAK_DTYPE)
+        ranking = np.empty((n_windows, self.n_pairs, max(m, 0)), np.float32)
+        self._check(self._lib.tdoa_xcorr_ranking(self._h, kind, win_start, win_len, n_windows, hop, _ptr(out),
+                                                 _ptr(ranking)))
+        return out, ranking
 
     def xcorr_bounded(self, kind: int, lo, hi, win_start: int = 0, win_len: int = 0, n_windows: int = 1,
                       hop: int = 0) -> np.ndarray:

@@ -119,6 +119,11 @@ struct tdoa_engine {
     tdoa::MultiState *multi = nullptr;   // engine_multi.cu; nullptr: one process, one GPU
     bool tgt_bounds = false;             // tdoa_set_tgt_bounds: the windowed calls bound their TGT lag search
     double tgt_guard = 0.0;              // samples added to each side of those intervals
+    // tdoa_xcorr_ranking: while rank_dump is set, run_fft copies each record's ranking plane to
+    // rank_dump + (record - rank_base) * rank_stride (device)
+    float *rank_dump = nullptr;
+    const tdoa::PeakRec *rank_base = nullptr;
+    int rank_stride = 0;
 };
 
 namespace tdoa {

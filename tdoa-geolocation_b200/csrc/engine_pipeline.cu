@@ -10,6 +10,7 @@
 #include <cstdio>
 #include <cstring>
 #include <string>
+#include <unordered_map>
 #include <vector>
 
 #include "engine_internal.h"
@@ -722,6 +723,12 @@ int run_fft(tdoa_engine *e, std::vector<CorrPlan *> &plans)
     std::vector<SpecGroup> spec_groups;
     std::vector<char> spec_plan(np, 0);
     const bool tiled = e->cfg.use_fft != 2;
+    // statistics (ST_SCALE) of every plane: the transforms scale planes of unusual power as they load them
+    std::unordered_map<const float *, const double *> stats_of;
+    for (const CorrPlan *pl : plans) {
+        stats_of[pl->job.t_re] = pl->job.t_stats;
+        stats_of[pl->job.s_re] = pl->job.s_stats;
+    }
     {
         std::vector<char> done(np, 0);
         for (int p0 = 0; p0 < np; p0++) {
@@ -797,6 +804,25 @@ int run_fft(tdoa_engine *e, std::vector<CorrPlan *> &plans)
             }
         }
     }
+    // the plane each plan's template (signal) shares its ranking transform with: the finish needs both planes'
+    // scales to know which the transform applied (rank_post, xcorr_fft.h).  This restates how the jobs below pack
+    // planes (t + i s; tile rows and columns two at a time; spectra rows 2m, 2m + 1): a change to one needs the
+    // other, and the weak-station cases of tests/test_gpu_ranking.py fail on any mismatch.
+    std::vector<const double *> t_pack(np), s_pack(np);
+    for (int p = 0; p < np; p++) { t_pack[p] = plans[p]->job.s_stats; s_pack[p] = plans[p]->job.t_stats; }   // t + i s
+    for (const Tile &T : tiles)
+        for (int q = 0; q < 4; q++)
+            if (T.plan[q] >= 0 && tiled) {
+                t_pack[T.plan[q]] = stats_of[T.t[1 - q / 2]];
+                s_pack[T.plan[q]] = stats_of[T.s[1 - q % 2]];
+            }
+    for (const SpecGroup &G : spec_groups)
+        for (int p : G.plans) {
+            const size_t tr = std::find(G.rows.begin(), G.rows.end(), plans[p]->job.t_re) - G.rows.begin();
+            const size_t sc = std::find(G.cols.begin(), G.cols.end(), plans[p]->job.s_re) - G.cols.begin();
+            t_pack[p] = stats_of[G.rows[(tr ^ 1) < G.rows.size() ? tr ^ 1 : tr]];
+            s_pack[p] = stats_of[G.cols[(sc ^ 1) < G.cols.size() ? sc ^ 1 : sc]];
+        }
     // lag chunks
     int n_fft_jobs = 0, n_tile_jobs = 0;
     for (int p = 0; p < np; p++)
@@ -848,6 +874,7 @@ int run_fft(tdoa_engine *e, std::vector<CorrPlan *> &plans)
         for (int c0 = 0; c0 < J.n_lags && !big_plan[p] && !spec_plan[p]; c0 += kLagW) {
             FftJob F{};
             F.t = J.t_re; F.s = J.s_re; F.t_stats = J.t_stats; F.s_stats = J.s_stats;
+            F.t_pack = t_pack[p]; F.s_pack = s_pack[p];
             F.t_off = J.t_off; F.n_t = J.n_t; F.sl = J.sl;
             F.s_off = (i64)J.lag0 + c0;
             F.n_lags = std::min(kLagW, J.n_lags - c0);
@@ -886,6 +913,8 @@ int run_fft(tdoa_engine *e, std::vector<CorrPlan *> &plans)
                 const FftJob &F0 = fjobs[first_job[lead] + ci];
                 TileJob TJ{};
                 TJ.t0 = T.t[0]; TJ.t1 = T.t[1]; TJ.s0 = T.s[0]; TJ.s1 = T.s[1];
+                TJ.t0_stats = stats_of[T.t[0]]; TJ.t1_stats = stats_of[T.t[1]];
+                TJ.s0_stats = stats_of[T.s[0]]; TJ.s1_stats = stats_of[T.s[1]];
                 TJ.t_off = F0.t_off; TJ.n_t = F0.n_t; TJ.sl = F0.sl; TJ.s_off = F0.s_off;
                 TJ.n_seg = F0.n_seg; TJ.n_cta = F0.n_cta;
                 for (int q = 0; q < 4; q++) TJ.partials[q] = T.plan[q] >= 0 ? fjobs[first_job[T.plan[q]] + ci].partials : nullptr;
@@ -934,6 +963,7 @@ int run_fft(tdoa_engine *e, std::vector<CorrPlan *> &plans)
                     const PairJob &J = plans[p]->job;
                     FftJob F{};
                     F.t = J.t_re; F.s = J.s_re; F.t_stats = J.t_stats; F.s_stats = J.s_stats;
+                    F.t_pack = t_pack[p]; F.s_pack = s_pack[p];
                     F.t_off = J.t_off; F.n_t = J.n_t; F.sl = J.sl; F.s_off = (i64)J.lag0 + c0;
                     F.n_lags = U.lw; F.n_seg = U.n_seg; F.n_cta = 0; F.partials = nullptr;
                     F.spectrum = static_cast<float2 *>(take((size_t)kFftBins * sizeof(float2)));
@@ -973,6 +1003,7 @@ int run_fft(tdoa_engine *e, std::vector<CorrPlan *> &plans)
                     const std::vector<const float *> &src = tpl ? G.rows : G.cols;
                     const size_t a = (size_t)2 * (tpl ? m : m - n_pk_t);
                     F.x0 = src[a]; F.x1 = a + 1 < src.size() ? src[a + 1] : src[a];
+                    F.x0_stats = stats_of[F.x0]; F.x1_stats = stats_of[F.x1];
                     F.stride = U.seg; F.n_seg = U.n_seg;
                     if (tpl) { F.base = K.t_off; F.lo = K.t_off; F.hi = K.t_off + K.n_t; F.seg_len = U.seg; }
                     else { F.base = (i64)K.lag0 + U.c0; F.lo = 0; F.hi = K.sl; F.seg_len = kFftN; }
@@ -1069,9 +1100,11 @@ int run_fft(tdoa_engine *e, std::vector<CorrPlan *> &plans)
                     const i64 first = (i64)g * G.Ts;
                     BigColJob a{};
                     a.x0 = T.t[0]; a.x1 = T.t[1]; a.base = G.t_off + first; a.lo = 0;
+                    a.x0_stats = stats_of[a.x0]; a.x1_stats = stats_of[a.x1];
                     a.hi = std::max<i64>(0, std::min<i64>(G.Ts, G.n_t - first)); a.out = buf(k, 0);
                     BigColJob b{};
                     b.x0 = T.s[0]; b.x1 = T.s[1]; b.base = G.lag0 + first;
+                    b.x0_stats = stats_of[b.x0]; b.x1_stats = stats_of[b.x1];
                     b.lo = std::max<i64>(0, -b.base); b.hi = std::max<i64>(b.lo, std::min<i64>(kBigN, G.sl - b.base));
                     b.out = buf(k, 1);
                     cj.push_back(a); cj.push_back(b);
@@ -1095,14 +1128,12 @@ int run_fft(tdoa_engine *e, std::vector<CorrPlan *> &plans)
                 for (int a = 0; a < 2; a++) {
                     const int q0 = T.plan[2 * a], q1 = T.plan[2 * a + 1];
                     if (q0 < 0 && q1 < 0) continue;
-                    const int any = q0 >= 0 ? q0 : q1;
                     BigOutJob O{};
                     O.G = buf(k, 2 + a);
                     O.approx0 = q0 >= 0 ? const_cast<float *>(sjobs[q0].approx) : nullptr;
                     O.approx1 = q1 >= 0 ? const_cast<float *>(sjobs[q1].approx) : nullptr;
-                    O.t_stats = plans[any]->job.t_stats;
-                    O.s0_stats = q0 >= 0 ? plans[q0]->job.s_stats : plans[any]->job.s_stats;
-                    O.s1_stats = q1 >= 0 ? plans[q1]->job.s_stats : plans[any]->job.s_stats;
+                    O.t_stats = stats_of[T.t[a]]; O.t_pack = stats_of[T.t[1 - a]];
+                    O.s0_stats = stats_of[T.s[0]]; O.s1_stats = stats_of[T.s[1]];
                     O.n_t = geo[k].n_t; O.n_lags = geo[k].n_lags;
                     irj.push_back(BigRowJob{buf(k, 2 + a), 1});
                     oj.push_back(O);
@@ -1118,6 +1149,11 @@ int run_fft(tdoa_engine *e, std::vector<CorrPlan *> &plans)
     }
     launch_select_candidates(d_s, np, e->stream);
     span_end(e, sp_fft);
+    if (e->rank_dump) {   // tdoa_xcorr_ranking: the planes leave the arena before the call frees it
+        for (int p = 0; p < np; p++)
+            CU(cudaMemcpyAsync(e->rank_dump + (size_t)(plans[p]->peak.out - e->rank_base) * e->rank_stride, sjobs[p].approx,
+                               (size_t)sjobs[p].n_lags * sizeof(float), cudaMemcpyDeviceToDevice, e->stream));
+    }
     {
         const int sp = span_begin(e, SPAN_CAND);
         launch_corr_candidates(d_p, d_c, np, max_nb, e->stream);
@@ -1476,6 +1512,7 @@ int xcorr_impl(tdoa_engine *e, int32_t kind, int64_t win_start, int64_t win_len,
     if (out_is_device) d_out = reinterpret_cast<PeakRec *>(out);
     else if (d_table) d_out = d_table;
     else if ((rc = alloc_t(e, &d_out, (size_t)n_windows * P))) return rc;
+    e->rank_base = d_out;   // record index of a ranking plane (tdoa_xcorr_ranking)
     stats_reset(e);
     cudaEventRecord(e->ev[0], e->stream);
     // Two halves of the windows side by side on two streams (as tdoa_process does with the two
@@ -1635,6 +1672,42 @@ int tdoa_xcorr_device(tdoa_engine *e, int32_t kind, int64_t win_start, int64_t w
                       int64_t hop, tdoa_peak *d_out)
 {
     return xcorr_impl(e, kind, win_start, win_len, n_windows, hop, d_out, true);
+}
+
+int tdoa_xcorr_ranking(tdoa_engine *e, int32_t kind, int64_t win_start, int64_t win_len, int32_t n_windows, int64_t hop,
+                       tdoa_peak *out, float *ranking)
+{
+    static const char *fn = "tdoa_xcorr_ranking";
+    if (!e) return TDOA_E_INVALID;
+    int rc = begin_call(e);
+    if (rc) return rc;
+    if (e->multi || e->cfg.n_devices > 1)
+        return fail(e, TDOA_E_INVALID, "%s: a probe of one GPU; this engine deals its windows over several", fn);
+    if (e->cfg.mode == TDOA_MODE_SOURCE) return fail(e, TDOA_E_INVALID, "%s: SOURCE mode has no FFT search", fn);
+    if (!out || !ranking) return fail(e, TDOA_E_INVALID, "%s: out or ranking is NULL", fn);
+    if (n_windows < 1) return fail(e, TDOA_E_INVALID, "%s: bad window arguments", fn);
+    const int S = e->cfg.n_stations, P = S * (S - 1) / 2;
+    const int stride = e->cfg.mode == TDOA_MODE_EXTENDED ? 2 * (e->cfg.max_lag / decimation(e)) + 1 : e->cfg.max_lag;
+    const size_t bytes = (size_t)n_windows * P * stride * sizeof(float);
+    float *d = nullptr;
+    CU(cudaMalloc(&d, bytes));
+    // all-ones bytes are a NaN: what every slot keeps that no ranking plane covers
+    if (cudaMemsetAsync(d, 0xff, bytes, e->stream) != cudaSuccess) { cudaFree(d); CU(cudaGetLastError()); }
+    e->rank_dump = d;
+    e->rank_stride = stride;
+    rc = xcorr_impl(e, kind, win_start, win_len, n_windows, hop, out, false);
+    e->rank_dump = nullptr;
+    e->rank_base = nullptr;
+    cudaError_t err = cudaSuccess;
+    if (rc == TDOA_OK) {
+        err = cudaMemcpyAsync(ranking, d, bytes, cudaMemcpyDeviceToHost, e->stream);
+        if (err == cudaSuccess) err = cudaStreamSynchronize(e->stream);
+    } else {
+        cudaStreamSynchronize(e->stream);
+    }
+    cudaFree(d);
+    if (err != cudaSuccess) return fail(e, TDOA_E_CUDA, "%s: ranking read-back failed: %s", fn, cudaGetErrorString(err));
+    return rc;
 }
 
 int tdoa_xcorr_bounded(tdoa_engine *e, int32_t kind, int64_t win_start, int64_t win_len, int32_t n_windows, int64_t hop,

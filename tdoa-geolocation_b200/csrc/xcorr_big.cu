@@ -100,8 +100,10 @@ __global__ void __launch_bounds__(kColThreads) k_big_cols(const BigColJob *jobs,
     const BigColJob &J = jobs[blockIdx.y];
     const int tid = threadIdx.x, c = tid & 31;
     const int n2 = blockIdx.x * kCols + c;
-    // z[n] = x0[base + n] + i x1[base + n] for lo <= n < hi, else 0
+    // z[n] = x0[base + n] sc0 + i x1[base + n] sc1 for lo <= n < hi, else 0; sc = rank_pre (xcorr_fft.h), 1 unless
+    // the two planes' powers differ widely
     const float *__restrict__ x0 = J.x0 + J.base, *__restrict__ x1 = J.x1 + J.base;
+    const float sc0 = rank_pre(J.x0_stats, J.x1_stats), sc1 = rank_pre(J.x1_stats, J.x0_stats);
     const i64 lo = J.lo, hi = J.hi;
 #pragma unroll 1
     for (int g = 0; g < 4; g++) {   // 8 rows per thread in flight
@@ -111,6 +113,10 @@ __global__ void __launch_bounds__(kColThreads) k_big_cols(const BigColJob *jobs,
             const int n1 = (tid >> 5) + 8 * (8 * g + u);
             const i64 n = (i64)n1 * kN2 + n2;
             z[u] = (n >= lo && n < hi) ? make_float2(x0[n], x1[n]) : make_float2(0.f, 0.f);
+        }
+        if (sc0 != 1.f || sc1 != 1.f) {
+#pragma unroll
+            for (int u = 0; u < 8; u++) z[u] = make_float2(__fmul_rn(z[u].x, sc0), __fmul_rn(z[u].y, sc1));
         }
 #pragma unroll
         for (int u = 0; u < 8; u++) sm[((tid >> 5) + 8 * (8 * g + u)) * kCols + c] = z[u];
@@ -223,10 +229,12 @@ __global__ void __launch_bounds__(kColThreads) k_big_out(const BigOutJob *jobs, 
     __syncthreads();
     strip_fft256(sm, tid, tw);
     // c[n] = conj(X): real part -> pair (a, 0), imaginary part -> pair (a, 1); coefficient units:
-    // scale_t scale_s / n_t (processor.go:347-349, :709-717), 1/N of the inverse, 1/4 of 2T 2S
+    // scale_t scale_s / n_t (processor.go:347-349, :709-717) less what k_big_cols applied (rank_pre), 1/N of the
+    // inverse, 1/4 of 2T 2S
     const double k = J.n_t > 0 ? 0.25 / ((double)J.n_t * (double)kBigN) : 0.0;
-    const double sc0 = J.approx0 ? (double)(float)J.t_stats[ST_SCALE] * (double)(float)J.s0_stats[ST_SCALE] * k : 0.0;
-    const double sc1 = J.approx1 ? (double)(float)J.t_stats[ST_SCALE] * (double)(float)J.s1_stats[ST_SCALE] * k : 0.0;
+    const double st = rank_post(J.t_stats, J.t_pack);
+    const double sc0 = J.approx0 ? st * rank_post(J.s0_stats, J.s1_stats) * k : 0.0;
+    const double sc1 = J.approx1 ? st * rank_post(J.s1_stats, J.s0_stats) * k : 0.0;
     const int rows = (J.n_lags + kN2 - 1) / kN2;
     for (int r = tid >> 5; r < kN1; r += 8) {
         const int n1 = (r >> 4) + 16 * (r & 15);

@@ -38,6 +38,9 @@ __global__ void __launch_bounds__(kThreads, 2) k_fft_segments(const FftJob *jobs
     const int tid = threadIdx.x;
     const float *__restrict__ tp = J.t + J.t_off;
     const float *__restrict__ sp = J.s;
+    // xcorr_fft.h: 1 unless the two planes' powers differ widely
+    const float sc_t = rank_pre(J.t_stats, J.s_stats), sc_s = rank_pre(J.s_stats, J.t_stats);
+    const bool pre = sc_t != 1.f || sc_s != 1.f;
     float2 *tab = sm + kPad;
     for (int idx = tid; idx < kTabLen; idx += kThreads) tab[idx] = tw[(16 * (idx & 31) * (idx >> 5)) & (kN - 1)];
     // (the first barrier inside the segment loop orders these writes before their use)
@@ -77,6 +80,10 @@ __global__ void __launch_bounds__(kThreads, 2) k_fft_segments(const FftJob *jobs
                     if (g >= 0 && g < J.sl) b = sp[g];
                     v[r] = make_float2(a, b);
                 }
+            }
+            if (pre) {
+#pragma unroll
+                for (int r = 0; r < 32; r++) v[r] = make_float2(__fmul_rn(v[r].x, sc_t), __fmul_rn(v[r].y, sc_s));
             }
             pass1_store(v, tid, sm);
         }
@@ -171,8 +178,9 @@ __global__ void __launch_bounds__(kThreads, 1) k_fft_finish(const FftJob *jobs, 
     pass_load16(sm, tid + 256, u1);
     pass3_compute(u0, tid, tw);
     pass3_compute(u1, tid + 256, tw);
-    // correlation coefficient units: scale_t * scale_s / n_t (processor.go:347-349, :709-717)
-    const double sc = J.n_t > 0 ? (double)(float)J.t_stats[ST_SCALE] * (double)(float)J.s_stats[ST_SCALE] /
+    // correlation coefficient units: scale_t * scale_s / n_t (processor.go:347-349, :709-717), less the scales the
+    // transforms applied as they loaded the planes (rank_pre)
+    const double sc = J.n_t > 0 ? rank_post(J.t_stats, J.t_pack) * rank_post(J.s_stats, J.s_pack) /
                                       ((double)J.n_t * (double)kN)
                                 : 0.0;
 #pragma unroll

@@ -10,10 +10,34 @@ constexpr int kSeg = kFftN - kLagW;       // template samples per segment (6144 
 constexpr int kMaxCand = 64;              // candidate lags re-evaluated exactly per pair
 constexpr int kFftBins = kFftN / 2 + 1;
 
+// The ranking transforms pack two real planes into one complex FFT and split the spectra with Z[k] +- conj Z[N-k],
+// so each spectrum carries rounding on the scale of the other plane: with planes of powers P_a, P_b the ranking's
+// error in coefficient units grows like eps log N sqrt(P_a / P_b) (a weak-branch station of near-constant bytes
+// beside strong ones reaches 2.5e9 and errors up to 1e-2, far over the selection tolerance:
+// profiles/r11_ranking.jsonl).  When the scales
+// f32(1 / sqrt(power)) of the two planes of a transform differ by more than kRankPackRatio, both are multiplied by
+// their scale as the transform loads them -- the very multiply k_corr_candidates applies -- and the finish leaves
+// them out; otherwise (stations of similar power: no multiply at all) the finish applies both scales.  Planes
+// that share a transform then differ in power by at most kRankPackRatio^2.
+constexpr float kRankPackRatio = 16.f;
+// a and b: statistics of the two planes of one transform
+__device__ __forceinline__ bool rank_scaled(const double *a, const double *b)
+{
+    const float sa = (float)a[ST_SCALE], sb = (float)b[ST_SCALE];
+    return fmaxf(sa, sb) > kRankPackRatio * fminf(sa, sb);
+}
+// the factor plane a is loaded with (packed with b), and the one the finish applies for it
+__device__ __forceinline__ float rank_pre(const double *a, const double *b) { return rank_scaled(a, b) ? (float)a[ST_SCALE] : 1.f; }
+__device__ __forceinline__ double rank_post(const double *a, const double *b)
+{
+    return rank_scaled(a, b) ? 1.0 : (double)(float)a[ST_SCALE];
+}
+
 // One (pair, lag chunk): approx[d] ~ corr(lag0 + d), d in [0, n_lags), n_lags <= kLagW.
 struct FftJob {
     const float *t, *s;              // real planes, pre-normalise
-    const double *t_stats, *s_stats; // ST_SCALE applied in the finish kernel
+    const double *t_stats, *s_stats; // ST_SCALE (rank_post in the finish)
+    const double *t_pack, *s_pack;   // statistics of the plane t (s) shares its ranking transform with
     i64 t_off;                       // template starts at t + t_off
     i64 n_t;                         // template samples that take part
     i64 sl;                          // signal length
@@ -32,6 +56,7 @@ struct FftJob {
 struct TileJob {
     const float *t0, *t1;   // template planes (t1 == t0 when the tile has one template)
     const float *s0, *s1;   // signal planes
+    const double *t0_stats, *t1_stats, *s0_stats, *s1_stats;   // their statistics (rank_pre as the samples are loaded)
     i64 t_off, n_t, sl, s_off;
     int n_seg, n_cta;
     float2 *partials[4];    // [n_cta][kFftBins] each
@@ -65,8 +90,9 @@ constexpr int kBigN1 = 256;
 constexpr i64 kBigN = (i64)kBigN1 * kFftN;     // 2 097 152 complex points
 constexpr int kBigMinLags = 8192;              // narrower searches stay with the segment kernel
 
-struct BigColJob {      // forward column pass of one transform: z[n] = x0[base+n] + i x1[base+n], lo <= n < hi
+struct BigColJob {      // forward column pass of one transform: z[n] = x0[base+n] sc0 + i x1[base+n] sc1, lo <= n < hi
     const float *x0, *x1;
+    const double *x0_stats, *x1_stats;              // sc0, sc1: rank_pre
     i64 base, lo, hi;
     float2 *out;        // [256][8192]
 };
@@ -82,7 +108,8 @@ struct BigCrossJob {    // G0 = C00 + i C01, G1 = C10 + i C11 with C_ab = 4 conj
 struct BigOutJob {      // inverse column pass of one packed pair of correlations
     const float2 *G;
     float *approx0, *approx1;                       // [n_lags] each, nullptr: pair absent
-    const double *t_stats, *s0_stats, *s1_stats;    // ST_SCALE of the template and the two signals
+    const double *t_stats, *t_pack;                 // the template and the plane it was packed with (rank_post)
+    const double *s0_stats, *s1_stats;              // the two signals (packed together)
     i64 n_t;
     int n_lags;
 };
@@ -106,7 +133,8 @@ constexpr int kSpecMaxTiles = 10;    // tiles per accumulation job (16 stations,
 __host__ __device__ inline size_t spec_seg_elems(int n_rows) { return (size_t)kSpecChunks * n_rows * kSpecBins; }
 
 struct SpecFftJob {     // one packed transform, all its segments
-    const float *x0, *x1;   // planes: z = x0 + i x1
+    const float *x0, *x1;   // planes: z = x0 sc0 + i x1 sc1
+    const double *x0_stats, *x1_stats;   // sc0, sc1: rank_pre
     i64 base;               // plane index of sample 0 of segment 0
     i64 stride;             // samples between segment starts
     i64 lo, hi;             // plane indices outside [lo, hi) read as zero

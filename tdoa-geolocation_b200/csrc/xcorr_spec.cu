@@ -51,9 +51,11 @@ __global__ void __launch_bounds__(kT, 2) k_spec_fft(const SpecFftJob *jobs, int 
     for (int idx = t; idx < kTab; idx += kT) tab[idx] = tw[(16 * (idx & 31) * (idx >> 5)) & (kN - 1)];
     const float2 w1a = tw[2 * t], w1b = tw[2 * t + 1];
     {
-        // z[m] = x0[i] + i x1[i], i = base + seg * stride + m, for m < seg_len and lo <= i < hi
+        // z[m] = x0[i] sc0 + i x1[i] sc1, i = base + seg * stride + m, for m < seg_len and lo <= i < hi; sc = rank_pre
+        // (xcorr_fft.h), 1 unless the two planes' powers differ widely
         const i64 first = J.base + (i64)seg * J.stride;
         const float *__restrict__ x0 = J.x0, *__restrict__ x1 = J.x1;
+        const float sc0 = rank_pre(J.x0_stats, J.x1_stats), sc1 = rank_pre(J.x1_stats, J.x0_stats);
         float2 v[32];
         if (first >= J.lo && first + J.seg_len <= J.hi && (J.seg_len & 255) == 0) {
             const int rows = J.seg_len >> 8;
@@ -66,6 +68,10 @@ __global__ void __launch_bounds__(kT, 2) k_spec_fft(const SpecFftJob *jobs, int 
                 const i64 i = first + m;
                 v[r] = (m < J.seg_len && i >= J.lo && i < J.hi) ? make_float2(x0[i], x1[i]) : make_float2(0.f, 0.f);
             }
+        }
+        if (sc0 != 1.f || sc1 != 1.f) {
+#pragma unroll
+            for (int r = 0; r < 32; r++) v[r] = make_float2(__fmul_rn(v[r].x, sc0), __fmul_rn(v[r].y, sc1));
         }
         pass1_store(v, t, buf);
     }

@@ -75,10 +75,11 @@ __device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.
 // barrier over the 256 threads of transform g (ids 1 and 2; 0 is __syncthreads)
 __device__ __forceinline__ void bar_transform(int g) { asm volatile("bar.sync %0, 256;" ::"r"(g + 1) : "memory"); }
 
-// samples m = t + 256 r of one segment as complex points (x0[m], x1[m]); CNT rows carry data
+// samples m = t + 256 r of one segment as complex points (x0[m] sc0, x1[m] sc1); CNT rows carry data.  sc0, sc1:
+// rank_pre (xcorr_fft.h), 1 unless the two planes' powers differ widely: no multiply at all then.
 template <int CNT>
-__device__ __forceinline__ void load_rows(const float *__restrict__ x0, const float *__restrict__ x1, i64 base, i64 lo,
-                                          i64 hi, int t, float2 (&v)[32])
+__device__ __forceinline__ void load_rows(const float *__restrict__ x0, const float *__restrict__ x1, float sc0,
+                                          float sc1, i64 base, i64 lo, i64 hi, int t, float2 (&v)[32])
 {
     if (lo <= 0 && hi >= 256 * CNT) {
         const float *__restrict__ p0 = x0 + base + t;
@@ -93,6 +94,10 @@ __device__ __forceinline__ void load_rows(const float *__restrict__ x0, const fl
             v[r] = ok ? make_float2(__ldg(x0 + base + m), __ldg(x1 + base + m)) : make_float2(0.f, 0.f);
         }
     }
+    if (sc0 != 1.f || sc1 != 1.f) {
+#pragma unroll
+        for (int r = 0; r < CNT; r++) v[r] = make_float2(__fmul_rn(v[r].x, sc0), __fmul_rn(v[r].y, sc1));
+    }
 }
 
 __global__ void __launch_bounds__(kTileThreads, 1) k_fft_tiles(const TileJob *jobs, const float2 *__restrict__ tw)
@@ -104,6 +109,9 @@ __global__ void __launch_bounds__(kTileThreads, 1) k_fft_tiles(const TileJob *jo
     if (cta >= J.n_cta) return;
     const int tid = threadIdx.x, warp = tid >> 5;
     const int g = tid >> 8, t = tid & (kT - 1);
+    // the scales first: their two dependent loads overlap the table fill and the tensor-memory set-up
+    const double *st0 = g ? J.s0_stats : J.t0_stats, *st1 = g ? J.s1_stats : J.t1_stats;
+    const float sc0 = rank_pre(st0, st1), sc1 = rank_pre(st1, st0);
     float2 *buf = sm + g * kBuf;
     float2 *tab = sm + 2 * kBuf;
     for (int idx = tid; idx < kTab; idx += kTileThreads) tab[idx] = tw[(16 * (idx & 31) * (idx >> 5)) & (kN - 1)];
@@ -133,10 +141,10 @@ __global__ void __launch_bounds__(kTileThreads, 1) k_fft_tiles(const TileJob *jo
     auto load_segment = [&](int seg, float2 (&v)[32]) {
         const i64 first = (i64)seg * kSeg;
         if (g == 0) {
-            load_rows<kSeg / 256>(x0, x1, J.t_off + first, 0, J.n_t - first, t, v);
+            load_rows<kSeg / 256>(x0, x1, sc0, sc1, J.t_off + first, 0, J.n_t - first, t, v);
         } else {
             const i64 base = J.s_off + first;
-            load_rows<32>(x0, x1, base, -base, J.sl - base, t, v);
+            load_rows<32>(x0, x1, sc0, sc1, base, -base, J.sl - base, t, v);
         }
     };
 
@@ -229,8 +237,8 @@ constexpr int kTile16Threads = 2 * fft16::kT16;
 __device__ __forceinline__ void bar_transform16(int g) { asm volatile("bar.sync %0, 512;" ::"r"(g + 1) : "memory"); }
 
 template <int CNT>
-__device__ __forceinline__ void load_rows16(const float *__restrict__ x0, const float *__restrict__ x1, i64 base, i64 lo,
-                                            i64 hi, int t, float2 (&v)[16])
+__device__ __forceinline__ void load_rows16(const float *__restrict__ x0, const float *__restrict__ x1, float sc0,
+                                            float sc1, i64 base, i64 lo, i64 hi, int t, float2 (&v)[16])
 {
     if (lo <= 0 && hi >= 512 * CNT) {
         const float *__restrict__ p0 = x0 + base + t;
@@ -245,6 +253,10 @@ __device__ __forceinline__ void load_rows16(const float *__restrict__ x0, const 
             v[r] = ok ? make_float2(__ldg(x0 + base + m), __ldg(x1 + base + m)) : make_float2(0.f, 0.f);
         }
     }
+    if (sc0 != 1.f || sc1 != 1.f) {
+#pragma unroll
+        for (int r = 0; r < CNT; r++) v[r] = make_float2(__fmul_rn(v[r].x, sc0), __fmul_rn(v[r].y, sc1));
+    }
 }
 
 __global__ void __launch_bounds__(kTile16Threads, 1) k_fft_tiles16(const TileJob *jobs, const float2 *__restrict__ tw)
@@ -257,6 +269,9 @@ __global__ void __launch_bounds__(kTile16Threads, 1) k_fft_tiles16(const TileJob
     if (cta >= J.n_cta) return;
     const int tid = threadIdx.x, warp = tid >> 5;
     const int g = tid >> 9, t = tid & (kT16 - 1);
+    // the scales first: their two dependent loads overlap the table fill and the tensor-memory set-up
+    const double *st0 = g ? J.s0_stats : J.t0_stats, *st1 = g ? J.s1_stats : J.t1_stats;
+    const float sc0 = rank_pre(st0, st1), sc1 = rank_pre(st1, st0);
     float2 *buf = sm + g * kBuf;
     float2 *tab = sm + 2 * kBuf;
     for (int idx = tid; idx < kTab; idx += kTile16Threads) tab[idx] = tw[(16 * (idx & 31) * (idx >> 5)) & (kN - 1)];
@@ -287,10 +302,10 @@ __global__ void __launch_bounds__(kTile16Threads, 1) k_fft_tiles16(const TileJob
     auto load_segment = [&](int seg, float2 (&v)[16]) {
         const i64 first = (i64)seg * kSeg;
         if (g == 0) {
-            load_rows16<kSeg / 512>(x0, x1, J.t_off + first, 0, J.n_t - first, t, v);
+            load_rows16<kSeg / 512>(x0, x1, sc0, sc1, J.t_off + first, 0, J.n_t - first, t, v);
         } else {
             const i64 base = J.s_off + first;
-            load_rows16<16>(x0, x1, base, -base, J.sl - base, t, v);
+            load_rows16<16>(x0, x1, sc0, sc1, base, -base, J.sl - base, t, v);
         }
     };
 

@@ -118,14 +118,17 @@ def binary_lags(raws, i: int = 0, j: int = 1, max_lag: int = BINARY_LAGS):
 
 def candidates(c, neighbours: bool, sanity: int = 0, tol: float = TOL):
     """The lags k_select_candidates keeps, on exact values: within tol of the maximum |c|, within tol of the
-    maximum over [0, sanity) when sanity > 0, and (neighbours) the lags either side of a lag of the first set."""
-    a = np.abs(np.asarray(c, np.float64))
+    maximum over [0, sanity) when sanity > 0, and (neighbours) the lags either side of a lag of the first set.
+    An f32 plane (the FFT ranking) is compared in f32, as the kernel does; anything else in f64."""
+    dt = np.float32 if np.asarray(c).dtype == np.float32 else np.float64
+    a = np.abs(np.asarray(c, dt))
+    tol = dt(tol)
     m1 = a.max()
-    take = a >= m1 - tol
+    take = a >= dt(m1 - tol)
     first = take.copy()
     if sanity > 0:
         m2 = a[:sanity].max()
-        take[:sanity] |= a[:sanity] >= m2 - tol
+        take[:sanity] |= a[:sanity] >= dt(m2 - tol)
     if neighbours:
         take[1:] |= first[:-1]
         take[:-1] |= first[1:]
@@ -135,7 +138,8 @@ def candidates(c, neighbours: bool, sanity: int = 0, tol: float = TOL):
 def selection_gap(c, sanity: int = 0):
     """How far the candidate set stands from changing: the smallest distance, in |c|, between a lag outside
     the set and the threshold it would need to cross (the maximum, or the [0, sanity) maximum).  A gap over
-    5 x TOL means the f32 ranking's error (~1e-6) cannot change which lags are candidates."""
+    5 x TOL means the f32 ranking's error (under 1e-6, tests/test_gpu_ranking.py) cannot change which lags are
+    candidates."""
     a = np.abs(np.asarray(c, np.float64))
     m1 = a.max()
     top = a >= m1 - TOL
